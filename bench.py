@@ -3,6 +3,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
                     [--workload poisson27|poisson5|rmat|rmat_c5|rect] [--dtype f64|f32]
+                    [--dump-outputs DIR]
 
 A "step" is one full C = A*B: all four stages of bhsparse::spgemm
 (SpGEMM_cuda/bhsparse.h:297-339) -- upper bound + binning, symbolic, row-pointer
@@ -182,6 +183,29 @@ class ClockSampler:
                 "samples": len(sm), "reasons": sorted(reasons)}
 
 
+DUMP_ENTRIES = 1 << 20      # sampled entries of a large C: 32 MB as float64, well within a 64 MB dump
+
+
+def dump_outputs(out_dir, rowptr, col, val, seed=0):
+    """Writes C = (rowptr, col, val), as a caller of the timed path receives it, to out_dir as .npy:
+    rowptr, col, val in full when they fit in 32 MB, else the entries at a fixed seeded sample of
+    positions: entry (position in col / val), row, col, val.  Indices are written as float64 (exact
+    below 2^53), values in their own float32 / float64, so two builds can be compared file by file."""
+    import torch
+    rowptr, col, val = (torch.as_tensor(x) for x in (rowptr, col, val))
+    if 8 * (rowptr.numel() + 2 * col.numel()) <= 32 * DUMP_ENTRIES:
+        arrays = {"rowptr": rowptr, "col": col, "val": val}
+    else:
+        entry = np.sort(np.random.default_rng(seed).choice(col.numel(), DUMP_ENTRIES, replace=False))
+        row = np.searchsorted(rowptr.cpu().numpy(), entry, side="right") - 1
+        at = torch.from_numpy(entry).to(col.device)
+        arrays = {"entry": entry, "row": row, "col": col[at], "val": val[at]}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        a = a.cpu().numpy() if torch.is_tensor(a) else a
+        np.save(os.path.join(out_dir, name + ".npy"), a if a.dtype in (np.float32, np.float64) else a.astype(np.float64))
+
+
 def config_dict(desc, m, nnzA, products, nnzC, world):
     """The `config` object: identical keys in both arms, so the driver can compare them."""
     return {"workload": desc, "values": VALUES, "m": int(m), "nnzA": int(nnzA), "products": int(products),
@@ -211,12 +235,14 @@ def run_reference(args, rank):
     rp = None
     for it in range(args.warmup + args.steps):
         t0 = time.perf_counter()
-        rp, _, _ = oracle.spgemm(A.rows, A.cols, B.cols, A.rowptr, A.col, A.val, B.rowptr, B.col, B.val)
+        rp, colC, valC = oracle.spgemm(A.rows, A.cols, B.cols, A.rowptr, A.col, A.val, B.rowptr, B.col, B.val)
         dt = time.perf_counter() - t0
         if it >= args.warmup:
             times.append(dt)
         if it == 0 and dt * (args.warmup + args.steps) > 240.0:
             break                                          # keep the arm within minutes: one step is the sample
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, rp, colC, valC)
     t = float(np.mean(times)) if times else dt
     val = 2.0 * P / t / 1e9
     sample = f"full {desc} ({A.rows} rows, {P} products) per step, {len(times) or 1} timed step(s)"
@@ -609,7 +635,13 @@ def main():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-rmat", action="store_true", help="skip the R-MAT sub-record of the default run")
     ap.add_argument("--no-parity", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write C of the last timed step to DIR/<name>.npy (one process, --gpus 1)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.gpus != 1:
+        ap.error("--dump-outputs writes one process's C: use it with --gpus 1")
     if args.dtype is None:
         args.dtype = "f32" if args.workload == "rect" else "f64"
     if args.warmup < 3 and args.impl == "ours":
@@ -640,6 +672,10 @@ def main():
     engine.set_profiling(True)
 
     t = timed_steps(run, rb, engine, args.steps, args.warmup, sample_clocks=True)
+    if args.dump_outputs:
+        res = engine.result()
+        dump_outputs(args.dump_outputs, res.rowptr64, res.col, res.val)
+        del res
     ms, st = t["ms"], t["st"]
     value = 2.0 * P_total / (ms * 1e-3) / 1e9
     bin_ms_sym, bin_ms_num = per_bin_times(engine, rb)       # same launches, per-bin events (profiling stays on)

@@ -1,7 +1,8 @@
-"""Inputs on which the oracle is pinned by outputs OF THE REFERENCE ITSELF (oracle/_ref run on a
-B200 by tests/golden/make_ref_golden.py).  One list, used by the generating script, by the CPU
-test that checks the oracle against the committed vectors (tests/test_oracle_pinned.py) and by
-the GPU test that re-runs the reference live (tests/test_reference_gpu.py).
+"""Inputs on which the oracle and the library are pinned by outputs OF THE REFERENCE ITSELF
+(oracle/_ref run on a B200 by tests/golden/make_ref_golden.py).  One list, used by the generating
+script, by the CPU test that checks the oracle against the committed vectors
+(tests/test_oracle_pinned.py) and by the GPU test that checks the library against them
+(tests/test_reference_gpu.py).
 
 A case is (name, builder) with builder(dtype) -> (A, B) host CSR.  Values are integers 1..9 as
 in the reference driver (main.cu:82,93), so every sum is exact in f32 and f64 and the compare is
@@ -90,3 +91,46 @@ DTYPES = {"f64": np.float64, "f32": np.float32}
 def digest(a: np.ndarray) -> str:
     import hashlib
     return hashlib.sha256(np.ascontiguousarray(a).tobytes()).hexdigest()
+
+
+SAMPLE = 4096          # stored values per real-valued case: their full arrays would not fit the golden file
+
+
+def row_sums(rp, val) -> np.ndarray:
+    rows = np.repeat(np.arange(rp.size - 1), np.diff(np.asarray(rp, dtype=np.int64)))
+    return np.bincount(rows, weights=val.astype(np.float64), minlength=rp.size - 1)
+
+
+def record(name: str, rp, col, val) -> dict:
+    """What tests/golden/ref_outputs.npz keeps of the reference's C = (rp, col, val) for one case, keyed
+    without the "<name>.<dtype>." prefix: nnzC and the SHA-256 digests of rowptrC (int32), colC and
+    valC; for the *_real cases, whose values are compared within a tolerance, also the per-row sums of
+    valC and valC at a fixed seeded sample of positions."""
+    rec = {"nnzC": np.int64(rp[-1]), "digest": np.array([digest(np.asarray(rp, np.int32)), digest(col), digest(val)])}
+    if name.endswith("_real"):
+        idx = np.random.default_rng(0).choice(val.size, min(SAMPLE, val.size), replace=False)
+        idx = np.sort(idx).astype(np.int32)
+        rec.update(sample_idx=idx, sample_val=val[idx], row_sum=row_sums(rp, val))
+    return rec
+
+
+def check(gold, name: str, dn: str, rp, col, val, rtol: float) -> None:
+    """Asserts that C = (rp, col, val) is the reference's output stored in `gold` for case `name` in
+    dtype `dn`: rowptrC and colC bit-exact; valC bit-exact, or for the *_real cases within rtol
+    relative at the sampled positions and in every row sum."""
+    key = f"{name}.{dn}"
+    assert int(gold[key + ".nnzC"]) == int(rp[-1]), f"{key}: nnzC differs"
+    d = gold[key + ".digest"]
+    assert d[0] == digest(np.asarray(rp, np.int32)), f"{key}: rowptrC differs"
+    assert d[1] == digest(col), f"{key}: colC differs"
+    if not name.endswith("_real"):
+        assert d[2] == digest(val), f"{key}: valC differs (exact compare)"
+        return
+    idx, want = gold[key + ".sample_idx"], gold[key + ".sample_val"]
+    assert want.dtype == val.dtype
+    err = np.abs(val[idx].astype(np.float64) - want.astype(np.float64)) / np.abs(want.astype(np.float64))
+    assert err.max() <= rtol, f"{key}: max rel err {err.max()} > {rtol}"
+    # every value within rtol of the reference's keeps each row sum within rtol of the row's sum of
+    # magnitudes; the factor 2 covers the rounding of the sums themselves
+    sum_err = np.abs(row_sums(rp, val) - gold[key + ".row_sum"])
+    assert (sum_err <= 2 * rtol * row_sums(rp, np.abs(val))).all(), f"{key}: a row sum differs beyond {rtol}"
