@@ -70,7 +70,6 @@ def build(force: bool = False, verbose: bool = False) -> str:
     cc = nvcc()
     hdr_time = _newest_header()
     extra = ["-Xptxas", "-v"] if verbose else []
-    extra += os.environ.get("BHB200_NVCC_DEFS", "").split()      # experiments: -DNAME=value
     # nvcc's host compiler: the image's $CC wrapper lacks some specs; use the system g++
     ccbin = ["-ccbin", "/usr/bin/g++"] if os.path.exists("/usr/bin/g++") else []
 

@@ -181,7 +181,7 @@ int reserve_word_lists(bhb200_ctx *ctx, int64_t products, WordLists &wl)
     CU(ctx->wl_cnt.reserve(m1 * 4, &ctx->dev_bytes), "alloc word-list counts");
     long long cap = products / 4 + (long long)ctx->m + 1024;
     if (cap > (1ll << 31)) cap = 1ll << 31;
-    if (const char *dbg = getenv("BHB200_DEBUG_WORDLIST_CAP")) cap = atoll(dbg);   // tests: force the fallback
+    if (ctx->wordlist_cap >= 0) cap = ctx->wordlist_cap;   // tests: force the fallback
     if (ctx->wl_idx.reserve((size_t)cap * 4, &ctx->dev_bytes) != cudaSuccess ||
         ctx->wl_bits.reserve((size_t)cap * 8, &ctx->dev_bytes) != cudaSuccess) {
         cudaGetLastError();
@@ -189,7 +189,7 @@ int reserve_word_lists(bhb200_ctx *ctx, int64_t products, WordLists &wl)
     } else {
         // grow-only buffers may be larger than this call's request: use all of it
         const long long have = (long long)(ctx->wl_idx.cap / 4 < ctx->wl_bits.cap / 8 ? ctx->wl_idx.cap / 4 : ctx->wl_bits.cap / 8);
-        if (have > cap && !getenv("BHB200_DEBUG_WORDLIST_CAP")) cap = have;
+        if (have > cap && ctx->wordlist_cap < 0) cap = have;
     }
     wl.off = ctx->wl_off.as<long long>();
     wl.cnt = ctx->wl_cnt.as<int>();
@@ -457,12 +457,7 @@ int bhb200_create(bhb200_ctx **out, int device)
         ctx->pattern_enable = strcmp(pm, "off") != 0;
         ctx->pattern_speculate = strcmp(pm, "detect") != 0;   // "detect": run the offset-set pass on every call
     }
-    if (const char *bh = getenv("BHB200_BUCKET_HEAVY")) ctx->bucket_heavy = strcmp(bh, "off") != 0;
-    if (const char *be = getenv("BHB200_BUCKET")) {
-        ctx->bucket_enable = strcmp(be, "off") != 0;
-        if (atoi(be) >= 512) ctx->bucket_min_cap = atoi(be);   // BHB200_BUCKET=<capacity>: smallest capacity that takes the bucket kernel
-    }
-    if (const char *dc = getenv("BHB200_DEBUG_DEVICE_CAP")) ctx->device_cap = (size_t)atoll(dc);
+    if (const char *bw = getenv("BHB200_BUCKET_W")) ctx->bucket_warp = strcmp(bw, "off") != 0;
     if (const char *dm = getenv("BHB200_DIRECT")) {
         ctx->direct_mode = strcmp(dm, "off") != 0;
         ctx->direct_wide = strcmp(dm, "tight") != 0;
@@ -472,6 +467,10 @@ int bhb200_create(bhb200_ctx **out, int device)
         else if (!strcmp(rm, "small")) ctx->max_span = SPAN_SMALL;
         else if (!strcmp(rm, "all")) ctx->max_span = SPAN_LARGE;
     }
+    if (const char *dc = getenv("BHB200_DEBUG_DEVICE_CAP")) ctx->device_cap = (size_t)atoll(dc);
+    if (const char *fc = getenv("BHB200_DEBUG_FORCE_CAP")) ctx->force_cap = atoi(fc) > 0 ? atoi(fc) : 0;
+    ctx->force_heavy = getenv("BHB200_DEBUG_FORCE_HEAVY") != nullptr;
+    if (const char *wc = getenv("BHB200_DEBUG_WORDLIST_CAP")) ctx->wordlist_cap = atoll(wc) > 0 ? atoll(wc) : 0;
     for (auto &ev : ctx->ev) {
         if (cudaEventCreate(&ev) != cudaSuccess) {
             cudaGetLastError();
@@ -710,7 +709,8 @@ int bhb200_spgemm(bhb200_ctx *ctx)
     long long spec_base[MAX_BINS] = {0};
     long long ct_entries = 0;
     const int SAMPLE_STRIDE = 64;
-    const int SPEC_MIN_ROWS = getenv("BHB200_DEBUG_FORCE_CAP") ? 1 : 4096;
+    const bool force = ctx->force_cap >= 0;
+    const int SPEC_MIN_ROWS = force ? 1 : 4096;
     static const int WIDE_CAP[7] = {128, 256, 512, 1024, 2048, 4096, 8192};   // SB_G128 .. SB_B8192
     if (ctx->direct_mode) {
         bool any = false;
@@ -725,7 +725,6 @@ int bhb200_spgemm(bhb200_ctx *ctx)
         if (any) {
             CU(cudaMemcpyAsync(ctx->h_ctr, d_ctr, sizeof(Counters), cudaMemcpyDeviceToHost, s), "D2H counters");
             CU(cudaStreamSynchronize(s), "direct-mode sampling");
-            const char *force = getenv("BHB200_DEBUG_FORCE_CAP");   // tests: speculate this capacity whatever the sample says
             bool wide_above = false;
             for (int b = SB_G128; b <= SB_B8192; ++b) {
                 if (hc.sym_bin[b] <= 0) continue;
@@ -737,15 +736,14 @@ int bhb200_spgemm(bhb200_ctx *ctx)
                 } else {
                     wide_above = false;
                     int smax = ctx->h_ctr->sample_max[b];
-                    if (force && hc.sym_bin[b] >= SPEC_MIN_ROWS) smax = atoi(force);
+                    if (force && hc.sym_bin[b] >= SPEC_MIN_ROWS) smax = ctx->force_cap;
                     if (hc.sym_bin[b] < SPEC_MIN_ROWS || smax < 1) continue;
                     const int nsample = (hc.sym_bin[b] + SAMPLE_STRIDE - 1) / SAMPLE_STRIDE;
                     const double mean = (double)ctx->h_ctr->sample_sum[b] / nsample;
                     const int wcap = WIDE_CAP[b - SB_G128];
                     // bins of at most 96 / 192 products whose sampled rows keep at least half of their products as outputs:
                     // sorting the products (k_num_bucket3w) beats hashing them (BHB200_BUCKET_W=off: hash kernels)
-                    static const bool w_on = [] { const char *e = getenv("BHB200_BUCKET_W"); return !(e && strcmp(e, "off") == 0); }();
-                    if (w_on && ctx->bucket_enable && b <= SB_G256 && !force && hc.sym_bin[b] > 0 &&
+                    if (ctx->bucket_warp && b <= SB_G256 && !force && hc.sym_bin[b] > 0 &&
                         mean * 2.0 * (double)hc.sym_bin[b] >= (double)hc.sym_bin_products[b])
                         spec_3w[b] = true;
                     if (smax <= 128) {
@@ -766,7 +764,7 @@ int bhb200_spgemm(bhb200_ctx *ctx)
         // rows with more products than the on-chip tables hold follow the largest sampled bin: if that one
         // does not compress they run once through the sliced bucket sort, staged at their product count
         // (BHB200_DEBUG_FORCE_HEAVY: tests send them there whatever the sample says)
-        bool top_wide = getenv("BHB200_DEBUG_FORCE_HEAVY") != nullptr;
+        bool top_wide = ctx->force_heavy;
         for (int b = SB_B8192; b >= SB_G128 && !top_wide; --b)
             if (hc.sym_bin[b] > 0) {
                 top_wide = ((spec_mask >> b) & 1u) && spec_wide[b];
@@ -774,7 +772,7 @@ int bhb200_spgemm(bhb200_ctx *ctx)
             }
         // (k_num_bucket_heavy2, measured on R-MAT 21, n = 2 M columns: 4.0 ms for these rows against 7.0 ms through the
         // two-pass tables + global column bitmap, whose cost also grows with n -- profiles/r02_notes.md section 5)
-        if (top_wide && ctx->bucket_enable && ctx->bucket_heavy && ctx->direct_wide) {
+        if (top_wide && ctx->direct_wide) {
             heavy_base = ct_entries;
             for (int b = SB_B16384; b <= SB_LARGE; ++b) {
                 if (hc.sym_bin[b] <= 0) continue;
@@ -827,11 +825,13 @@ int bhb200_spgemm(bhb200_ctx *ctx)
     CU(cudaEventRecord(ctx->ev[1], s), "event");
 
     // wide bins with 512+ entries per row: bucket-sort kernels, which need the column CDF of the products
+    // (k_num_bucket3 beats the hash kernels from a capacity of 512 up, profiles/r02_notes.md section 5)
+    constexpr int BUCKET_MIN_CAP = 512;
     bool use_bucket = false;
     int cdf_shift = 0;
-    if (ctx->bucket_enable && spec_mask) {
+    if (spec_mask) {
         for (int b = SB_G128; b <= SB_G256; ++b) use_bucket |= ((spec_mask >> b) & 1u) && spec_3w[b];
-        for (int b = SB_G512; b <= SB_B8192; ++b) use_bucket |= ((spec_mask >> b) & 1u) && spec_wide[b] && spec_cap[b] >= ctx->bucket_min_cap;
+        for (int b = SB_G512; b <= SB_B8192; ++b) use_bucket |= ((spec_mask >> b) & 1u) && spec_wide[b] && spec_cap[b] >= BUCKET_MIN_CAP;
         for (int b = SB_B16384; b <= SB_LARGE; ++b) use_bucket |= ((spec_mask >> b) & 1u) && spec_heavy[b];
         if (use_bucket && (ctx->cdf_colcount.reserve(((size_t)ctx->k + 1) * 4, &ctx->dev_bytes) != cudaSuccess ||
                            ctx->cdf_hist.reserve((size_t)CDF_KNOTS * 8, &ctx->dev_bytes) != cudaSuccess ||
@@ -844,8 +844,7 @@ int bhb200_spgemm(bhb200_ctx *ctx)
                     spec_mask &= ~(1u << b);
                 }
         }
-        static const bool cdf_rebuild = [] { const char *e = getenv("BHB200_CDF"); return e && strcmp(e, "rebuild") == 0; }();
-        if (use_bucket && ctx->cdf_valid && !cdf_rebuild) {
+        if (use_bucket && ctx->cdf_valid) {
             cdf_shift = ctx->cdf_shift_cached;
         } else if (use_bucket) {
             CU(launch_build_cdf(lc, ctx->m, ctx->k, ctx->n, ctx->nnzA, ctx->A, ctx->B, ctx->cdf_colcount.as<int>(),
@@ -857,9 +856,7 @@ int bhb200_spgemm(bhb200_ctx *ctx)
     }
     // Rows with more products than the on-chip tables hold (bins SB_B16384 .. SB_LARGE), single pass, staged by atomic
     // bump at heavy_base: rows of at most 8192 products by k_num_bucket3 itself, the rest by k_num_bucket_heavy2
-    // (partitioned by slice through the row's own staging area), what that kernel cannot slice by k_num_bucket_heavy
-    // (BHB200_HEAVY_V=1: everything by k_num_bucket_heavy).
-    static const bool heavy_v1 = [] { const char *e = getenv("BHB200_HEAVY_V"); return e && atoi(e) == 1; }();
+    // (partitioned by slice through the row's own staging area), what that kernel cannot slice by k_num_bucket_heavy.
     auto run_heavy_bin = [&](const int b) -> cudaError_t {
         const bool f64 = ctx->dtype == BHB200_DTYPE_F64;
         const unsigned *cdf = ctx->cdf_tab.as<unsigned>();
@@ -868,12 +865,8 @@ int bhb200_spgemm(bhb200_ctx *ctx)
         DirectOut d{rcnt, ctx->ct_off.as<long long>(), ctx->ct_col.as<int>(), ctx->ct_val.p, heavy_base, nullptr, nullptr};
         d.prod = prod;
         cudaError_t e;
-        if (heavy_v1)
-            return f64 ? launch_num_bucket_heavy_f64(lc, bq, rows, ctx->A, ctx->B, d, cdf, cdf_shift, &d_ctr->heavy_cursor)
-                       : launch_num_bucket_heavy_f32(lc, bq, rows, ctx->A, ctx->B, d, cdf, cdf_shift, &d_ctr->heavy_cursor);
         int p_lo = 0;
-        static const bool bucket_v1 = [] { const char *e = getenv("BHB200_BUCKET_V"); return e && atoi(e) == 1; }();
-        if (b == SB_B16384 && !bucket_v1) {   // 6144 < products <= 12288: up to 8192 fit k_num_bucket3's largest capacity
+        if (b == SB_B16384) {   // 6144 < products <= 12288: up to 8192 fit k_num_bucket3's largest capacity
             DirectOut d3 = d;
             d3.p_lo = 0;
             d3.p_hi = 8192;
@@ -933,7 +926,7 @@ int bhb200_spgemm(bhb200_ctx *ctx)
                     d.p_hi = pass == 0 ? spec_cap[b] / 2 : 0x7fffffff;
                     if (pass == 0) cap = spec_cap[b] / 2;
                 }
-                if (spec_wide[b] && use_bucket && cap >= ctx->bucket_min_cap) {
+                if (spec_wide[b] && use_bucket && cap >= BUCKET_MIN_CAP) {
                     if (ctx->dtype == BHB200_DTYPE_F64)
                         CU(launch_num_bucket_f64(lc, cap, queue + so.off[b], hc.sym_bin[b], ctx->A, ctx->B, d, ctx->cdf_tab.as<unsigned>(), cdf_shift),
                            "bucket numeric f64");

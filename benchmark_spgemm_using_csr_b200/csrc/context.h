@@ -103,12 +103,10 @@ struct bhb200_ctx {
     bhb::DevBuf brange, rlo, rspan, wl_off, wl_cnt, wl_idx, wl_bits;   // span info + word-list pool (range kernels)
     bhb::DevBuf cdf_colcount, cdf_hist, cdf_tab;                          // bucket-sort kernels: column CDF of the products
     // the table of the previous product on these operands is kept: it only balances the buckets (any monotone table gives
-    // the same C), and it depends on the patterns alone; reset whenever operands are (re)initialised (BHB200_CDF=rebuild: every call)
+    // the same C), and it depends on the patterns alone; reset whenever operands are (re)initialised
     bool cdf_valid = false;
     int cdf_shift_cached = 0;
-    int bucket_min_cap = 512;                                             // smallest wide-bin capacity that takes the bucket kernel (k_num_bucket3 wins from 512 up, r02_notes.md section 5)
-    int bucket_heavy = 1;                                                 // BHB200_BUCKET_HEAVY=off: global-bitmap kernels for rows beyond the on-chip tables
-    int bucket_enable = 1;                                                // BHB200_BUCKET=off: hash kernels for the wide bins
+    int bucket_warp = 1;                                                  // BHB200_BUCKET_W=off: hash kernels instead of k_num_bucket3w
     bhb::DevBuf ct_off, ct_col, ct_val, retry_q;                       // direct mode: staging buffer (Ct) + retry queues
     // diagonal-pattern mode (stage_pattern.cuh): offset sets, per-entry codes, masks, tables
     bhb::DevBuf pat_sets, pat_ta, pat_tb, pat_maskB, pat_outmask, pat_tables, pat_fullbits;
@@ -122,6 +120,9 @@ struct bhb200_ctx {
     const unsigned char *last_ta = nullptr, *last_tb = nullptr;
     int direct_mode = 1;                                          // BHB200_DIRECT=off disables
     int direct_wide = 1;                                          // BHB200_DIRECT=tight: speculated capacities <= 128 only
+    int force_cap = -1;            // BHB200_DEBUG_FORCE_CAP (tests): speculate this capacity whatever the sample says; -1: off
+    bool force_heavy = false;      // BHB200_DEBUG_FORCE_HEAVY (tests): rows beyond the on-chip tables take the sliced bucket sort
+    long long wordlist_cap = -1;   // BHB200_DEBUG_WORDLIST_CAP (tests): size of the range kernels' word-list pool; -1: by product count
     size_t bitmap_zeroed_bytes = 0;
     bhb::DevBuf colC, valC;
     bhb::Counters *h_ctr = nullptr;   // pinned

@@ -3,21 +3,21 @@
 // R-MAT rows (BASELINE configs 3 and 5): nnz(C_i) is within a fraction of a percent of the row's
 // intermediate products, so hashing buys nothing and the work is a sort of p (column, value) pairs.
 // The hash kernels sort with a bitonic network -- O(log^2 p) compare-exchanges per key, ~200 of their
-// ~240 instructions per product at p = 1024 (profiles/r02_notes.md).  This kernel sorts in O(1) passes:
+// ~240 instructions per product at p = 1024 (profiles/r02_notes.md).  These kernels sort in O(1) passes:
 //
 //   * a MONOTONE bucket function  bucket(c) = floor(F(c) * NB),  F = the cumulative distribution of the
 //     columns of all intermediate products of the whole multiplication (a 4096-knot piecewise-linear
 //     table built once per product by k_cdf_*: every entry (k, c) of B weighted by the number of entries
 //     of A in column k).  Under F the products of a row spread almost evenly over the buckets, whatever
 //     the skew of the matrix (R-MAT: a third of all products fall into 1 % of the column range);
-//   * pass 1 counts the products of the row per bucket (shared-memory integer atomics), a CTA-wide scan
-//     turns the counts into segments, pass 2 scatters (column, a*b) into them;
-//   * one thread per bucket sorts its few entries by insertion and merges equal columns; the buckets are
-//     in column order, so the row is sorted; a second scan gives the compacted positions.
+//   * the products of a row are counted per bucket (shared-memory integer atomics), a CTA-wide scan turns
+//     the counts into segments, and the (column, a*b) pairs are placed into them;
+//   * each bucket is sorted by column and equal columns are merged; the buckets are in column order, so the
+//     row is sorted; a second scan gives the compacted positions.
 //
-// It plays the role of the reference's EM_mergepath rounds (bhsparse_cuda.h:1902-2157) for these rows.
-// One CTA per row; direct (single-pass) mode only: the row is staged at ct_base + q*ct_stride, its
-// length goes to rc[], k_copy_ct moves it to its final place after the scan.
+// They play the role of the reference's EM_mergepath rounds (bhsparse_cuda.h:1902-2157) for these rows.
+// Direct (single-pass) mode only: the row is staged in Ct (at ct_base + q*ct_stride, or by atomic bump),
+// its length goes to rc[], k_copy_ct moves it to its final place after the scan.
 #pragma once
 #include "common.cuh"
 
@@ -30,14 +30,6 @@ struct ColumnCdf {
     const unsigned *cdf;   // [CDF_KNOTS + 1], non-decreasing, cdf[0] = 0
     int shift;             // column >> shift < CDF_KNOTS
 };
-
-__device__ __forceinline__ unsigned cdf_eval(const ColumnCdf &f, const int c)
-{
-    const int i = c >> f.shift;
-    const unsigned lo = __ldg(f.cdf + i), hi = __ldg(f.cdf + i + 1);
-    const unsigned frac = (unsigned)c & ((1u << f.shift) - 1u);
-    return lo + (unsigned)(((unsigned long long)(hi - lo) * frac) >> f.shift);
-}
 
 // exclusive scan of a[0..n) in place by the whole CTA; returns the total.  scratch: 33 ints.
 template <int THREADS>
@@ -77,109 +69,11 @@ __device__ __forceinline__ int cta_exclusive_scan(int *a, const int n, int *scra
     return total;
 }
 
-template <typename VT, int THREADS>
-__global__ void __launch_bounds__(THREADS)
-k_num_bucket(const int *__restrict__ queue, const int count, const int *__restrict__ rowptrA, const int *__restrict__ colA,
-             const VT *__restrict__ valA, const int *__restrict__ rowptrB, const int *__restrict__ colB,
-             const VT *__restrict__ valB, const ColumnCdf cdf, const int cap, const int nb, int *__restrict__ rc,
-             long long *__restrict__ ct_off, int *__restrict__ ctcol, VT *__restrict__ ctval, const long long ct_base,
-             const int *__restrict__ prod, const int p_lo, const int p_hi, const int ct_stride)
-{
-    extern __shared__ __align__(16) unsigned char smem_raw[];
-    VT *vals = reinterpret_cast<VT *>(smem_raw);                              // [cap]
-    int *keys = reinterpret_cast<int *>(smem_raw + (size_t)cap * sizeof(VT));   // [cap]
-    int *cnt = keys + cap;                                                    // [nb]  bucket counts -> segment ends
-    int *ocnt = cnt + nb;                                                     // [nb + 1] merged counts -> output positions
-    int *scratch = ocnt + nb + 1;                                             // [34]: scan scratch + the B-row counter
-    const int lane = threadIdx.x & 31;
-
-    for (int q = blockIdx.x; q < count; q += gridDim.x) {
-        const int row = queue[q];
-        const int p = prod[row];
-        if (p <= p_lo || p > p_hi) continue;   // CTA-uniform
-        for (int i = threadIdx.x; i < nb; i += THREADS) cnt[i] = 0;
-        if (threadIdx.x == 0) scratch[33] = 0;
-        __syncthreads();
-        const int a0 = rowptrA[row], a1 = rowptrA[row + 1];
-        // ---- pass 1: products per bucket (warps take B rows from a shared counter, see k_num_block) ----
-        for (int j = a0 + take_next(&scratch[33], lane); j < a1; j = a0 + take_next(&scratch[33], lane)) {
-            const int k = colA[j];
-            const int bs = rowptrB[k], be = rowptrB[k + 1];
-            for (int e = bs + lane; e < be; e += 32)
-                atomicAdd(&cnt[__umulhi(cdf_eval(cdf, colB[e]), (unsigned)nb)], 1);
-        }
-        __syncthreads();
-        cta_exclusive_scan<THREADS>(cnt, nb, scratch);   // cnt[b] = first slot of bucket b
-        if (threadIdx.x == 0) scratch[33] = 0;
-        __syncthreads();
-        // ---- pass 2: scatter (column, a*b) into the segments; afterwards cnt[b] = END of bucket b ----
-        for (int j = a0 + take_next(&scratch[33], lane); j < a1; j = a0 + take_next(&scratch[33], lane)) {
-            const int k = colA[j];
-            const VT av = valA[j];
-            const int bs = rowptrB[k], be = rowptrB[k + 1];
-            for (int e = bs + lane; e < be; e += 32) {
-                const int c = colB[e];
-                const int slot = atomicAdd(&cnt[__umulhi(cdf_eval(cdf, c), (unsigned)nb)], 1);
-                keys[slot] = c;
-                vals[slot] = av * valB[e];
-            }
-        }
-        __syncthreads();
-        // ---- per bucket: insertion sort by column, equal columns merged.  (Measured and dropped: one ENTRY
-        // per thread ranking itself inside its bucket, rows permuted through registers -- 64 registers and
-        // twice the threads per row made every bin slower, profiles/r02_notes.md.) ----
-        for (int b = threadIdx.x; b < nb; b += THREADS) {
-            const int s = b ? cnt[b - 1] : 0, e = cnt[b];
-            for (int i = s + 1; i < e; ++i) {
-                const int kc = keys[i];
-                const VT kv = vals[i];
-                int j = i - 1;
-                while (j >= s && keys[j] > kc) {
-                    keys[j + 1] = keys[j];
-                    vals[j + 1] = vals[j];
-                    --j;
-                }
-                keys[j + 1] = kc;
-                vals[j + 1] = kv;
-            }
-            int w = s;
-            for (int i = s; i < e; ++i) {
-                if (i > s && keys[i] == keys[w - 1]) {
-                    vals[w - 1] += vals[i];
-                } else {
-                    keys[w] = keys[i];
-                    vals[w] = vals[i];
-                    ++w;
-                }
-            }
-            ocnt[b] = w - s;
-        }
-        if (threadIdx.x == 0) ocnt[nb] = 0;
-        __syncthreads();
-        const int total = cta_exclusive_scan<THREADS>(ocnt, nb + 1, scratch);   // ocnt[b] = output position of bucket b
-        // ---- emit ----
-        const long long o = ct_base + (long long)q * ct_stride;
-        if (threadIdx.x == 0) {
-            rc[row] = total;
-            ct_off[row] = o;
-        }
-        for (int b = threadIdx.x; b < nb; b += THREADS) {
-            const int s = b ? cnt[b - 1] : 0;
-            const int o0 = ocnt[b], n = ocnt[b + 1] - o0;
-            for (int i = 0; i < n; ++i) {
-                ctcol[o + o0 + i] = keys[s + i];
-                ctval[o + o0 + i] = vals[s + i];
-            }
-        }
-        __syncthreads();
-    }
-}
-
 // ---------------------------------------------------------------------------------------------------
-// k_num_bucket3 (round 2, second pass): the same sort with ONE pass over the B rows and no per-bucket loops
-// by single threads.  ncu of k_num_bucket (profiles/r02_ncu_bucket_v1.txt): L1TEX 74 % -- 7.5 sectors per
-// global load request, because every product looks the CDF table up twice per pass through L1 (32 lanes,
-// ~25 different sectors) -- and 45 % of its instructions run at 3-4 active lanes (a thread per bucket).
+// k_num_bucket3: one CTA per row, ONE pass over the B rows and no per-bucket loops by single threads.  A
+// two-pass kernel with a thread per bucket measured (profiles/r02_ncu_bucket_v1.txt) L1TEX 74 % -- 7.5 sectors
+// per global load request, because every product looked the CDF table up twice per pass through L1 (32 lanes,
+// ~25 different sectors) -- and 45 % of its instructions ran at 3-4 active lanes.
 //   * the CDF table sits in shared memory (all 4096 knots, or every fourth for the small capacities);
 //   * the row's A entries are staged a chunk at a time as {B row start, length, first product index}: the
 //     colA -> rowptrB -> colB chain of dependent loads is paid once per chunk by all threads in parallel,
@@ -652,21 +546,24 @@ k_num_bucket3w(const int *__restrict__ queue, const int count, const int *__rest
 }
 
 // ---------------------------------------------------------------------------------------------------
-// k_num_bucket_heavy: the same bucket sort for rows with MORE products than fit on chip (the rows the
+// k_num_bucket_heavy: the bucket sort for rows with MORE products than fit on chip (the rows the
 // reference sends through EM_mergepath_global, bhsparse_cuda.h:2270-2525, and round 1 sent through a global
 // column bitmap -- at n = 16.8 M columns, config 5, that kernel ran at 6 products/ns and held rank 0 at 99 ms
-// while the other ranks finished in 67, profiles/r02_notes.md).  The row is cut into slices of the
+// while the other ranks finished in 67, profiles/r02_notes.md).  It runs the rows k_num_bucket_heavy2 (below)
+// cannot slice, from that kernel's retry queue.  The row is cut into slices of the
 // F-axis (F = the product-column CDF): 2^k equal slices sized for 1.5x headroom; a slice whose products
-// exceed the capacity is halved, recursively (an explicit stack, CTA-uniform control flow).  Every slice is
-// counted, scattered, sorted and emitted like a row of k_num_bucket; slices are processed in ascending F, so
-// their outputs concatenate into the sorted row.  The row's products are re-read once per slice and pass
+// exceed the capacity is halved, recursively (an explicit stack, CTA-uniform control flow).  Every slice takes
+// two passes over the row's B rows: the first counts its products per bucket, a CTA scan turns the counts into
+// segments, the second scatters (column, a*b) into them; then one thread per bucket insertion-sorts its entries
+// and merges equal columns, and a second scan gives the compacted positions.  Slices are processed in ascending F,
+// so their outputs concatenate into the sorted row.  The row's products are re-read once per slice and pass
 // (they sit in L1/L2).  A slice of a single F value that still overflows (thousands of products in one
 // column: possible only for rows of A with more entries than the capacity) is reduced column by column.
 // (Measured and dropped: finding a long B row's share of a slice by a warp-wide 32-ary search of its sorted
 // columns instead of scanning it with the filter -- 8 % slower on R-MAT 24 rank 0: the scans hit L1/L2, the searches
 // are chains of dependent loads.)
 // Direct mode: the row is staged at ct_base + [running sum of the products of the rows before it in the
-// launch, by atomic bump]; rc / ct_off as in k_num_bucket.
+// launch, by atomic bump]; its length goes to rc[row], its staging offset to ct_off[row].
 // ---------------------------------------------------------------------------------------------------
 template <typename VT, int THREADS>
 __global__ void __launch_bounds__(THREADS)

@@ -22,9 +22,6 @@
 #include "common.cuh"
 #include "stage_bucket.cuh"
 
-#include <cstdlib>
-#include <cstring>
-
 namespace bhb {
 
 template <typename VT, int G, int LOG2T, int R>
@@ -795,32 +792,12 @@ template <typename VT, int THREADS>
 static cudaError_t launch_num_bucket_tt(const LaunchCtx &lc, int cap, const int *queue, int count, Csr A, Csr B, DirectOut d,
                                         ColumnCdf cdf)
 {
-    // buckets per row: cap / BHB200_BUCKET_DIV (default 4: about four entries per bucket for a full row)
-    // BHB200_BUCKET_V=1: the first bucket kernel (two passes over B, a thread per bucket); default: k_num_bucket3
-    static const int version = [] { const char *e = getenv("BHB200_BUCKET_V"); return (e && atoi(e) == 1) ? 1 : 3; }();
-    if (version == 3 && cap <= 8192) {
-        // (one bucket per entry for the capacities up to 2048 instead of one per two: measured equal, R-MAT 21 39.46 vs 39.56 ms)
-        const int nb3 = cap / 2 < 32 ? 32 : cap / 2;
-        const bool small = cap <= 2048 || THREADS == 768;   // every fourth knot of the CDF: enough for <= 1024 buckets, and what lets two 4096-entry CTAs share an SM
-        const size_t smem3 = b3_smem_bytes<VT, THREADS>(cap, nb3, small ? 1024 : CDF_KNOTS);
-        auto k3 = small ? k_num_bucket3<VT, THREADS, 10> : k_num_bucket3<VT, THREADS, CDF_BITS>;
-        if (smem3 > 48 * 1024) {
-            cudaError_t e = cudaFuncSetAttribute(k3, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem3);
-            if (e != cudaSuccess) return e;
-        }
-        long long blocks3 = count;
-        const long long lim3 = (long long)lc.sm_count * resident_blocks(k3, THREADS, smem3);
-        if (blocks3 > lim3) blocks3 = lim3;
-        ++*lc.launches;
-        k3<<<(int)blocks3, THREADS, smem3, lc.stream>>>(queue, count, A.rowptr, A.col, (const VT *)A.val, B.rowptr, B.col,
-                                                         (const VT *)B.val, cdf, cap, nb3, d.rc, d.ct_off, d.ctcol, (VT *)d.ctval,
-                                                         d.ct_base, d.prod, d.p_lo, d.p_hi, d.ct_stride ? d.ct_stride : cap, d.bump);
-        return cudaGetLastError();
-    }
-    static const int div = [] { const char *e = getenv("BHB200_BUCKET_DIV"); const int v = e ? atoi(e) : 4; return (v == 1 || v == 2 || v == 4 || v == 8) ? v : 4; }();
-    const int nb = cap / div < 32 ? 32 : cap / div;
-    const size_t smem = (size_t)cap * (sizeof(VT) + 4) + (size_t)(2 * nb + 1 + 34) * 4;
-    auto kern = k_num_bucket<VT, THREADS>;
+    // (one bucket per entry for the capacities up to 2048 instead of one per two: measured equal, R-MAT 21 39.46 vs 39.56 ms)
+    const int nb = cap / 2;
+    // below 1024 threads every fourth knot of the CDF: enough for <= 1024 buckets, and what lets two 4096-entry CTAs share an SM
+    constexpr int KB = THREADS < 1024 ? 10 : CDF_BITS;
+    const size_t smem = b3_smem_bytes<VT, THREADS>(cap, nb, 1 << KB);
+    auto kern = k_num_bucket3<VT, THREADS, KB>;
     if (smem > 48 * 1024) {
         cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         if (e != cudaSuccess) return e;
@@ -831,7 +808,7 @@ static cudaError_t launch_num_bucket_tt(const LaunchCtx &lc, int cap, const int 
     ++*lc.launches;
     kern<<<(int)blocks, THREADS, smem, lc.stream>>>(queue, count, A.rowptr, A.col, (const VT *)A.val, B.rowptr, B.col,
                                                     (const VT *)B.val, cdf, cap, nb, d.rc, d.ct_off, d.ctcol, (VT *)d.ctval,
-                                                    d.ct_base, d.prod, d.p_lo, d.p_hi, d.ct_stride ? d.ct_stride : cap);
+                                                    d.ct_base, d.prod, d.p_lo, d.p_hi, d.ct_stride ? d.ct_stride : cap, d.bump);
     return cudaGetLastError();
 }
 
@@ -841,24 +818,15 @@ static cudaError_t launch_num_bucket_t(const LaunchCtx &lc, int cap, const int *
                                        ColumnCdf cdf)
 {
     if (count <= 0) return cudaSuccess;
-    // k_num_bucket3: a thread per BHB200_B3_EPT (default 4) entries of the capacity (its working set per entry is larger, so
-    // it needs more threads per row than k_num_bucket for the same occupancy)
-    static const int version = [] { const char *e = getenv("BHB200_BUCKET_V"); return (e && atoi(e) == 1) ? 1 : 3; }();
-    static const int ept = [] { const char *e = getenv("BHB200_B3_EPT"); const int v = e ? atoi(e) : 4; return (v == 2 || v == 4 || v == 8) ? v : 4; }();
-    if (version == 3 && cap <= 8192) {
-        const int thr = cap / ept;
-        if (thr <= 128) return launch_num_bucket_tt<VT, 128>(lc, cap, queue, count, A, B, d, cdf);
-        if (thr <= 256) return launch_num_bucket_tt<VT, 256>(lc, cap, queue, count, A, B, d, cdf);
-        if (thr <= 512) return launch_num_bucket_tt<VT, 512>(lc, cap, queue, count, A, B, d, cdf);
-        // 4096 entries: 2 x 768 threads per SM (109 KB each) instead of 1 x 1024 (BHB200_B3_768=off: the latter)
-        static const bool use768 = [] { const char *e = getenv("BHB200_B3_768"); return !(e && strcmp(e, "off") == 0); }();
-        if (cap == 4096 && use768) return launch_num_bucket_tt<VT, 768>(lc, cap, queue, count, A, B, d, cdf);
-        return launch_num_bucket_tt<VT, 1024>(lc, cap, queue, count, A, B, d, cdf);
+    // k_num_bucket3: a thread per four entries of the capacity, at most 1024
+    switch (cap) {
+    case 512: return launch_num_bucket_tt<VT, 128>(lc, cap, queue, count, A, B, d, cdf);
+    case 1024: return launch_num_bucket_tt<VT, 256>(lc, cap, queue, count, A, B, d, cdf);
+    case 2048: return launch_num_bucket_tt<VT, 512>(lc, cap, queue, count, A, B, d, cdf);
+    case 4096: return launch_num_bucket_tt<VT, 768>(lc, cap, queue, count, A, B, d, cdf);   // 2 x 768 threads per SM (109 KB each) beat 1 x 1024
+    case 8192: return launch_num_bucket_tt<VT, 1024>(lc, cap, queue, count, A, B, d, cdf);
+    default: return cudaErrorInvalidValue;
     }
-    if (cap <= 1024) return launch_num_bucket_tt<VT, 128>(lc, cap, queue, count, A, B, d, cdf);
-    if (cap <= 2048) return launch_num_bucket_tt<VT, 256>(lc, cap, queue, count, A, B, d, cdf);
-    if (cap <= 4096) return launch_num_bucket_tt<VT, 512>(lc, cap, queue, count, A, B, d, cdf);
-    return launch_num_bucket_tt<VT, 1024>(lc, cap, queue, count, A, B, d, cdf);
 }
 
 // warp-per-row bucket sort for the bins of at most 96 (capw 128) / 192 (capw 256) products; rows staged `stride` apart
@@ -903,9 +871,8 @@ static cudaError_t launch_num_bucket_heavy_t(const LaunchCtx &lc, const int *que
     if (count <= 0) return cudaSuccess;
     constexpr int THREADS = 1024;
     constexpr int cap = sizeof(VT) == 8 ? 12288 : 16384;   // entries of a slice held on chip
-    // buckets per slice: capacity / BHB200_HEAVY_DIV (default 2; measured on R-MAT 24 rank 0: /2 70.3, /4 72.5, /8 72.8 ms)
-    static const int div = [] { const char *e = getenv("BHB200_HEAVY_DIV"); const int v = e ? atoi(e) : 2; return (v == 2 || v == 4 || v == 8) ? v : 2; }();
-    const int nb = cap / div;
+    // buckets per slice: half the capacity (measured best on R-MAT 24 rank 0: /2 70.3, /4 72.5, /8 72.8 ms)
+    constexpr int nb = cap / 2;
     const size_t smem = (size_t)cap * (sizeof(VT) + 4) + (size_t)(2 * nb + 1 + 34) * 4 + (size_t)(CDF_KNOTS + 1) * 4;
     auto kern = k_num_bucket_heavy<VT, THREADS>;
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);

@@ -1,12 +1,6 @@
 // stage_pattern.cu -- kernels of the diagonal-pattern mode (see stage_pattern.cuh).
 #include "stage_pattern.cuh"
 
-#include <cstdlib>
-
-#ifndef PAT_DEFAULT_MINB
-#define PAT_DEFAULT_MINB 6
-#endif
-
 namespace bhb {
 
 // ---------------------------------------------------------------------------------------------
@@ -586,8 +580,9 @@ struct PatRec<float> {
 };
 
 // LONGB: rows of B may hold more than G entries (only possible for G = 32 with more than 32 diagonals in B)
-template <typename VT, int G, int MINB, bool LONGB>
-__global__ void __launch_bounds__(256, MINB)
+// 6 CTAs per SM (40 registers): per-warp memory-level parallelism beat 8 CTAs at 32 registers (profiles/r02_notes.md)
+template <typename VT, int G, bool LONGB>
+__global__ void __launch_bounds__(256, 6)
 k_pat_numeric(const int m, const int *__restrict__ rowptrA, const int *__restrict__ colA, const VT *__restrict__ valA,
               const unsigned char *__restrict__ ta, const int *__restrict__ rowptrB, const unsigned char *__restrict__ tb,
               const VT *__restrict__ valB, const PatTables t, const unsigned *__restrict__ outmask,
@@ -707,7 +702,7 @@ k_pat_numeric(const int m, const int *__restrict__ rowptrA, const int *__restric
     }
 }
 
-template <typename VT, int G, int MINB, bool LONGB>
+template <typename VT, int G, bool LONGB>
 static cudaError_t launch_pat_numeric_tbl(const LaunchCtx &lc, int m, Csr A, Csr B, const unsigned char *ta,
                                         const unsigned char *tb, const PatTables &t, const unsigned *outmask,
                                         const int64_t *rowoff, int *colC, VT *valC)
@@ -716,7 +711,7 @@ static cudaError_t launch_pat_numeric_tbl(const LaunchCtx &lc, int m, Csr A, Csr
     const int groups = threads / G;
     const size_t tab_bytes = ((size_t)t.nD * 4 + (size_t)t.nDA * t.nDB + (size_t)t.nD + 15) & ~(size_t)15;
     const size_t smem = tab_bytes + (size_t)groups * ((size_t)t.acc_len * sizeof(VT) + (size_t)G * 16);
-    auto kern = k_pat_numeric<VT, G, MINB, LONGB>;
+    auto kern = k_pat_numeric<VT, G, LONGB>;
     if (smem > 48 * 1024) {
         cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         if (e != cudaSuccess) return e;
@@ -730,215 +725,15 @@ static cudaError_t launch_pat_numeric_tbl(const LaunchCtx &lc, int m, Csr A, Csr
     return cudaGetLastError();
 }
 
-template <typename VT, int G, int MINB>
-static cudaError_t launch_pat_numeric_tb(const LaunchCtx &lc, int m, Csr A, Csr B, const unsigned char *ta,
-                                         const unsigned char *tb, const PatTables &t, const unsigned *outmask,
-                                         const int64_t *rowoff, int *colC, VT *valC)
-{
-    if constexpr (G == 32) {
-        if (t.nDB > 32) return launch_pat_numeric_tbl<VT, G, MINB, true>(lc, m, A, B, ta, tb, t, outmask, rowoff, colC, valC);
-    }
-    return launch_pat_numeric_tbl<VT, G, MINB, false>(lc, m, A, B, ta, tb, t, outmask, rowoff, colC, valC);
-}
-
-// ---------------------------------------------------------------------------------------------
-// k_pat_numeric_tma (EXPERIMENT, BHB200_PAT_TMA=1; G = 32, B rows of at most 32 entries): the same
-// kernel with the B rows staged by the TMA unit.  Lane 0 of a warp issues two 1-D bulk copies per
-// B row (cp.async.bulk.shared::cluster.global, SASS UBLKCP) -- the code bytes and the values, each
-// widened to the enclosing 16-byte-aligned range -- into a per-warp ring of PAT_TMA_STAGES stages,
-// completion signalled on an mbarrier per stage (SYNCS); the lanes read their element from shared
-// memory.  Three B rows are in flight per warp without a single register holding them.
-// Measured against the register-pipelined kernel in profiles/r02_notes.md.
-// ---------------------------------------------------------------------------------------------
-constexpr int PAT_TMA_STAGES = 4;
-constexpr int PAT_TMA_VAL_BYTES = 32 * 8 + 16;    // 32 values + alignment slack
-constexpr int PAT_TMA_CODE_BYTES = 48;            // 32 codes + alignment slack, 16-byte multiple
-
-__device__ __forceinline__ unsigned smem_u32(const void *p) { return (unsigned)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(unsigned bar, int count)
-{
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count) : "memory");
-}
-__device__ __forceinline__ void mbar_expect_tx(unsigned bar, unsigned bytes)
-{
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void bulk_g2s(unsigned dst, const void *src, unsigned bytes, unsigned bar)
-{
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(dst), "l"(src),
-                 "r"(bytes), "r"(bar)
-                 : "memory");
-}
-__device__ __forceinline__ void mbar_wait(unsigned bar, unsigned parity)
-{
-    asm volatile(
-        "{\n"
-        ".reg .pred p;\n"
-        "PAT_WAIT:\n"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n"
-        "@p bra PAT_DONE;\n"
-        "bra PAT_WAIT;\n"
-        "PAT_DONE:\n"
-        "}\n" ::"r"(bar),
-        "r"(parity)
-        : "memory");
-}
-
-template <typename VT>
-__global__ void __launch_bounds__(256, 6)
-k_pat_numeric_tma(const int m, const int *__restrict__ rowptrA, const int *__restrict__ colA, const VT *__restrict__ valA,
-                  const unsigned char *__restrict__ ta, const int *__restrict__ rowptrB, const unsigned char *__restrict__ tb,
-                  const VT *__restrict__ valB, const PatTables t, const unsigned *__restrict__ outmask,
-                  const int64_t *__restrict__ rowoff, int *__restrict__ colC, VT *__restrict__ valC)
-{
-    extern __shared__ __align__(16) unsigned char smem_raw[];
-    int *s_dcol = reinterpret_cast<int *>(smem_raw);
-    unsigned char *s_mphys = smem_raw + (size_t)t.nD * 4;
-    unsigned char *s_pos = s_mphys + (size_t)t.nDA * t.nDB;
-    const size_t tab_bytes = ((size_t)t.nD * 4 + (size_t)t.nDA * t.nDB + (size_t)t.nD + 15) & ~(size_t)15;
-    for (int i = threadIdx.x; i < t.nD; i += blockDim.x) {
-        s_dcol[i] = t.dcol[i];
-        s_pos[i] = t.pos[i];
-    }
-    for (int i = threadIdx.x; i < t.nDA * t.nDB; i += blockDim.x) s_mphys[i] = t.mphys[i];
-
-    const int lane = threadIdx.x & 31;
-    const int wib = threadIdx.x >> 5;
-    const int warps_per_block = blockDim.x >> 5;
-    const int acc_len = t.acc_len;
-    constexpr int STAGE_BYTES = PAT_TMA_VAL_BYTES + PAT_TMA_CODE_BYTES;
-    const size_t per_warp = (size_t)acc_len * sizeof(VT) + 32 * 16 + (size_t)PAT_TMA_STAGES * STAGE_BYTES + PAT_TMA_STAGES * 8;
-    unsigned char *mine = smem_raw + tab_bytes + (size_t)wib * per_warp;
-    VT *acc = reinterpret_cast<VT *>(mine);
-    int4 *rec = reinterpret_cast<int4 *>(mine + (size_t)acc_len * sizeof(VT));
-    unsigned char *ring = mine + (size_t)acc_len * sizeof(VT) + 32 * 16;
-    const unsigned bar0 = smem_u32(ring + (size_t)PAT_TMA_STAGES * STAGE_BYTES);
-    if (lane == 0) {
-#pragma unroll
-        for (int sgi = 0; sgi < PAT_TMA_STAGES; ++sgi) mbar_init(bar0 + 8 * sgi, 1);
-        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-    }
-    __syncthreads();
-    const int nDB = t.nDB, nD = t.nD, nw = t.nw;
-    unsigned phase = 0u;   // bit sg: parity to wait for on stage sg (warp-uniform)
-
-    // lane 0: start the two bulk copies of the B row of record r into stage sg
-    auto issue = [&](const int4 &r, const int sg) {
-        const int len = r.y & 0xffff;
-        if (len == 0) return;
-        const size_t v0 = (size_t)r.x * sizeof(VT), v1 = v0 + (size_t)len * sizeof(VT);
-        const size_t va = v0 & ~(size_t)15, vb = (v1 + 15) & ~(size_t)15;
-        const size_t c0 = (size_t)r.x, c1 = c0 + len;
-        const size_t ca = c0 & ~(size_t)15, cb = (c1 + 15) & ~(size_t)15;
-        const unsigned bar = bar0 + 8 * sg;
-        unsigned char *dst = ring + (size_t)sg * STAGE_BYTES;
-        mbar_expect_tx(bar, (unsigned)((vb - va) + (cb - ca)));
-        bulk_g2s(smem_u32(dst), reinterpret_cast<const unsigned char *>(valB) + va, (unsigned)(vb - va), bar);
-        bulk_g2s(smem_u32(dst + PAT_TMA_VAL_BYTES), tb + ca, (unsigned)(cb - ca), bar);
-    };
-
-    for (long long q = (long long)blockIdx.x * warps_per_block + wib; q < m; q += (long long)gridDim.x * warps_per_block) {
-        const int row = (int)q;
-        for (int s = lane; s < acc_len; s += 32) acc[s] = VT(0);
-        const int a0 = rowptrA[row];
-        const int na = rowptrA[row + 1] - a0;
-        for (int base = 0; base < na; base += 32) {
-            const int j = base + lane;
-            if (j < na) {
-                const int k = colA[a0 + j];
-                const int bs = rowptrB[k];
-                const int len = rowptrB[k + 1] - bs;
-                rec[lane] = PatRec<VT>::pack(bs, len | (((int)ta[a0 + j] * nDB) << 16), valA[a0 + j]);
-            }
-            __syncwarp();
-            const int cnt = min(32, na - base);
-            if (lane == 0) {
-                for (int u = 0; u < PAT_TMA_STAGES - 1 && u < cnt; ++u) issue(rec[u], u);
-            }
-            for (int tt = 0; tt < cnt; ++tt) {
-                const int sg = tt & (PAT_TMA_STAGES - 1);
-                if (lane == 0 && tt + PAT_TMA_STAGES - 1 < cnt)
-                    issue(rec[tt + PAT_TMA_STAGES - 1], (tt + PAT_TMA_STAGES - 1) & (PAT_TMA_STAGES - 1));
-                const int4 r = rec[tt];
-                const int len = r.y & 0xffff;
-                if (len > 0) {
-                    mbar_wait(bar0 + 8 * sg, (phase >> sg) & 1u);
-                    phase ^= 1u << sg;
-                    if (lane < len) {
-                        const unsigned char *st = ring + (size_t)sg * STAGE_BYTES;
-                        const VT bv = *reinterpret_cast<const VT *>(st + (((size_t)r.x * sizeof(VT)) & 15) + (size_t)lane * sizeof(VT));
-                        const int jb = st[PAT_TMA_VAL_BYTES + (r.x & 15) + lane];
-                        const int p = s_mphys[(r.y >> 16) + jb];
-                        acc[p] = fma(PatRec<VT>::val(r), bv, acc[p]);
-                    }
-                }
-                __syncwarp();   // accumulators of the next B row; the stage may be refilled
-            }
-        }
-        const int64_t o0 = rowoff[row];
-        const unsigned *mrow = outmask + (size_t)row * nw;
-        int rank0 = 0;
-        for (int ob = 0; ob < nD; ob += 32) {
-            const unsigned bits = __ldg(mrow + (ob >> 5));
-            const int o = ob + lane;
-            if ((bits >> lane) & 1u) {
-                const int rnk = rank0 + __popc(bits & ((1u << lane) - 1u));
-                colC[o0 + rnk] = row + s_dcol[o];
-                valC[o0 + rnk] = acc[s_pos[o]];
-            }
-            rank0 += __popc(bits);
-        }
-        __syncwarp();
-    }
-}
-
-template <typename VT>
-static cudaError_t launch_pat_numeric_tma(const LaunchCtx &lc, int m, Csr A, Csr B, const unsigned char *ta,
-                                          const unsigned char *tb, const PatTables &t, const unsigned *outmask,
-                                          const int64_t *rowoff, int *colC, VT *valC)
-{
-    const int threads = 256;
-    const size_t tab_bytes = ((size_t)t.nD * 4 + (size_t)t.nDA * t.nDB + (size_t)t.nD + 15) & ~(size_t)15;
-    const size_t per_warp = (size_t)t.acc_len * sizeof(VT) + 32 * 16 +
-                            (size_t)PAT_TMA_STAGES * (PAT_TMA_VAL_BYTES + PAT_TMA_CODE_BYTES) + PAT_TMA_STAGES * 8;
-    const size_t smem = tab_bytes + 8 * per_warp;
-    auto kern = k_pat_numeric_tma<VT>;
-    if (smem > 48 * 1024) {
-        cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e != cudaSuccess) return e;
-    }
-    long long blocks = ((long long)m + 7) / 8;
-    const long long cap = (long long)lc.sm_count * resident_blocks(kern, threads, smem);
-    if (blocks > cap) blocks = cap;
-    ++*lc.launches;
-    kern<<<(int)blocks, threads, smem, lc.stream>>>(m, A.rowptr, A.col, (const VT *)A.val, ta, B.rowptr, tb,
-                                                    (const VT *)B.val, t, outmask, rowoff, colC, valC);
-    return cudaGetLastError();
-}
-
-// resident CTAs per SM the compiler is asked for (register budget 32 / 36 / 40): BHB200_PAT_MINB=8|7|6
-// (experiments; see profiles/r02_notes.md for the measured choice)
-static int pat_minb()
-{
-    static int v = -1;
-    if (v < 0) {
-        const char *e = getenv("BHB200_PAT_MINB");
-        v = e ? atoi(e) : PAT_DEFAULT_MINB;
-        if (v != 6 && v != 7 && v != 8) v = PAT_DEFAULT_MINB;
-    }
-    return v;
-}
-
 template <typename VT, int G>
 static cudaError_t launch_pat_numeric_t(const LaunchCtx &lc, int m, Csr A, Csr B, const unsigned char *ta,
                                         const unsigned char *tb, const PatTables &t, const unsigned *outmask,
                                         const int64_t *rowoff, int *colC, VT *valC)
 {
-    switch (pat_minb()) {
-    case 6: return launch_pat_numeric_tb<VT, G, 6>(lc, m, A, B, ta, tb, t, outmask, rowoff, colC, valC);
-    case 7: return launch_pat_numeric_tb<VT, G, 7>(lc, m, A, B, ta, tb, t, outmask, rowoff, colC, valC);
-    default: return launch_pat_numeric_tb<VT, G, 8>(lc, m, A, B, ta, tb, t, outmask, rowoff, colC, valC);
+    if constexpr (G == 32) {
+        if (t.nDB > 32) return launch_pat_numeric_tbl<VT, G, true>(lc, m, A, B, ta, tb, t, outmask, rowoff, colC, valC);
     }
+    return launch_pat_numeric_tbl<VT, G, false>(lc, m, A, B, ta, tb, t, outmask, rowoff, colC, valC);
 }
 
 cudaError_t launch_pat_numeric(const LaunchCtx &lc, int dtype, int m, Csr A, Csr B, const unsigned char *ta,
@@ -947,11 +742,6 @@ cudaError_t launch_pat_numeric(const LaunchCtx &lc, int dtype, int m, Csr A, Csr
 {
     if (m <= 0) return cudaSuccess;
     const int G = t.nDB <= 8 ? 8 : t.nDB <= 16 ? 16 : 32;
-    static const bool use_tma = getenv("BHB200_PAT_TMA") && atoi(getenv("BHB200_PAT_TMA")) != 0;
-    if (use_tma && G == 32 && t.nDB <= 32 && (((size_t)B.val | (size_t)tb) & 15) == 0) {
-        if (dtype == 1) return launch_pat_numeric_tma<double>(lc, m, A, B, ta, tb, t, outmask, rowoff, colC, (double *)valC);
-        return launch_pat_numeric_tma<float>(lc, m, A, B, ta, tb, t, outmask, rowoff, colC, (float *)valC);
-    }
     if (dtype == 1) {   // BHB200_DTYPE_F64
         double *v = (double *)valC;
         if (G == 8) return launch_pat_numeric_t<double, 8>(lc, m, A, B, ta, tb, t, outmask, rowoff, colC, v);

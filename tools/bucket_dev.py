@@ -2,7 +2,7 @@
 """Development check of the wide-row kernels on R-MAT (needs a GPU): parity against the CPU oracle at
 the given scales in both precisions (`check`), or the per-bin report (`bins`, = tools/bin_report.py rmat).
 usage: python tools/bucket_dev.py check 16 18 | python tools/bucket_dev.py bins 21 [f32]
-The kernel variants are chosen by the library's environment switches (BHB200_BUCKET, BHB200_BUCKET_V, ...)."""
+The library picks the kernels; its environment switches (tools/README.md) are read when spgemm() creates its context."""
 import subprocess
 import sys
 import time
