@@ -64,14 +64,16 @@ class bhsparse:
 
     # -- data (bhsparse.h:180-258) -------------------------------------------
     def initData(self, m, k, n, nnzA, csrValA, csrRowPtrA, csrColIndA,
-                 nnzB, csrValB, csrRowPtrB, csrColIndB, csrRowPtrC) -> int:
+                 nnzB, csrValB, csrRowPtrB, csrColIndB, csrRowPtrC, transA=False, transB=False) -> int:
+        """C = op(A)*op(B): m, k, n are the dimensions of op(A) (m x k) and op(B) (k x n); with
+        transA / transB the arrays hold A / B as stored, i.e. k x m / n x k (bhb200_init_data_op_*)."""
         if not self._ctx:
             return capi.ERR_INVALID
         valA = np.ascontiguousarray(csrValA)
         if valA.dtype == np.float64:
-            fn, dt = self._lib.bhb200_init_data_f64, np.float64
+            fn, dt = self._lib.bhb200_init_data_op_f64, np.float64
         elif valA.dtype == np.float32:
-            fn, dt = self._lib.bhb200_init_data_f32, np.float32
+            fn, dt = self._lib.bhb200_init_data_op_f32, np.float32
         else:
             return capi.ERR_INVALID
         valB = np.ascontiguousarray(csrValB, dtype=dt)
@@ -79,14 +81,19 @@ class bhsparse:
         cA = np.ascontiguousarray(csrColIndA, dtype=np.int32)
         rpB = np.ascontiguousarray(csrRowPtrB, dtype=np.int32)
         cB = np.ascontiguousarray(csrColIndB, dtype=np.int32)
-        if rpA.size != m + 1 or rpB.size != k + 1 or cA.size < nnzA or cB.size < nnzB:
+        rows_a = k if transA else m            # rows of A / B as stored
+        rows_b = n if transB else k
+        if rpA.size != rows_a + 1 or rpB.size != rows_b + 1 or cA.size < nnzA or cB.size < nnzB:
             return capi.ERR_INVALID
         if csrRowPtrC is not None and (csrRowPtrC.dtype != np.int32 or csrRowPtrC.size < m + 1):
             return capi.ERR_INVALID
         self._rowptrC = csrRowPtrC           # caller-owned, written by get_C (main.cu:100)
         self._dtype = dt
         self._m = m
-        return fn(self._ctx, m, k, n, nnzA, _ptr(valA), _ptr(rpA), _ptr(cA), nnzB, _ptr(valB), _ptr(rpB), _ptr(cB))
+        # (the same host arrays for A and B stay the same objects here, so the library can upload them once)
+        opA = capi.OP_T if transA else capi.OP_N
+        opB = capi.OP_T if transB else capi.OP_N
+        return fn(self._ctx, opA, opB, m, k, n, nnzA, _ptr(valA), _ptr(rpA), _ptr(cA), nnzB, _ptr(valB), _ptr(rpB), _ptr(cB))
 
     def aliased_operands(self) -> bool:
         """True if initData got the same host arrays for A and B and uploaded them once."""
@@ -183,13 +190,17 @@ class bhsparse:
             pass
 
 
-def spgemm(A, B, device: int = 0, return_stats: bool = False, return_row_products: bool = False):
-    """Convenience driver following main.cu:104-135: C = A*B for two
-    generators.CSR operands; returns (rowptrC int32, colC int32, valC)."""
+def spgemm(A, B, device: int = 0, return_stats: bool = False, return_row_products: bool = False,
+           transA: bool = False, transB: bool = False):
+    """Convenience driver following main.cu:104-135: C = op(A)*op(B) for two
+    generators.CSR operands (op = transpose with transA / transB); returns
+    (rowptrC int32, colC int32, valC)."""
     platforms = [False] * NUM_PLATFORMS
     platforms[BHSPARSE_CUDA] = True
     bh = bhsparse(device)
-    rowptrC = np.zeros(A.rows + 1, dtype=np.int32)
+    m, k = (A.cols, A.rows) if transA else (A.rows, A.cols)
+    n = B.rows if transB else B.cols
+    rowptrC = np.zeros(m + 1, dtype=np.int32)
 
     def ok(err, what):
         if err != BHSPARSE_SUCCESS:
@@ -198,8 +209,8 @@ def spgemm(A, B, device: int = 0, return_stats: bool = False, return_row_product
             raise capi.BhsparseError(err, f"{what}: {msg}")
 
     ok(bh.initPlatform(platforms), "initPlatform")
-    ok(bh.initData(A.rows, A.cols, B.cols, A.nnz, A.val, A.rowptr, A.col,
-                   B.nnz, B.val, B.rowptr, B.col, rowptrC), "initData")
+    ok(bh.initData(m, k, n, A.nnz, A.val, A.rowptr, A.col,
+                   B.nnz, B.val, B.rowptr, B.col, rowptrC, transA, transB), "initData")
     ok(bh.spgemm(), "spgemm")
     nnzC = bh.get_nnzC()
     colC = np.empty(max(nnzC, 0), dtype=np.int32)

@@ -21,6 +21,8 @@ ERR_ALLOC = -4
 ERR_NO_DEVICE = -5
 DTYPE_F32 = 0
 DTYPE_F64 = 1
+OP_N = 0
+OP_T = 1
 NUM_BINS = 24
 
 SYM_BIN_NAMES = ["p=0", "p=1", "esc<=32", "g128", "g256", "g512", "g1024", "g2048", "g4096",
@@ -39,6 +41,7 @@ EXPORTED = [
     "bhb200_dist_unique_id", "bhb200_dist_init", "bhb200_dist_setup_square", "bhb200_dist_spgemm",
     "bhb200_dist_get_layout", "bhb200_dist_get_block_products", "bhb200_dist_get_global_rowptr_device",
     "bhb200_dist_broadcast_ms", "bhb200_dist_finalize", "bhb200_pattern_plan_probe",
+    "bhb200_init_data_op_f64", "bhb200_init_data_op_f32", "bhb200_init_data_device_op",
 ]
 DIST_ID_BYTES = 128
 
@@ -59,6 +62,7 @@ class Stats(ctypes.Structure):
         ("direct_bin_mask", c_int64),
         ("pattern_mode", c_int64), ("pattern_nDA", c_int64), ("pattern_nDB", c_int64), ("pattern_nD", c_int64),
         ("pattern_acc_len", c_int64), ("spill_bytes", c_int64),
+        ("transposed_ops", c_int64), ("ms_transpose", c_float),
     ]
 
     def as_dict(self) -> dict:
@@ -108,6 +112,9 @@ def load(build_if_missing: bool = False):
     L.bhb200_init_data_f32.argtypes = L.bhb200_init_data_f64.argtypes
     L.bhb200_init_data_device.argtypes = [ctxp, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p,
                                           c_int, c_void_p, c_void_p, c_void_p]
+    L.bhb200_init_data_op_f64.argtypes = [ctxp, c_int, c_int] + L.bhb200_init_data_f64.argtypes[1:]
+    L.bhb200_init_data_op_f32.argtypes = L.bhb200_init_data_op_f64.argtypes
+    L.bhb200_init_data_device_op.argtypes = [ctxp, c_int, c_int, c_int] + L.bhb200_init_data_device.argtypes[2:]
     L.bhb200_operands_aliased.argtypes = [ctxp]
     L.bhb200_get_operands_device.argtypes = [ctxp, POINTER(c_int32)] + [POINTER(c_void_p)] * 6
     L.bhb200_warmup.argtypes = [ctxp]

@@ -11,6 +11,7 @@
 // (:2527-2780) do not exist here: step 3 sizes C exactly.
 #pragma once
 #include <cuda_runtime.h>
+#include <stddef.h>
 #include <stdint.h>
 
 namespace bhb {
@@ -138,7 +139,12 @@ struct Counters {
     unsigned long long num_bin_products[MAX_BINS];
     unsigned long long num_bin_nnzc[MAX_BINS];
     unsigned long long num_bin_nnza[MAX_BINS];
+    // transposed operands (stage_transpose.cu): bit 0 / 1 = a column of the stored A / B outside its range.
+    // Last member: written by the transposition only, so a transposition done by bhb200_warmup is still
+    // reported by the next bhb200_spgemm (the per-call zeroing stops at CTR_ZERO_BYTES)
+    int bad_T;
 };
+constexpr size_t CTR_ZERO_BYTES = offsetof(Counters, bad_T);
 struct BinOffsets {
     int off[MAX_BINS + 1];
 };
@@ -557,6 +563,20 @@ cudaError_t launch_scan(const LaunchCtx &lc, int m, const int *rowptrA, const in
                         const int *rspan, unsigned spec_mask, const long long *ct_off, int64_t *rowoff64,
                         int *rowptr32, long long *blocksums, Counters *ctr);
 size_t scan_blocksum_count(int m);
+// stage_transpose.cu: X (rows x cols, nnz entries, int32 CSR) -> X^T (cols x rows) and perm with
+// out.val[p] = X.val[perm[p]]; a stored column outside [0, cols) is replaced by 0 and raises bad_bit in *bad
+struct TransposeOut {
+    int *rowptr;   // [cols + 1]
+    int *col;      // [nnz]
+    void *val;     // [nnz]
+    int *perm;     // [nnz]
+};
+size_t transpose_scratch_bytes(int nnz, int cols);
+int transpose_passes(int cols);
+cudaError_t launch_transpose(const LaunchCtx &lc, int dtype, int rows, int cols, int nnz, Csr X, TransposeOut out,
+                             void *scratch, int *bad, int bad_bit);
+// values again through the permutation of the last transposition: valT[p] = val[perm[p]]
+cudaError_t launch_regather(const LaunchCtx &lc, int dtype, int nnz, const void *val, const int *perm, void *valT);
 // stage_small.cu
 cudaError_t launch_sym_esc(const LaunchCtx &lc, const int *queue, int count, int n, Csr A, Csr B, int *rc);
 cudaError_t launch_num_single(const LaunchCtx &lc, int dtype, const int *queue, int count, Csr A, Csr B,

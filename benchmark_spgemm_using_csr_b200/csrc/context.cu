@@ -54,8 +54,15 @@ void release_operands(bhb200_ctx *ctx)
     ctx->b_rowptr.release(&ctx->dev_bytes);
     ctx->b_col.release(&ctx->dev_bytes);
     ctx->b_val.release(&ctx->dev_bytes);
+    DevBuf *tbufs[] = {&ctx->at_rowptr, &ctx->at_col, &ctx->at_val, &ctx->at_perm,
+                       &ctx->bt_rowptr, &ctx->bt_col, &ctx->bt_val, &ctx->bt_perm};
+    for (DevBuf *b : tbufs) b->release(&ctx->dev_bytes);
     ctx->A = Csr{nullptr, nullptr, nullptr};
     ctx->B = Csr{nullptr, nullptr, nullptr};
+    ctx->As = Csr{nullptr, nullptr, nullptr};
+    ctx->Bs = Csr{nullptr, nullptr, nullptr};
+    ctx->opA = ctx->opB = BHB200_OP_N;
+    ctx->t_pending = ctx->t_shared = false;
     ctx->have_data = false;
     ctx->borrowed = false;
     ctx->aliased = false;
@@ -76,31 +83,113 @@ int check_dims(bhb200_ctx *ctx, int m, int k, int n, int nnzA, int nnzB, const v
     return BHB200_SUCCESS;
 }
 
-int init_host(bhb200_ctx *ctx, int dtype, int m, int k, int n, int nnzA, const void *valA, const int32_t *rowptrA,
-              const int32_t *colA, int nnzB, const void *valB, const int32_t *rowptrB, const int32_t *colB)
+int check_ops(bhb200_ctx *ctx, int opA, int opB)
+{
+    if ((opA != BHB200_OP_N && opA != BHB200_OP_T) || (opB != BHB200_OP_N && opB != BHB200_OP_T))
+        return fail(ctx, BHB200_ERR_INVALID, "op must be BHB200_OP_N or BHB200_OP_T");
+    return BHB200_SUCCESS;
+}
+
+// ctx->A / ctx->B from the stored operands: the transposed copies (reserved here, filled by run_transposes) for op = T
+int set_effective(bhb200_ctx *ctx)
+{
+    const size_t vs = vsize(ctx->dtype);
+    ctx->A = ctx->As;
+    ctx->B = ctx->Bs;
+    if (ctx->opA) {
+        CU(ctx->at_rowptr.reserve(((size_t)ctx->m + 1) * 4, &ctx->dev_bytes), "alloc rowptr of A^T");
+        CU(ctx->at_col.reserve((size_t)ctx->nnzA * 4 + 4, &ctx->dev_bytes), "alloc col of A^T");
+        CU(ctx->at_val.reserve((size_t)ctx->nnzA * vs + 16, &ctx->dev_bytes), "alloc val of A^T");
+        CU(ctx->at_perm.reserve((size_t)ctx->nnzA * 4 + 4, &ctx->dev_bytes), "alloc perm of A^T");
+        ctx->A = Csr{ctx->at_rowptr.as<int>(), ctx->at_col.as<int>(), ctx->at_val.p};
+    }
+    if (ctx->opB && ctx->t_shared) {
+        ctx->B = ctx->A;
+    } else if (ctx->opB) {
+        CU(ctx->bt_rowptr.reserve(((size_t)ctx->k + 1) * 4, &ctx->dev_bytes), "alloc rowptr of B^T");
+        CU(ctx->bt_col.reserve((size_t)ctx->nnzB * 4 + 4, &ctx->dev_bytes), "alloc col of B^T");
+        CU(ctx->bt_val.reserve((size_t)ctx->nnzB * vs + 16, &ctx->dev_bytes), "alloc val of B^T");
+        CU(ctx->bt_perm.reserve((size_t)ctx->nnzB * 4 + 4, &ctx->dev_bytes), "alloc perm of B^T");
+        ctx->B = Csr{ctx->bt_rowptr.as<int>(), ctx->bt_col.as<int>(), ctx->bt_val.p};
+    }
+    ctx->t_pending = ctx->opA || ctx->opB;
+    return BHB200_SUCCESS;
+}
+
+// The transposed structure and values of every op = T operand, on the context's stream (no host sync).
+// A column of a stored operand outside its range raises a bit of Counters::bad_T, read with the counters.
+int run_transposes(bhb200_ctx *ctx, const LaunchCtx &lc)
+{
+    const bool tb = ctx->opB && !ctx->t_shared;
+    size_t need = 0;
+    if (ctx->opA) need = transpose_scratch_bytes(ctx->nnzA, ctx->m);
+    if (tb) need = std::max(need, transpose_scratch_bytes(ctx->nnzB, ctx->k));
+    if (need) CU(ctx->t_scratch.reserve(need, &ctx->dev_bytes), "alloc transpose scratch");
+    Counters *d_ctr = ctx->counters.as<Counters>();
+    CU(cudaMemsetAsync(&d_ctr->bad_T, 0, sizeof(int), lc.stream), "zero transpose flag");
+    if (ctx->opA)
+        CU(launch_transpose(lc, ctx->dtype, ctx->k, ctx->m, ctx->nnzA, ctx->As,
+                            TransposeOut{ctx->at_rowptr.as<int>(), ctx->at_col.as<int>(), ctx->at_val.p, ctx->at_perm.as<int>()},
+                            ctx->t_scratch.p, &d_ctr->bad_T, 1),
+           "transpose A");
+    if (tb)
+        CU(launch_transpose(lc, ctx->dtype, ctx->n, ctx->k, ctx->nnzB, ctx->Bs,
+                            TransposeOut{ctx->bt_rowptr.as<int>(), ctx->bt_col.as<int>(), ctx->bt_val.p, ctx->bt_perm.as<int>()},
+                            ctx->t_scratch.p, &d_ctr->bad_T, 2),
+           "transpose B");
+    ctx->t_pending = false;
+    return BHB200_SUCCESS;
+}
+
+// values of the op = T operands again from the stored values, through the permutation of the last transposition
+int run_regathers(bhb200_ctx *ctx, const LaunchCtx &lc)
+{
+    if (ctx->opA)
+        CU(launch_regather(lc, ctx->dtype, ctx->nnzA, ctx->As.val, ctx->at_perm.as<int>(), ctx->at_val.p), "re-gather values of A^T");
+    if (ctx->opB && !ctx->t_shared)
+        CU(launch_regather(lc, ctx->dtype, ctx->nnzB, ctx->Bs.val, ctx->bt_perm.as<int>(), ctx->bt_val.p), "re-gather values of B^T");
+    return BHB200_SUCCESS;
+}
+
+// Counters::bad_T of the transposition of this call's operands (read back with the other counters)
+int check_transposed(bhb200_ctx *ctx, int bad_T)
+{
+    if (!(ctx->opA || ctx->opB) || !bad_T) return BHB200_SUCCESS;
+    if (bad_T & 1) return fail(ctx, BHB200_ERR_INVALID, "a column index of the stored A (opA = T) is outside [0, m)");
+    return fail(ctx, BHB200_ERR_INVALID, "a column index of the stored B (opB = T) is outside [0, k)");
+}
+
+int init_host(bhb200_ctx *ctx, int dtype, int opA, int opB, int m, int k, int n, int nnzA, const void *valA,
+              const int32_t *rowptrA, const int32_t *colA, int nnzB, const void *valB, const int32_t *rowptrB,
+              const int32_t *colB)
 {
     if (!ctx) return BHB200_ERR_INVALID;
-    int rc = check_dims(ctx, m, k, n, nnzA, nnzB, valA, rowptrA, colA, valB, rowptrB, colB);
+    int rc = check_ops(ctx, opA, opB);
     if (rc) return rc;
-    if (rowptrA[0] != 0 || rowptrA[m] != nnzA) return fail(ctx, BHB200_ERR_INVALID, "rowptrA does not span [0, nnzA]");
-    if (rowptrB[0] != 0 || rowptrB[k] != nnzB) return fail(ctx, BHB200_ERR_INVALID, "rowptrB does not span [0, nnzB]");
+    rc = check_dims(ctx, m, k, n, nnzA, nnzB, valA, rowptrA, colA, valB, rowptrB, colB);
+    if (rc) return rc;
+    // stored shapes: A is m x k (k x m for opA = T), B is k x n (n x k for opB = T)
+    const int ra = opA ? k : m, ca = opA ? m : k, rb = opB ? n : k, cb = opB ? k : n;
+    if (rowptrA[0] != 0 || rowptrA[ra] != nnzA) return fail(ctx, BHB200_ERR_INVALID, "rowptrA does not span [0, nnzA]");
+    if (rowptrB[0] != 0 || rowptrB[rb] != nnzB) return fail(ctx, BHB200_ERR_INVALID, "rowptrB does not span [0, nnzB]");
     CU(cudaSetDevice(ctx->device), "cudaSetDevice");
     if (ctx->borrowed) release_operands(ctx);
     const size_t vs = vsize(dtype);
-    CU(ctx->a_rowptr.reserve((size_t)(m + 1) * 4, &ctx->dev_bytes), "alloc rowptrA");
+    CU(ctx->a_rowptr.reserve((size_t)(ra + 1) * 4, &ctx->dev_bytes), "alloc rowptrA");
     CU(ctx->a_col.reserve((size_t)nnzA * 4 + 4, &ctx->dev_bytes), "alloc colA");
     CU(ctx->a_val.reserve((size_t)nnzA * vs + 16, &ctx->dev_bytes), "alloc valA");
     // C = A*A with the SAME host arrays passed twice (the reference driver's stock workloads build
-    // A and B identically, main.cu:32-51): one upload, both operands point at it
-    const bool alias = m == k && nnzA == nnzB && rowptrA == rowptrB && colA == colB && valA == valB;
+    // A and B identically, main.cu:32-51): one upload, both operands point at it (also A*A^T, A^T*A)
+    const bool alias = ra == rb && (!(opA || opB) || ca == cb) && nnzA == nnzB && rowptrA == rowptrB && colA == colB &&
+                       valA == valB;
     if (!alias) {
-        CU(ctx->b_rowptr.reserve((size_t)(k + 1) * 4, &ctx->dev_bytes), "alloc rowptrB");
+        CU(ctx->b_rowptr.reserve((size_t)(rb + 1) * 4, &ctx->dev_bytes), "alloc rowptrB");
         CU(ctx->b_col.reserve((size_t)nnzB * 4 + 4, &ctx->dev_bytes), "alloc colB");
         CU(ctx->b_val.reserve((size_t)nnzB * vs + 16, &ctx->dev_bytes), "alloc valB");
     }
     cudaStream_t s = ctx->stream;
-    CU(cudaMemcpyAsync(ctx->a_rowptr.p, rowptrA, (size_t)(m + 1) * 4, cudaMemcpyHostToDevice, s), "H2D rowptrA");
-    if (!alias) CU(cudaMemcpyAsync(ctx->b_rowptr.p, rowptrB, (size_t)(k + 1) * 4, cudaMemcpyHostToDevice, s), "H2D rowptrB");
+    CU(cudaMemcpyAsync(ctx->a_rowptr.p, rowptrA, (size_t)(ra + 1) * 4, cudaMemcpyHostToDevice, s), "H2D rowptrA");
+    if (!alias) CU(cudaMemcpyAsync(ctx->b_rowptr.p, rowptrB, (size_t)(rb + 1) * 4, cudaMemcpyHostToDevice, s), "H2D rowptrB");
     if (nnzA > 0) {
         CU(cudaMemcpyAsync(ctx->a_col.p, colA, (size_t)nnzA * 4, cudaMemcpyHostToDevice, s), "H2D colA");
         CU(cudaMemcpyAsync(ctx->a_val.p, valA, (size_t)nnzA * vs, cudaMemcpyHostToDevice, s), "H2D valA");
@@ -110,8 +199,8 @@ int init_host(bhb200_ctx *ctx, int dtype, int m, int k, int n, int nnzA, const v
         CU(cudaMemcpyAsync(ctx->b_val.p, valB, (size_t)nnzB * vs, cudaMemcpyHostToDevice, s), "H2D valB");
     }
     CU(cudaStreamSynchronize(s), "H2D operands");
-    ctx->A = Csr{ctx->a_rowptr.as<int>(), ctx->a_col.as<int>(), ctx->a_val.p};
-    ctx->B = alias ? ctx->A : Csr{ctx->b_rowptr.as<int>(), ctx->b_col.as<int>(), ctx->b_val.p};
+    ctx->As = Csr{ctx->a_rowptr.as<int>(), ctx->a_col.as<int>(), ctx->a_val.p};
+    ctx->Bs = alias ? ctx->As : Csr{ctx->b_rowptr.as<int>(), ctx->b_col.as<int>(), ctx->b_val.p};
     ctx->aliased = alias;
     ctx->dtype = dtype;
     ctx->m = m;
@@ -119,6 +208,12 @@ int init_host(bhb200_ctx *ctx, int dtype, int m, int k, int n, int nnzA, const v
     ctx->n = n;
     ctx->nnzA = nnzA;
     ctx->nnzB = nnzB;
+    ctx->opA = opA;
+    ctx->opB = opB;
+    ctx->t_shared = alias && opA && opB;
+    ctx->have_data = false;
+    rc = set_effective(ctx);
+    if (rc) return rc;
     ctx->have_data = true;
     ctx->cdf_valid = false;   // new operands: the column CDF of the previous ones is not reused
     ctx->borrowed = false;
@@ -366,6 +461,7 @@ int run_pattern(bhb200_ctx *ctx, const LaunchCtx &lc, bool same_ab, bool specula
        "row pointer scan");
     CU(cudaMemcpyAsync(ctx->h_ctr, d_ctr, sizeof(Counters), cudaMemcpyDeviceToHost, s), "D2H counters");
     CU(cudaStreamSynchronize(s), "pattern symbolic / scan");
+    if (int rc = check_transposed(ctx, ctx->h_ctr->bad_T)) return rc;
     if (ctx->h_ctr->pat_miss) {
         ctx->plan = PatternPlan();   // (speculative or not: these lists do not describe the operands)
         return speculative ? PATTERN_PLAN_STALE : fail(ctx, BHB200_ERR_CUDA, "pattern mode: offset lists inconsistent with the operands");
@@ -494,7 +590,7 @@ int bhb200_free_mem(bhb200_ctx *ctx)
                       &ctx->cdf_colcount, &ctx->cdf_hist, &ctx->cdf_tab, &ctx->ct_off, &ctx->ct_col, &ctx->ct_val, &ctx->retry_q,
                       &ctx->brange, &ctx->rlo, &ctx->rspan, &ctx->wl_off, &ctx->wl_cnt, &ctx->wl_idx, &ctx->wl_bits,
                       &ctx->prod, &ctx->rc, &ctx->queue, &ctx->rowoff64, &ctx->rowptr32, &ctx->blocksums,
-                      &ctx->counters, &ctx->bitmap, &ctx->prefix, &ctx->colC, &ctx->valC, &ctx->slice_range};
+                      &ctx->counters, &ctx->bitmap, &ctx->prefix, &ctx->colC, &ctx->valC, &ctx->slice_range, &ctx->t_scratch};
     for (DevBuf *b : bufs) b->release(&ctx->dev_bytes);
     ctx->bitmap_zeroed_bytes = 0;
     cudaGetLastError();
@@ -545,33 +641,61 @@ int bhb200_init_data_f64(bhb200_ctx *ctx, int m, int k, int n, int nnzA, const d
                          const int32_t *colA, int nnzB, const double *valB, const int32_t *rowptrB,
                          const int32_t *colB)
 {
-    return init_host(ctx, BHB200_DTYPE_F64, m, k, n, nnzA, valA, rowptrA, colA, nnzB, valB, rowptrB, colB);
+    return init_host(ctx, BHB200_DTYPE_F64, BHB200_OP_N, BHB200_OP_N, m, k, n, nnzA, valA, rowptrA, colA, nnzB, valB,
+                     rowptrB, colB);
 }
 int bhb200_init_data_f32(bhb200_ctx *ctx, int m, int k, int n, int nnzA, const float *valA, const int32_t *rowptrA,
                          const int32_t *colA, int nnzB, const float *valB, const int32_t *rowptrB,
                          const int32_t *colB)
 {
-    return init_host(ctx, BHB200_DTYPE_F32, m, k, n, nnzA, valA, rowptrA, colA, nnzB, valB, rowptrB, colB);
+    return init_host(ctx, BHB200_DTYPE_F32, BHB200_OP_N, BHB200_OP_N, m, k, n, nnzA, valA, rowptrA, colA, nnzB, valB,
+                     rowptrB, colB);
+}
+int bhb200_init_data_op_f64(bhb200_ctx *ctx, int opA, int opB, int m, int k, int n, int nnzA, const double *valA,
+                            const int32_t *rowptrA, const int32_t *colA, int nnzB, const double *valB, const int32_t *rowptrB,
+                            const int32_t *colB)
+{
+    return init_host(ctx, BHB200_DTYPE_F64, opA, opB, m, k, n, nnzA, valA, rowptrA, colA, nnzB, valB, rowptrB, colB);
+}
+int bhb200_init_data_op_f32(bhb200_ctx *ctx, int opA, int opB, int m, int k, int n, int nnzA, const float *valA,
+                            const int32_t *rowptrA, const int32_t *colA, int nnzB, const float *valB, const int32_t *rowptrB,
+                            const int32_t *colB)
+{
+    return init_host(ctx, BHB200_DTYPE_F32, opA, opB, m, k, n, nnzA, valA, rowptrA, colA, nnzB, valB, rowptrB, colB);
 }
 
 int bhb200_init_data_device(bhb200_ctx *ctx, int dtype, int m, int k, int n, int nnzA, const void *valA,
                             const int32_t *rowptrA, const int32_t *colA, int nnzB, const void *valB,
                             const int32_t *rowptrB, const int32_t *colB)
 {
+    return bhb200_init_data_device_op(ctx, dtype, BHB200_OP_N, BHB200_OP_N, m, k, n, nnzA, valA, rowptrA, colA, nnzB, valB,
+                                      rowptrB, colB);
+}
+
+int bhb200_init_data_device_op(bhb200_ctx *ctx, int dtype, int opA, int opB, int m, int k, int n, int nnzA,
+                               const void *valA, const int32_t *rowptrA, const int32_t *colA, int nnzB, const void *valB,
+                               const int32_t *rowptrB, const int32_t *colB)
+{
     if (!ctx) return BHB200_ERR_INVALID;
     if (dtype != BHB200_DTYPE_F32 && dtype != BHB200_DTYPE_F64) return fail(ctx, BHB200_ERR_INVALID, "bad dtype");
-    int rc = check_dims(ctx, m, k, n, nnzA, nnzB, valA, rowptrA, colA, valB, rowptrB, colB);
+    int rc = check_ops(ctx, opA, opB);
+    if (rc) return rc;
+    rc = check_dims(ctx, m, k, n, nnzA, nnzB, valA, rowptrA, colA, valB, rowptrB, colB);
     if (rc) return rc;
     CU(cudaSetDevice(ctx->device), "cudaSetDevice");
     release_operands(ctx);
-    ctx->A = Csr{rowptrA, colA, valA};
-    ctx->B = Csr{rowptrB, colB, valB};
+    ctx->As = Csr{rowptrA, colA, valA};
+    ctx->Bs = Csr{rowptrB, colB, valB};
     ctx->dtype = dtype;
     ctx->m = m;
     ctx->k = k;
     ctx->n = n;
     ctx->nnzA = nnzA;
     ctx->nnzB = nnzB;
+    ctx->opA = opA;
+    ctx->opB = opB;
+    rc = set_effective(ctx);
+    if (rc) return rc;
     ctx->have_data = true;
     ctx->cdf_valid = false;   // new operands: the column CDF of the previous ones is not reused
     ctx->borrowed = true;
@@ -586,11 +710,15 @@ int bhb200_warmup(bhb200_ctx *ctx)
     int rc = reserve_workspace(ctx);
     if (rc) return rc;
     LaunchCtx lc{ctx->stream, ctx->sm_count, &ctx->launches, ctx->max_span};
+    if (ctx->t_pending) {   // (its column check is reported by the next spgemm)
+        rc = run_transposes(ctx, lc);
+        if (rc) return rc;
+    }
     CU(launch_b_row_ranges(lc, ctx->k, ctx->n, ctx->B, ctx->brange.as<int4>(), ctx->counters.as<Counters>()), "B row ranges kernel");
     // like the reference's warm-up (bhsparse.h:341-363: compute_nnzCt only) this must leave an existing
     // result intact: k_row_products rewrites rc[] and the counters, so it is skipped once C exists
     if (ctx->have_C) return BHB200_SUCCESS;
-    CU(cudaMemsetAsync(ctx->counters.p, 0, sizeof(Counters), ctx->stream), "zero counters");
+    CU(cudaMemsetAsync(ctx->counters.p, 0, CTR_ZERO_BYTES, ctx->stream), "zero counters");
     CU(launch_row_products(lc, ctx->m, ctx->k, ctx->nnzA, ctx->A, ctx->B, ctx->brange.as<int4>(), ctx->prod.as<int>(),
                            ctx->rc.as<int>(), ctx->rlo.as<int>(), ctx->rspan.as<int>(), ctx->counters.as<Counters>()),
        "row products kernel");
@@ -605,8 +733,10 @@ int bhb200_spgemm(bhb200_ctx *ctx)
     ctx->reuse_bins_valid = false;
     ctx->timing_valid = false;
     ctx->launches = 0;
+    ctx->t_ran = false;
     bhb200_stats &st = ctx->stats;
     memset(&st, 0, sizeof(st));
+    st.transposed_ops = (ctx->opA ? 1 : 0) | (ctx->opB ? 2 : 0);
     st.m = ctx->m;
     st.k = ctx->k;
     st.n = ctx->n;
@@ -626,7 +756,14 @@ int bhb200_spgemm(bhb200_ctx *ctx)
 
     // ---- stage 1: upper bound per row + symbolic bins ----
     CU(cudaEventRecord(ctx->ev[0], s), "event");
-    CU(cudaMemsetAsync(d_ctr, 0, sizeof(Counters), s), "zero counters");
+    // transposed operands: built once for host copies, on every call for borrowed ones (the caller may have rewritten them)
+    if (ctx->t_pending || (ctx->borrowed && (ctx->opA || ctx->opB))) {
+        rc = run_transposes(ctx, lc);
+        if (rc) return rc;
+        CU(cudaEventRecord(ctx->ev[5], s), "event");
+        ctx->t_ran = true;
+    }
+    CU(cudaMemsetAsync(d_ctr, 0, CTR_ZERO_BYTES, s), "zero counters");
     // diagonal-pattern mode: exact offset sets of A and B, read back with the stage-1 counters
     ctx->last_pattern = false;
     const bool same_ab = ctx->A.rowptr == ctx->B.rowptr && ctx->A.col == ctx->B.col && ctx->m == ctx->k;
@@ -644,7 +781,7 @@ int bhb200_spgemm(bhb200_ctx *ctx)
         }
         rc = run_pattern(ctx, lc, same_ab, true);
         if (rc != PATTERN_NOT_APPLICABLE && rc != PATTERN_PLAN_STALE) return rc;
-        CU(cudaMemsetAsync(d_ctr, 0, sizeof(Counters), s), "zero counters");
+        CU(cudaMemsetAsync(d_ctr, 0, CTR_ZERO_BYTES, s), "zero counters");
         st.pattern_mode = 0;
     }
     if (try_pattern) {
@@ -664,7 +801,7 @@ int bhb200_spgemm(bhb200_ctx *ctx)
         rc = run_pattern(ctx, lc, same_ab, false);
         if (rc != PATTERN_NOT_APPLICABLE) return rc;
         ctx->plan = PatternPlan();   // these operands are not diagonal-structured: no speculation next time
-        CU(cudaMemsetAsync(d_ctr, 0, sizeof(Counters), s), "zero counters");
+        CU(cudaMemsetAsync(d_ctr, 0, CTR_ZERO_BYTES, s), "zero counters");
     }
     int *rlo = ctx->rlo.as<int>();
     int *rspan = ctx->rspan.as<int>();
@@ -674,6 +811,8 @@ int bhb200_spgemm(bhb200_ctx *ctx)
     CU(cudaMemcpyAsync(ctx->h_ctr, d_ctr, sizeof(Counters), cudaMemcpyDeviceToHost, s), "D2H counters");
     CU(cudaStreamSynchronize(s), "stage 1");
     Counters hc = *ctx->h_ctr;
+    rc = check_transposed(ctx, hc.bad_T);
+    if (rc) return rc;
     if (hc.bad_B) return fail(ctx, BHB200_ERR_INVALID, "rows of B must be sorted by column, duplicate-free and inside [0, n)");
     if (hc.bad_A) return fail(ctx, BHB200_ERR_INVALID, "a column index of A is outside [0, k)");
     if (hc.row_overflow) return fail(ctx, BHB200_ERR_OVERFLOW, "a row has more than INT32_MAX intermediate products");
@@ -1043,11 +1182,19 @@ int bhb200_spgemm_numeric(bhb200_ctx *ctx)
     CU(cudaSetDevice(ctx->device), "cudaSetDevice");
     ctx->timing_valid = false;
     ctx->launches = 0;
+    ctx->t_ran = false;
     bhb200_stats &st = ctx->stats;
     cudaStream_t s = ctx->stream;
     LaunchCtx lc{s, ctx->sm_count, &ctx->launches, ctx->max_span};
     Counters *d_ctr = ctx->counters.as<Counters>();
     CU(cudaEventRecord(ctx->ev[0], s), "event");
+    if (ctx->borrowed && (ctx->opA || ctx->opB)) {
+        // borrowed operands are rewritten in place by the caller: their values again through perm
+        int rc = run_regathers(ctx, lc);
+        if (rc) return rc;
+        CU(cudaEventRecord(ctx->ev[5], s), "event");
+        ctx->t_ran = true;
+    }
     CU(cudaEventRecord(ctx->ev[1], s), "event");
     CU(cudaEventRecord(ctx->ev[2], s), "event");
     memset(ctx->ev_bin_used, 0, sizeof(ctx->ev_bin_used));
@@ -1064,7 +1211,7 @@ int bhb200_spgemm_numeric(bhb200_ctx *ctx)
     }
     if (!ctx->reuse_bins_valid) {
         // numeric bins of ALL rows (the direct-mode rows of the full product sit in the copy bin)
-        CU(cudaMemsetAsync(d_ctr, 0, sizeof(Counters), s), "zero counters");
+        CU(cudaMemsetAsync(d_ctr, 0, CTR_ZERO_BYTES, s), "zero counters");
         CU(launch_scan(lc, ctx->m, ctx->A.rowptr, ctx->prod.as<int>(), ctx->rc.as<int>(), ctx->rspan.as<int>(), 0u, nullptr,
                        ctx->rowoff64.as<int64_t>(), ctx->rowptr32.as<int>(), ctx->blocksums.as<long long>(), d_ctr),
            "row pointer scan");
@@ -1104,21 +1251,46 @@ static int update_values_any(bhb200_ctx *ctx, int dtype, const void *valA, const
     if (ctx->aliased && (valA || valB) && valA != valB) {
         // A and B share one device copy (same host arrays in initData) but now get different values:
         // give B its own copy (patterns unchanged, so every cached structure stays valid)
-        CU(ctx->b_rowptr.reserve((size_t)(ctx->k + 1) * 4, &ctx->dev_bytes), "alloc rowptrB");
+        const int rb = ctx->opB ? ctx->n : ctx->k;   // rows of B as stored
+        CU(ctx->b_rowptr.reserve((size_t)(rb + 1) * 4, &ctx->dev_bytes), "alloc rowptrB");
         CU(ctx->b_col.reserve((size_t)ctx->nnzB * 4 + 4, &ctx->dev_bytes), "alloc colB");
         CU(ctx->b_val.reserve((size_t)ctx->nnzB * vs + 8, &ctx->dev_bytes), "alloc valB");
-        CU(cudaMemcpyAsync(ctx->b_rowptr.p, ctx->a_rowptr.p, (size_t)(ctx->k + 1) * 4, cudaMemcpyDeviceToDevice, ctx->stream), "D2D rowptrB");
+        CU(cudaMemcpyAsync(ctx->b_rowptr.p, ctx->a_rowptr.p, (size_t)(rb + 1) * 4, cudaMemcpyDeviceToDevice, ctx->stream), "D2D rowptrB");
         if (ctx->nnzB > 0) {
             CU(cudaMemcpyAsync(ctx->b_col.p, ctx->a_col.p, (size_t)ctx->nnzB * 4, cudaMemcpyDeviceToDevice, ctx->stream), "D2D colB");
             CU(cudaMemcpyAsync(ctx->b_val.p, ctx->a_val.p, (size_t)ctx->nnzB * vs, cudaMemcpyDeviceToDevice, ctx->stream), "D2D valB");
         }
-        ctx->B = Csr{ctx->b_rowptr.as<int>(), ctx->b_col.as<int>(), ctx->b_val.p};
+        ctx->Bs = Csr{ctx->b_rowptr.as<int>(), ctx->b_col.as<int>(), ctx->b_val.p};
+        if (!ctx->opB) {
+            ctx->B = ctx->Bs;
+        } else if (ctx->t_shared) {
+            // op(B) shared op(A)'s transposed copy: B gets its own (same structure and permutation)
+            const bool pending = ctx->t_pending;
+            ctx->t_shared = false;
+            int rc = set_effective(ctx);
+            if (rc) return rc;
+            ctx->t_pending = pending;
+            cudaStream_t s = ctx->stream;
+            if (!pending)
+                CU(cudaMemcpyAsync(ctx->bt_rowptr.p, ctx->at_rowptr.p, (size_t)(ctx->k + 1) * 4, cudaMemcpyDeviceToDevice, s),
+                   "D2D rowptr of B^T");
+            if (!pending && ctx->nnzB > 0) {
+                CU(cudaMemcpyAsync(ctx->bt_col.p, ctx->at_col.p, (size_t)ctx->nnzB * 4, cudaMemcpyDeviceToDevice, s), "D2D col of B^T");
+                CU(cudaMemcpyAsync(ctx->bt_perm.p, ctx->at_perm.p, (size_t)ctx->nnzB * 4, cudaMemcpyDeviceToDevice, s), "D2D perm of B^T");
+            }
+        }
         ctx->aliased = false;
     }
     if (valA && ctx->nnzA > 0)
         CU(cudaMemcpyAsync(ctx->a_val.p, valA, (size_t)ctx->nnzA * vs, cudaMemcpyHostToDevice, ctx->stream), "H2D valA");
     if (valB && ctx->nnzB > 0 && !ctx->aliased)   // (still aliased: valB == valA, the shared copy has just been written)
         CU(cudaMemcpyAsync(ctx->b_val.p, valB, (size_t)ctx->nnzB * vs, cudaMemcpyHostToDevice, ctx->stream), "H2D valB");
+    if (!ctx->t_pending && (ctx->opA || ctx->opB)) {
+        // transposed operands: their values through the permutation of the transposition
+        LaunchCtx lc{ctx->stream, ctx->sm_count, &ctx->launches, ctx->max_span};
+        int rc = run_regathers(ctx, lc);
+        if (rc) return rc;
+    }
     CU(cudaStreamSynchronize(ctx->stream), "update values");
     return BHB200_SUCCESS;
 }
@@ -1309,6 +1481,11 @@ int bhb200_get_stats(const bhb200_ctx *cctx, bhb200_stats *out)
         bhb200_stats &st = ctx->stats;
         cudaEventElapsedTime(&st.ms_total, ctx->ev[0], ctx->ev[4]);
         cudaEventElapsedTime(&st.ms_count, ctx->ev[0], ctx->ev[1]);
+        st.ms_transpose = 0.f;
+        if (ctx->t_ran) {   // (ms_count then starts after the transposition)
+            cudaEventElapsedTime(&st.ms_transpose, ctx->ev[0], ctx->ev[5]);
+            cudaEventElapsedTime(&st.ms_count, ctx->ev[5], ctx->ev[1]);
+        }
         cudaEventElapsedTime(&st.ms_symbolic, ctx->ev[1], ctx->ev[2]);
         cudaEventElapsedTime(&st.ms_scan, ctx->ev[2], ctx->ev[3]);
         cudaEventElapsedTime(&st.ms_numeric, ctx->ev[3], ctx->ev[4]);

@@ -96,7 +96,15 @@ struct bhb200_ctx {
     int dtype = BHB200_DTYPE_F64;
     int m = 0, k = 0, n = 0, nnzA = 0, nnzB = 0;
     bhb::DevBuf a_rowptr, a_col, a_val, b_rowptr, b_col, b_val;
-    bhb::Csr A{nullptr, nullptr, nullptr}, B{nullptr, nullptr, nullptr};
+    bhb::Csr A{nullptr, nullptr, nullptr}, B{nullptr, nullptr, nullptr};   // the effective operands op(A), op(B)
+    // transposed operands (stage_transpose.cu): As / Bs are the operands as stored (host copies or borrowed);
+    // with op = BHB200_OP_T, A / B point at the library's transposed copy at_* / bt_* (grow-only)
+    int opA = BHB200_OP_N, opB = BHB200_OP_N;
+    bhb::Csr As{nullptr, nullptr, nullptr}, Bs{nullptr, nullptr, nullptr};
+    bhb::DevBuf at_rowptr, at_col, at_val, at_perm, bt_rowptr, bt_col, bt_val, bt_perm, t_scratch;
+    bool t_pending = false;   // the transposed structure is not built yet (host operands: once after init_data)
+    bool t_shared = false;    // same host arrays and both ops T: op(B) IS op(A) (one transposed copy)
+    bool t_ran = false;       // the last call transposed or re-gathered: ev[5] marks its end
 
     // workspace (grow-only, reused across calls)
     bhb::DevBuf prod, rc, queue, rowoff64, rowptr32, blocksums, counters, bitmap, prefix;
@@ -135,7 +143,7 @@ struct bhb200_ctx {
     bhb::WordLists last_wl{nullptr, nullptr, nullptr, nullptr, 0};
     bool reuse_bins_valid = false;   // queue holds the numeric bins without the copy bin
     int reuse_num_bin[bhb::MAX_BINS] = {0};
-    cudaEvent_t ev[5] = {nullptr, nullptr, nullptr, nullptr, nullptr};
+    cudaEvent_t ev[6] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};   // [5]: after the transposition
     bool timing_valid = false;
     bool profiling = false;
     int max_span = bhb::SPAN_SMALL;   // BHB200_RANGE=off|small|all overrides (experiments)

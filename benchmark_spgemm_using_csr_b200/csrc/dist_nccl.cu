@@ -404,6 +404,8 @@ int bhb200_dist_setup_square(bhb200_ctx *ctx, int root, int dtype, int n, int64_
     ctx->cdf_valid = false;   // new operands: the column CDF of the previous ones is not reused
     ctx->borrowed = true;    // (update_values does not apply; the b_* buffers stay library-owned)
     ctx->aliased = false;
+    ctx->opA = ctx->opB = BHB200_OP_N;   // (no transposed operands in the multi-GPU driver)
+    ctx->t_pending = ctx->t_shared = false;
     ctx->wait_before_values = d->ev_val;   // the first spgemm waits for the values after its stage 1
     DCU(cudaEventRecord(d->ev_t1, d->val_stream), "event");
     return BHB200_SUCCESS;

@@ -62,19 +62,22 @@ public:
         return err;
     }
 
-    /* bhsparse.h:180-258.  csrRowPtrC (m+1 ints) is caller-owned and written by get_C. */
+    /* bhsparse.h:180-258.  csrRowPtrC (m+1 ints) is caller-owned and written by get_C.
+     * Addition: transA / transB compute C = op(A)*op(B) with op(X) = X^T (bhb200_init_data_op_*);
+     * m, k, n are then the dimensions of op(A) (m x k) and op(B) (k x n), the arrays hold A / B as stored. */
     int initData(int m, int k, int n, int nnzA, value_type *csrValA, index_type *csrRowPtrA, index_type *csrColIndA,
                  int nnzB, value_type *csrValB, index_type *csrRowPtrB, index_type *csrColIndB,
-                 index_type *csrRowPtrC)
+                 index_type *csrRowPtrC, bool transA = false, bool transB = false)
     {
         if (!_ctx) return BHB200_ERR_INVALID;
         _rowptrC = csrRowPtrC;
+        const int opA = transA ? BHB200_OP_T : BHB200_OP_N, opB = transB ? BHB200_OP_T : BHB200_OP_N;
 #ifdef BHSPARSE_VALUE_FLOAT
-        return bhb200_init_data_f32(_ctx, m, k, n, nnzA, csrValA, csrRowPtrA, csrColIndA, nnzB, csrValB, csrRowPtrB,
-                                    csrColIndB);
+        return bhb200_init_data_op_f32(_ctx, opA, opB, m, k, n, nnzA, csrValA, csrRowPtrA, csrColIndA, nnzB, csrValB,
+                                       csrRowPtrB, csrColIndB);
 #else
-        return bhb200_init_data_f64(_ctx, m, k, n, nnzA, csrValA, csrRowPtrA, csrColIndA, nnzB, csrValB, csrRowPtrB,
-                                    csrColIndB);
+        return bhb200_init_data_op_f64(_ctx, opA, opB, m, k, n, nnzA, csrValA, csrRowPtrA, csrColIndA, nnzB, csrValB,
+                                       csrRowPtrB, csrColIndB);
 #endif
     }
 

@@ -45,6 +45,10 @@ extern "C" {
 #define BHB200_DTYPE_F32 0
 #define BHB200_DTYPE_F64 1
 
+/* op(X) of bhb200_init_data_op_* / bhb200_init_data_device_op: X as stored, or its transpose */
+#define BHB200_OP_N 0
+#define BHB200_OP_T 1
+
 #define BHB200_NUM_SYM_BINS 24
 #define BHB200_NUM_NUM_BINS 24
 
@@ -89,6 +93,11 @@ typedef struct bhb200_stats {
     /* host-memory spill: bytes of C / of the staging buffer that live in pinned, device-mapped host
      * memory because the device could not hold them (0 normally) */
     int64_t spill_bytes;
+    /* transposed operands: bit 0 = op(A) is A^T, bit 1 = op(B) is B^T.  ms_transpose: device time of the
+     * transposition (or value re-gather) this call ran, included in ms_total; its kernels count in
+     * kernel_launches */
+    int64_t transposed_ops;
+    float ms_transpose;
 } bhb200_stats;
 
 /* -- platform --------------------------------------------------------------
@@ -116,12 +125,33 @@ BHB200_API int bhb200_init_data_f64(bhb200_ctx *ctx, int m, int k, int n,
 BHB200_API int bhb200_init_data_f32(bhb200_ctx *ctx, int m, int k, int n,
                                     int nnzA, const float *valA, const int32_t *rowptrA, const int32_t *colA,
                                     int nnzB, const float *valB, const int32_t *rowptrB, const int32_t *colB);
-/* 1 if the last bhb200_init_data_{f64,f32} received the SAME host arrays for A and B (C = A*A as
- * the reference driver's stock workloads set it up, main.cu:32-51): they are uploaded once and both
- * operands share the device copy.  bhb200_update_values_* then takes one set of values. */
+/* C = op(A)*op(B) with op(X) = X (BHB200_OP_N) or X^T (BHB200_OP_T), as the transpose flags of
+ * cuSPARSE's legacy csrgemm: m, k, n are the dimensions of op(A) (m x k) and op(B) (k x n); the stored
+ * arrays have the stored row count + 1 row pointers (rowptrA: k+1 entries for opA = T, rowptrB: n+1 for
+ * opB = T).  The library transposes on the device (stable: the rows of X^T in increasing column order,
+ * whatever the order inside the stored rows, so with opB = T the rows of the stored B need not be
+ * sorted; they must still be duplicate-free).  A column of a stored operand outside its range makes
+ * bhb200_spgemm return BHB200_ERR_INVALID naming the operand.  When the transposition runs:
+ *   host operands (bhb200_init_data_op_*): once, at the first bhb200_warmup or bhb200_spgemm after
+ *     init_data; bhb200_update_values_* carries new values into the transposed copies;
+ *   borrowed operands (bhb200_init_data_device_op): at every bhb200_spgemm (the caller may have rewritten
+ *     them); bhb200_spgemm_numeric re-gathers the values of the transposed copies from the caller's arrays,
+ *     so values rewritten in place take effect with the structure kept.
+ * With the same host arrays for A and B (A*A^T, A^T*A) they are uploaded once; with both ops T one
+ * transposed copy serves both operands.  The two functions without _op are the OP_N, OP_N case. */
+BHB200_API int bhb200_init_data_op_f64(bhb200_ctx *ctx, int opA, int opB, int m, int k, int n,
+                                       int nnzA, const double *valA, const int32_t *rowptrA, const int32_t *colA,
+                                       int nnzB, const double *valB, const int32_t *rowptrB, const int32_t *colB);
+BHB200_API int bhb200_init_data_op_f32(bhb200_ctx *ctx, int opA, int opB, int m, int k, int n,
+                                       int nnzA, const float *valA, const int32_t *rowptrA, const int32_t *colA,
+                                       int nnzB, const float *valB, const int32_t *rowptrB, const int32_t *colB);
+/* 1 if the last bhb200_init_data_{f64,f32} (or _op_) received the SAME host arrays for A and B (C = A*A as
+ * the reference driver's stock workloads set it up, main.cu:32-51; also A*A^T, A^T*A): they are uploaded
+ * once and both operands share the device copy.  bhb200_update_values_* then takes one set of values. */
 BHB200_API int bhb200_operands_aliased(const bhb200_ctx *ctx);
 /* The operands as the library holds them on the device (borrowed views, valid until the next
- * init_data / dist_setup / free_mem): dims = {m, k, n, nnzA, nnzB, dtype}.  After
+ * init_data / dist_setup / free_mem): dims = {m, k, n, nnzA, nnzB, dtype}.  These are the effective
+ * operands op(A) and op(B): the transposed copies for BHB200_OP_T.  After
  * bhb200_dist_setup_square this is the rank's row block of A and its replica of B.  Any pointer may
  * be NULL. */
 BHB200_API int bhb200_get_operands_device(const bhb200_ctx *ctx, int32_t *dims, const int32_t **rowptrA,
@@ -133,6 +163,10 @@ BHB200_API int bhb200_get_operands_device(const bhb200_ctx *ctx, int32_t *dims, 
 BHB200_API int bhb200_init_data_device(bhb200_ctx *ctx, int dtype, int m, int k, int n,
                                        int nnzA, const void *valA, const int32_t *rowptrA, const int32_t *colA,
                                        int nnzB, const void *valB, const int32_t *rowptrB, const int32_t *colB);
+/* Device operands with transpose flags (see bhb200_init_data_op_f64 above for m, k, n and the rules). */
+BHB200_API int bhb200_init_data_device_op(bhb200_ctx *ctx, int dtype, int opA, int opB, int m, int k, int n,
+                                          int nnzA, const void *valA, const int32_t *rowptrA, const int32_t *colA,
+                                          int nnzB, const void *valB, const int32_t *rowptrB, const int32_t *colB);
 
 /* -- the hot path --------------------------------------------------------------
  * bhb200_warmup replaces bhsparse::warmup (bhsparse.h:341-363): runs the
