@@ -28,13 +28,14 @@ SOURCES = [
     "stage_range.cu",
     "stage_pattern.cu",
     "pattern_plan.cu",
+    "direct_plan.cu",
     "dist_nccl.cu",
     "stage_bucket.cu",
     "stage_numeric_f32.cu",
     "stage_numeric_f64.cu",
     "stage_transpose.cu",
 ]
-HEADERS = ["common.cuh", "stage_numeric.cuh", "stage_range.cuh", "stage_range_vec.cuh", "stage_pattern.cuh", "pattern_plan.h", "context.h", "stage_bucket.cuh", os.path.join(INCLUDE, "bhsparse_b200.h")]
+HEADERS = ["common.cuh", "stage_numeric.cuh", "stage_range.cuh", "stage_range_vec.cuh", "stage_pattern.cuh", "pattern_plan.h", "direct_plan.h", "context.h", "stage_bucket.cuh", os.path.join(INCLUDE, "bhsparse_b200.h")]
 
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",
@@ -49,6 +50,11 @@ def nvcc() -> str:
         if cand and os.path.exists(cand):
             return cand
     raise RuntimeError("nvcc not found: the CUDA library cannot be built (there is no CPU fallback)")
+
+
+def ccbin() -> list[str]:
+    """nvcc's host compiler: the image's $CC wrapper lacks some specs; use the system g++"""
+    return ["-ccbin", "/usr/bin/g++"] if os.path.exists("/usr/bin/g++") else []
 
 
 def _newest_header() -> float:
@@ -71,8 +77,6 @@ def build(force: bool = False, verbose: bool = False) -> str:
     cc = nvcc()
     hdr_time = _newest_header()
     extra = ["-Xptxas", "-v"] if verbose else []
-    # nvcc's host compiler: the image's $CC wrapper lacks some specs; use the system g++
-    ccbin = ["-ccbin", "/usr/bin/g++"] if os.path.exists("/usr/bin/g++") else []
 
     jobs = []
     for s in SOURCES:
@@ -83,7 +87,7 @@ def build(force: bool = False, verbose: bool = False) -> str:
 
     def compile_one(job):
         src, obj = job
-        cmd = [cc] + ccbin + NVCC_FLAGS + extra + ["-c", src, "-o", obj]
+        cmd = [cc] + ccbin() + NVCC_FLAGS + extra + ["-c", src, "-o", obj]
         r = subprocess.run(cmd, capture_output=True, text=True)
         return job, r
 
@@ -96,7 +100,7 @@ def build(force: bool = False, verbose: bool = False) -> str:
                     raise RuntimeError(f"nvcc failed on {src}:\n{r.stdout}\n{r.stderr}")
     objs = [os.path.join(OBJ, s.replace(".cu", ".o")) for s in SOURCES]
     if jobs or not os.path.exists(LIB) or any(os.path.getmtime(o) > os.path.getmtime(LIB) for o in objs):
-        cmd = [cc] + ccbin + ["-shared", "-o", LIB] + objs + ["-gencode", "arch=compute_100a,code=sm_100a", "-ldl"]
+        cmd = [cc] + ccbin() + ["-shared", "-o", LIB] + objs + ["-gencode", "arch=compute_100a,code=sm_100a", "-ldl"]
         r = subprocess.run(cmd, capture_output=True, text=True)
         if r.returncode != 0:
             raise RuntimeError(f"link failed:\n{r.stdout}\n{r.stderr}")

@@ -5,6 +5,7 @@
 // 300-byte counter block (bin sizes; nnz(C)) -- the reference has >= 8 blocking copies of
 // O(m) data plus 3 per merge round (SURVEY.md 3.2).
 #include "context.h"
+#include "direct_plan.h"
 #include "stage_bucket.cuh"
 
 #include <algorithm>
@@ -379,6 +380,48 @@ void finish_stats(bhb200_ctx *ctx)
     st.workspace_bytes = (int64_t)ctx->dev_bytes;
 }
 
+// per-call state common to bhb200_spgemm and bhb200_spgemm_numeric
+int begin_call(bhb200_ctx *ctx)
+{
+    CU(cudaSetDevice(ctx->device), "cudaSetDevice");
+    ctx->timing_valid = false;
+    ctx->launches = 0;
+    ctx->t_ran = false;
+    return BHB200_SUCCESS;
+}
+
+int read_counters(bhb200_ctx *ctx, const char *what)
+{
+    CU(cudaMemcpyAsync(ctx->h_ctr, ctx->counters.p, sizeof(Counters), cudaMemcpyDeviceToHost, ctx->stream), "D2H counters");
+    CU(cudaStreamSynchronize(ctx->stream), what);
+    return BHB200_SUCCESS;
+}
+
+// multi-GPU set-up (bhb200_dist_setup_square): the broadcast of B's values overlapped what ran so far; the rest reads them
+int wait_for_values(bhb200_ctx *ctx)
+{
+    if (ctx->wait_before_values) {
+        CU(cudaStreamWaitEvent(ctx->stream, ctx->wait_before_values, 0), "wait for the broadcast of B's values");
+        ctx->wait_before_values = nullptr;
+    }
+    return BHB200_SUCCESS;
+}
+
+int64_t spilled_bytes(const DevBuf &b)
+{
+    return b.host ? (int64_t)b.cap : 0;
+}
+
+// colC / valC for nnzC entries, spilled to host memory if the device cannot hold them
+int reserve_C(bhb200_ctx *ctx)
+{
+    CU(ctx->colC.reserve_spillable((size_t)ctx->nnzC * 4 + 16, &ctx->dev_bytes, ctx->device_cap, nullptr), "alloc colC");
+    CU(ctx->valC.reserve_spillable((size_t)ctx->nnzC * vsize(ctx->dtype) + 16, &ctx->dev_bytes, ctx->device_cap, nullptr),
+       "alloc valC");
+    ctx->stats.spill_bytes += spilled_bytes(ctx->colC) + spilled_bytes(ctx->valC);
+    return BHB200_SUCCESS;
+}
+
 // Diagonal-pattern mode (stage_pattern.cuh).  Called after the stage-1 sync with the offset sets of
 // A and B in ctx->h_sets.  Returns PATTERN_NOT_APPLICABLE if the operands do not qualify (the
 // caller continues with the general path), otherwise the result of the whole product.
@@ -459,8 +502,7 @@ int run_pattern(bhb200_ctx *ctx, const LaunchCtx &lc, bool same_ab, bool specula
     CU(launch_scan(lc, ctx->m, ctx->A.rowptr, ctx->prod.as<int>(), rcnt, nullptr, 0u, nullptr,
                    ctx->rowoff64.as<int64_t>(), ctx->rowptr32.as<int>(), ctx->blocksums.as<long long>(), d_ctr),
        "row pointer scan");
-    CU(cudaMemcpyAsync(ctx->h_ctr, d_ctr, sizeof(Counters), cudaMemcpyDeviceToHost, s), "D2H counters");
-    CU(cudaStreamSynchronize(s), "pattern symbolic / scan");
+    if (int rc = read_counters(ctx, "pattern symbolic / scan")) return rc;
     if (int rc = check_transposed(ctx, ctx->h_ctr->bad_T)) return rc;
     if (ctx->h_ctr->pat_miss) {
         ctx->plan = PatternPlan();   // (speculative or not: these lists do not describe the operands)
@@ -472,12 +514,7 @@ int run_pattern(bhb200_ctx *ctx, const LaunchCtx &lc, bool same_ab, bool specula
     st.nnzC = ctx->nnzC;
     st.products = (int64_t)ctx->h_ctr->products;
     st.max_row_products = ctx->h_ctr->max_row_products;
-    {
-        bool spilled = false;
-        CU(ctx->colC.reserve_spillable((size_t)ctx->nnzC * 4 + 16, &ctx->dev_bytes, ctx->device_cap, &spilled), "alloc colC");
-        CU(ctx->valC.reserve_spillable((size_t)ctx->nnzC * vs + 16, &ctx->dev_bytes, ctx->device_cap, &spilled), "alloc valC");
-        st.spill_bytes += (ctx->colC.host ? (int64_t)ctx->colC.cap : 0) + (ctx->valC.host ? (int64_t)ctx->valC.cap : 0);
-    }
+    if (int rc = reserve_C(ctx)) return rc;
     CU(cudaEventRecord(ctx->ev[3], s), "event");
     CU(launch_pat_numeric(lc, ctx->dtype, ctx->m, ctx->A, ctx->B, ta, tb, t, ctx->pat_outmask.as<unsigned>(),
                           ctx->rowoff64.as<int64_t>(), ctx->colC.as<int>(), ctx->valC.p),
@@ -498,6 +535,317 @@ int run_pattern(bhb200_ctx *ctx, const LaunchCtx &lc, bool same_ab, bool specula
     return BHB200_SUCCESS;
 }
 
+
+// ---- general mode: the stages of one bhb200_spgemm call ----
+
+// what the stages hand on to each other
+struct Product {
+    LaunchCtx lc;
+    Counters hc{};             // stage-1 counters, then those after the scan
+    int G = 32;                // lanes per row group of the hash kernels
+    BinOffsets so{}, no{};     // symbolic / numeric bin queues
+    DirectPlan plan{};
+    int cdf_shift = 0;
+    WordLists wl{nullptr, nullptr, nullptr, nullptr, 0};
+};
+
+// transposed operands: built once for host copies, on every call for borrowed ones (the caller may have rewritten them)
+int transpose_operands(bhb200_ctx *ctx, const LaunchCtx &lc)
+{
+    if (!ctx->t_pending && !(ctx->borrowed && (ctx->opA || ctx->opB))) return BHB200_SUCCESS;
+    const int rc = run_transposes(ctx, lc);
+    if (rc) return rc;
+    CU(cudaEventRecord(ctx->ev[5], ctx->stream), "event");
+    ctx->t_ran = true;
+    return BHB200_SUCCESS;
+}
+
+// diagonal-pattern mode, speculative on the previous product's plan, then with the exact offset sets of A and B
+// (read back by a sync of their own).  PATTERN_NOT_APPLICABLE: the general path follows, on zeroed counters.
+int try_pattern(bhb200_ctx *ctx, const LaunchCtx &lc)
+{
+    cudaStream_t s = ctx->stream;
+    Counters *d_ctr = ctx->counters.as<Counters>();
+    ctx->last_pattern = false;
+    const bool same_ab = ctx->A.rowptr == ctx->B.rowptr && ctx->A.col == ctx->B.col && ctx->m == ctx->k;
+    if (!(ctx->pattern_enable && ctx->m > 0 && ctx->nnzA > 0 && ctx->nnzB > 0)) return PATTERN_NOT_APPLICABLE;
+    if (ctx->pat_sets.reserve(2 * sizeof(PatSet), &ctx->dev_bytes) != cudaSuccess) {
+        cudaGetLastError();
+        return PATTERN_NOT_APPLICABLE;
+    }
+    int rc;
+    if (ctx->plan.valid && ctx->pattern_speculate) {
+        // the previous product on this context ran in pattern mode: reuse its plan without the detection
+        // pass; every entry is verified against it (k_pat_codes), a miss brings us back here
+        if ((rc = wait_for_values(ctx))) return rc;
+        rc = run_pattern(ctx, lc, same_ab, true);
+        if (rc != PATTERN_NOT_APPLICABLE && rc != PATTERN_PLAN_STALE) return rc;
+        CU(cudaMemsetAsync(d_ctr, 0, CTR_ZERO_BYTES, s), "zero counters");
+    }
+    PatSet *sets = ctx->pat_sets.as<PatSet>();
+    CU(cudaMemsetAsync(sets, 0x80, 2 * sizeof(PatSet), s), "init offset sets");   // slots = PAT_EMPTY
+    CU(cudaMemsetAsync(&sets[0], 0, 8, s), "init offset sets");
+    CU(cudaMemsetAsync(&sets[1], 0, 8, s), "init offset sets");
+    CU(launch_offset_set(lc, ctx->k, ctx->B.rowptr, ctx->B.col, &sets[1]), "offset set of B");
+    if (!same_ab) CU(launch_offset_set(lc, ctx->m, ctx->A.rowptr, ctx->A.col, &sets[0]), "offset set of A");
+    CU(cudaMemcpyAsync(ctx->h_sets, ctx->pat_sets.p, 2 * sizeof(PatSet), cudaMemcpyDeviceToHost, s), "D2H offset sets");
+    CU(cudaStreamSynchronize(s), "offset sets");
+    if ((rc = wait_for_values(ctx))) return rc;
+    rc = run_pattern(ctx, lc, same_ab, false);
+    if (rc != PATTERN_NOT_APPLICABLE) return rc;
+    ctx->plan = PatternPlan();   // these operands are not diagonal-structured: no speculation next time
+    CU(cudaMemsetAsync(d_ctr, 0, CTR_ZERO_BYTES, s), "zero counters");
+    return PATTERN_NOT_APPLICABLE;
+}
+
+// ---- stage 1: upper bound per row + symbolic bins ----
+int stage1_counts(bhb200_ctx *ctx, Product &p)
+{
+    Counters *d_ctr = ctx->counters.as<Counters>();
+    bhb200_stats &st = ctx->stats;
+    CU(launch_b_row_ranges(p.lc, ctx->k, ctx->n, ctx->B, ctx->brange.as<int4>(), d_ctr), "B row ranges kernel");
+    CU(launch_row_products(p.lc, ctx->m, ctx->k, ctx->nnzA, ctx->A, ctx->B, ctx->brange.as<int4>(), ctx->prod.as<int>(),
+                           ctx->rc.as<int>(), ctx->rlo.as<int>(), ctx->rspan.as<int>(), d_ctr),
+       "row products kernel");
+    int rc = read_counters(ctx, "stage 1");
+    if (rc) return rc;
+    p.hc = *ctx->h_ctr;
+    const Counters &hc = p.hc;
+    if ((rc = check_transposed(ctx, hc.bad_T))) return rc;
+    if (hc.bad_B) return fail(ctx, BHB200_ERR_INVALID, "rows of B must be sorted by column, duplicate-free and inside [0, n)");
+    if (hc.bad_A) return fail(ctx, BHB200_ERR_INVALID, "a column index of A is outside [0, k)");
+    if (hc.row_overflow) return fail(ctx, BHB200_ERR_OVERFLOW, "a row has more than INT32_MAX intermediate products");
+    st.products = (int64_t)hc.products;
+    st.max_row_products = hc.max_row_products;
+    for (int b = 0; b < BHB200_NUM_SYM_BINS && b < MAX_BINS; ++b) st.sym_bin_rows[b] = hc.sym_bin[b];
+    if ((rc = wait_for_values(ctx))) return rc;
+    // lanes per row group: follow the average length of the B rows actually referenced
+    const double avg_b = ctx->nnzA > 0 ? (double)hc.products / (double)ctx->nnzA : 0.0;
+    p.G = avg_b <= 10.0 ? 8 : 32;
+    offsets_from_counts(hc.sym_bin, p.so);
+    CU(launch_bin_scatter(p.lc, false, ctx->m, ctx->prod.as<int>(), ctx->rc.as<int>(), ctx->rspan.as<int>(), 0u, nullptr, p.so,
+                          d_ctr, ctx->queue.as<int>()),
+       "symbolic bin scatter");
+    return BHB200_SUCCESS;
+}
+
+// ---- direct (single-pass) mode: sample the group-hash bins, plan (direct_plan.cu), staging buffer, column CDF ----
+int choose_direct(bhb200_ctx *ctx, Product &p)
+{
+    Counters *d_ctr = ctx->counters.as<Counters>();
+    bhb200_stats &st = ctx->stats;
+    const size_t vs = vsize(ctx->dtype);
+    const DirectSwitches sw{ctx->direct_mode != 0, ctx->direct_wide != 0, ctx->bucket_warp != 0, ctx->force_cap,
+                            ctx->force_heavy};
+    const unsigned sampled = direct_sample_bins(p.hc, sw);
+    for (int b = SB_G128; b <= SB_G4096; ++b)
+        if ((sampled >> b) & 1u)
+            CU(launch_sym_hash(p.lc, b, p.G, ctx->queue.as<int>() + p.so.off[b], direct_sample_rows(p.hc.sym_bin[b]), ctx->A,
+                               ctx->B, ctx->rc.as<int>(), DIRECT_SAMPLE_STRIDE, &d_ctr->sample_max[b], nullptr,
+                               &d_ctr->sample_sum[b]),
+               "symbolic sample");
+    int rc = sampled ? read_counters(ctx, "direct-mode sampling") : BHB200_SUCCESS;
+    if (rc) return rc;
+    p.plan = plan_direct(*ctx->h_ctr, sw, vs);   // (*h_ctr: the stage-1 counters, sampled or not)
+    DirectPlan &plan = p.plan;
+    // the wide staging buffer must not crowd out C itself (at most `products` entries)
+    // (only checked when the staging buffer has to grow: cudaMemGetInfo can take milliseconds)
+    if (plan.mask() &&
+        ((size_t)plan.ct_entries * 4 + 16 > ctx->ct_col.cap || (size_t)plan.ct_entries * vs + 16 > ctx->ct_val.cap)) {
+        size_t free_b = 0, total_b = 0;
+        cudaMemGetInfo(&free_b, &total_b);
+        const double avail = (double)free_b + (double)ctx->ct_col.cap + (double)ctx->ct_val.cap + (double)ctx->colC.cap +
+                             (double)ctx->valC.cap;
+        const double need = ((double)plan.ct_entries + (double)st.products) * (4.0 + vs);
+        if (need > 0.9 * avail) plan.drop_wide();
+    }
+    if (plan.mask()) {
+        const size_t m1 = (size_t)ctx->m + 1;
+        // the staging buffer (the reference's Ct) may spill to host memory like C itself
+        if (ctx->ct_off.reserve(m1 * 8, &ctx->dev_bytes) != cudaSuccess ||
+            ctx->retry_q.reserve(m1 * 4, &ctx->dev_bytes) != cudaSuccess ||
+            ctx->ct_col.reserve_spillable((size_t)plan.ct_entries * 4 + 16, &ctx->dev_bytes, ctx->device_cap, nullptr) != cudaSuccess ||
+            ctx->ct_val.reserve_spillable((size_t)plan.ct_entries * vs + 16, &ctx->dev_bytes, ctx->device_cap, nullptr) != cudaSuccess) {
+            cudaGetLastError();
+            plan.drop_all();   // no room for the staging buffer: two-pass path for everything
+        } else {
+            st.spill_bytes += spilled_bytes(ctx->ct_col) + spilled_bytes(ctx->ct_val);
+        }
+    }
+    st.direct_ct_bytes = plan.ct_bytes();
+    st.direct_bin_mask = (int64_t)plan.mask();
+    CU(cudaEventRecord(ctx->ev[1], ctx->stream), "event");
+    if (plan.uses_bucket() && (ctx->cdf_colcount.reserve(((size_t)ctx->k + 1) * 4, &ctx->dev_bytes) != cudaSuccess ||
+                               ctx->cdf_hist.reserve((size_t)CDF_KNOTS * 8, &ctx->dev_bytes) != cudaSuccess ||
+                               ctx->cdf_tab.reserve((size_t)(CDF_KNOTS + 1) * 4, &ctx->dev_bytes) != cudaSuccess)) {
+        cudaGetLastError();
+        plan.drop_bucket();
+    }
+    if (plan.uses_bucket() && ctx->cdf_valid) {
+        p.cdf_shift = ctx->cdf_shift_cached;
+    } else if (plan.uses_bucket()) {
+        CU(launch_build_cdf(p.lc, ctx->m, ctx->k, ctx->n, ctx->nnzA, ctx->A, ctx->B, ctx->cdf_colcount.as<int>(),
+                            ctx->cdf_hist.as<unsigned long long>(), ctx->cdf_tab.as<unsigned>(), &p.cdf_shift),
+           "column CDF");
+        ctx->cdf_valid = true;
+        ctx->cdf_shift_cached = p.cdf_shift;
+    }
+    return BHB200_SUCCESS;
+}
+
+// the launches DirectPlan::launches lists for direct-mode bin b, in the value type of the operands
+int run_direct_bin(bhb200_ctx *ctx, const Product &p, int b)
+{
+    struct Kernels {
+        decltype(&launch_num_direct_f32) direct;
+        decltype(&launch_num_bucket_f32) bucket;
+        decltype(&launch_num_bucket3w_f32) bucket3w;
+        decltype(&launch_num_bucket_heavy2_f32) heavy2;
+        decltype(&launch_num_bucket_heavy_f32) heavy;
+    };
+    static const Kernels F32{launch_num_direct_f32, launch_num_bucket_f32, launch_num_bucket3w_f32,
+                             launch_num_bucket_heavy2_f32, launch_num_bucket_heavy_f32};
+    static const Kernels F64{launch_num_direct_f64, launch_num_bucket_f64, launch_num_bucket3w_f64,
+                             launch_num_bucket_heavy2_f64, launch_num_bucket_heavy_f64};
+    const Kernels &k = ctx->dtype == BHB200_DTYPE_F64 ? F64 : F32;
+    const DirectBin &db = p.plan.bin[b];
+    Counters *d_ctr = ctx->counters.as<Counters>();
+    const int *queue = ctx->queue.as<int>() + p.so.off[b];
+    int *retry_queue = ctx->retry_q.as<int>() + p.so.off[b];
+    const unsigned *cdf = ctx->cdf_tab.as<unsigned>();
+    const DirectLaunches ls = p.plan.launches(b, p.G);
+    for (int i = 0; i < ls.n; ++i) {
+        const DirectLaunch &l = ls.at[i];
+        DirectOut d{ctx->rc.as<int>(), ctx->ct_off.as<long long>(), ctx->ct_col.as<int>(), ctx->ct_val.p, db.base,
+                    retry_queue, &d_ctr->retry_cnt[b]};
+        // tight bins take every row of the queue; wide and heavy ones choose and stage rows by their product count
+        if (db.mode != DirectMode::TIGHT) d.prod = ctx->prod.as<int>();
+        if (db.mode == DirectMode::HEAVY) d.bump = &d_ctr->heavy_cursor;
+        d.p_lo = l.p_lo;
+        d.p_hi = l.p_hi;
+        d.ct_stride = l.stride;
+        switch (l.kernel) {
+        case DirectKernel::DIRECT:
+            CU(k.direct(p.lc, l.cap, l.sg, queue, db.rows, ctx->A, ctx->B, d), "direct numeric");
+            break;
+        case DirectKernel::BUCKET:
+            CU(k.bucket(p.lc, l.cap, queue, db.rows, ctx->A, ctx->B, d, cdf, p.cdf_shift), "bucket numeric");
+            break;
+        case DirectKernel::BUCKET3W:
+            CU(k.bucket3w(p.lc, l.cap, l.sg, queue, db.rows, ctx->A, ctx->B, d, cdf, p.cdf_shift, l.stride), "warp bucket numeric");
+            break;
+        case DirectKernel::HEAVY:
+            CU(k.heavy2(p.lc, queue, db.rows, ctx->A, ctx->B, d, cdf, p.cdf_shift, &d_ctr->heavy_cursor), "heavy rows");
+            d.count_dev = d.retry_cnt;   // what k_num_bucket_heavy2 could not slice
+            CU(k.heavy(p.lc, retry_queue, db.rows, ctx->A, ctx->B, d, cdf, p.cdf_shift, &d_ctr->heavy_cursor), "heavy rows");
+            break;
+        }
+    }
+    // rows that did not fit: ordinary symbolic pass, row count read on the device
+    if (ls.retry)
+        CU(launch_sym_hash(p.lc, b, p.G, retry_queue, db.rows, ctx->A, ctx->B, ctx->rc.as<int>(), 1, nullptr, &d_ctr->retry_cnt[b]),
+           "symbolic retry");
+    return BHB200_SUCCESS;
+}
+
+// ---- stage 2: symbolic, one launch per non-empty bin (direct-mode bins: the numeric kernel itself) ----
+int stage2_symbolic(bhb200_ctx *ctx, Product &p)
+{
+    const Counters &hc = p.hc;
+    const int *queue = ctx->queue.as<int>();
+    int *rcnt = ctx->rc.as<int>();
+    int rc;
+    memset(ctx->ev_bin_used, 0, sizeof(ctx->ev_bin_used));
+    if (hc.sym_bin[SB_ESC] > 0) CU(stamp(ctx, 0, SB_ESC), "event");
+    CU(launch_sym_esc(p.lc, queue + p.so.off[SB_ESC], hc.sym_bin[SB_ESC], ctx->n, ctx->A, ctx->B, rcnt), "symbolic ESC");
+    for (int b = SB_G128; b <= SB_LARGE; ++b) {
+        const int rows = hc.sym_bin[b];
+        if (p.plan.bin[b].mode != DirectMode::TWO_PASS) {
+            CU(stamp(ctx, 0, b), "event");
+            if ((rc = run_direct_bin(ctx, p, b))) return rc;
+            ctx->stats.direct_rows += rows;
+        } else if (b < SB_LARGE) {
+            if (rows > 0) CU(stamp(ctx, 0, b), "event");
+            CU(launch_sym_hash(p.lc, b, p.G, queue + p.so.off[b], rows, ctx->A, ctx->B, rcnt), "symbolic hash");
+        } else if (rows > 0) {
+            if ((rc = reserve_large_scratch(ctx, false))) return rc;
+            CU(stamp(ctx, 0, SB_LARGE), "event");
+            CU(launch_sym_large(p.lc, queue + p.so.off[SB_LARGE], rows, ctx->n, ctx->A, ctx->B, rcnt, ctx->bitmap.as<unsigned>(),
+                                large_scratch_blocks(ctx->sm_count, ctx->n)),
+               "symbolic large");
+        }
+    }
+    if (hc.sym_bin[SB_RANGE_S] + hc.sym_bin[SB_RANGE_L] > 0) {
+        if ((rc = reserve_word_lists(ctx, ctx->stats.products, p.wl))) return rc;
+        int *rlo = ctx->rlo.as<int>();
+        Counters *d_ctr = ctx->counters.as<Counters>();
+        if (hc.sym_bin[SB_RANGE_S] > 0) {
+            CU(stamp(ctx, 0, SB_RANGE_S), "event");
+            CU(launch_sym_range(p.lc, NSUM_SMALL, queue + p.so.off[SB_RANGE_S], hc.sym_bin[SB_RANGE_S], ctx->A, ctx->B, rlo,
+                                rcnt, d_ctr, p.wl),
+               "symbolic range (small span)");
+        }
+        if (hc.sym_bin[SB_RANGE_L] > 0) {
+            CU(stamp(ctx, 0, SB_RANGE_L), "event");
+            CU(launch_sym_range(p.lc, NSUM_LARGE, queue + p.so.off[SB_RANGE_L], hc.sym_bin[SB_RANGE_L], ctx->A, ctx->B, rlo,
+                                rcnt, d_ctr, p.wl),
+               "symbolic range (large span)");
+        }
+    }
+    CU(stamp(ctx, 0, MAX_BINS), "event");
+    CU(cudaEventRecord(ctx->ev[2], ctx->stream), "event");
+    return BHB200_SUCCESS;
+}
+
+// ---- stage 3: row pointers, numeric bins, exact allocation of C ----
+int stage3_scan_alloc(bhb200_ctx *ctx, Product &p)
+{
+    const unsigned mask = p.plan.mask();
+    Counters *d_ctr = ctx->counters.as<Counters>();
+    bhb200_stats &st = ctx->stats;
+    CU(launch_scan(p.lc, ctx->m, ctx->A.rowptr, ctx->prod.as<int>(), ctx->rc.as<int>(), ctx->rspan.as<int>(), mask,
+                   ctx->ct_off.as<long long>(), ctx->rowoff64.as<int64_t>(), ctx->rowptr32.as<int>(),
+                   ctx->blocksums.as<long long>(), d_ctr),
+       "row pointer scan");
+    int rc = read_counters(ctx, "stage 2/3");
+    if (rc) return rc;
+    p.hc = *ctx->h_ctr;
+    const Counters &hc = p.hc;
+    ctx->nnzC = (int64_t)hc.nnzC;
+    st.nnzC = ctx->nnzC;
+    for (int b = 0; b < BHB200_NUM_NUM_BINS && b < MAX_BINS; ++b) {
+        st.num_bin_rows[b] = hc.num_bin[b];
+        st.num_bin_products[b] = (int64_t)hc.num_bin_products[b];
+        st.num_bin_nnzC[b] = (int64_t)hc.num_bin_nnzc[b];
+        st.num_bin_nnzA[b] = (int64_t)hc.num_bin_nnza[b];
+    }
+    if ((rc = reserve_C(ctx))) return rc;
+    offsets_from_counts(hc.num_bin, p.no);
+    CU(launch_bin_scatter(p.lc, true, ctx->m, ctx->prod.as<int>(), ctx->rc.as<int>(), ctx->rspan.as<int>(), mask,
+                          ctx->ct_off.as<long long>(), p.no, d_ctr, ctx->queue.as<int>()),
+       "numeric bin scatter");
+    for (int b = 0; b < MAX_BINS; ++b) st.direct_retry_rows += hc.retry_cnt[b];
+    CU(cudaEventRecord(ctx->ev[3], ctx->stream), "event");
+    return BHB200_SUCCESS;
+}
+
+// ---- stage 4: numeric, C written in place ----
+int stage4_numeric(bhb200_ctx *ctx, const Product &p)
+{
+    const Counters &hc = p.hc;
+    const int rc = run_numeric_bins(ctx, p.lc, hc.num_bin, p.no, p.G, p.wl);
+    if (rc) return rc;
+    if (hc.num_bin[NB_COPY] > 0) {
+        CU(stamp(ctx, 1, NB_COPY), "event");
+        CU(launch_copy_ct(p.lc, ctx->dtype, ctx->queue.as<int>() + p.no.off[NB_COPY], hc.num_bin[NB_COPY], ctx->rowoff64.as<int64_t>(),
+                          ctx->ct_off.as<long long>(), ctx->ct_col.as<int>(), ctx->ct_val.p, ctx->colC.as<int>(), ctx->valC.p,
+                          (double)hc.num_bin_nnzc[NB_COPY] / (double)hc.num_bin[NB_COPY]),
+           "Ct -> C copy");
+    }
+    CU(stamp(ctx, 1, MAX_BINS), "event");
+    CU(cudaEventRecord(ctx->ev[4], ctx->stream), "event");
+    return BHB200_SUCCESS;
+}
 
 }  // namespace
 
@@ -728,12 +1076,10 @@ int bhb200_warmup(bhb200_ctx *ctx)
 int bhb200_spgemm(bhb200_ctx *ctx)
 {
     if (!ctx || !ctx->have_data) return fail(ctx, BHB200_ERR_INVALID, "spgemm before initData");
-    CU(cudaSetDevice(ctx->device), "cudaSetDevice");
+    int rc = begin_call(ctx);
+    if (rc) return rc;
     ctx->have_C = false;
     ctx->reuse_bins_valid = false;
-    ctx->timing_valid = false;
-    ctx->launches = 0;
-    ctx->t_ran = false;
     bhb200_stats &st = ctx->stats;
     memset(&st, 0, sizeof(st));
     st.transposed_ops = (ctx->opA ? 1 : 0) | (ctx->opB ? 2 : 0);
@@ -743,429 +1089,21 @@ int bhb200_spgemm(bhb200_ctx *ctx)
     st.nnzA = ctx->nnzA;
     st.nnzB = ctx->nnzB;
     st.dtype = ctx->dtype;
-    const size_t vs = vsize(ctx->dtype);
-    cudaStream_t s = ctx->stream;
-    int rc = reserve_workspace(ctx);
-    if (rc) return rc;
-    LaunchCtx lc{s, ctx->sm_count, &ctx->launches, ctx->max_span};
-    Counters *d_ctr = ctx->counters.as<Counters>();
-    int *prod = ctx->prod.as<int>();
-    int *rcnt = ctx->rc.as<int>();
-    int *queue = ctx->queue.as<int>();
-    int64_t *rowoff = ctx->rowoff64.as<int64_t>();
-
-    // ---- stage 1: upper bound per row + symbolic bins ----
-    CU(cudaEventRecord(ctx->ev[0], s), "event");
-    // transposed operands: built once for host copies, on every call for borrowed ones (the caller may have rewritten them)
-    if (ctx->t_pending || (ctx->borrowed && (ctx->opA || ctx->opB))) {
-        rc = run_transposes(ctx, lc);
-        if (rc) return rc;
-        CU(cudaEventRecord(ctx->ev[5], s), "event");
-        ctx->t_ran = true;
-    }
-    CU(cudaMemsetAsync(d_ctr, 0, CTR_ZERO_BYTES, s), "zero counters");
-    // diagonal-pattern mode: exact offset sets of A and B, read back with the stage-1 counters
-    ctx->last_pattern = false;
-    const bool same_ab = ctx->A.rowptr == ctx->B.rowptr && ctx->A.col == ctx->B.col && ctx->m == ctx->k;
-    bool try_pattern = ctx->pattern_enable && ctx->m > 0 && ctx->nnzA > 0 && ctx->nnzB > 0;
-    if (try_pattern && ctx->pat_sets.reserve(2 * sizeof(PatSet), &ctx->dev_bytes) != cudaSuccess) {
-        cudaGetLastError();
-        try_pattern = false;
-    }
-    if (try_pattern && ctx->plan.valid && ctx->pattern_speculate) {
-        // the previous product on this context ran in pattern mode: reuse its plan without the detection
-        // pass; every entry is verified against it (k_pat_codes), a miss brings us back here
-        if (ctx->wait_before_values) {
-            CU(cudaStreamWaitEvent(s, ctx->wait_before_values, 0), "wait for the broadcast of B's values");
-            ctx->wait_before_values = nullptr;
-        }
-        rc = run_pattern(ctx, lc, same_ab, true);
-        if (rc != PATTERN_NOT_APPLICABLE && rc != PATTERN_PLAN_STALE) return rc;
-        CU(cudaMemsetAsync(d_ctr, 0, CTR_ZERO_BYTES, s), "zero counters");
-        st.pattern_mode = 0;
-    }
-    if (try_pattern) {
-        PatSet *sets = ctx->pat_sets.as<PatSet>();
-        CU(cudaMemsetAsync(sets, 0x80, 2 * sizeof(PatSet), s), "init offset sets");   // slots = PAT_EMPTY
-        CU(cudaMemsetAsync(&sets[0], 0, 8, s), "init offset sets");
-        CU(cudaMemsetAsync(&sets[1], 0, 8, s), "init offset sets");
-        CU(launch_offset_set(lc, ctx->k, ctx->B.rowptr, ctx->B.col, &sets[1]), "offset set of B");
-        if (!same_ab) CU(launch_offset_set(lc, ctx->m, ctx->A.rowptr, ctx->A.col, &sets[0]), "offset set of A");
-        CU(cudaMemcpyAsync(ctx->h_sets, ctx->pat_sets.p, 2 * sizeof(PatSet), cudaMemcpyDeviceToHost, s), "D2H offset sets");
-        CU(cudaStreamSynchronize(s), "offset sets");
-        if (ctx->wait_before_values) {
-            // multi-GPU set-up: the broadcast of B's values overlapped the detection; the rest reads them
-            CU(cudaStreamWaitEvent(s, ctx->wait_before_values, 0), "wait for the broadcast of B's values");
-            ctx->wait_before_values = nullptr;
-        }
-        rc = run_pattern(ctx, lc, same_ab, false);
-        if (rc != PATTERN_NOT_APPLICABLE) return rc;
-        ctx->plan = PatternPlan();   // these operands are not diagonal-structured: no speculation next time
-        CU(cudaMemsetAsync(d_ctr, 0, CTR_ZERO_BYTES, s), "zero counters");
-    }
-    int *rlo = ctx->rlo.as<int>();
-    int *rspan = ctx->rspan.as<int>();
-    CU(launch_b_row_ranges(lc, ctx->k, ctx->n, ctx->B, ctx->brange.as<int4>(), ctx->counters.as<Counters>()), "B row ranges kernel");
-    CU(launch_row_products(lc, ctx->m, ctx->k, ctx->nnzA, ctx->A, ctx->B, ctx->brange.as<int4>(), prod, rcnt, rlo, rspan, d_ctr),
-       "row products kernel");
-    CU(cudaMemcpyAsync(ctx->h_ctr, d_ctr, sizeof(Counters), cudaMemcpyDeviceToHost, s), "D2H counters");
-    CU(cudaStreamSynchronize(s), "stage 1");
-    Counters hc = *ctx->h_ctr;
-    rc = check_transposed(ctx, hc.bad_T);
-    if (rc) return rc;
-    if (hc.bad_B) return fail(ctx, BHB200_ERR_INVALID, "rows of B must be sorted by column, duplicate-free and inside [0, n)");
-    if (hc.bad_A) return fail(ctx, BHB200_ERR_INVALID, "a column index of A is outside [0, k)");
-    if (hc.row_overflow) return fail(ctx, BHB200_ERR_OVERFLOW, "a row has more than INT32_MAX intermediate products");
-    st.products = (int64_t)hc.products;
-    st.max_row_products = hc.max_row_products;
-    for (int b = 0; b < BHB200_NUM_SYM_BINS && b < MAX_BINS; ++b) st.sym_bin_rows[b] = hc.sym_bin[b];
-    if (ctx->wait_before_values) {
-        // multi-GPU set-up: the broadcast of B's values overlapped stage 1; everything below reads them
-        CU(cudaStreamWaitEvent(s, ctx->wait_before_values, 0), "wait for the broadcast of B's values");
-        ctx->wait_before_values = nullptr;
-    }
-    // lanes per row group: follow the average length of the B rows actually referenced
-    const double avg_b = ctx->nnzA > 0 ? (double)hc.products / (double)ctx->nnzA : 0.0;
-    const int G = avg_b <= 10.0 ? 8 : 32;
-    BinOffsets so;
-    offsets_from_counts(hc.sym_bin, so);
-    CU(launch_bin_scatter(lc, false, ctx->m, prod, rcnt, rspan, 0u, nullptr, so, d_ctr, queue), "symbolic bin scatter");
-
-    // ---- direct (single-pass) mode: sample the group-hash bins, pick a staging capacity ----
-    // (DirectOut in common.cuh). Two cases per bin:
-    //  * tight: every sampled row has nnz(C_i) <= 128 -> speculate 32/64/128 entries per row,
-    //    rows that overflow go through the two-pass path (stencils: 1728 products -> 125);
-    //  * wide: the sampled rows barely compress (mean nnz(C_i) >= a quarter of the bin's table
-    //    capacity, R-MAT: nnz(C_i) ~ products) -> the numeric kernel would use the table the
-    //    product bound dictates anyway, so it runs once, staged, and the symbolic pass is
-    //    skipped; the bound is below the capacity, nothing can overflow.
-    unsigned spec_mask = 0;
-    int spec_cap[MAX_BINS] = {0};
-    bool spec_wide[MAX_BINS] = {false};
-    bool spec_heavy[MAX_BINS] = {false};   // rows beyond the on-chip tables: sliced bucket sort (k_num_bucket_heavy)
-    bool spec_3w[MAX_BINS] = {false};      // SB_G128 / SB_G256 whose rows barely compress: warp-per-row bucket sort (k_num_bucket3w)
-    long long heavy_base = 0;
-    long long spec_base[MAX_BINS] = {0};
-    long long ct_entries = 0;
-    const int SAMPLE_STRIDE = 64;
-    const bool force = ctx->force_cap >= 0;
-    const int SPEC_MIN_ROWS = force ? 1 : 4096;
-    static const int WIDE_CAP[7] = {128, 256, 512, 1024, 2048, 4096, 8192};   // SB_G128 .. SB_B8192
-    if (ctx->direct_mode) {
-        bool any = false;
-        for (int b = SB_G128; b <= SB_G4096; ++b) {
-            if (hc.sym_bin[b] < SPEC_MIN_ROWS) continue;
-            const int nsample = (hc.sym_bin[b] + SAMPLE_STRIDE - 1) / SAMPLE_STRIDE;
-            CU(launch_sym_hash(lc, b, G, queue + so.off[b], nsample, ctx->A, ctx->B, rcnt, SAMPLE_STRIDE,
-                               &d_ctr->sample_max[b], nullptr, &d_ctr->sample_sum[b]),
-               "symbolic sample");
-            any = true;
-        }
-        if (any) {
-            CU(cudaMemcpyAsync(ctx->h_ctr, d_ctr, sizeof(Counters), cudaMemcpyDeviceToHost, s), "D2H counters");
-            CU(cudaStreamSynchronize(s), "direct-mode sampling");
-            bool wide_above = false;
-            for (int b = SB_G128; b <= SB_B8192; ++b) {
-                if (hc.sym_bin[b] <= 0) continue;
-                if (b == SB_B8192) {
-                    // not sampled (the group kernels stop at 4096 slots): follows its neighbour
-                    if (!wide_above) continue;
-                    spec_cap[b] = WIDE_CAP[b - SB_G128];
-                    spec_wide[b] = true;
-                } else {
-                    wide_above = false;
-                    int smax = ctx->h_ctr->sample_max[b];
-                    if (force && hc.sym_bin[b] >= SPEC_MIN_ROWS) smax = ctx->force_cap;
-                    if (hc.sym_bin[b] < SPEC_MIN_ROWS || smax < 1) continue;
-                    const int nsample = (hc.sym_bin[b] + SAMPLE_STRIDE - 1) / SAMPLE_STRIDE;
-                    const double mean = (double)ctx->h_ctr->sample_sum[b] / nsample;
-                    const int wcap = WIDE_CAP[b - SB_G128];
-                    // bins of at most 96 / 192 products whose sampled rows keep at least half of their products as outputs:
-                    // sorting the products (k_num_bucket3w) beats hashing them (BHB200_BUCKET_W=off: hash kernels)
-                    if (ctx->bucket_warp && b <= SB_G256 && !force && hc.sym_bin[b] > 0 &&
-                        mean * 2.0 * (double)hc.sym_bin[b] >= (double)hc.sym_bin_products[b])
-                        spec_3w[b] = true;
-                    if (smax <= 128) {
-                        spec_cap[b] = smax <= 32 ? 32 : smax <= 64 ? 64 : 128;
-                    } else if (ctx->direct_wide && !force && mean * 4.0 >= wcap) {
-                        spec_cap[b] = wcap;
-                        spec_wide[b] = true;
-                        wide_above = true;
-                    } else {
-                        continue;
-                    }
-                }
-                spec_base[b] = ct_entries;
-                ct_entries += (long long)hc.sym_bin[b] * spec_cap[b];
-                spec_mask |= 1u << b;
-            }
-        }
-        // rows with more products than the on-chip tables hold follow the largest sampled bin: if that one
-        // does not compress they run once through the sliced bucket sort, staged at their product count
-        // (BHB200_DEBUG_FORCE_HEAVY: tests send them there whatever the sample says)
-        bool top_wide = ctx->force_heavy;
-        for (int b = SB_B8192; b >= SB_G128 && !top_wide; --b)
-            if (hc.sym_bin[b] > 0) {
-                top_wide = ((spec_mask >> b) & 1u) && spec_wide[b];
-                break;
-            }
-        // (k_num_bucket_heavy2, measured on R-MAT 21, n = 2 M columns: 4.0 ms for these rows against 7.0 ms through the
-        // two-pass tables + global column bitmap, whose cost also grows with n -- profiles/r02_notes.md section 5)
-        if (top_wide && ctx->direct_wide) {
-            heavy_base = ct_entries;
-            for (int b = SB_B16384; b <= SB_LARGE; ++b) {
-                if (hc.sym_bin[b] <= 0) continue;
-                spec_heavy[b] = spec_wide[b] = true;
-                spec_base[b] = heavy_base;
-                ct_entries += (long long)hc.sym_bin_products[b];
-                spec_mask |= 1u << b;
-            }
-        }
-        // the wide staging buffer must not crowd out C itself (at most `products` entries)
-        if (spec_mask && ((size_t)ct_entries * 4 + 16 > ctx->ct_col.cap || (size_t)ct_entries * vs + 16 > ctx->ct_val.cap)) {
-            // (only when the staging buffer has to grow: cudaMemGetInfo can take milliseconds)
-            size_t free_b = 0, total_b = 0;
-            cudaMemGetInfo(&free_b, &total_b);
-            const double avail = (double)free_b + (double)ctx->ct_col.cap + (double)ctx->ct_val.cap +
-                                 (double)ctx->colC.cap + (double)ctx->valC.cap;
-            const double need = ((double)ct_entries + (double)st.products) * (4.0 + vs);
-            if (need > 0.9 * avail) {
-                ct_entries = 0;
-                for (int b = SB_G128; b <= SB_LARGE; ++b) {
-                    if (!((spec_mask >> b) & 1u)) continue;
-                    if (spec_wide[b]) {
-                        spec_mask &= ~(1u << b);
-                        spec_heavy[b] = false;
-                        continue;
-                    }
-                    spec_base[b] = ct_entries;
-                    ct_entries += (long long)hc.sym_bin[b] * spec_cap[b];
-                }
-            }
-        }
-        if (spec_mask) {
-            const size_t m1 = (size_t)ctx->m + 1;
-            // the staging buffer (the reference's Ct) may spill to host memory like C itself
-            bool spilled = false;
-            if (ctx->ct_off.reserve(m1 * 8, &ctx->dev_bytes) != cudaSuccess ||
-                ctx->retry_q.reserve(m1 * 4, &ctx->dev_bytes) != cudaSuccess ||
-                ctx->ct_col.reserve_spillable((size_t)ct_entries * 4 + 16, &ctx->dev_bytes, ctx->device_cap, &spilled) != cudaSuccess ||
-                ctx->ct_val.reserve_spillable((size_t)ct_entries * vs + 16, &ctx->dev_bytes, ctx->device_cap, &spilled) != cudaSuccess) {
-                cudaGetLastError();
-                spec_mask = 0;   // no room for the staging buffer: two-pass path for everything
-            }
-            if (spec_mask)
-                st.spill_bytes += (ctx->ct_col.host ? (int64_t)ctx->ct_col.cap : 0) + (ctx->ct_val.host ? (int64_t)ctx->ct_val.cap : 0);
-        }
-    }
-    st.direct_rows = 0;
-    st.direct_ct_bytes = spec_mask ? ct_entries * (4 + (int64_t)vs) : 0;
-    st.direct_bin_mask = (int64_t)spec_mask;
-    CU(cudaEventRecord(ctx->ev[1], s), "event");
-
-    // wide bins with 512+ entries per row: bucket-sort kernels, which need the column CDF of the products
-    // (k_num_bucket3 beats the hash kernels from a capacity of 512 up, profiles/r02_notes.md section 5)
-    constexpr int BUCKET_MIN_CAP = 512;
-    bool use_bucket = false;
-    int cdf_shift = 0;
-    if (spec_mask) {
-        for (int b = SB_G128; b <= SB_G256; ++b) use_bucket |= ((spec_mask >> b) & 1u) && spec_3w[b];
-        for (int b = SB_G512; b <= SB_B8192; ++b) use_bucket |= ((spec_mask >> b) & 1u) && spec_wide[b] && spec_cap[b] >= BUCKET_MIN_CAP;
-        for (int b = SB_B16384; b <= SB_LARGE; ++b) use_bucket |= ((spec_mask >> b) & 1u) && spec_heavy[b];
-        if (use_bucket && (ctx->cdf_colcount.reserve(((size_t)ctx->k + 1) * 4, &ctx->dev_bytes) != cudaSuccess ||
-                           ctx->cdf_hist.reserve((size_t)CDF_KNOTS * 8, &ctx->dev_bytes) != cudaSuccess ||
-                           ctx->cdf_tab.reserve((size_t)(CDF_KNOTS + 1) * 4, &ctx->dev_bytes) != cudaSuccess)) {
-            cudaGetLastError();
-            use_bucket = false;
-            for (int b = SB_B16384; b <= SB_LARGE; ++b)
-                if (spec_heavy[b]) {   // (their staging stays allocated but unused: two-pass path)
-                    spec_heavy[b] = false;
-                    spec_mask &= ~(1u << b);
-                }
-        }
-        if (use_bucket && ctx->cdf_valid) {
-            cdf_shift = ctx->cdf_shift_cached;
-        } else if (use_bucket) {
-            CU(launch_build_cdf(lc, ctx->m, ctx->k, ctx->n, ctx->nnzA, ctx->A, ctx->B, ctx->cdf_colcount.as<int>(),
-                                ctx->cdf_hist.as<unsigned long long>(), ctx->cdf_tab.as<unsigned>(), &cdf_shift),
-               "column CDF");
-            ctx->cdf_valid = true;
-            ctx->cdf_shift_cached = cdf_shift;
-        }
-    }
-    // Rows with more products than the on-chip tables hold (bins SB_B16384 .. SB_LARGE), single pass, staged by atomic
-    // bump at heavy_base: rows of at most 8192 products by k_num_bucket3 itself, the rest by k_num_bucket_heavy2
-    // (partitioned by slice through the row's own staging area), what that kernel cannot slice by k_num_bucket_heavy.
-    auto run_heavy_bin = [&](const int b) -> cudaError_t {
-        const bool f64 = ctx->dtype == BHB200_DTYPE_F64;
-        const unsigned *cdf = ctx->cdf_tab.as<unsigned>();
-        const int *bq = queue + so.off[b];
-        const int rows = hc.sym_bin[b];
-        DirectOut d{rcnt, ctx->ct_off.as<long long>(), ctx->ct_col.as<int>(), ctx->ct_val.p, heavy_base, nullptr, nullptr};
-        d.prod = prod;
-        cudaError_t e;
-        int p_lo = 0;
-        if (b == SB_B16384) {   // 6144 < products <= 12288: up to 8192 fit k_num_bucket3's largest capacity
-            DirectOut d3 = d;
-            d3.p_lo = 0;
-            d3.p_hi = 8192;
-            d3.bump = &d_ctr->heavy_cursor;
-            e = f64 ? launch_num_bucket_f64(lc, 8192, bq, rows, ctx->A, ctx->B, d3, cdf, cdf_shift)
-                    : launch_num_bucket_f32(lc, 8192, bq, rows, ctx->A, ctx->B, d3, cdf, cdf_shift);
-            if (e != cudaSuccess) return e;
-            p_lo = 8192;
-        }
-        d.p_lo = p_lo;
-        d.retry_queue = ctx->retry_q.as<int>() + so.off[b];
-        d.retry_cnt = &d_ctr->retry_cnt[b];
-        e = f64 ? launch_num_bucket_heavy2_f64(lc, bq, rows, ctx->A, ctx->B, d, cdf, cdf_shift, &d_ctr->heavy_cursor)
-                : launch_num_bucket_heavy2_f32(lc, bq, rows, ctx->A, ctx->B, d, cdf, cdf_shift, &d_ctr->heavy_cursor);
-        if (e != cudaSuccess) return e;
-        d.count_dev = d.retry_cnt;
-        return f64 ? launch_num_bucket_heavy_f64(lc, d.retry_queue, rows, ctx->A, ctx->B, d, cdf, cdf_shift, &d_ctr->heavy_cursor)
-                   : launch_num_bucket_heavy_f32(lc, d.retry_queue, rows, ctx->A, ctx->B, d, cdf, cdf_shift, &d_ctr->heavy_cursor);
-    };
-    // ---- stage 2: symbolic, one launch per non-empty bin (direct-mode bins: the numeric kernel itself) ----
-    memset(ctx->ev_bin_used, 0, sizeof(ctx->ev_bin_used));
-    if (hc.sym_bin[SB_ESC] > 0) CU(stamp(ctx, 0, SB_ESC), "event");
-    CU(launch_sym_esc(lc, queue + so.off[SB_ESC], hc.sym_bin[SB_ESC], ctx->n, ctx->A, ctx->B, rcnt), "symbolic ESC");
-    for (int b = SB_G128; b <= SB_B32768; ++b) {
-        if (hc.sym_bin[b] > 0) CU(stamp(ctx, 0, b), "event");
-        if (((spec_mask >> b) & 1u) && spec_heavy[b]) {
-            CU(run_heavy_bin(b), "heavy rows");
-            st.direct_rows += hc.sym_bin[b];
-            continue;
-        }
-        if ((spec_mask >> b) & 1u) {
-            DirectOut d{rcnt, ctx->ct_off.as<long long>(), ctx->ct_col.as<int>(), ctx->ct_val.p, spec_base[b],
-                        ctx->retry_q.as<int>() + so.off[b], &d_ctr->retry_cnt[b]};
-            if (spec_3w[b] && use_bucket) {
-                const int capw = b == SB_G128 ? 128 : 256;
-                if (ctx->dtype == BHB200_DTYPE_F64)
-                    CU(launch_num_bucket3w_f64(lc, capw, G, queue + so.off[b], hc.sym_bin[b], ctx->A, ctx->B, d, ctx->cdf_tab.as<unsigned>(), cdf_shift, spec_cap[b]),
-                       "warp bucket numeric f64");
-                else
-                    CU(launch_num_bucket3w_f32(lc, capw, G, queue + so.off[b], hc.sym_bin[b], ctx->A, ctx->B, d, ctx->cdf_tab.as<unsigned>(), cdf_shift, spec_cap[b]),
-                       "warp bucket numeric f32");
-                if (!spec_wide[b])
-                    CU(launch_sym_hash(lc, b, G, ctx->retry_q.as<int>() + so.off[b], hc.sym_bin[b], ctx->A, ctx->B, rcnt, 1,
-                                       nullptr, &d_ctr->retry_cnt[b]),
-                       "symbolic retry");
-                st.direct_rows += hc.sym_bin[b];
-                continue;
-            }
-            // wide bins: the rows up to half the capacity run with the half-size table
-            const int passes = spec_wide[b] ? 2 : 1;
-            for (int pass = 0; pass < passes; ++pass) {
-                int cap = spec_cap[b];
-                if (spec_wide[b]) {
-                    d.prod = prod;
-                    d.ct_stride = spec_cap[b];
-                    d.p_lo = pass == 0 ? 0 : spec_cap[b] / 2;
-                    d.p_hi = pass == 0 ? spec_cap[b] / 2 : 0x7fffffff;
-                    if (pass == 0) cap = spec_cap[b] / 2;
-                }
-                if (spec_wide[b] && use_bucket && cap >= BUCKET_MIN_CAP) {
-                    if (ctx->dtype == BHB200_DTYPE_F64)
-                        CU(launch_num_bucket_f64(lc, cap, queue + so.off[b], hc.sym_bin[b], ctx->A, ctx->B, d, ctx->cdf_tab.as<unsigned>(), cdf_shift),
-                           "bucket numeric f64");
-                    else
-                        CU(launch_num_bucket_f32(lc, cap, queue + so.off[b], hc.sym_bin[b], ctx->A, ctx->B, d, ctx->cdf_tab.as<unsigned>(), cdf_shift),
-                           "bucket numeric f32");
-                } else if (ctx->dtype == BHB200_DTYPE_F64)
-                    CU(launch_num_direct_f64(lc, cap, spec_wide[b] ? 32 : G, queue + so.off[b], hc.sym_bin[b], ctx->A, ctx->B, d),
-                       "direct numeric f64");
-                else
-                    CU(launch_num_direct_f32(lc, cap, spec_wide[b] ? 32 : G, queue + so.off[b], hc.sym_bin[b], ctx->A, ctx->B, d),
-                       "direct numeric f32");
-            }
-            // rows that did not fit: ordinary symbolic pass, row count read on the device
-            if (!spec_wide[b])
-                CU(launch_sym_hash(lc, b, G, ctx->retry_q.as<int>() + so.off[b], hc.sym_bin[b], ctx->A, ctx->B, rcnt, 1,
-                                   nullptr, &d_ctr->retry_cnt[b]),
-                   "symbolic retry");
-            st.direct_rows += hc.sym_bin[b];
-            continue;
-        }
-        CU(launch_sym_hash(lc, b, G, queue + so.off[b], hc.sym_bin[b], ctx->A, ctx->B, rcnt), "symbolic hash");
-    }
-    if (hc.sym_bin[SB_LARGE] > 0 && ((spec_mask >> SB_LARGE) & 1u) && spec_heavy[SB_LARGE]) {
-        CU(stamp(ctx, 0, SB_LARGE), "event");
-        CU(run_heavy_bin(SB_LARGE), "heavy rows");
-        st.direct_rows += hc.sym_bin[SB_LARGE];
-    } else if (hc.sym_bin[SB_LARGE] > 0) {
-        rc = reserve_large_scratch(ctx, false);
-        if (rc) return rc;
-        CU(stamp(ctx, 0, SB_LARGE), "event");
-        CU(launch_sym_large(lc, queue + so.off[SB_LARGE], hc.sym_bin[SB_LARGE], ctx->n, ctx->A, ctx->B, rcnt,
-                            ctx->bitmap.as<unsigned>(), large_scratch_blocks(ctx->sm_count, ctx->n)),
-           "symbolic large");
-    }
-    WordLists wl{nullptr, nullptr, nullptr, nullptr, 0};
-    if (hc.sym_bin[SB_RANGE_S] + hc.sym_bin[SB_RANGE_L] > 0) {
-        rc = reserve_word_lists(ctx, st.products, wl);
-        if (rc) return rc;
-        if (hc.sym_bin[SB_RANGE_S] > 0) {
-            CU(stamp(ctx, 0, SB_RANGE_S), "event");
-            CU(launch_sym_range(lc, NSUM_SMALL, queue + so.off[SB_RANGE_S], hc.sym_bin[SB_RANGE_S], ctx->A, ctx->B, rlo,
-                                rcnt, d_ctr, wl),
-               "symbolic range (small span)");
-        }
-        if (hc.sym_bin[SB_RANGE_L] > 0) {
-            CU(stamp(ctx, 0, SB_RANGE_L), "event");
-            CU(launch_sym_range(lc, NSUM_LARGE, queue + so.off[SB_RANGE_L], hc.sym_bin[SB_RANGE_L], ctx->A, ctx->B, rlo,
-                                rcnt, d_ctr, wl),
-               "symbolic range (large span)");
-        }
-    }
-    CU(stamp(ctx, 0, MAX_BINS), "event");
-    CU(cudaEventRecord(ctx->ev[2], s), "event");
-
-    // ---- stage 3: row pointers, numeric bins, exact allocation of C ----
-    CU(launch_scan(lc, ctx->m, ctx->A.rowptr, prod, rcnt, rspan, spec_mask, ctx->ct_off.as<long long>(), rowoff, ctx->rowptr32.as<int>(), ctx->blocksums.as<long long>(), d_ctr),
-       "row pointer scan");
-    CU(cudaMemcpyAsync(ctx->h_ctr, d_ctr, sizeof(Counters), cudaMemcpyDeviceToHost, s), "D2H counters");
-    CU(cudaStreamSynchronize(s), "stage 2/3");
-    hc = *ctx->h_ctr;
-    ctx->nnzC = (int64_t)hc.nnzC;
-    st.nnzC = ctx->nnzC;
-    for (int b = 0; b < BHB200_NUM_NUM_BINS && b < MAX_BINS; ++b) {
-        st.num_bin_rows[b] = hc.num_bin[b];
-        st.num_bin_products[b] = (int64_t)hc.num_bin_products[b];
-        st.num_bin_nnzC[b] = (int64_t)hc.num_bin_nnzc[b];
-        st.num_bin_nnzA[b] = (int64_t)hc.num_bin_nnza[b];
-    }
-    {
-        bool spilled = false;
-        CU(ctx->colC.reserve_spillable((size_t)ctx->nnzC * 4 + 16, &ctx->dev_bytes, ctx->device_cap, &spilled), "alloc colC");
-        CU(ctx->valC.reserve_spillable((size_t)ctx->nnzC * vs + 16, &ctx->dev_bytes, ctx->device_cap, &spilled), "alloc valC");
-        st.spill_bytes += (ctx->colC.host ? (int64_t)ctx->colC.cap : 0) + (ctx->valC.host ? (int64_t)ctx->valC.cap : 0);
-    }
-    BinOffsets no;
-    offsets_from_counts(hc.num_bin, no);
-    CU(launch_bin_scatter(lc, true, ctx->m, prod, rcnt, rspan, spec_mask, ctx->ct_off.as<long long>(), no, d_ctr, queue),
-       "numeric bin scatter");
-    for (int b = 0; b < MAX_BINS; ++b) st.direct_retry_rows += hc.retry_cnt[b];
-    CU(cudaEventRecord(ctx->ev[3], s), "event");
-
-    // ---- stage 4: numeric, C written in place ----
-    rc = run_numeric_bins(ctx, lc, hc.num_bin, no, G, wl);
-    if (rc) return rc;
-    int *colC = ctx->colC.as<int>();
-    void *valC = ctx->valC.p;
-    if (hc.num_bin[NB_COPY] > 0) {
-        CU(stamp(ctx, 1, NB_COPY), "event");
-        CU(launch_copy_ct(lc, ctx->dtype, queue + no.off[NB_COPY], hc.num_bin[NB_COPY], rowoff, ctx->ct_off.as<long long>(),
-                          ctx->ct_col.as<int>(), ctx->ct_val.p, colC, valC,
-                          (double)hc.num_bin_nnzc[NB_COPY] / (double)hc.num_bin[NB_COPY]),
-           "Ct -> C copy");
-    }
-    CU(stamp(ctx, 1, MAX_BINS), "event");
-    CU(cudaEventRecord(ctx->ev[4], s), "event");
-
+    if ((rc = reserve_workspace(ctx))) return rc;
+    Product p{LaunchCtx{ctx->stream, ctx->sm_count, &ctx->launches, ctx->max_span}};
+    CU(cudaEventRecord(ctx->ev[0], ctx->stream), "event");
+    if ((rc = transpose_operands(ctx, p.lc))) return rc;
+    CU(cudaMemsetAsync(ctx->counters.p, 0, CTR_ZERO_BYTES, ctx->stream), "zero counters");
+    rc = try_pattern(ctx, p.lc);
+    if (rc != PATTERN_NOT_APPLICABLE) return rc;
+    if ((rc = stage1_counts(ctx, p))) return rc;
+    if ((rc = choose_direct(ctx, p))) return rc;
+    if ((rc = stage2_symbolic(ctx, p))) return rc;
+    if ((rc = stage3_scan_alloc(ctx, p))) return rc;
+    if ((rc = stage4_numeric(ctx, p))) return rc;
     finish_stats(ctx);
-    ctx->last_G = G;
-    ctx->last_wl = wl;
+    ctx->last_G = p.G;
+    ctx->last_wl = p.wl;
     ctx->have_C = true;
     ctx->timing_valid = true;
     return BHB200_SUCCESS;
@@ -1179,10 +1117,8 @@ int bhb200_spgemm_numeric(bhb200_ctx *ctx)
 {
     if (!ctx || !ctx->have_data || !ctx->have_C)
         return fail(ctx, BHB200_ERR_INVALID, "spgemm_numeric needs a completed spgemm on the same operands");
-    CU(cudaSetDevice(ctx->device), "cudaSetDevice");
-    ctx->timing_valid = false;
-    ctx->launches = 0;
-    ctx->t_ran = false;
+    int rc = begin_call(ctx);
+    if (rc) return rc;
     bhb200_stats &st = ctx->stats;
     cudaStream_t s = ctx->stream;
     LaunchCtx lc{s, ctx->sm_count, &ctx->launches, ctx->max_span};
@@ -1190,8 +1126,7 @@ int bhb200_spgemm_numeric(bhb200_ctx *ctx)
     CU(cudaEventRecord(ctx->ev[0], s), "event");
     if (ctx->borrowed && (ctx->opA || ctx->opB)) {
         // borrowed operands are rewritten in place by the caller: their values again through perm
-        int rc = run_regathers(ctx, lc);
-        if (rc) return rc;
+        if ((rc = run_regathers(ctx, lc))) return rc;
         CU(cudaEventRecord(ctx->ev[5], s), "event");
         ctx->t_ran = true;
     }
@@ -1215,8 +1150,7 @@ int bhb200_spgemm_numeric(bhb200_ctx *ctx)
         CU(launch_scan(lc, ctx->m, ctx->A.rowptr, ctx->prod.as<int>(), ctx->rc.as<int>(), ctx->rspan.as<int>(), 0u, nullptr,
                        ctx->rowoff64.as<int64_t>(), ctx->rowptr32.as<int>(), ctx->blocksums.as<long long>(), d_ctr),
            "row pointer scan");
-        CU(cudaMemcpyAsync(ctx->h_ctr, d_ctr, sizeof(Counters), cudaMemcpyDeviceToHost, s), "D2H counters");
-        CU(cudaStreamSynchronize(s), "numeric-only binning");
+        if ((rc = read_counters(ctx, "numeric-only binning"))) return rc;
         if ((int64_t)ctx->h_ctr->nnzC != ctx->nnzC) return fail(ctx, BHB200_ERR_INVALID, "structure of C changed");
         memcpy(ctx->reuse_num_bin, ctx->h_ctr->num_bin, sizeof(ctx->reuse_num_bin));
         BinOffsets no0;
@@ -1229,8 +1163,7 @@ int bhb200_spgemm_numeric(bhb200_ctx *ctx)
     BinOffsets no;
     offsets_from_counts(ctx->reuse_num_bin, no);
     CU(cudaEventRecord(ctx->ev[3], s), "event");
-    int rc = run_numeric_bins(ctx, lc, ctx->reuse_num_bin, no, ctx->last_G, ctx->last_wl);
-    if (rc) return rc;
+    if ((rc = run_numeric_bins(ctx, lc, ctx->reuse_num_bin, no, ctx->last_G, ctx->last_wl))) return rc;
     CU(stamp(ctx, 1, MAX_BINS), "event");
     CU(cudaEventRecord(ctx->ev[4], s), "event");
     for (int b = 0; b < BHB200_NUM_NUM_BINS && b < MAX_BINS; ++b) st.num_bin_rows[b] = ctx->reuse_num_bin[b];
