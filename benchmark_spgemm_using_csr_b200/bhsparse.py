@@ -156,6 +156,20 @@ class bhsparse:
         """Values of C again after update_values; structure of C reused (bhb200_spgemm_numeric)."""
         return self._lib.bhb200_spgemm_numeric(self._ctx) if self._ctx else capi.ERR_INVALID
 
+    def set_mask(self, csrRowPtrM, csrColIndM) -> int:
+        """Masked products C = M .* (op(A)*op(B)) on the pattern of M (bhb200_set_mask; host arrays,
+        copied).  Call after initData; initData clears it."""
+        if not self._ctx:
+            return capi.ERR_INVALID
+        rp = np.ascontiguousarray(csrRowPtrM, dtype=np.int32)
+        col = np.ascontiguousarray(csrColIndM, dtype=np.int32)
+        if rp.size != self._m + 1:
+            return capi.ERR_INVALID
+        return self._lib.bhb200_set_mask(self._ctx, int(col.size), _ptr(rp), _ptr(col) if col.size else None)
+
+    def clear_mask(self) -> int:
+        return self._lib.bhb200_clear_mask(self._ctx) if self._ctx else capi.ERR_INVALID
+
     def get_rowptrC_i64(self) -> np.ndarray:
         out = np.empty(self._m + 1, dtype=np.int64)
         capi.check(self._lib, self._ctx, self._lib.bhb200_get_rowptrC_i64(self._ctx, ctypes.c_void_p(out.ctypes.data)))
@@ -191,10 +205,11 @@ class bhsparse:
 
 
 def spgemm(A, B, device: int = 0, return_stats: bool = False, return_row_products: bool = False,
-           transA: bool = False, transB: bool = False):
+           transA: bool = False, transB: bool = False, mask=None):
     """Convenience driver following main.cu:104-135: C = op(A)*op(B) for two
     generators.CSR operands (op = transpose with transA / transB); returns
-    (rowptrC int32, colC int32, valC)."""
+    (rowptrC int32, colC int32, valC).  mask: a generators.CSR or (rowptr, col)
+    whose pattern restricts C (masked product, bhb200_set_mask)."""
     platforms = [False] * NUM_PLATFORMS
     platforms[BHSPARSE_CUDA] = True
     bh = bhsparse(device)
@@ -211,6 +226,9 @@ def spgemm(A, B, device: int = 0, return_stats: bool = False, return_row_product
     ok(bh.initPlatform(platforms), "initPlatform")
     ok(bh.initData(m, k, n, A.nnz, A.val, A.rowptr, A.col,
                    B.nnz, B.val, B.rowptr, B.col, rowptrC, transA, transB), "initData")
+    if mask is not None:
+        rpM, colM = (mask.rowptr, mask.col) if hasattr(mask, "rowptr") else mask
+        ok(bh.set_mask(rpM, colM), "set_mask")
     ok(bh.spgemm(), "spgemm")
     nnzC = bh.get_nnzC()
     colC = np.empty(max(nnzC, 0), dtype=np.int32)

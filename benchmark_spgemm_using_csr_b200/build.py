@@ -34,6 +34,7 @@ SOURCES = [
     "stage_numeric_f32.cu",
     "stage_numeric_f64.cu",
     "stage_transpose.cu",
+    "stage_masked.cu",
 ]
 HEADERS = ["common.cuh", "stage_numeric.cuh", "stage_range.cuh", "stage_range_vec.cuh", "stage_pattern.cuh", "pattern_plan.h", "direct_plan.h", "context.h", "stage_bucket.cuh", os.path.join(INCLUDE, "bhsparse_b200.h")]
 

@@ -24,6 +24,8 @@ DTYPE_F64 = 1
 OP_N = 0
 OP_T = 1
 NUM_BINS = 24
+NUM_MASK_BINS = 9
+MASK_BIN_NAMES = ["none", "esc<=32", "w64", "w256", "w1024", "c1024", "c4096", "c16384", "global"]
 
 SYM_BIN_NAMES = ["p=0", "p=1", "esc<=32", "g128", "g256", "g512", "g1024", "g2048", "g4096",
                  "b8192", "b16384", "b32768", "large", "range_s", "range_l"]
@@ -42,6 +44,7 @@ EXPORTED = [
     "bhb200_dist_get_layout", "bhb200_dist_get_block_products", "bhb200_dist_get_global_rowptr_device",
     "bhb200_dist_broadcast_ms", "bhb200_dist_finalize", "bhb200_pattern_plan_probe",
     "bhb200_init_data_op_f64", "bhb200_init_data_op_f32", "bhb200_init_data_device_op",
+    "bhb200_set_mask", "bhb200_set_mask_device", "bhb200_clear_mask",
 ]
 DIST_ID_BYTES = 128
 
@@ -63,6 +66,7 @@ class Stats(ctypes.Structure):
         ("pattern_mode", c_int64), ("pattern_nDA", c_int64), ("pattern_nDB", c_int64), ("pattern_nD", c_int64),
         ("pattern_acc_len", c_int64), ("spill_bytes", c_int64),
         ("transposed_ops", c_int64), ("ms_transpose", c_float),
+        ("masked", c_int64), ("nnzM", c_int64), ("mask_bin_rows", c_int64 * NUM_MASK_BINS),
     ]
 
     def as_dict(self) -> dict:
@@ -117,6 +121,9 @@ def load(build_if_missing: bool = False):
     L.bhb200_init_data_device_op.argtypes = [ctxp, c_int, c_int, c_int] + L.bhb200_init_data_device.argtypes[2:]
     L.bhb200_operands_aliased.argtypes = [ctxp]
     L.bhb200_get_operands_device.argtypes = [ctxp, POINTER(c_int32)] + [POINTER(c_void_p)] * 6
+    L.bhb200_set_mask.argtypes = [ctxp, c_int, c_void_p, c_void_p]
+    L.bhb200_set_mask_device.argtypes = [ctxp, c_int, c_void_p, c_void_p]
+    L.bhb200_clear_mask.argtypes = [ctxp]
     L.bhb200_warmup.argtypes = [ctxp]
     L.bhb200_spgemm.argtypes = [ctxp]
     L.bhb200_synchronize.argtypes = [ctxp]

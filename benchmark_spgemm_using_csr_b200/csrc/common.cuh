@@ -78,6 +78,32 @@ enum NumBin {
 };
 constexpr int MAX_BINS = 24;
 
+// Masked products (stage_masked.cu): the table size follows m = nnz(M_i), the parallelism p = products
+enum MaskBin {
+    MB_ZERO = 0,     // p == 0 or m == 0    -> nnz(C_i) = 0, no kernel
+    MB_ESC = 1,      // p <= 32             -> warp per row, one product per lane
+    MB_W64 = 2,      // m <= 32, p <= MASK_WARP_MAX_P -> warp per row, T = 64
+    MB_W256 = 3,     // m <= 128
+    MB_W1024 = 4,    // m <= 512
+    MB_C1024 = 5,    // m <= 512, more products -> CTA per row, T = 1024
+    MB_C4096 = 6,    // m <= 2048
+    MB_C16384 = 7,   // m <= 8192
+    MB_GLOBAL = 8,   // beyond the shared-memory tables: binary search in M_i, values in global scratch
+    MB_COUNT = 9
+};
+constexpr int MASK_WARP_MAX_P = 2048;
+constexpr int MASK_TABLE_MAX = 8192;
+__host__ __device__ __forceinline__ int mask_bin_of(int p, int m)
+{
+    if (p == 0 || m == 0) return MB_ZERO;
+    if (p <= 32) return MB_ESC;
+    if (m > MASK_TABLE_MAX) return MB_GLOBAL;
+    if (p <= MASK_WARP_MAX_P && m <= 512) return m <= 32 ? MB_W64 : m <= 128 ? MB_W256 : MB_W1024;
+    return m <= 512 ? MB_C1024 : m <= 2048 ? MB_C4096 : MB_C16384;
+}
+// Counters::bad_M bits
+constexpr int MASK_BAD_ROWPTR = 1, MASK_BAD_ORDER = 2, MASK_BAD_COL = 4;
+
 __host__ __device__ __forceinline__ int sym_bin_of(int p, int span)
 {
     if (p <= 1) return p;
@@ -139,6 +165,9 @@ struct Counters {
     unsigned long long num_bin_products[MAX_BINS];
     unsigned long long num_bin_nnzc[MAX_BINS];
     unsigned long long num_bin_nnza[MAX_BINS];
+    int mask_bin[MB_COUNT];        // masked product: rows per masked bin (k_mask_bins)
+    int mask_cursor[MB_COUNT];
+    int bad_M;                     // masked product: MASK_BAD_* of the mask
     // transposed operands (stage_transpose.cu): bit 0 / 1 = a column of the stored A / B outside its range.
     // Last member: written by the transposition only, so a transposition done by bhb200_warmup is still
     // reported by the next bhb200_spgemm (the per-call zeroing stops at CTR_ZERO_BYTES)
@@ -577,6 +606,25 @@ cudaError_t launch_transpose(const LaunchCtx &lc, int dtype, int rows, int cols,
                              void *scratch, int *bad, int bad_bit);
 // values again through the permutation of the last transposition: valT[p] = val[perm[p]]
 cudaError_t launch_regather(const LaunchCtx &lc, int dtype, int nnz, const void *val, const int *perm, void *valT);
+// stage_masked.cu: the mask M (m x n, structural) and where the masked kernels put their rows
+struct MaskCsr {
+    const int *rowptr;
+    const int *col;
+    int nnz;
+};
+struct MaskOut {
+    int *rc;                // [m] nnz(C_i)
+    long long *ct_off;      // [m] = rowptrM[i]: rows are staged at their mask offsets
+    int *ctcol;             // staging columns (nnzM)
+    void *ctval;            // staging values (nnzM)
+    void *acc;              // MB_GLOBAL: values per mask entry (nnzM), or null
+    unsigned char *hit;     // MB_GLOBAL: hit flag per mask entry (nnzM), or null
+};
+cudaError_t launch_mask_bins(const LaunchCtx &lc, int m, int n, MaskCsr M, const int *prod, Counters *ctr);
+cudaError_t launch_mask_scatter(const LaunchCtx &lc, int m, MaskCsr M, const int *prod, const BinOffsets &offs, Counters *ctr,
+                                int *queue, int *rc, long long *ct_off);
+cudaError_t launch_mask_bin(const LaunchCtx &lc, int dtype, int bin, const int *queue, int count, Csr A, Csr B,
+                            const int4 *brange, MaskCsr M, MaskOut o);
 // stage_small.cu
 cudaError_t launch_sym_esc(const LaunchCtx &lc, const int *queue, int count, int n, Csr A, Csr B, int *rc);
 cudaError_t launch_num_single(const LaunchCtx &lc, int dtype, const int *queue, int count, Csr A, Csr B,

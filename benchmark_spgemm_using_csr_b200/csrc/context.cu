@@ -47,6 +47,14 @@ size_t vsize(int dtype)
     return dtype == BHB200_DTYPE_F64 ? 8 : 4;
 }
 
+// forget the mask (the library's copy stays allocated for the next bhb200_set_mask)
+void drop_mask(bhb200_ctx *ctx)
+{
+    ctx->mask_set = false;
+    ctx->M = MaskCsr{nullptr, nullptr, 0};
+    ctx->last_masked = false;
+}
+
 void release_operands(bhb200_ctx *ctx)
 {
     ctx->a_rowptr.release(&ctx->dev_bytes);
@@ -72,6 +80,7 @@ void release_operands(bhb200_ctx *ctx)
     ctx->have_C = false;
     ctx->last_pattern = false;
     ctx->nnzC = 0;
+    drop_mask(ctx);
 }
 
 int check_dims(bhb200_ctx *ctx, int m, int k, int n, int nnzA, int nnzB, const void *valA, const int32_t *rowptrA,
@@ -220,6 +229,7 @@ int init_host(bhb200_ctx *ctx, int dtype, int opA, int opB, int m, int k, int n,
     ctx->borrowed = false;
     ctx->have_C = false;
     ctx->nnzC = 0;
+    drop_mask(ctx);
     return BHB200_SUCCESS;
 }
 
@@ -375,6 +385,8 @@ void finish_stats(bhb200_ctx *ctx)
     const int64_t m1 = (int64_t)ctx->m + 1;
     st.bytes_algorithmic = (m1 * 4 + (int64_t)ctx->nnzA * (4 + v)) + ((int64_t)ctx->nnzA * 8 + st.products * (4 + v)) +
                            (m1 * 4 + ctx->nnzC * (4 + v));
+    // masked: + M read twice (validation, tables) + the staged rows written and read once (DESIGN.md 4.10)
+    if (st.masked) st.bytes_algorithmic += (m1 * 4 + 2 * st.nnzM * 4) + 2 * ctx->nnzC * (4 + v);
     st.bytes_compulsory = (m1 * 4 + (int64_t)ctx->nnzA * (4 + v)) + (((int64_t)ctx->k + 1) * 4 + (int64_t)ctx->nnzB * (4 + v)) +
                           (m1 * 4 + ctx->nnzC * (4 + v));
     st.workspace_bytes = (int64_t)ctx->dev_bytes;
@@ -607,6 +619,7 @@ int stage1_counts(bhb200_ctx *ctx, Product &p)
     CU(launch_row_products(p.lc, ctx->m, ctx->k, ctx->nnzA, ctx->A, ctx->B, ctx->brange.as<int4>(), ctx->prod.as<int>(),
                            ctx->rc.as<int>(), ctx->rlo.as<int>(), ctx->rspan.as<int>(), d_ctr),
        "row products kernel");
+    if (ctx->mask_set) CU(launch_mask_bins(p.lc, ctx->m, ctx->n, ctx->M, ctx->prod.as<int>(), d_ctr), "mask bins kernel");
     int rc = read_counters(ctx, "stage 1");
     if (rc) return rc;
     p.hc = *ctx->h_ctr;
@@ -619,6 +632,13 @@ int stage1_counts(bhb200_ctx *ctx, Product &p)
     st.max_row_products = hc.max_row_products;
     for (int b = 0; b < BHB200_NUM_SYM_BINS && b < MAX_BINS; ++b) st.sym_bin_rows[b] = hc.sym_bin[b];
     if ((rc = wait_for_values(ctx))) return rc;
+    if (ctx->mask_set) {   // (the masked product bins its rows by the mask: stage_masked)
+        if (hc.bad_M & MASK_BAD_ROWPTR)
+            return fail(ctx, BHB200_ERR_INVALID, "mask: row pointers must rise from 0 to nnzM");
+        if (hc.bad_M & MASK_BAD_COL) return fail(ctx, BHB200_ERR_INVALID, "mask: a column index is outside [0, n)");
+        if (hc.bad_M) return fail(ctx, BHB200_ERR_INVALID, "mask: rows must be sorted by column and duplicate-free");
+        return BHB200_SUCCESS;
+    }
     // lanes per row group: follow the average length of the B rows actually referenced
     const double avg_b = ctx->nnzA > 0 ? (double)hc.products / (double)ctx->nnzA : 0.0;
     p.G = avg_b <= 10.0 ? 8 : 32;
@@ -847,6 +867,104 @@ int stage4_numeric(bhb200_ctx *ctx, const Product &p)
     return BHB200_SUCCESS;
 }
 
+// ---- masked product (stage_masked.cu): the masked kernels of every bin, rows staged at their mask offsets ----
+int run_mask_bins(bhb200_ctx *ctx, const LaunchCtx &lc, const int *mask_bin)
+{
+    const MaskOut o{ctx->rc.as<int>(), ctx->ct_off.as<long long>(), ctx->ct_col.as<int>(), ctx->ct_val.p, ctx->mask_acc.p,
+                    ctx->mask_hit.as<unsigned char>()};
+    memset(ctx->ev_bin_used, 0, sizeof(ctx->ev_bin_used));
+    int off = 0;
+    for (int b = 0; b < MB_COUNT; ++b) {
+        if (b != MB_ZERO && mask_bin[b] > 0) {
+            CU(stamp(ctx, 0, b), "event");
+            CU(launch_mask_bin(lc, ctx->dtype, b, ctx->mask_q.as<int>() + off, mask_bin[b], ctx->A, ctx->B, ctx->brange.as<int4>(),
+                               ctx->M, o),
+               "masked kernel");
+        }
+        if (b != MB_ZERO) off += mask_bin[b];   // (MB_ZERO rows are not queued)
+    }
+    CU(stamp(ctx, 0, MAX_BINS), "event");
+    return BHB200_SUCCESS;
+}
+
+// the k_copy_ct launch of the copy bin the numeric bin scatter left in the queue
+int run_mask_copy(bhb200_ctx *ctx, const LaunchCtx &lc)
+{
+    if (ctx->last_copy_rows <= 0) return BHB200_SUCCESS;
+    CU(launch_copy_ct(lc, ctx->dtype, ctx->queue.as<int>() + ctx->last_copy_off, ctx->last_copy_rows, ctx->rowoff64.as<int64_t>(),
+                      ctx->ct_off.as<long long>(), ctx->ct_col.as<int>(), ctx->ct_val.p, ctx->colC.as<int>(), ctx->valC.p,
+                      ctx->last_copy_avg),
+       "Ct -> C copy");
+    return BHB200_SUCCESS;
+}
+
+// In place of the direct-mode choice and stages 2-4.  Host synchronisations: the one of stage 1 (which
+// brought the masked bin sizes and the mask check) and the one after the scan (nnz(C)).
+int stage_masked(bhb200_ctx *ctx, Product &p)
+{
+    Counters *d_ctr = ctx->counters.as<Counters>();
+    bhb200_stats &st = ctx->stats;
+    cudaStream_t s = ctx->stream;
+    const size_t vs = vsize(ctx->dtype);
+    const size_t m1 = (size_t)ctx->m + 1, nM = (size_t)ctx->M.nnz;
+    const int *prod = ctx->prod.as<int>();
+    st.masked = 1;
+    st.nnzM = (int64_t)nM;
+    for (int b = 0; b < BHB200_NUM_MASK_BINS && b < MB_COUNT; ++b) st.mask_bin_rows[b] = p.hc.mask_bin[b];
+    // staging: exactly nnzM entries, row i at rowptrM[i]; it may spill to host memory like C
+    CU(ctx->ct_off.reserve(m1 * 8, &ctx->dev_bytes), "alloc staging offsets");
+    CU(ctx->mask_q.reserve(m1 * 4, &ctx->dev_bytes), "alloc masked bin queue");
+    CU(ctx->ct_col.reserve_spillable(nM * 4 + 16, &ctx->dev_bytes, ctx->device_cap, nullptr), "alloc staging columns");
+    CU(ctx->ct_val.reserve_spillable(nM * vs + 16, &ctx->dev_bytes, ctx->device_cap, nullptr), "alloc staging values");
+    st.spill_bytes += spilled_bytes(ctx->ct_col) + spilled_bytes(ctx->ct_val);
+    if (p.hc.mask_bin[MB_GLOBAL] > 0) {
+        CU(ctx->mask_acc.reserve(nM * vs + 16, &ctx->dev_bytes), "alloc masked accumulator");
+        CU(ctx->mask_hit.reserve(nM + 16, &ctx->dev_bytes), "alloc masked hit flags");
+    }
+    memcpy(ctx->last_mask_bin, p.hc.mask_bin, sizeof(ctx->last_mask_bin));
+    BinOffsets mo{};
+    for (int b = 1, acc = 0; b < MB_COUNT; ++b) {
+        mo.off[b] = acc;
+        acc += p.hc.mask_bin[b];
+    }
+    CU(launch_mask_scatter(p.lc, ctx->m, ctx->M, prod, mo, d_ctr, ctx->mask_q.as<int>(), ctx->rc.as<int>(),
+                           ctx->ct_off.as<long long>()),
+       "masked bin scatter");
+    CU(cudaEventRecord(ctx->ev[1], s), "event");
+    int rc = run_mask_bins(ctx, p.lc, ctx->last_mask_bin);
+    if (rc) return rc;
+    CU(cudaEventRecord(ctx->ev[2], s), "event");
+    // every row with a kernel has ct_off >= 0: with all bins marked direct, the scan and the bin scatter put it in NB_COPY
+    const unsigned all = ~0u;
+    CU(launch_scan(p.lc, ctx->m, ctx->A.rowptr, prod, ctx->rc.as<int>(), ctx->rspan.as<int>(), all, ctx->ct_off.as<long long>(),
+                   ctx->rowoff64.as<int64_t>(), ctx->rowptr32.as<int>(), ctx->blocksums.as<long long>(), d_ctr),
+       "row pointer scan");
+    if ((rc = read_counters(ctx, "masked product / scan"))) return rc;
+    p.hc = *ctx->h_ctr;
+    const Counters &hc = p.hc;
+    ctx->nnzC = (int64_t)hc.nnzC;
+    st.nnzC = ctx->nnzC;
+    for (int b = 0; b < BHB200_NUM_NUM_BINS && b < MAX_BINS; ++b) {
+        st.num_bin_rows[b] = hc.num_bin[b];
+        st.num_bin_products[b] = (int64_t)hc.num_bin_products[b];
+        st.num_bin_nnzC[b] = (int64_t)hc.num_bin_nnzc[b];
+        st.num_bin_nnzA[b] = (int64_t)hc.num_bin_nnza[b];
+    }
+    if ((rc = reserve_C(ctx))) return rc;
+    offsets_from_counts(hc.num_bin, p.no);
+    CU(launch_bin_scatter(p.lc, true, ctx->m, prod, ctx->rc.as<int>(), ctx->rspan.as<int>(), all, ctx->ct_off.as<long long>(), p.no,
+                          d_ctr, ctx->queue.as<int>()),
+       "numeric bin scatter");
+    CU(cudaEventRecord(ctx->ev[3], s), "event");
+    ctx->last_copy_rows = hc.num_bin[NB_COPY];
+    ctx->last_copy_off = p.no.off[NB_COPY];
+    ctx->last_copy_avg = hc.num_bin[NB_COPY] > 0 ? (double)hc.num_bin_nnzc[NB_COPY] / (double)hc.num_bin[NB_COPY] : 0.0;
+    if ((rc = run_mask_copy(ctx, p.lc))) return rc;
+    CU(cudaEventRecord(ctx->ev[4], s), "event");
+    ctx->last_masked = true;
+    return BHB200_SUCCESS;
+}
+
 }  // namespace
 
 // ============================================================================
@@ -938,7 +1056,8 @@ int bhb200_free_mem(bhb200_ctx *ctx)
                       &ctx->cdf_colcount, &ctx->cdf_hist, &ctx->cdf_tab, &ctx->ct_off, &ctx->ct_col, &ctx->ct_val, &ctx->retry_q,
                       &ctx->brange, &ctx->rlo, &ctx->rspan, &ctx->wl_off, &ctx->wl_cnt, &ctx->wl_idx, &ctx->wl_bits,
                       &ctx->prod, &ctx->rc, &ctx->queue, &ctx->rowoff64, &ctx->rowptr32, &ctx->blocksums,
-                      &ctx->counters, &ctx->bitmap, &ctx->prefix, &ctx->colC, &ctx->valC, &ctx->slice_range, &ctx->t_scratch};
+                      &ctx->counters, &ctx->bitmap, &ctx->prefix, &ctx->colC, &ctx->valC, &ctx->slice_range, &ctx->t_scratch,
+                      &ctx->mask_rowptr, &ctx->mask_col, &ctx->mask_q, &ctx->mask_acc, &ctx->mask_hit};
     for (DevBuf *b : bufs) b->release(&ctx->dev_bytes);
     ctx->bitmap_zeroed_bytes = 0;
     cudaGetLastError();
@@ -1050,6 +1169,50 @@ int bhb200_init_data_device_op(bhb200_ctx *ctx, int dtype, int opA, int opB, int
     return BHB200_SUCCESS;
 }
 
+static int set_mask_any(bhb200_ctx *ctx, bool device, int nnzM, const int32_t *rowptrM, const int32_t *colM)
+{
+    if (!ctx) return BHB200_ERR_INVALID;
+    if (!ctx->have_data) return fail(ctx, BHB200_ERR_INVALID, "mask: set_mask needs operands (initData) for its shape");
+    if (ctx->dist) return fail(ctx, BHB200_ERR_INVALID, "mask: masked products are not available on a multi-GPU context");
+    if (nnzM < 0 || !rowptrM || (nnzM > 0 && !colM)) return fail(ctx, BHB200_ERR_INVALID, "mask: null array or negative nnzM");
+    ctx->mask_changed = true;
+    drop_mask(ctx);
+    if (device) {
+        ctx->M = MaskCsr{rowptrM, colM, nnzM};
+    } else {
+        CU(cudaSetDevice(ctx->device), "cudaSetDevice");
+        const size_t m1 = (size_t)ctx->m + 1;
+        CU(ctx->mask_rowptr.reserve(m1 * 4, &ctx->dev_bytes), "alloc mask row pointers");
+        CU(ctx->mask_col.reserve((size_t)nnzM * 4 + 4, &ctx->dev_bytes), "alloc mask columns");
+        // (the stream may still be reading the previous mask: the copies are ordered after it)
+        CU(cudaMemcpyAsync(ctx->mask_rowptr.p, rowptrM, m1 * 4, cudaMemcpyHostToDevice, ctx->stream), "H2D mask row pointers");
+        if (nnzM > 0)
+            CU(cudaMemcpyAsync(ctx->mask_col.p, colM, (size_t)nnzM * 4, cudaMemcpyHostToDevice, ctx->stream), "H2D mask columns");
+        CU(cudaStreamSynchronize(ctx->stream), "H2D mask");
+        ctx->M = MaskCsr{ctx->mask_rowptr.as<int>(), ctx->mask_col.as<int>(), nnzM};
+    }
+    ctx->mask_set = true;
+    return BHB200_SUCCESS;
+}
+
+int bhb200_set_mask(bhb200_ctx *ctx, int nnzM, const int32_t *rowptrM, const int32_t *colM)
+{
+    return set_mask_any(ctx, false, nnzM, rowptrM, colM);
+}
+
+int bhb200_set_mask_device(bhb200_ctx *ctx, int nnzM, const int32_t *rowptrM, const int32_t *colM)
+{
+    return set_mask_any(ctx, true, nnzM, rowptrM, colM);
+}
+
+int bhb200_clear_mask(bhb200_ctx *ctx)
+{
+    if (!ctx) return BHB200_ERR_INVALID;
+    if (ctx->mask_set) ctx->mask_changed = true;
+    drop_mask(ctx);
+    return BHB200_SUCCESS;
+}
+
 int bhb200_warmup(bhb200_ctx *ctx)
 {
     if (!ctx || !ctx->have_data) return fail(ctx, BHB200_ERR_INVALID, "warmup before initData");
@@ -1080,6 +1243,8 @@ int bhb200_spgemm(bhb200_ctx *ctx)
     if (rc) return rc;
     ctx->have_C = false;
     ctx->reuse_bins_valid = false;
+    ctx->last_masked = false;
+    ctx->mask_changed = false;
     bhb200_stats &st = ctx->stats;
     memset(&st, 0, sizeof(st));
     st.transposed_ops = (ctx->opA ? 1 : 0) | (ctx->opB ? 2 : 0);
@@ -1094,13 +1259,19 @@ int bhb200_spgemm(bhb200_ctx *ctx)
     CU(cudaEventRecord(ctx->ev[0], ctx->stream), "event");
     if ((rc = transpose_operands(ctx, p.lc))) return rc;
     CU(cudaMemsetAsync(ctx->counters.p, 0, CTR_ZERO_BYTES, ctx->stream), "zero counters");
-    rc = try_pattern(ctx, p.lc);
-    if (rc != PATTERN_NOT_APPLICABLE) return rc;
-    if ((rc = stage1_counts(ctx, p))) return rc;
-    if ((rc = choose_direct(ctx, p))) return rc;
-    if ((rc = stage2_symbolic(ctx, p))) return rc;
-    if ((rc = stage3_scan_alloc(ctx, p))) return rc;
-    if ((rc = stage4_numeric(ctx, p))) return rc;
+    if (ctx->mask_set) {
+        ctx->last_pattern = false;   // (a masked product never takes the diagonal-pattern mode)
+        if ((rc = stage1_counts(ctx, p))) return rc;
+        if ((rc = stage_masked(ctx, p))) return rc;
+    } else {
+        rc = try_pattern(ctx, p.lc);
+        if (rc != PATTERN_NOT_APPLICABLE) return rc;
+        if ((rc = stage1_counts(ctx, p))) return rc;
+        if ((rc = choose_direct(ctx, p))) return rc;
+        if ((rc = stage2_symbolic(ctx, p))) return rc;
+        if ((rc = stage3_scan_alloc(ctx, p))) return rc;
+        if ((rc = stage4_numeric(ctx, p))) return rc;
+    }
     finish_stats(ctx);
     ctx->last_G = p.G;
     ctx->last_wl = p.wl;
@@ -1117,6 +1288,7 @@ int bhb200_spgemm_numeric(bhb200_ctx *ctx)
 {
     if (!ctx || !ctx->have_data || !ctx->have_C)
         return fail(ctx, BHB200_ERR_INVALID, "spgemm_numeric needs a completed spgemm on the same operands");
+    if (ctx->mask_changed) return fail(ctx, BHB200_ERR_INVALID, "spgemm_numeric: the mask changed since the last spgemm");
     int rc = begin_call(ctx);
     if (rc) return rc;
     bhb200_stats &st = ctx->stats;
@@ -1131,6 +1303,17 @@ int bhb200_spgemm_numeric(bhb200_ctx *ctx)
         ctx->t_ran = true;
     }
     CU(cudaEventRecord(ctx->ev[1], s), "event");
+    if (ctx->last_masked) {
+        // masked product: the masked kernels on the cached bin queues, then the copy of the cached copy bin
+        if ((rc = run_mask_bins(ctx, lc, ctx->last_mask_bin))) return rc;
+        CU(cudaEventRecord(ctx->ev[2], s), "event");
+        CU(cudaEventRecord(ctx->ev[3], s), "event");
+        if ((rc = run_mask_copy(ctx, lc))) return rc;
+        CU(cudaEventRecord(ctx->ev[4], s), "event");
+        st.kernel_launches = ctx->launches;
+        ctx->timing_valid = true;
+        return BHB200_SUCCESS;
+    }
     CU(cudaEventRecord(ctx->ev[2], s), "event");
     memset(ctx->ev_bin_used, 0, sizeof(ctx->ev_bin_used));
     if (ctx->last_pattern) {

@@ -132,6 +132,16 @@ struct bhb200_ctx {
     bool force_heavy = false;      // BHB200_DEBUG_FORCE_HEAVY (tests): rows beyond the on-chip tables take the sliced bucket sort
     long long wordlist_cap = -1;   // BHB200_DEBUG_WORDLIST_CAP (tests): size of the range kernels' word-list pool; -1: by product count
     size_t bitmap_zeroed_bytes = 0;
+    // masked product (stage_masked.cu): M is the library's copy (bhb200_set_mask) or the caller's arrays
+    // (bhb200_set_mask_device); mask_q holds the masked bin queues of the last masked product
+    bool mask_set = false;
+    bool mask_changed = false;   // set / cleared since the last bhb200_spgemm: no bhb200_spgemm_numeric
+    bhb::MaskCsr M{nullptr, nullptr, 0};
+    bhb::DevBuf mask_rowptr, mask_col, mask_q, mask_acc, mask_hit;
+    bool last_masked = false;
+    int last_mask_bin[bhb::MB_COUNT] = {0};
+    int last_copy_rows = 0, last_copy_off = 0;
+    double last_copy_avg = 0.0;
     bhb::DevBuf colC, valC;
     bhb::Counters *h_ctr = nullptr;   // pinned
     size_t dev_bytes = 0;

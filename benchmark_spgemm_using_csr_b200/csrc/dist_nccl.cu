@@ -295,6 +295,9 @@ int bhb200_dist_setup_square(bhb200_ctx *ctx, int root, int dtype, int n, int64_
     ctx->have_C = false;
     ctx->last_pattern = false;
     ctx->reuse_bins_valid = false;
+    ctx->mask_set = false;   // (a mask set before bhb200_dist_init: masked products are single-GPU)
+    ctx->M = MaskCsr{nullptr, nullptr, 0};
+    ctx->last_masked = false;
     d->have_layout = false;
     Partition *dp = d->d_part.as<Partition>();
     DCU(cudaEventRecord(d->ev_t0, s), "event");

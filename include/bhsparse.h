@@ -81,6 +81,14 @@ public:
 #endif
     }
 
+    /* Addition: masked products C = M .* (op(A)*op(B)) on the structure of M (host arrays, copied;
+     * bhb200_set_mask), until clearMask() or the next initData. */
+    int setMask(int nnzM, index_type *csrRowPtrM, index_type *csrColIndM)
+    {
+        return _ctx ? bhb200_set_mask(_ctx, nnzM, csrRowPtrM, csrColIndM) : BHB200_ERR_INVALID;
+    }
+    int clearMask() { return _ctx ? bhb200_clear_mask(_ctx) : BHB200_ERR_INVALID; }
+
     int warmup() { return _ctx ? bhb200_warmup(_ctx) : BHB200_ERR_INVALID; }   /* bhsparse.h:341-363 */
 
     /* bhsparse.h:260-339 */

@@ -51,6 +51,7 @@ extern "C" {
 
 #define BHB200_NUM_SYM_BINS 24
 #define BHB200_NUM_NUM_BINS 24
+#define BHB200_NUM_MASK_BINS 9
 
 typedef struct bhb200_ctx bhb200_ctx;
 
@@ -98,6 +99,16 @@ typedef struct bhb200_stats {
      * kernel_launches */
     int64_t transposed_ops;
     float ms_transpose;
+    /* masked product (bhb200_set_mask): 1 if the last product was masked, nnz(M), and the rows per
+     * masked kernel bin: 0 no products or no mask entries (no kernel), 1 <= 32 products (warp, binary
+     * search), 2-4 warp per row with a table for <= 32 / 128 / 512 mask entries (<= 2048 products),
+     * 5-7 CTA per row with a table for <= 512 / 2048 / 8192 mask entries, 8 more mask entries (binary
+     * search, values in global memory).  The stage times then read: ms_count = stage 1 + mask binning,
+     * ms_symbolic = the masked kernels (ms_sym_bin[b]: masked bin b, with profiling), ms_scan = scan +
+     * allocation of C, ms_numeric = the copy of the staged rows into C. */
+    int64_t masked;
+    int64_t nnzM;
+    int64_t mask_bin_rows[BHB200_NUM_MASK_BINS];
 } bhb200_stats;
 
 /* -- platform --------------------------------------------------------------
@@ -167,6 +178,30 @@ BHB200_API int bhb200_init_data_device(bhb200_ctx *ctx, int dtype, int m, int k,
 BHB200_API int bhb200_init_data_device_op(bhb200_ctx *ctx, int dtype, int opA, int opB, int m, int k, int n,
                                           int nnzA, const void *valA, const int32_t *rowptrA, const int32_t *colA,
                                           int nnzB, const void *valB, const int32_t *rowptrB, const int32_t *colB);
+
+/* -- masked products: C = M .* (op(A)*op(B)) (GraphBLAS C<M> = A*B) ----------------------------------
+ * M is m x n and structural: row pointers (m+1) and column indices, no values; its rows must be sorted
+ * and duplicate-free with columns in [0, n), as the rows of B.  C_ij is present iff M_ij is present and
+ * at least one product A_ik*B_kj exists; its value is the sum of those products (explicit zeros from
+ * cancellation are kept).  So C is the unmasked C restricted to the pattern of M.  Rows of C are
+ * sorted; the row pointers, get_C*, get_C_range, get_C_device and copy_C_to_device work as for
+ * unmasked products.  Only nnz(M) entries are staged and no product is sorted.
+ *   bhb200_set_mask         HOST arrays, copied before the call returns.  Needs operands (m, n).
+ *   bhb200_set_mask_device  DEVICE arrays, borrowed and read by every bhb200_spgemm, like borrowed
+ *                           operands; they may be the operands' own arrays (triangle counting: L as A,
+ *                           B and M).
+ *   bhb200_clear_mask       back to unmasked products.
+ * The mask is checked on the device by bhb200_spgemm: unsorted or duplicate columns, a column outside
+ * [0, n), row pointers that do not rise from 0 to nnzM all return BHB200_ERR_INVALID naming the mask.
+ * Every init_data*, init_data_device*, dist_setup_square and free_mem clears the mask.  Setting or
+ * clearing it leaves an existing C readable, but bhb200_spgemm_numeric returns BHB200_ERR_INVALID until
+ * the next bhb200_spgemm; after a masked bhb200_spgemm, update_values_* + spgemm_numeric recompute the
+ * masked values with the structure kept.  A masked product never takes the diagonal-pattern mode.
+ * Complemented masks and masks with values are not supported; on a multi-GPU context (after
+ * bhb200_dist_init) bhb200_set_mask* returns BHB200_ERR_INVALID. */
+BHB200_API int bhb200_set_mask(bhb200_ctx *ctx, int nnzM, const int32_t *rowptrM, const int32_t *colM);
+BHB200_API int bhb200_set_mask_device(bhb200_ctx *ctx, int nnzM, const int32_t *rowptrM, const int32_t *colM);
+BHB200_API int bhb200_clear_mask(bhb200_ctx *ctx);
 
 /* -- the hot path --------------------------------------------------------------
  * bhb200_warmup replaces bhsparse::warmup (bhsparse.h:341-363): runs the
