@@ -10,6 +10,7 @@
 // bhsparse_cuda.h:285-301, 2813-2911) and its host re-allocation loop
 // (:2527-2780) do not exist here: step 3 sizes C exactly.
 #pragma once
+#include "../../include/bhsparse_b200.h"   // BHB200_DTYPE_*
 #include <cuda_runtime.h>
 #include <stddef.h>
 #include <stdint.h>
@@ -639,59 +640,54 @@ cudaError_t launch_sym_hash(const LaunchCtx &lc, int bin, int G, const int *queu
                             unsigned long long *bin_sum = nullptr);
 cudaError_t launch_sym_large(const LaunchCtx &lc, const int *queue, int count, int n, Csr A, Csr B, int *rc,
                              unsigned *bitmap_scratch, int scratch_blocks);
-// stage_numeric_f32.cu / stage_numeric_f64.cu
-cudaError_t launch_num_hash_f32(const LaunchCtx &lc, int bin, int G, const int *queue, int count, Csr A, Csr B,
-                                const int64_t *rowoff, int *colC, float *valC);
-cudaError_t launch_num_hash_f64(const LaunchCtx &lc, int bin, int G, const int *queue, int count, Csr A, Csr B,
-                                const int64_t *rowoff, int *colC, double *valC);
-// direct mode: cap in {32, 64, 128} speculated (rows may overflow into the retry queue), or
-// {256, ..., 8192} for bins whose product bound is below cap (no overflow possible)
-cudaError_t launch_num_direct_f32(const LaunchCtx &lc, int cap, int G, const int *queue, int count, Csr A, Csr B,
-                                  DirectOut d);
-cudaError_t launch_num_direct_f64(const LaunchCtx &lc, int cap, int G, const int *queue, int count, Csr A, Csr B,
-                                  DirectOut d);
-// bucket-sort ESC for rows that barely compress (stage_bucket.cuh): wide direct bins, cap >= 512
-cudaError_t launch_num_bucket_f32(const LaunchCtx &lc, int cap, const int *queue, int count, Csr A, Csr B, DirectOut d,
-                                  const unsigned *cdf, int cdf_shift);
-cudaError_t launch_num_bucket_f64(const LaunchCtx &lc, int cap, const int *queue, int count, Csr A, Csr B, DirectOut d,
-                                  const unsigned *cdf, int cdf_shift);
-// heavy rows (more products than fit on chip): sliced bucket sort, staged at ct_base + bump(cursor, products)
-cudaError_t launch_num_bucket_heavy_f32(const LaunchCtx &lc, const int *queue, int count, Csr A, Csr B, DirectOut d,
-                                        const unsigned *cdf, int cdf_shift, unsigned long long *cursor);
-cudaError_t launch_num_bucket_heavy_f64(const LaunchCtx &lc, const int *queue, int count, Csr A, Csr B, DirectOut d,
-                                        const unsigned *cdf, int cdf_shift, unsigned long long *cursor);
-// warp-per-row bucket sort (k_num_bucket3w): bins SB_G128 (capw 128) / SB_G256 (capw 256) whose rows barely compress;
-// sg = lanes per B row (8 | 32); rows staged `stride` apart, rows with more outputs go to d.retry_queue
-cudaError_t launch_num_bucket3w_f32(const LaunchCtx &lc, int capw, int sg, const int *queue, int count, Csr A, Csr B, DirectOut d,
-                                    const unsigned *cdf, int cdf_shift, int stride);
-cudaError_t launch_num_bucket3w_f64(const LaunchCtx &lc, int capw, int sg, const int *queue, int count, Csr A, Csr B, DirectOut d,
-                                    const unsigned *cdf, int cdf_shift, int stride);
-// second formulation (k_num_bucket_heavy2): rows with more than d.p_lo products, partitioned by slice through their own
-// staging area; rows it cannot slice go to d.retry_queue / d.retry_cnt for launch_num_bucket_heavy_* (d.count_dev)
-cudaError_t launch_num_bucket_heavy2_f32(const LaunchCtx &lc, const int *queue, int count, Csr A, Csr B, DirectOut d,
-                                         const unsigned *cdf, int cdf_shift, unsigned long long *cursor);
-cudaError_t launch_num_bucket_heavy2_f64(const LaunchCtx &lc, const int *queue, int count, Csr A, Csr B, DirectOut d,
-                                         const unsigned *cdf, int cdf_shift, unsigned long long *cursor);
 // column CDF of the intermediate products (stage_bucket.cu): colcountA [k+1] ints, hist [4096] u64, cdf [4097] u32
 cudaError_t launch_build_cdf(const LaunchCtx &lc, int m, int k, int n, int nnzA, Csr A, Csr B, int *colcountA,
                              unsigned long long *hist, unsigned *cdf, int *shift_out);
-cudaError_t launch_copy_ct(const LaunchCtx &lc, int dtype, const int *queue, int count, const int64_t *rowoff,
-                           const long long *ct_off, const int *ctcol, const void *ctval, int *colC, void *valC, double avg_row);
-cudaError_t launch_num_large_f32(const LaunchCtx &lc, const int *queue, int count, int n, Csr A, Csr B,
-                                 const int64_t *rowoff, int *colC, float *valC, unsigned *bitmap_scratch,
-                                 int *prefix_scratch, int scratch_blocks);
-cudaError_t launch_num_large_f64(const LaunchCtx &lc, const int *queue, int count, int n, Csr A, Csr B,
-                                 const int64_t *rowoff, int *colC, double *valC, unsigned *bitmap_scratch,
-                                 int *prefix_scratch, int scratch_blocks);
 // resident CTAs (= private scratch sets) of the large-row kernels for n columns
 int large_scratch_blocks(int sm_count, int n);
 // stage_range.cu (symbolic) / stage_numeric (numeric) -- shared-memory bitmap kernels
 // (the launchers pick the 128-bit vectorised kernels of stage_range_vec.cuh when B is 16-byte aligned)
 cudaError_t launch_sym_range(const LaunchCtx &lc, int nsum, const int *queue, int count, Csr A, Csr B, const int *rlo,
                              int *rc, Counters *ctr, WordLists wl);
-cudaError_t launch_num_range_f32(const LaunchCtx &lc, int nsum, int nacc, const int *queue, int count, Csr A, Csr B,
-                                 const int *rlo, const int64_t *rowoff, int *colC, float *valC, WordLists wl);
-cudaError_t launch_num_range_f64(const LaunchCtx &lc, int nsum, int nacc, const int *queue, int count, Csr A, Csr B,
-                                 const int *rlo, const int64_t *rowoff, int *colC, double *valC, WordLists wl);
+
+// The numeric kernels of one value type (stage_numeric_f32.cu / stage_numeric_f64.cu); values are float or double
+// as the operands are.  The two types compile in two translation units, in parallel.
+struct ColumnCdf {
+    const unsigned *cdf;   // [CDF_KNOTS + 1], non-decreasing, cdf[0] = 0
+    int shift;             // column >> shift < CDF_KNOTS
+};
+struct NumericKernels {
+    cudaError_t (*hash)(const LaunchCtx &lc, int bin, int G, const int *queue, int count, Csr A, Csr B,
+                        const int64_t *rowoff, int *colC, void *valC);
+    cudaError_t (*large)(const LaunchCtx &lc, const int *queue, int count, int n, Csr A, Csr B, const int64_t *rowoff,
+                         int *colC, void *valC, unsigned *bitmap_scratch, int *prefix_scratch, int scratch_blocks);
+    cudaError_t (*range)(const LaunchCtx &lc, int nsum, int nacc, const int *queue, int count, Csr A, Csr B,
+                         const int *rlo, const int64_t *rowoff, int *colC, void *valC, WordLists wl);
+    // direct mode: cap in {32, 64, 128} speculated (rows may overflow into the retry queue), or
+    // {256, ..., 8192} for bins whose product bound is below cap (no overflow possible)
+    cudaError_t (*direct)(const LaunchCtx &lc, int cap, int G, const int *queue, int count, Csr A, Csr B, DirectOut d);
+    // bucket-sort ESC for rows that barely compress (stage_bucket.cuh): wide direct bins, cap >= 512
+    cudaError_t (*bucket)(const LaunchCtx &lc, int cap, const int *queue, int count, Csr A, Csr B, DirectOut d,
+                          ColumnCdf cdf);
+    // warp-per-row bucket sort (k_num_bucket3w): bins SB_G128 (capw 128) / SB_G256 (capw 256) whose rows barely compress;
+    // sg = lanes per B row (8 | 32); rows staged `stride` apart, rows with more outputs go to d.retry_queue
+    cudaError_t (*bucket3w)(const LaunchCtx &lc, int capw, int sg, const int *queue, int count, Csr A, Csr B, DirectOut d,
+                            ColumnCdf cdf, int stride);
+    // heavy rows (more products than fit on chip): sliced bucket sort, staged at ct_base + bump(cursor, products)
+    cudaError_t (*heavy)(const LaunchCtx &lc, const int *queue, int count, Csr A, Csr B, DirectOut d, ColumnCdf cdf,
+                         unsigned long long *cursor);
+    // second formulation (k_num_bucket_heavy2): rows with more than d.p_lo products, partitioned by slice through their own
+    // staging area; rows it cannot slice go to d.retry_queue / d.retry_cnt for `heavy` (d.count_dev)
+    cudaError_t (*heavy2)(const LaunchCtx &lc, const int *queue, int count, Csr A, Csr B, DirectOut d, ColumnCdf cdf,
+                          unsigned long long *cursor);
+    // staged rows -> C; avg_row = staged entries per row of the launch: short rows are copied 32 rows per warp
+    cudaError_t (*copy_ct)(const LaunchCtx &lc, const int *queue, int count, const int64_t *rowoff, const long long *ct_off,
+                           const int *ctcol, const void *ctval, int *colC, void *valC, double avg_row);
+};
+extern const NumericKernels NUMERIC_F32, NUMERIC_F64;
+inline const NumericKernels &numeric_kernels(int dtype)
+{
+    return dtype == BHB200_DTYPE_F64 ? NUMERIC_F64 : NUMERIC_F32;
+}
 
 }  // namespace bhb

@@ -321,6 +321,8 @@ int run_numeric_bins(bhb200_ctx *ctx, const LaunchCtx &lc, const int *num_bin, c
                      const WordLists &wl)
 {
     int rc = 0;
+    const NumericKernels &nk = numeric_kernels(ctx->dtype);
+    const bool f64 = ctx->dtype == BHB200_DTYPE_F64;   // (for the error messages)
     int *queue = ctx->queue.as<int>();
     int64_t *rowoff = ctx->rowoff64.as<int64_t>();
     int *rlo = ctx->rlo.as<int>();
@@ -334,26 +336,17 @@ int run_numeric_bins(bhb200_ctx *ctx, const LaunchCtx &lc, const int *num_bin, c
        "numeric ESC");
     for (int b = NB_G64; b <= NB_B16384; ++b) {
         if (num_bin[b] > 0) CU(stamp(ctx, 1, b), "event");
-        if (ctx->dtype == BHB200_DTYPE_F64)
-            CU(launch_num_hash_f64(lc, b, G, queue + no.off[b], num_bin[b], ctx->A, ctx->B, rowoff, colC, (double *)valC),
-               "numeric hash f64");
-        else
-            CU(launch_num_hash_f32(lc, b, G, queue + no.off[b], num_bin[b], ctx->A, ctx->B, rowoff, colC, (float *)valC),
-               "numeric hash f32");
+        CU(nk.hash(lc, b, G, queue + no.off[b], num_bin[b], ctx->A, ctx->B, rowoff, colC, valC),
+           f64 ? "numeric hash f64" : "numeric hash f32");
     }
     if (num_bin[NB_LARGE] > 0) {
         rc = reserve_large_scratch(ctx, true);
         if (rc) return rc;
         const int sb = large_scratch_blocks(ctx->sm_count, ctx->n);
         CU(stamp(ctx, 1, NB_LARGE), "event");
-        if (ctx->dtype == BHB200_DTYPE_F64)
-            CU(launch_num_large_f64(lc, queue + no.off[NB_LARGE], num_bin[NB_LARGE], ctx->n, ctx->A, ctx->B, rowoff, colC,
-                                    (double *)valC, ctx->bitmap.as<unsigned>(), ctx->prefix.as<int>(), sb),
-               "numeric large f64");
-        else
-            CU(launch_num_large_f32(lc, queue + no.off[NB_LARGE], num_bin[NB_LARGE], ctx->n, ctx->A, ctx->B, rowoff, colC,
-                                    (float *)valC, ctx->bitmap.as<unsigned>(), ctx->prefix.as<int>(), sb),
-               "numeric large f32");
+        CU(nk.large(lc, queue + no.off[NB_LARGE], num_bin[NB_LARGE], ctx->n, ctx->A, ctx->B, rowoff, colC, valC,
+                    ctx->bitmap.as<unsigned>(), ctx->prefix.as<int>(), sb),
+           f64 ? "numeric large f64" : "numeric large f32");
     }
     {
         const int rb[4] = {NB_RANGE_S128, NB_RANGE_S512, NB_RANGE_L128, NB_RANGE_L512};
@@ -363,14 +356,8 @@ int run_numeric_bins(bhb200_ctx *ctx, const LaunchCtx &lc, const int *num_bin, c
             const int b = rb[i];
             if (num_bin[b] <= 0) continue;
             CU(stamp(ctx, 1, b), "event");
-            if (ctx->dtype == BHB200_DTYPE_F64)
-                CU(launch_num_range_f64(lc, rnsum[i], rnacc[i], queue + no.off[b], num_bin[b], ctx->A, ctx->B, rlo, rowoff,
-                                        colC, (double *)valC, wl),
-                   "numeric range f64");
-            else
-                CU(launch_num_range_f32(lc, rnsum[i], rnacc[i], queue + no.off[b], num_bin[b], ctx->A, ctx->B, rlo, rowoff,
-                                        colC, (float *)valC, wl),
-                   "numeric range f32");
+            CU(nk.range(lc, rnsum[i], rnacc[i], queue + no.off[b], num_bin[b], ctx->A, ctx->B, rlo, rowoff, colC, valC, wl),
+               f64 ? "numeric range f64" : "numeric range f32");
         }
     }
     return BHB200_SUCCESS;
@@ -716,23 +703,12 @@ int choose_direct(bhb200_ctx *ctx, Product &p)
 // the launches DirectPlan::launches lists for direct-mode bin b, in the value type of the operands
 int run_direct_bin(bhb200_ctx *ctx, const Product &p, int b)
 {
-    struct Kernels {
-        decltype(&launch_num_direct_f32) direct;
-        decltype(&launch_num_bucket_f32) bucket;
-        decltype(&launch_num_bucket3w_f32) bucket3w;
-        decltype(&launch_num_bucket_heavy2_f32) heavy2;
-        decltype(&launch_num_bucket_heavy_f32) heavy;
-    };
-    static const Kernels F32{launch_num_direct_f32, launch_num_bucket_f32, launch_num_bucket3w_f32,
-                             launch_num_bucket_heavy2_f32, launch_num_bucket_heavy_f32};
-    static const Kernels F64{launch_num_direct_f64, launch_num_bucket_f64, launch_num_bucket3w_f64,
-                             launch_num_bucket_heavy2_f64, launch_num_bucket_heavy_f64};
-    const Kernels &k = ctx->dtype == BHB200_DTYPE_F64 ? F64 : F32;
+    const NumericKernels &nk = numeric_kernels(ctx->dtype);
     const DirectBin &db = p.plan.bin[b];
     Counters *d_ctr = ctx->counters.as<Counters>();
     const int *queue = ctx->queue.as<int>() + p.so.off[b];
     int *retry_queue = ctx->retry_q.as<int>() + p.so.off[b];
-    const unsigned *cdf = ctx->cdf_tab.as<unsigned>();
+    const ColumnCdf cdf{ctx->cdf_tab.as<unsigned>(), p.cdf_shift};
     const DirectLaunches ls = p.plan.launches(b, p.G);
     for (int i = 0; i < ls.n; ++i) {
         const DirectLaunch &l = ls.at[i];
@@ -746,18 +722,18 @@ int run_direct_bin(bhb200_ctx *ctx, const Product &p, int b)
         d.ct_stride = l.stride;
         switch (l.kernel) {
         case DirectKernel::DIRECT:
-            CU(k.direct(p.lc, l.cap, l.sg, queue, db.rows, ctx->A, ctx->B, d), "direct numeric");
+            CU(nk.direct(p.lc, l.cap, l.sg, queue, db.rows, ctx->A, ctx->B, d), "direct numeric");
             break;
         case DirectKernel::BUCKET:
-            CU(k.bucket(p.lc, l.cap, queue, db.rows, ctx->A, ctx->B, d, cdf, p.cdf_shift), "bucket numeric");
+            CU(nk.bucket(p.lc, l.cap, queue, db.rows, ctx->A, ctx->B, d, cdf), "bucket numeric");
             break;
         case DirectKernel::BUCKET3W:
-            CU(k.bucket3w(p.lc, l.cap, l.sg, queue, db.rows, ctx->A, ctx->B, d, cdf, p.cdf_shift, l.stride), "warp bucket numeric");
+            CU(nk.bucket3w(p.lc, l.cap, l.sg, queue, db.rows, ctx->A, ctx->B, d, cdf, l.stride), "warp bucket numeric");
             break;
         case DirectKernel::HEAVY:
-            CU(k.heavy2(p.lc, queue, db.rows, ctx->A, ctx->B, d, cdf, p.cdf_shift, &d_ctr->heavy_cursor), "heavy rows");
+            CU(nk.heavy2(p.lc, queue, db.rows, ctx->A, ctx->B, d, cdf, &d_ctr->heavy_cursor), "heavy rows");
             d.count_dev = d.retry_cnt;   // what k_num_bucket_heavy2 could not slice
-            CU(k.heavy(p.lc, retry_queue, db.rows, ctx->A, ctx->B, d, cdf, p.cdf_shift, &d_ctr->heavy_cursor), "heavy rows");
+            CU(nk.heavy(p.lc, retry_queue, db.rows, ctx->A, ctx->B, d, cdf, &d_ctr->heavy_cursor), "heavy rows");
             break;
         }
     }
@@ -817,17 +793,17 @@ int stage2_symbolic(bhb200_ctx *ctx, Product &p)
     return BHB200_SUCCESS;
 }
 
-// ---- stage 3: row pointers, numeric bins, exact allocation of C ----
-int stage3_scan_alloc(bhb200_ctx *ctx, Product &p)
+// Row pointers of C, nnz(C) and the numeric bins read back (one host sync), C allocated exactly, rows scattered to
+// the numeric bin queues.  spec_mask: symbolic bins whose rows were staged; those with ct_off >= 0 go to NB_COPY.
+int scan_and_bin(bhb200_ctx *ctx, Product &p, unsigned spec_mask, const char *what)
 {
-    const unsigned mask = p.plan.mask();
     Counters *d_ctr = ctx->counters.as<Counters>();
     bhb200_stats &st = ctx->stats;
-    CU(launch_scan(p.lc, ctx->m, ctx->A.rowptr, ctx->prod.as<int>(), ctx->rc.as<int>(), ctx->rspan.as<int>(), mask,
+    CU(launch_scan(p.lc, ctx->m, ctx->A.rowptr, ctx->prod.as<int>(), ctx->rc.as<int>(), ctx->rspan.as<int>(), spec_mask,
                    ctx->ct_off.as<long long>(), ctx->rowoff64.as<int64_t>(), ctx->rowptr32.as<int>(),
                    ctx->blocksums.as<long long>(), d_ctr),
        "row pointer scan");
-    int rc = read_counters(ctx, "stage 2/3");
+    int rc = read_counters(ctx, what);
     if (rc) return rc;
     p.hc = *ctx->h_ctr;
     const Counters &hc = p.hc;
@@ -841,60 +817,62 @@ int stage3_scan_alloc(bhb200_ctx *ctx, Product &p)
     }
     if ((rc = reserve_C(ctx))) return rc;
     offsets_from_counts(hc.num_bin, p.no);
-    CU(launch_bin_scatter(p.lc, true, ctx->m, ctx->prod.as<int>(), ctx->rc.as<int>(), ctx->rspan.as<int>(), mask,
+    CU(launch_bin_scatter(p.lc, true, ctx->m, ctx->prod.as<int>(), ctx->rc.as<int>(), ctx->rspan.as<int>(), spec_mask,
                           ctx->ct_off.as<long long>(), p.no, d_ctr, ctx->queue.as<int>()),
        "numeric bin scatter");
-    for (int b = 0; b < MAX_BINS; ++b) st.direct_retry_rows += hc.retry_cnt[b];
+    for (int b = 0; b < MAX_BINS; ++b) st.direct_retry_rows += hc.retry_cnt[b];   // (zero in a masked product)
     CU(cudaEventRecord(ctx->ev[3], ctx->stream), "event");
+    const int copy_rows = hc.num_bin[NB_COPY];
+    ctx->last_copy_rows = copy_rows;
+    ctx->last_copy_off = p.no.off[NB_COPY];
+    ctx->last_copy_avg = copy_rows > 0 ? (double)hc.num_bin_nnzc[NB_COPY] / (double)copy_rows : 0.0;
     return BHB200_SUCCESS;
+}
+
+// the k_copy_ct launch of the copy bin that scan_and_bin recorded
+int run_copy_bin(bhb200_ctx *ctx, const LaunchCtx &lc)
+{
+    if (ctx->last_copy_rows <= 0) return BHB200_SUCCESS;
+    CU(numeric_kernels(ctx->dtype)
+           .copy_ct(lc, ctx->queue.as<int>() + ctx->last_copy_off, ctx->last_copy_rows, ctx->rowoff64.as<int64_t>(),
+                    ctx->ct_off.as<long long>(), ctx->ct_col.as<int>(), ctx->ct_val.p, ctx->colC.as<int>(), ctx->valC.p,
+                    ctx->last_copy_avg),
+       "Ct -> C copy");
+    return BHB200_SUCCESS;
+}
+
+// ---- stage 3: row pointers, numeric bins, exact allocation of C ----
+int stage3_scan_alloc(bhb200_ctx *ctx, Product &p)
+{
+    return scan_and_bin(ctx, p, p.plan.mask(), "stage 2/3");
 }
 
 // ---- stage 4: numeric, C written in place ----
 int stage4_numeric(bhb200_ctx *ctx, const Product &p)
 {
-    const Counters &hc = p.hc;
-    const int rc = run_numeric_bins(ctx, p.lc, hc.num_bin, p.no, p.G, p.wl);
+    int rc = run_numeric_bins(ctx, p.lc, p.hc.num_bin, p.no, p.G, p.wl);
     if (rc) return rc;
-    if (hc.num_bin[NB_COPY] > 0) {
-        CU(stamp(ctx, 1, NB_COPY), "event");
-        CU(launch_copy_ct(p.lc, ctx->dtype, ctx->queue.as<int>() + p.no.off[NB_COPY], hc.num_bin[NB_COPY], ctx->rowoff64.as<int64_t>(),
-                          ctx->ct_off.as<long long>(), ctx->ct_col.as<int>(), ctx->ct_val.p, ctx->colC.as<int>(), ctx->valC.p,
-                          (double)hc.num_bin_nnzc[NB_COPY] / (double)hc.num_bin[NB_COPY]),
-           "Ct -> C copy");
-    }
+    if (ctx->last_copy_rows > 0) CU(stamp(ctx, 1, NB_COPY), "event");
+    if ((rc = run_copy_bin(ctx, p.lc))) return rc;
     CU(stamp(ctx, 1, MAX_BINS), "event");
     CU(cudaEventRecord(ctx->ev[4], ctx->stream), "event");
     return BHB200_SUCCESS;
 }
 
 // ---- masked product (stage_masked.cu): the masked kernels of every bin, rows staged at their mask offsets ----
-int run_mask_bins(bhb200_ctx *ctx, const LaunchCtx &lc, const int *mask_bin)
+int run_mask_bins(bhb200_ctx *ctx, const LaunchCtx &lc)
 {
     const MaskOut o{ctx->rc.as<int>(), ctx->ct_off.as<long long>(), ctx->ct_col.as<int>(), ctx->ct_val.p, ctx->mask_acc.p,
                     ctx->mask_hit.as<unsigned char>()};
     memset(ctx->ev_bin_used, 0, sizeof(ctx->ev_bin_used));
-    int off = 0;
-    for (int b = 0; b < MB_COUNT; ++b) {
-        if (b != MB_ZERO && mask_bin[b] > 0) {
-            CU(stamp(ctx, 0, b), "event");
-            CU(launch_mask_bin(lc, ctx->dtype, b, ctx->mask_q.as<int>() + off, mask_bin[b], ctx->A, ctx->B, ctx->brange.as<int4>(),
-                               ctx->M, o),
-               "masked kernel");
-        }
-        if (b != MB_ZERO) off += mask_bin[b];   // (MB_ZERO rows are not queued)
+    for (int b = MB_ZERO + 1; b < MB_COUNT; ++b) {
+        if (ctx->last_mask_bin[b] <= 0) continue;
+        CU(stamp(ctx, 0, b), "event");
+        CU(launch_mask_bin(lc, ctx->dtype, b, ctx->mask_q.as<int>() + ctx->last_mask_off.off[b], ctx->last_mask_bin[b], ctx->A,
+                           ctx->B, ctx->brange.as<int4>(), ctx->M, o),
+           "masked kernel");
     }
     CU(stamp(ctx, 0, MAX_BINS), "event");
-    return BHB200_SUCCESS;
-}
-
-// the k_copy_ct launch of the copy bin the numeric bin scatter left in the queue
-int run_mask_copy(bhb200_ctx *ctx, const LaunchCtx &lc)
-{
-    if (ctx->last_copy_rows <= 0) return BHB200_SUCCESS;
-    CU(launch_copy_ct(lc, ctx->dtype, ctx->queue.as<int>() + ctx->last_copy_off, ctx->last_copy_rows, ctx->rowoff64.as<int64_t>(),
-                      ctx->ct_off.as<long long>(), ctx->ct_col.as<int>(), ctx->ct_val.p, ctx->colC.as<int>(), ctx->valC.p,
-                      ctx->last_copy_avg),
-       "Ct -> C copy");
     return BHB200_SUCCESS;
 }
 
@@ -922,44 +900,21 @@ int stage_masked(bhb200_ctx *ctx, Product &p)
         CU(ctx->mask_hit.reserve(nM + 16, &ctx->dev_bytes), "alloc masked hit flags");
     }
     memcpy(ctx->last_mask_bin, p.hc.mask_bin, sizeof(ctx->last_mask_bin));
-    BinOffsets mo{};
-    for (int b = 1, acc = 0; b < MB_COUNT; ++b) {
-        mo.off[b] = acc;
+    ctx->last_mask_off = BinOffsets{};
+    for (int b = MB_ZERO + 1, acc = 0; b < MB_COUNT; ++b) {   // (MB_ZERO rows are not queued)
+        ctx->last_mask_off.off[b] = acc;
         acc += p.hc.mask_bin[b];
     }
-    CU(launch_mask_scatter(p.lc, ctx->m, ctx->M, prod, mo, d_ctr, ctx->mask_q.as<int>(), ctx->rc.as<int>(),
+    CU(launch_mask_scatter(p.lc, ctx->m, ctx->M, prod, ctx->last_mask_off, d_ctr, ctx->mask_q.as<int>(), ctx->rc.as<int>(),
                            ctx->ct_off.as<long long>()),
        "masked bin scatter");
     CU(cudaEventRecord(ctx->ev[1], s), "event");
-    int rc = run_mask_bins(ctx, p.lc, ctx->last_mask_bin);
+    int rc = run_mask_bins(ctx, p.lc);
     if (rc) return rc;
     CU(cudaEventRecord(ctx->ev[2], s), "event");
     // every row with a kernel has ct_off >= 0: with all bins marked direct, the scan and the bin scatter put it in NB_COPY
-    const unsigned all = ~0u;
-    CU(launch_scan(p.lc, ctx->m, ctx->A.rowptr, prod, ctx->rc.as<int>(), ctx->rspan.as<int>(), all, ctx->ct_off.as<long long>(),
-                   ctx->rowoff64.as<int64_t>(), ctx->rowptr32.as<int>(), ctx->blocksums.as<long long>(), d_ctr),
-       "row pointer scan");
-    if ((rc = read_counters(ctx, "masked product / scan"))) return rc;
-    p.hc = *ctx->h_ctr;
-    const Counters &hc = p.hc;
-    ctx->nnzC = (int64_t)hc.nnzC;
-    st.nnzC = ctx->nnzC;
-    for (int b = 0; b < BHB200_NUM_NUM_BINS && b < MAX_BINS; ++b) {
-        st.num_bin_rows[b] = hc.num_bin[b];
-        st.num_bin_products[b] = (int64_t)hc.num_bin_products[b];
-        st.num_bin_nnzC[b] = (int64_t)hc.num_bin_nnzc[b];
-        st.num_bin_nnzA[b] = (int64_t)hc.num_bin_nnza[b];
-    }
-    if ((rc = reserve_C(ctx))) return rc;
-    offsets_from_counts(hc.num_bin, p.no);
-    CU(launch_bin_scatter(p.lc, true, ctx->m, prod, ctx->rc.as<int>(), ctx->rspan.as<int>(), all, ctx->ct_off.as<long long>(), p.no,
-                          d_ctr, ctx->queue.as<int>()),
-       "numeric bin scatter");
-    CU(cudaEventRecord(ctx->ev[3], s), "event");
-    ctx->last_copy_rows = hc.num_bin[NB_COPY];
-    ctx->last_copy_off = p.no.off[NB_COPY];
-    ctx->last_copy_avg = hc.num_bin[NB_COPY] > 0 ? (double)hc.num_bin_nnzc[NB_COPY] / (double)hc.num_bin[NB_COPY] : 0.0;
-    if ((rc = run_mask_copy(ctx, p.lc))) return rc;
+    if ((rc = scan_and_bin(ctx, p, ~0u, "masked product / scan"))) return rc;
+    if ((rc = run_copy_bin(ctx, p.lc))) return rc;
     CU(cudaEventRecord(ctx->ev[4], s), "event");
     ctx->last_masked = true;
     return BHB200_SUCCESS;
@@ -1305,10 +1260,10 @@ int bhb200_spgemm_numeric(bhb200_ctx *ctx)
     CU(cudaEventRecord(ctx->ev[1], s), "event");
     if (ctx->last_masked) {
         // masked product: the masked kernels on the cached bin queues, then the copy of the cached copy bin
-        if ((rc = run_mask_bins(ctx, lc, ctx->last_mask_bin))) return rc;
+        if ((rc = run_mask_bins(ctx, lc))) return rc;
         CU(cudaEventRecord(ctx->ev[2], s), "event");
         CU(cudaEventRecord(ctx->ev[3], s), "event");
-        if ((rc = run_mask_copy(ctx, lc))) return rc;
+        if ((rc = run_copy_bin(ctx, lc))) return rc;
         CU(cudaEventRecord(ctx->ev[4], s), "event");
         st.kernel_launches = ctx->launches;
         ctx->timing_valid = true;

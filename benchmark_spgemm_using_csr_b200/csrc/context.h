@@ -140,6 +140,8 @@ struct bhb200_ctx {
     bhb::DevBuf mask_rowptr, mask_col, mask_q, mask_acc, mask_hit;
     bool last_masked = false;
     int last_mask_bin[bhb::MB_COUNT] = {0};
+    bhb::BinOffsets last_mask_off{};   // where each masked bin's queue starts in mask_q
+    // copy bin (NB_COPY) of the last scan: rows, their place in `queue`, staged entries per row
     int last_copy_rows = 0, last_copy_off = 0;
     double last_copy_avg = 0.0;
     bhb::DevBuf colC, valC;

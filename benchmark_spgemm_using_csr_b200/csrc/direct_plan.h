@@ -31,9 +31,9 @@ enum class DirectMode {
 };
 
 enum class DirectKernel {
-    DIRECT,     // k_num_direct / k_num_block (launch_num_direct_*)
-    BUCKET,     // k_num_bucket3 (launch_num_bucket_*); in a heavy bin staged by atomic bump
-    BUCKET3W,   // k_num_bucket3w (launch_num_bucket3w_*)
+    DIRECT,     // k_num_direct / k_num_block (NumericKernels::direct)
+    BUCKET,     // k_num_bucket3 (NumericKernels::bucket); in a heavy bin staged by atomic bump
+    BUCKET3W,   // k_num_bucket3w (NumericKernels::bucket3w)
     HEAVY,      // k_num_bucket_heavy2, then k_num_bucket_heavy on the rows it could not slice
 };
 

@@ -24,12 +24,7 @@
 namespace bhb {
 
 constexpr int CDF_BITS = 12;
-constexpr int CDF_KNOTS = 1 << CDF_BITS;   // cdf[0 .. CDF_KNOTS], cdf[i] = F(i << shift) scaled to 2^32
-
-struct ColumnCdf {
-    const unsigned *cdf;   // [CDF_KNOTS + 1], non-decreasing, cdf[0] = 0
-    int shift;             // column >> shift < CDF_KNOTS
-};
+constexpr int CDF_KNOTS = 1 << CDF_BITS;   // cdf[0 .. CDF_KNOTS], cdf[i] = F(i << shift) scaled to 2^32 (ColumnCdf)
 
 // exclusive scan of a[0..n) in place by the whole CTA; returns the total.  scratch: 33 ints.
 template <int THREADS>

@@ -519,8 +519,8 @@ cudaError_t launch_mask_bin(const LaunchCtx &lc, int dtype, int bin, const int *
                             const int4 *brange, MaskCsr M, MaskOut o)
 {
     if (count <= 0) return cudaSuccess;
-    return dtype == 1 ? launch_mask_bin_t<double>(lc, bin, queue, count, A, B, brange, M, o)
-                      : launch_mask_bin_t<float>(lc, bin, queue, count, A, B, brange, M, o);
+    return dtype == BHB200_DTYPE_F64 ? launch_mask_bin_t<double>(lc, bin, queue, count, A, B, brange, M, o)
+                                     : launch_mask_bin_t<float>(lc, bin, queue, count, A, B, brange, M, o);
 }
 
 }  // namespace bhb

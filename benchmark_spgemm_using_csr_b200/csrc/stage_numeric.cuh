@@ -593,7 +593,7 @@ k_num_large(const int *__restrict__ queue, const int count, const int *__restric
 // ---- launchers ---------------------------------------------------------------
 template <typename VT, int G, int LOG2T, int R>
 static cudaError_t launch_num_group_t(const LaunchCtx &lc, const int *queue, int count, Csr A, Csr B,
-                                      const int64_t *rowoff, int *colC, VT *valC)
+                                      const int64_t *rowoff, int *colC, void *valC)
 {
     constexpr int T = 1 << LOG2T;
     constexpr int N = (R > 0) ? G * R : T / 2;
@@ -616,13 +616,13 @@ static cudaError_t launch_num_group_t(const LaunchCtx &lc, const int *queue, int
     if (blocks > cap) blocks = cap;
     ++*lc.launches;
     k_num_group<VT, G, LOG2T, R><<<(int)blocks, threads, smem, lc.stream>>>(
-        queue, count, A.rowptr, A.col, (const VT *)A.val, B.rowptr, B.col, (const VT *)B.val, rowoff, colC, valC);
+        queue, count, A.rowptr, A.col, (const VT *)A.val, B.rowptr, B.col, (const VT *)B.val, rowoff, colC, (VT *)valC);
     return cudaGetLastError();
 }
 
 template <typename VT, int LOG2T, int THREADS = 512>
 static cudaError_t launch_num_block_t(const LaunchCtx &lc, const int *queue, int count, Csr A, Csr B,
-                                      const int64_t *rowoff, int *colC, VT *valC)
+                                      const int64_t *rowoff, int *colC, void *valC)
 {
     constexpr int T = 1 << LOG2T;
     const size_t smem = (size_t)T * sizeof(VT) + (size_t)T * 4 + (size_t)(T / 2) * 4;
@@ -636,13 +636,13 @@ static cudaError_t launch_num_block_t(const LaunchCtx &lc, const int *queue, int
     if (blocks > cap) blocks = cap;
     ++*lc.launches;
     k_num_block<VT, LOG2T, THREADS><<<(int)blocks, THREADS, smem, lc.stream>>>(
-        queue, count, A.rowptr, A.col, (const VT *)A.val, B.rowptr, B.col, (const VT *)B.val, rowoff, colC, valC);
+        queue, count, A.rowptr, A.col, (const VT *)A.val, B.rowptr, B.col, (const VT *)B.val, rowoff, colC, (VT *)valC);
     return cudaGetLastError();
 }
 
 template <typename VT>
 static cudaError_t launch_num_hash_t(const LaunchCtx &lc, int bin, int G, const int *queue, int count, Csr A, Csr B,
-                                     const int64_t *rowoff, int *colC, VT *valC)
+                                     const int64_t *rowoff, int *colC, void *valC)
 {
     if (count <= 0) return cudaSuccess;
     // register-sort widths: G=32 -> R = N/32; G=8 -> R = N/8 while <= 16, else shared-memory sort
@@ -673,7 +673,7 @@ static cudaError_t launch_num_hash_t(const LaunchCtx &lc, int bin, int G, const 
 
 template <typename VT>
 static cudaError_t launch_num_large_t(const LaunchCtx &lc, const int *queue, int count, int n, Csr A, Csr B,
-                                      const int64_t *rowoff, int *colC, VT *valC, unsigned *bitmap_scratch,
+                                      const int64_t *rowoff, int *colC, void *valC, unsigned *bitmap_scratch,
                                       int *prefix_scratch, int scratch_blocks)
 {
     if (count <= 0) return cudaSuccess;
@@ -681,7 +681,7 @@ static cudaError_t launch_num_large_t(const LaunchCtx &lc, const int *queue, int
     const int blocks = count < scratch_blocks ? count : scratch_blocks;
     ++*lc.launches;
     k_num_large<VT><<<blocks, 1024, 0, lc.stream>>>(queue, count, A.rowptr, A.col, (const VT *)A.val, B.rowptr, B.col,
-                                                    (const VT *)B.val, rowoff, colC, valC, bitmap_scratch,
+                                                    (const VT *)B.val, rowoff, colC, (VT *)valC, bitmap_scratch,
                                                     prefix_scratch, nwords);
     return cudaGetLastError();
 }
@@ -910,7 +910,7 @@ static cudaError_t launch_num_bucket_heavy2_t(const LaunchCtx &lc, const int *qu
 
 template <typename VT>
 static cudaError_t launch_copy_ct_t(const LaunchCtx &lc, const int *queue, int count, const int64_t *rowoff,
-                                    const long long *ct_off, const int *ctcol, const VT *ctval, int *colC, VT *valC,
+                                    const long long *ct_off, const int *ctcol, const void *ctval, int *colC, void *valC,
                                     double avg_row)
 {
     if (count <= 0) return cudaSuccess;
@@ -920,10 +920,12 @@ static cudaError_t launch_copy_ct_t(const LaunchCtx &lc, const int *queue, int c
     // config 4's copy 1.50 -> 1.52 ms)
     if (avg_row <= 12.0) {
         const long long blocks = ((long long)count * 8 + threads - 1) / threads;
-        k_copy_ct<VT, 8><<<(int)blocks, threads, 0, lc.stream>>>(queue, count, rowoff, ct_off, ctcol, ctval, colC, valC);
+        k_copy_ct<VT, 8><<<(int)blocks, threads, 0, lc.stream>>>(queue, count, rowoff, ct_off, ctcol, (const VT *)ctval,
+                                                                 colC, (VT *)valC);
     } else {
         const long long blocks = ((long long)count * 32 + threads - 1) / threads;
-        k_copy_ct<VT, 32><<<(int)blocks, threads, 0, lc.stream>>>(queue, count, rowoff, ct_off, ctcol, ctval, colC, valC);
+        k_copy_ct<VT, 32><<<(int)blocks, threads, 0, lc.stream>>>(queue, count, rowoff, ct_off, ctcol, (const VT *)ctval,
+                                                                  colC, (VT *)valC);
     }
     return cudaGetLastError();
 }

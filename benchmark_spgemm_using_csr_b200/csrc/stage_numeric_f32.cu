@@ -4,56 +4,10 @@
 
 namespace bhb {
 
-cudaError_t launch_num_hash_f32(const LaunchCtx &lc, int bin, int G, const int *queue, int count, Csr A, Csr B,
-                                const int64_t *rowoff, int *colC, float *valC)
-{
-    return launch_num_hash_t<float>(lc, bin, G, queue, count, A, B, rowoff, colC, valC);
-}
-
-cudaError_t launch_num_large_f32(const LaunchCtx &lc, const int *queue, int count, int n, Csr A, Csr B,
-                                 const int64_t *rowoff, int *colC, float *valC, unsigned *bitmap_scratch,
-                                 int *prefix_scratch, int scratch_blocks)
-{
-    return launch_num_large_t<float>(lc, queue, count, n, A, B, rowoff, colC, valC, bitmap_scratch, prefix_scratch,
-                                   scratch_blocks);
-}
-
-cudaError_t launch_num_range_f32(const LaunchCtx &lc, int nsum, int nacc, const int *queue, int count, Csr A, Csr B,
-                                 const int *rlo, const int64_t *rowoff, int *colC, float *valC, WordLists wl)
-{
-    if (nacc <= 128 && range_vec_aligned(B))
-        return launch_num_range_vec_t<float>(lc, nsum, nacc, queue, count, A, B, rlo, rowoff, colC, valC, wl);
-    return launch_num_range_t<float>(lc, nsum, nacc, queue, count, A, B, rlo, rowoff, colC, valC, wl);
-}
-
-cudaError_t launch_num_direct_f32(const LaunchCtx &lc, int cap, int G, const int *queue, int count, Csr A, Csr B,
-                                  DirectOut d)
-{
-    return launch_num_direct_t<float>(lc, cap, G, queue, count, A, B, d);
-}
-
-cudaError_t launch_num_bucket_f32(const LaunchCtx &lc, int cap, const int *queue, int count, Csr A, Csr B, DirectOut d,
-                                  const unsigned *cdf, int cdf_shift)
-{
-    return launch_num_bucket_t<float>(lc, cap, queue, count, A, B, d, ColumnCdf{cdf, cdf_shift});
-}
-
-cudaError_t launch_num_bucket_heavy_f32(const LaunchCtx &lc, const int *queue, int count, Csr A, Csr B, DirectOut d,
-                                        const unsigned *cdf, int cdf_shift, unsigned long long *cursor)
-{
-    return launch_num_bucket_heavy_t<float>(lc, queue, count, A, B, d, ColumnCdf{cdf, cdf_shift}, cursor);
-}
-
-cudaError_t launch_num_bucket_heavy2_f32(const LaunchCtx &lc, const int *queue, int count, Csr A, Csr B, DirectOut d,
-                                         const unsigned *cdf, int cdf_shift, unsigned long long *cursor)
-{
-    return launch_num_bucket_heavy2_t<float>(lc, queue, count, A, B, d, ColumnCdf{cdf, cdf_shift}, cursor);
-}
-
-cudaError_t launch_num_bucket3w_f32(const LaunchCtx &lc, int capw, int sg, const int *queue, int count, Csr A, Csr B, DirectOut d,
-                                     const unsigned *cdf, int cdf_shift, int stride)
-{
-    return launch_num_bucket3w_t<float>(lc, capw, sg, queue, count, A, B, d, ColumnCdf{cdf, cdf_shift}, stride);
-}
+const NumericKernels NUMERIC_F32{&launch_num_hash_t<float>,        &launch_num_large_t<float>,
+                                 &launch_num_range_pick_t<float>,  &launch_num_direct_t<float>,
+                                 &launch_num_bucket_t<float>,      &launch_num_bucket3w_t<float>,
+                                 &launch_num_bucket_heavy_t<float>, &launch_num_bucket_heavy2_t<float>,
+                                 &launch_copy_ct_t<float>};
 
 }  // namespace bhb

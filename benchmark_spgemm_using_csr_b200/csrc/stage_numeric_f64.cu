@@ -4,66 +4,10 @@
 
 namespace bhb {
 
-cudaError_t launch_num_hash_f64(const LaunchCtx &lc, int bin, int G, const int *queue, int count, Csr A, Csr B,
-                                const int64_t *rowoff, int *colC, double *valC)
-{
-    return launch_num_hash_t<double>(lc, bin, G, queue, count, A, B, rowoff, colC, valC);
-}
-
-cudaError_t launch_num_large_f64(const LaunchCtx &lc, const int *queue, int count, int n, Csr A, Csr B,
-                                 const int64_t *rowoff, int *colC, double *valC, unsigned *bitmap_scratch,
-                                 int *prefix_scratch, int scratch_blocks)
-{
-    return launch_num_large_t<double>(lc, queue, count, n, A, B, rowoff, colC, valC, bitmap_scratch, prefix_scratch,
-                                   scratch_blocks);
-}
-
-cudaError_t launch_num_range_f64(const LaunchCtx &lc, int nsum, int nacc, const int *queue, int count, Csr A, Csr B,
-                                 const int *rlo, const int64_t *rowoff, int *colC, double *valC, WordLists wl)
-{
-    if (nacc <= 128 && range_vec_aligned(B))
-        return launch_num_range_vec_t<double>(lc, nsum, nacc, queue, count, A, B, rlo, rowoff, colC, valC, wl);
-    return launch_num_range_t<double>(lc, nsum, nacc, queue, count, A, B, rlo, rowoff, colC, valC, wl);
-}
-
-cudaError_t launch_num_direct_f64(const LaunchCtx &lc, int cap, int G, const int *queue, int count, Csr A, Csr B,
-                                  DirectOut d)
-{
-    return launch_num_direct_t<double>(lc, cap, G, queue, count, A, B, d);
-}
-
-cudaError_t launch_copy_ct(const LaunchCtx &lc, int dtype, const int *queue, int count, const int64_t *rowoff,
-                           const long long *ct_off, const int *ctcol, const void *ctval, int *colC, void *valC, double avg_row)
-{
-    // avg_row = staged entries per row of the launch: short rows are copied 32 rows per warp
-    return dtype ? launch_copy_ct_t<double>(lc, queue, count, rowoff, ct_off, ctcol, (const double *)ctval, colC,
-                                            (double *)valC, avg_row)
-                 : launch_copy_ct_t<float>(lc, queue, count, rowoff, ct_off, ctcol, (const float *)ctval, colC,
-                                           (float *)valC, avg_row);
-}
-
-cudaError_t launch_num_bucket_f64(const LaunchCtx &lc, int cap, const int *queue, int count, Csr A, Csr B, DirectOut d,
-                                  const unsigned *cdf, int cdf_shift)
-{
-    return launch_num_bucket_t<double>(lc, cap, queue, count, A, B, d, ColumnCdf{cdf, cdf_shift});
-}
-
-cudaError_t launch_num_bucket_heavy_f64(const LaunchCtx &lc, const int *queue, int count, Csr A, Csr B, DirectOut d,
-                                        const unsigned *cdf, int cdf_shift, unsigned long long *cursor)
-{
-    return launch_num_bucket_heavy_t<double>(lc, queue, count, A, B, d, ColumnCdf{cdf, cdf_shift}, cursor);
-}
-
-cudaError_t launch_num_bucket_heavy2_f64(const LaunchCtx &lc, const int *queue, int count, Csr A, Csr B, DirectOut d,
-                                         const unsigned *cdf, int cdf_shift, unsigned long long *cursor)
-{
-    return launch_num_bucket_heavy2_t<double>(lc, queue, count, A, B, d, ColumnCdf{cdf, cdf_shift}, cursor);
-}
-
-cudaError_t launch_num_bucket3w_f64(const LaunchCtx &lc, int capw, int sg, const int *queue, int count, Csr A, Csr B, DirectOut d,
-                                     const unsigned *cdf, int cdf_shift, int stride)
-{
-    return launch_num_bucket3w_t<double>(lc, capw, sg, queue, count, A, B, d, ColumnCdf{cdf, cdf_shift}, stride);
-}
+const NumericKernels NUMERIC_F64{&launch_num_hash_t<double>,        &launch_num_large_t<double>,
+                                 &launch_num_range_pick_t<double>,  &launch_num_direct_t<double>,
+                                 &launch_num_bucket_t<double>,      &launch_num_bucket3w_t<double>,
+                                 &launch_num_bucket_heavy_t<double>, &launch_num_bucket_heavy2_t<double>,
+                                 &launch_copy_ct_t<double>};
 
 }  // namespace bhb

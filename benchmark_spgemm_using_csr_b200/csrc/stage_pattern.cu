@@ -742,7 +742,7 @@ cudaError_t launch_pat_numeric(const LaunchCtx &lc, int dtype, int m, Csr A, Csr
 {
     if (m <= 0) return cudaSuccess;
     const int G = t.nDB <= 8 ? 8 : t.nDB <= 16 ? 16 : 32;
-    if (dtype == 1) {   // BHB200_DTYPE_F64
+    if (dtype == BHB200_DTYPE_F64) {
         double *v = (double *)valC;
         if (G == 8) return launch_pat_numeric_t<double, 8>(lc, m, A, B, ta, tb, t, outmask, rowoff, colC, v);
         if (G == 16) return launch_pat_numeric_t<double, 16>(lc, m, A, B, ta, tb, t, outmask, rowoff, colC, v);

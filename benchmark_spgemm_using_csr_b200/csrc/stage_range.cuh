@@ -290,7 +290,7 @@ inline void range_launch_shape(size_t warp_bytes, int &wpb, int &blocks_per_sm)
 
 template <typename VT>
 static cudaError_t launch_num_range_t(const LaunchCtx &lc, int nsum, int nacc, const int *queue, int count, Csr A,
-                                      Csr B, const int *rlo, const int64_t *rowoff, int *colC, VT *valC, WordLists wl)
+                                      Csr B, const int *rlo, const int64_t *rowoff, int *colC, void *valC, WordLists wl)
 {
     if (count <= 0) return cudaSuccess;
     const size_t wb = num_range_warp_bytes(nsum, nacc, sizeof(VT));
@@ -306,7 +306,7 @@ static cudaError_t launch_num_range_t(const LaunchCtx &lc, int nsum, int nacc, c
     ++*lc.launches;
     k_num_range<VT><<<(int)blocks, wpb * 32, smem, lc.stream>>>(queue, count, A.rowptr, A.col, (const VT *)A.val,
                                                                 B.rowptr, B.col, (const VT *)B.val, rlo, nsum, nacc,
-                                                                rowoff, colC, valC, wl);
+                                                                rowoff, colC, (VT *)valC, wl);
     return cudaGetLastError();
 }
 

@@ -262,7 +262,7 @@ k_num_range_vec(const int *__restrict__ queue, const int count, const int *__res
 
 template <typename VT>
 static cudaError_t launch_num_range_vec_t(const LaunchCtx &lc, int nsum, int nacc, const int *queue, int count, Csr A,
-                                          Csr B, const int *rlo, const int64_t *rowoff, int *colC, VT *valC,
+                                          Csr B, const int *rlo, const int64_t *rowoff, int *colC, void *valC,
                                           WordLists wl)
 {
     if (count <= 0) return cudaSuccess;
@@ -279,13 +279,24 @@ static cudaError_t launch_num_range_vec_t(const LaunchCtx &lc, int nsum, int nac
     ++*lc.launches;
     k_num_range_vec<VT><<<(int)blocks, wpb * 32, smem, lc.stream>>>(queue, count, A.rowptr, A.col, (const VT *)A.val,
                                                                     B.rowptr, B.col, (const VT *)B.val, rlo, nsum, nacc,
-                                                                    rowoff, colC, valC, wl);
+                                                                    rowoff, colC, (VT *)valC, wl);
     return cudaGetLastError();
 }
 
 inline bool range_vec_aligned(const Csr &B)
 {
     return (((uintptr_t)B.col | (uintptr_t)B.val) & 15u) == 0;
+}
+
+// numeric range bins: the vectorised kernel for rows of at most 128 outputs when B is 16-byte aligned
+template <typename VT>
+static cudaError_t launch_num_range_pick_t(const LaunchCtx &lc, int nsum, int nacc, const int *queue, int count, Csr A,
+                                           Csr B, const int *rlo, const int64_t *rowoff, int *colC, void *valC,
+                                           WordLists wl)
+{
+    if (nacc <= 128 && range_vec_aligned(B))
+        return launch_num_range_vec_t<VT>(lc, nsum, nacc, queue, count, A, B, rlo, rowoff, colC, valC, wl);
+    return launch_num_range_t<VT>(lc, nsum, nacc, queue, count, A, B, rlo, rowoff, colC, valC, wl);
 }
 
 }  // namespace bhb

@@ -15,7 +15,6 @@
 // lower bound per column in the sorted keys (k_tr_rowptr).  A column outside [0, cols) is replaced by
 // 0 (so every array written stays in bounds) and raises `bad_bit` in *bad.
 #include "common.cuh"
-#include "../../include/bhsparse_b200.h"
 
 #include <algorithm>
 
