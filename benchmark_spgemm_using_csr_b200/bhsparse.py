@@ -12,7 +12,9 @@ tests read like the reference driver (main.cu:104-135).
 
 Host arrays are numpy (or anything exposing a writable buffer of the right
 dtype); the value dtype (float32/float64) is taken from valA -- the reference
-needs a recompile for that (common.h:31, README.md:84-86).
+needs a recompile for that (common.h:31, README.md:84-86).  With valA and valB both
+None the product is structure-only (BHB200_DTYPE_NONE): C has row pointers and
+columns, and get_C takes None for the values.
 """
 from __future__ import annotations
 
@@ -39,6 +41,7 @@ class bhsparse:
         self._verbose = verbose
         self._rowptrC = None
         self._dtype = None
+        self._structure = False   # structure-only operands (no values)
         self._m = 0
 
     # -- platform (bhsparse.h:96-148) ---------------------------------------
@@ -66,17 +69,24 @@ class bhsparse:
     def initData(self, m, k, n, nnzA, csrValA, csrRowPtrA, csrColIndA,
                  nnzB, csrValB, csrRowPtrB, csrColIndB, csrRowPtrC, transA=False, transB=False) -> int:
         """C = op(A)*op(B): m, k, n are the dimensions of op(A) (m x k) and op(B) (k x n); with
-        transA / transB the arrays hold A / B as stored, i.e. k x m / n x k (bhb200_init_data_op_*)."""
+        transA / transB the arrays hold A / B as stored, i.e. k x m / n x k (bhb200_init_data_op_*).
+        csrValA and csrValB both None: structure-only product (bhb200_init_data_structure)."""
         if not self._ctx:
             return capi.ERR_INVALID
-        valA = np.ascontiguousarray(csrValA)
-        if valA.dtype == np.float64:
-            fn, dt = self._lib.bhb200_init_data_op_f64, np.float64
-        elif valA.dtype == np.float32:
-            fn, dt = self._lib.bhb200_init_data_op_f32, np.float32
-        else:
+        structure = csrValA is None and csrValB is None
+        if structure:
+            dt = None
+        elif csrValA is None or csrValB is None:
             return capi.ERR_INVALID
-        valB = np.ascontiguousarray(csrValB, dtype=dt)
+        else:
+            valA = np.ascontiguousarray(csrValA)
+            if valA.dtype == np.float64:
+                fn, dt = self._lib.bhb200_init_data_op_f64, np.float64
+            elif valA.dtype == np.float32:
+                fn, dt = self._lib.bhb200_init_data_op_f32, np.float32
+            else:
+                return capi.ERR_INVALID
+            valB = np.ascontiguousarray(csrValB, dtype=dt)
         rpA = np.ascontiguousarray(csrRowPtrA, dtype=np.int32)
         cA = np.ascontiguousarray(csrColIndA, dtype=np.int32)
         rpB = np.ascontiguousarray(csrRowPtrB, dtype=np.int32)
@@ -89,10 +99,14 @@ class bhsparse:
             return capi.ERR_INVALID
         self._rowptrC = csrRowPtrC           # caller-owned, written by get_C (main.cu:100)
         self._dtype = dt
+        self._structure = structure
         self._m = m
         # (the same host arrays for A and B stay the same objects here, so the library can upload them once)
         opA = capi.OP_T if transA else capi.OP_N
         opB = capi.OP_T if transB else capi.OP_N
+        if structure:
+            return self._lib.bhb200_init_data_structure(self._ctx, opA, opB, m, k, n, nnzA, _ptr(rpA), _ptr(cA), nnzB,
+                                                        _ptr(rpB), _ptr(cB))
         return fn(self._ctx, opA, opB, m, k, n, nnzA, _ptr(valA), _ptr(rpA), _ptr(cA), nnzB, _ptr(valB), _ptr(rpB), _ptr(cB))
 
     def aliased_operands(self) -> bool:
@@ -109,8 +123,7 @@ class bhsparse:
         err = self._lib.bhb200_spgemm(self._ctx)
         # create_C leaves rowptrC in the caller's array at the end of spgemm() (bhsparse_cuda.h:2787-2808)
         if err == BHSPARSE_SUCCESS and self._rowptrC is not None and 0 <= self.get_nnzC() <= 0x7fffffff:
-            fn = self._lib.bhb200_get_C_f64 if self._dtype == np.float64 else self._lib.bhb200_get_C_f32
-            err = fn(self._ctx, ctypes.c_void_p(self._rowptrC.ctypes.data), None, None)
+            err = self._lib.bhb200_get_C_structure(self._ctx, ctypes.c_void_p(self._rowptrC.ctypes.data), None)
         if err == BHSPARSE_SUCCESS and self._verbose:
             st = self.stats()
             t = st["ms_total"]
@@ -124,17 +137,19 @@ class bhsparse:
         return int(self._lib.bhb200_get_nnzC(self._ctx)) if self._ctx else -1
 
     def get_C(self, csrColIndC, csrValC) -> int:
+        """Columns (and values) of C; csrValC None skips the values, and must be None for a structure-only product."""
         if not self._ctx:
             return capi.ERR_INVALID
-        if csrValC is not None and csrValC.dtype != self._dtype:
+        if csrValC is not None and (self._structure or csrValC.dtype != self._dtype):
             return capi.ERR_INVALID
         if csrColIndC is not None and csrColIndC.dtype != np.int32:
             return capi.ERR_INVALID
-        fn = self._lib.bhb200_get_C_f64 if self._dtype == np.float64 else self._lib.bhb200_get_C_f32
         rp = ctypes.c_void_p(self._rowptrC.ctypes.data) if self._rowptrC is not None else None
         cp = ctypes.c_void_p(csrColIndC.ctypes.data) if csrColIndC is not None else None
-        vp = ctypes.c_void_p(csrValC.ctypes.data) if csrValC is not None else None
-        return fn(self._ctx, rp, cp, vp)
+        if csrValC is None:
+            return self._lib.bhb200_get_C_structure(self._ctx, rp, cp)
+        fn = self._lib.bhb200_get_C_f64 if self._dtype == np.float64 else self._lib.bhb200_get_C_f32
+        return fn(self._ctx, rp, cp, ctypes.c_void_p(csrValC.ctypes.data))
 
     def free_mem(self) -> int:
         return self._lib.bhb200_free_mem(self._ctx) if self._ctx else BHSPARSE_SUCCESS
@@ -176,11 +191,13 @@ class bhsparse:
         return out
 
     def get_C_range(self, first: int, count: int):
-        """Entries [first, first+count) of (colC, valC): piecewise access for results beyond INT32_MAX."""
+        """Entries [first, first+count) of (colC, valC): piecewise access for results beyond INT32_MAX.
+        valC is None for a structure-only product."""
         col = np.empty(max(count, 0), dtype=np.int32)
-        val = np.empty(max(count, 0), dtype=self._dtype)
+        val = None if self._structure else np.empty(max(count, 0), dtype=self._dtype)
         capi.check(self._lib, self._ctx, self._lib.bhb200_get_C_range(
-            self._ctx, int(first), int(count), ctypes.c_void_p(col.ctypes.data), ctypes.c_void_p(val.ctypes.data)))
+            self._ctx, int(first), int(count), ctypes.c_void_p(col.ctypes.data),
+            ctypes.c_void_p(val.ctypes.data) if val is not None else None))
         return col, val
 
     def get_row_products(self) -> np.ndarray:
@@ -205,11 +222,12 @@ class bhsparse:
 
 
 def spgemm(A, B, device: int = 0, return_stats: bool = False, return_row_products: bool = False,
-           transA: bool = False, transB: bool = False, mask=None):
+           transA: bool = False, transB: bool = False, mask=None, structure_only: bool = False):
     """Convenience driver following main.cu:104-135: C = op(A)*op(B) for two
     generators.CSR operands (op = transpose with transA / transB); returns
     (rowptrC int32, colC int32, valC).  mask: a generators.CSR or (rowptr, col)
-    whose pattern restricts C (masked product, bhb200_set_mask)."""
+    whose pattern restricts C (masked product, bhb200_set_mask).  structure_only:
+    the pattern of C alone, from the operands' patterns (valC is None)."""
     platforms = [False] * NUM_PLATFORMS
     platforms[BHSPARSE_CUDA] = True
     bh = bhsparse(device)
@@ -224,15 +242,15 @@ def spgemm(A, B, device: int = 0, return_stats: bool = False, return_row_product
             raise capi.BhsparseError(err, f"{what}: {msg}")
 
     ok(bh.initPlatform(platforms), "initPlatform")
-    ok(bh.initData(m, k, n, A.nnz, A.val, A.rowptr, A.col,
-                   B.nnz, B.val, B.rowptr, B.col, rowptrC, transA, transB), "initData")
+    ok(bh.initData(m, k, n, A.nnz, None if structure_only else A.val, A.rowptr, A.col,
+                   B.nnz, None if structure_only else B.val, B.rowptr, B.col, rowptrC, transA, transB), "initData")
     if mask is not None:
         rpM, colM = (mask.rowptr, mask.col) if hasattr(mask, "rowptr") else mask
         ok(bh.set_mask(rpM, colM), "set_mask")
     ok(bh.spgemm(), "spgemm")
     nnzC = bh.get_nnzC()
     colC = np.empty(max(nnzC, 0), dtype=np.int32)
-    valC = np.empty(max(nnzC, 0), dtype=A.val.dtype)
+    valC = None if structure_only else np.empty(max(nnzC, 0), dtype=A.val.dtype)
     ok(bh.get_C(colC, valC), "get_C")
     st = bh.stats() if return_stats else None
     prods = bh.get_row_products() if return_row_products else None

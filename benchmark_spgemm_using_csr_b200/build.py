@@ -33,6 +33,7 @@ SOURCES = [
     "stage_bucket.cu",
     "stage_numeric_f32.cu",
     "stage_numeric_f64.cu",
+    "stage_numeric_none.cu",
     "stage_transpose.cu",
     "stage_masked.cu",
 ]

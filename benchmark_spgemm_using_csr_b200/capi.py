@@ -21,6 +21,7 @@ ERR_ALLOC = -4
 ERR_NO_DEVICE = -5
 DTYPE_F32 = 0
 DTYPE_F64 = 1
+DTYPE_NONE = 2   # structure only: row pointers and columns, no values
 OP_N = 0
 OP_T = 1
 NUM_BINS = 24
@@ -45,6 +46,7 @@ EXPORTED = [
     "bhb200_dist_broadcast_ms", "bhb200_dist_finalize", "bhb200_pattern_plan_probe",
     "bhb200_init_data_op_f64", "bhb200_init_data_op_f32", "bhb200_init_data_device_op",
     "bhb200_set_mask", "bhb200_set_mask_device", "bhb200_clear_mask",
+    "bhb200_init_data_structure", "bhb200_get_C_structure",
 ]
 DIST_ID_BYTES = 128
 
@@ -119,6 +121,9 @@ def load(build_if_missing: bool = False):
     L.bhb200_init_data_op_f64.argtypes = [ctxp, c_int, c_int] + L.bhb200_init_data_f64.argtypes[1:]
     L.bhb200_init_data_op_f32.argtypes = L.bhb200_init_data_op_f64.argtypes
     L.bhb200_init_data_device_op.argtypes = [ctxp, c_int, c_int, c_int] + L.bhb200_init_data_device.argtypes[2:]
+    L.bhb200_init_data_structure.argtypes = [ctxp, c_int, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_int,
+                                             c_void_p, c_void_p]
+    L.bhb200_get_C_structure.argtypes = [ctxp, c_void_p, c_void_p]
     L.bhb200_operands_aliased.argtypes = [ctxp]
     L.bhb200_get_operands_device.argtypes = [ctxp, POINTER(c_int32)] + [POINTER(c_void_p)] * 6
     L.bhb200_set_mask.argtypes = [ctxp, c_int, c_void_p, c_void_p]

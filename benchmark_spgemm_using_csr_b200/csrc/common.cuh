@@ -21,6 +21,36 @@ constexpr int EMPTY_KEY = -1;
 constexpr int SORT_PAD = 0x7fffffff;
 constexpr unsigned FULL = 0xffffffffu;
 
+// ---- value types -------------------------------------------------------------
+// The numeric kernels are templates on the value type VT (float, double).  Structure-only
+// products (BHB200_DTYPE_NONE) instantiate them with NoVal: an empty type whose arithmetic,
+// shuffles, loads and atomics do nothing, so every value load, store and shared-memory access
+// compiles away and only the column work is left.  Shared-memory layouts are sized with
+// value_bytes<VT> (0 for NoVal, not sizeof = 1) and step over value arrays with vslots<VT>.
+namespace novalue {   // (its own namespace: the overloads below would hide CUDA's for int and float inside bhb)
+struct NoVal {
+    __host__ __device__ constexpr NoVal() {}
+    __host__ __device__ constexpr explicit NoVal(int) {}
+    __host__ __device__ constexpr NoVal operator*(NoVal) const { return NoVal(); }
+    __host__ __device__ constexpr NoVal operator+(NoVal) const { return NoVal(); }
+    __host__ __device__ NoVal &operator+=(NoVal) { return *this; }
+};
+// found by argument-dependent lookup from the kernel templates
+__device__ __forceinline__ NoVal __shfl_sync(unsigned, NoVal, int, int = 32) { return NoVal(); }
+__device__ __forceinline__ NoVal __shfl_down_sync(unsigned, NoVal, unsigned, int = 32) { return NoVal(); }
+__device__ __forceinline__ NoVal __ldg(const NoVal *) { return NoVal(); }
+__device__ __forceinline__ NoVal atomicAdd(NoVal *, NoVal) { return NoVal(); }
+}  // namespace novalue
+using novalue::NoVal;
+template <typename VT>
+constexpr size_t value_bytes = sizeof(VT);
+template <>
+constexpr size_t value_bytes<NoVal> = 0;
+
+// elements per value slot when stepping over a value array: p + n * vslots<VT> (NoVal's arrays take no space)
+template <typename VT>
+constexpr int vslots = value_bytes<VT> ? 1 : 0;
+
 // ---- bins ------------------------------------------------------------------
 // Symbolic bins are chosen by p = upper bound of the row (products) and by the row's
 // column span; numeric bins by c = exact nnz(C_i), p and the span.  They play the role
@@ -650,8 +680,9 @@ int large_scratch_blocks(int sm_count, int n);
 cudaError_t launch_sym_range(const LaunchCtx &lc, int nsum, const int *queue, int count, Csr A, Csr B, const int *rlo,
                              int *rc, Counters *ctr, WordLists wl);
 
-// The numeric kernels of one value type (stage_numeric_f32.cu / stage_numeric_f64.cu); values are float or double
-// as the operands are.  The two types compile in two translation units, in parallel.
+// The numeric kernels of one value type (stage_numeric_f32.cu / _f64.cu / _none.cu); values are float or double
+// as the operands are, or none (NoVal: columns only, value pointers never read).  The three types compile in three
+// translation units, in parallel.
 struct ColumnCdf {
     const unsigned *cdf;   // [CDF_KNOTS + 1], non-decreasing, cdf[0] = 0
     int shift;             // column >> shift < CDF_KNOTS
@@ -684,10 +715,10 @@ struct NumericKernels {
     cudaError_t (*copy_ct)(const LaunchCtx &lc, const int *queue, int count, const int64_t *rowoff, const long long *ct_off,
                            const int *ctcol, const void *ctval, int *colC, void *valC, double avg_row);
 };
-extern const NumericKernels NUMERIC_F32, NUMERIC_F64;
+extern const NumericKernels NUMERIC_F32, NUMERIC_F64, NUMERIC_NONE;
 inline const NumericKernels &numeric_kernels(int dtype)
 {
-    return dtype == BHB200_DTYPE_F64 ? NUMERIC_F64 : NUMERIC_F32;
+    return dtype == BHB200_DTYPE_F64 ? NUMERIC_F64 : dtype == BHB200_DTYPE_NONE ? NUMERIC_NONE : NUMERIC_F32;
 }
 
 }  // namespace bhb

@@ -44,7 +44,14 @@ int fail(bhb200_ctx *c, int code, const char *what, cudaError_t e = cudaSuccess)
 
 size_t vsize(int dtype)
 {
-    return dtype == BHB200_DTYPE_F64 ? 8 : 4;
+    return dtype == BHB200_DTYPE_F64 ? 8 : dtype == BHB200_DTYPE_NONE ? 0 : 4;
+}
+
+int refuse_structure(bhb200_ctx *ctx, const char *what)
+{
+    std::string msg = what;
+    msg += ": the operands are structure-only (BHB200_DTYPE_NONE), C has no values";
+    return fail(ctx, BHB200_ERR_INVALID, msg.c_str());
 }
 
 // forget the mask (the library's copy stays allocated for the next bhb200_set_mask)
@@ -83,13 +90,15 @@ void release_operands(bhb200_ctx *ctx)
     drop_mask(ctx);
 }
 
-int check_dims(bhb200_ctx *ctx, int m, int k, int n, int nnzA, int nnzB, const void *valA, const int32_t *rowptrA,
+// (structure-only operands: the values are never read and may be null)
+int check_dims(bhb200_ctx *ctx, int dtype, int m, int k, int n, int nnzA, int nnzB, const void *valA, const int32_t *rowptrA,
                const int32_t *colA, const void *valB, const int32_t *rowptrB, const int32_t *colB)
 {
+    const bool values = dtype != BHB200_DTYPE_NONE;
     if (m < 0 || k < 0 || n < 0 || nnzA < 0 || nnzB < 0) return fail(ctx, BHB200_ERR_INVALID, "negative dimension");
     if (!rowptrA || !rowptrB) return fail(ctx, BHB200_ERR_INVALID, "null row pointer array");
-    if (nnzA > 0 && (!colA || !valA)) return fail(ctx, BHB200_ERR_INVALID, "null A arrays");
-    if (nnzB > 0 && (!colB || !valB)) return fail(ctx, BHB200_ERR_INVALID, "null B arrays");
+    if (nnzA > 0 && (!colA || (values && !valA))) return fail(ctx, BHB200_ERR_INVALID, "null A arrays");
+    if (nnzB > 0 && (!colB || (values && !valB))) return fail(ctx, BHB200_ERR_INVALID, "null B arrays");
     return BHB200_SUCCESS;
 }
 
@@ -100,7 +109,9 @@ int check_ops(bhb200_ctx *ctx, int opA, int opB)
     return BHB200_SUCCESS;
 }
 
-// ctx->A / ctx->B from the stored operands: the transposed copies (reserved here, filled by run_transposes) for op = T
+// ctx->A / ctx->B from the stored operands: the transposed copies (reserved here, filled by run_transposes) for op = T.
+// Structure-only operands have no values to transpose and keep no permutation (nothing is ever re-gathered): the sort
+// still writes one, into the transpose scratch (run_transposes).
 int set_effective(bhb200_ctx *ctx)
 {
     const size_t vs = vsize(ctx->dtype);
@@ -109,18 +120,22 @@ int set_effective(bhb200_ctx *ctx)
     if (ctx->opA) {
         CU(ctx->at_rowptr.reserve(((size_t)ctx->m + 1) * 4, &ctx->dev_bytes), "alloc rowptr of A^T");
         CU(ctx->at_col.reserve((size_t)ctx->nnzA * 4 + 4, &ctx->dev_bytes), "alloc col of A^T");
-        CU(ctx->at_val.reserve((size_t)ctx->nnzA * vs + 16, &ctx->dev_bytes), "alloc val of A^T");
-        CU(ctx->at_perm.reserve((size_t)ctx->nnzA * 4 + 4, &ctx->dev_bytes), "alloc perm of A^T");
-        ctx->A = Csr{ctx->at_rowptr.as<int>(), ctx->at_col.as<int>(), ctx->at_val.p};
+        if (vs) {
+            CU(ctx->at_val.reserve((size_t)ctx->nnzA * vs + 16, &ctx->dev_bytes), "alloc val of A^T");
+            CU(ctx->at_perm.reserve((size_t)ctx->nnzA * 4 + 4, &ctx->dev_bytes), "alloc perm of A^T");
+        }
+        ctx->A = Csr{ctx->at_rowptr.as<int>(), ctx->at_col.as<int>(), vs ? ctx->at_val.p : nullptr};
     }
     if (ctx->opB && ctx->t_shared) {
         ctx->B = ctx->A;
     } else if (ctx->opB) {
         CU(ctx->bt_rowptr.reserve(((size_t)ctx->k + 1) * 4, &ctx->dev_bytes), "alloc rowptr of B^T");
         CU(ctx->bt_col.reserve((size_t)ctx->nnzB * 4 + 4, &ctx->dev_bytes), "alloc col of B^T");
-        CU(ctx->bt_val.reserve((size_t)ctx->nnzB * vs + 16, &ctx->dev_bytes), "alloc val of B^T");
-        CU(ctx->bt_perm.reserve((size_t)ctx->nnzB * 4 + 4, &ctx->dev_bytes), "alloc perm of B^T");
-        ctx->B = Csr{ctx->bt_rowptr.as<int>(), ctx->bt_col.as<int>(), ctx->bt_val.p};
+        if (vs) {
+            CU(ctx->bt_val.reserve((size_t)ctx->nnzB * vs + 16, &ctx->dev_bytes), "alloc val of B^T");
+            CU(ctx->bt_perm.reserve((size_t)ctx->nnzB * 4 + 4, &ctx->dev_bytes), "alloc perm of B^T");
+        }
+        ctx->B = Csr{ctx->bt_rowptr.as<int>(), ctx->bt_col.as<int>(), vs ? ctx->bt_val.p : nullptr};
     }
     ctx->t_pending = ctx->opA || ctx->opB;
     return BHB200_SUCCESS;
@@ -131,20 +146,26 @@ int set_effective(bhb200_ctx *ctx)
 int run_transposes(bhb200_ctx *ctx, const LaunchCtx &lc)
 {
     const bool tb = ctx->opB && !ctx->t_shared;
+    const bool keep_perm = ctx->dtype != BHB200_DTYPE_NONE;
     size_t need = 0;
     if (ctx->opA) need = transpose_scratch_bytes(ctx->nnzA, ctx->m);
     if (tb) need = std::max(need, transpose_scratch_bytes(ctx->nnzB, ctx->k));
+    const size_t perm_at = need;   // structure only: the sort still produces the permutation, into the scratch after the rest
+    if (!keep_perm) need += (size_t)std::max(ctx->opA ? ctx->nnzA : 0, tb ? ctx->nnzB : 0) * 4 + 4;
     if (need) CU(ctx->t_scratch.reserve(need, &ctx->dev_bytes), "alloc transpose scratch");
+    int *scratch_perm = reinterpret_cast<int *>(static_cast<unsigned char *>(ctx->t_scratch.p) + perm_at);
     Counters *d_ctr = ctx->counters.as<Counters>();
     CU(cudaMemsetAsync(&d_ctr->bad_T, 0, sizeof(int), lc.stream), "zero transpose flag");
     if (ctx->opA)
         CU(launch_transpose(lc, ctx->dtype, ctx->k, ctx->m, ctx->nnzA, ctx->As,
-                            TransposeOut{ctx->at_rowptr.as<int>(), ctx->at_col.as<int>(), ctx->at_val.p, ctx->at_perm.as<int>()},
+                            TransposeOut{ctx->at_rowptr.as<int>(), ctx->at_col.as<int>(), keep_perm ? ctx->at_val.p : nullptr,
+                                         keep_perm ? ctx->at_perm.as<int>() : scratch_perm},
                             ctx->t_scratch.p, &d_ctr->bad_T, 1),
            "transpose A");
     if (tb)
         CU(launch_transpose(lc, ctx->dtype, ctx->n, ctx->k, ctx->nnzB, ctx->Bs,
-                            TransposeOut{ctx->bt_rowptr.as<int>(), ctx->bt_col.as<int>(), ctx->bt_val.p, ctx->bt_perm.as<int>()},
+                            TransposeOut{ctx->bt_rowptr.as<int>(), ctx->bt_col.as<int>(), keep_perm ? ctx->bt_val.p : nullptr,
+                                         keep_perm ? ctx->bt_perm.as<int>() : scratch_perm},
                             ctx->t_scratch.p, &d_ctr->bad_T, 2),
            "transpose B");
     ctx->t_pending = false;
@@ -176,7 +197,7 @@ int init_host(bhb200_ctx *ctx, int dtype, int opA, int opB, int m, int k, int n,
     if (!ctx) return BHB200_ERR_INVALID;
     int rc = check_ops(ctx, opA, opB);
     if (rc) return rc;
-    rc = check_dims(ctx, m, k, n, nnzA, nnzB, valA, rowptrA, colA, valB, rowptrB, colB);
+    rc = check_dims(ctx, dtype, m, k, n, nnzA, nnzB, valA, rowptrA, colA, valB, rowptrB, colB);
     if (rc) return rc;
     // stored shapes: A is m x k (k x m for opA = T), B is k x n (n x k for opB = T)
     const int ra = opA ? k : m, ca = opA ? m : k, rb = opB ? n : k, cb = opB ? k : n;
@@ -187,7 +208,7 @@ int init_host(bhb200_ctx *ctx, int dtype, int opA, int opB, int m, int k, int n,
     const size_t vs = vsize(dtype);
     CU(ctx->a_rowptr.reserve((size_t)(ra + 1) * 4, &ctx->dev_bytes), "alloc rowptrA");
     CU(ctx->a_col.reserve((size_t)nnzA * 4 + 4, &ctx->dev_bytes), "alloc colA");
-    CU(ctx->a_val.reserve((size_t)nnzA * vs + 16, &ctx->dev_bytes), "alloc valA");
+    if (vs) CU(ctx->a_val.reserve((size_t)nnzA * vs + 16, &ctx->dev_bytes), "alloc valA");
     // C = A*A with the SAME host arrays passed twice (the reference driver's stock workloads build
     // A and B identically, main.cu:32-51): one upload, both operands point at it (also A*A^T, A^T*A)
     const bool alias = ra == rb && (!(opA || opB) || ca == cb) && nnzA == nnzB && rowptrA == rowptrB && colA == colB &&
@@ -195,22 +216,22 @@ int init_host(bhb200_ctx *ctx, int dtype, int opA, int opB, int m, int k, int n,
     if (!alias) {
         CU(ctx->b_rowptr.reserve((size_t)(rb + 1) * 4, &ctx->dev_bytes), "alloc rowptrB");
         CU(ctx->b_col.reserve((size_t)nnzB * 4 + 4, &ctx->dev_bytes), "alloc colB");
-        CU(ctx->b_val.reserve((size_t)nnzB * vs + 16, &ctx->dev_bytes), "alloc valB");
+        if (vs) CU(ctx->b_val.reserve((size_t)nnzB * vs + 16, &ctx->dev_bytes), "alloc valB");
     }
     cudaStream_t s = ctx->stream;
     CU(cudaMemcpyAsync(ctx->a_rowptr.p, rowptrA, (size_t)(ra + 1) * 4, cudaMemcpyHostToDevice, s), "H2D rowptrA");
     if (!alias) CU(cudaMemcpyAsync(ctx->b_rowptr.p, rowptrB, (size_t)(rb + 1) * 4, cudaMemcpyHostToDevice, s), "H2D rowptrB");
     if (nnzA > 0) {
         CU(cudaMemcpyAsync(ctx->a_col.p, colA, (size_t)nnzA * 4, cudaMemcpyHostToDevice, s), "H2D colA");
-        CU(cudaMemcpyAsync(ctx->a_val.p, valA, (size_t)nnzA * vs, cudaMemcpyHostToDevice, s), "H2D valA");
+        if (vs) CU(cudaMemcpyAsync(ctx->a_val.p, valA, (size_t)nnzA * vs, cudaMemcpyHostToDevice, s), "H2D valA");
     }
     if (nnzB > 0 && !alias) {
         CU(cudaMemcpyAsync(ctx->b_col.p, colB, (size_t)nnzB * 4, cudaMemcpyHostToDevice, s), "H2D colB");
-        CU(cudaMemcpyAsync(ctx->b_val.p, valB, (size_t)nnzB * vs, cudaMemcpyHostToDevice, s), "H2D valB");
+        if (vs) CU(cudaMemcpyAsync(ctx->b_val.p, valB, (size_t)nnzB * vs, cudaMemcpyHostToDevice, s), "H2D valB");
     }
     CU(cudaStreamSynchronize(s), "H2D operands");
-    ctx->As = Csr{ctx->a_rowptr.as<int>(), ctx->a_col.as<int>(), ctx->a_val.p};
-    ctx->Bs = alias ? ctx->As : Csr{ctx->b_rowptr.as<int>(), ctx->b_col.as<int>(), ctx->b_val.p};
+    ctx->As = Csr{ctx->a_rowptr.as<int>(), ctx->a_col.as<int>(), vs ? ctx->a_val.p : nullptr};
+    ctx->Bs = alias ? ctx->As : Csr{ctx->b_rowptr.as<int>(), ctx->b_col.as<int>(), vs ? ctx->b_val.p : nullptr};
     ctx->aliased = alias;
     ctx->dtype = dtype;
     ctx->m = m;
@@ -411,13 +432,15 @@ int64_t spilled_bytes(const DevBuf &b)
     return b.host ? (int64_t)b.cap : 0;
 }
 
-// colC / valC for nnzC entries, spilled to host memory if the device cannot hold them
+// colC / valC for nnzC entries, spilled to host memory if the device cannot hold them (structure only: no valC)
 int reserve_C(bhb200_ctx *ctx)
 {
+    const size_t vs = vsize(ctx->dtype);
     CU(ctx->colC.reserve_spillable((size_t)ctx->nnzC * 4 + 16, &ctx->dev_bytes, ctx->device_cap, nullptr), "alloc colC");
-    CU(ctx->valC.reserve_spillable((size_t)ctx->nnzC * vsize(ctx->dtype) + 16, &ctx->dev_bytes, ctx->device_cap, nullptr),
-       "alloc valC");
-    ctx->stats.spill_bytes += spilled_bytes(ctx->colC) + spilled_bytes(ctx->valC);
+    ctx->stats.spill_bytes += spilled_bytes(ctx->colC);
+    if (!vs) return BHB200_SUCCESS;
+    CU(ctx->valC.reserve_spillable((size_t)ctx->nnzC * vs + 16, &ctx->dev_bytes, ctx->device_cap, nullptr), "alloc valC");
+    ctx->stats.spill_bytes += spilled_bytes(ctx->valC);
     return BHB200_SUCCESS;
 }
 
@@ -658,7 +681,7 @@ int choose_direct(bhb200_ctx *ctx, Product &p)
     // the wide staging buffer must not crowd out C itself (at most `products` entries)
     // (only checked when the staging buffer has to grow: cudaMemGetInfo can take milliseconds)
     if (plan.mask() &&
-        ((size_t)plan.ct_entries * 4 + 16 > ctx->ct_col.cap || (size_t)plan.ct_entries * vs + 16 > ctx->ct_val.cap)) {
+        ((size_t)plan.ct_entries * 4 + 16 > ctx->ct_col.cap || (vs && (size_t)plan.ct_entries * vs + 16 > ctx->ct_val.cap))) {
         size_t free_b = 0, total_b = 0;
         cudaMemGetInfo(&free_b, &total_b);
         const double avail = (double)free_b + (double)ctx->ct_col.cap + (double)ctx->ct_val.cap + (double)ctx->colC.cap +
@@ -672,11 +695,12 @@ int choose_direct(bhb200_ctx *ctx, Product &p)
         if (ctx->ct_off.reserve(m1 * 8, &ctx->dev_bytes) != cudaSuccess ||
             ctx->retry_q.reserve(m1 * 4, &ctx->dev_bytes) != cudaSuccess ||
             ctx->ct_col.reserve_spillable((size_t)plan.ct_entries * 4 + 16, &ctx->dev_bytes, ctx->device_cap, nullptr) != cudaSuccess ||
-            ctx->ct_val.reserve_spillable((size_t)plan.ct_entries * vs + 16, &ctx->dev_bytes, ctx->device_cap, nullptr) != cudaSuccess) {
+            (vs && ctx->ct_val.reserve_spillable((size_t)plan.ct_entries * vs + 16, &ctx->dev_bytes, ctx->device_cap, nullptr) !=
+                       cudaSuccess)) {
             cudaGetLastError();
             plan.drop_all();   // no room for the staging buffer: two-pass path for everything
         } else {
-            st.spill_bytes += spilled_bytes(ctx->ct_col) + spilled_bytes(ctx->ct_val);
+            st.spill_bytes += spilled_bytes(ctx->ct_col) + (vs ? spilled_bytes(ctx->ct_val) : 0);
         }
     }
     st.direct_ct_bytes = plan.ct_bytes();
@@ -893,10 +917,10 @@ int stage_masked(bhb200_ctx *ctx, Product &p)
     CU(ctx->ct_off.reserve(m1 * 8, &ctx->dev_bytes), "alloc staging offsets");
     CU(ctx->mask_q.reserve(m1 * 4, &ctx->dev_bytes), "alloc masked bin queue");
     CU(ctx->ct_col.reserve_spillable(nM * 4 + 16, &ctx->dev_bytes, ctx->device_cap, nullptr), "alloc staging columns");
-    CU(ctx->ct_val.reserve_spillable(nM * vs + 16, &ctx->dev_bytes, ctx->device_cap, nullptr), "alloc staging values");
-    st.spill_bytes += spilled_bytes(ctx->ct_col) + spilled_bytes(ctx->ct_val);
-    if (p.hc.mask_bin[MB_GLOBAL] > 0) {
-        CU(ctx->mask_acc.reserve(nM * vs + 16, &ctx->dev_bytes), "alloc masked accumulator");
+    if (vs) CU(ctx->ct_val.reserve_spillable(nM * vs + 16, &ctx->dev_bytes, ctx->device_cap, nullptr), "alloc staging values");
+    st.spill_bytes += spilled_bytes(ctx->ct_col) + (vs ? spilled_bytes(ctx->ct_val) : 0);
+    if (p.hc.mask_bin[MB_GLOBAL] > 0) {   // (structure only: hit flags, no accumulator)
+        if (vs) CU(ctx->mask_acc.reserve(nM * vs + 16, &ctx->dev_bytes), "alloc masked accumulator");
         CU(ctx->mask_hit.reserve(nM + 16, &ctx->dev_bytes), "alloc masked hit flags");
     }
     memcpy(ctx->last_mask_bin, p.hc.mask_bin, sizeof(ctx->last_mask_bin));
@@ -1086,6 +1110,12 @@ int bhb200_init_data_op_f32(bhb200_ctx *ctx, int opA, int opB, int m, int k, int
     return init_host(ctx, BHB200_DTYPE_F32, opA, opB, m, k, n, nnzA, valA, rowptrA, colA, nnzB, valB, rowptrB, colB);
 }
 
+int bhb200_init_data_structure(bhb200_ctx *ctx, int opA, int opB, int m, int k, int n, int nnzA, const int32_t *rowptrA,
+                               const int32_t *colA, int nnzB, const int32_t *rowptrB, const int32_t *colB)
+{
+    return init_host(ctx, BHB200_DTYPE_NONE, opA, opB, m, k, n, nnzA, nullptr, rowptrA, colA, nnzB, nullptr, rowptrB, colB);
+}
+
 int bhb200_init_data_device(bhb200_ctx *ctx, int dtype, int m, int k, int n, int nnzA, const void *valA,
                             const int32_t *rowptrA, const int32_t *colA, int nnzB, const void *valB,
                             const int32_t *rowptrB, const int32_t *colB)
@@ -1099,15 +1129,17 @@ int bhb200_init_data_device_op(bhb200_ctx *ctx, int dtype, int opA, int opB, int
                                const int32_t *rowptrB, const int32_t *colB)
 {
     if (!ctx) return BHB200_ERR_INVALID;
-    if (dtype != BHB200_DTYPE_F32 && dtype != BHB200_DTYPE_F64) return fail(ctx, BHB200_ERR_INVALID, "bad dtype");
+    if (dtype != BHB200_DTYPE_F32 && dtype != BHB200_DTYPE_F64 && dtype != BHB200_DTYPE_NONE)
+        return fail(ctx, BHB200_ERR_INVALID, "bad dtype");
     int rc = check_ops(ctx, opA, opB);
     if (rc) return rc;
-    rc = check_dims(ctx, m, k, n, nnzA, nnzB, valA, rowptrA, colA, valB, rowptrB, colB);
+    rc = check_dims(ctx, dtype, m, k, n, nnzA, nnzB, valA, rowptrA, colA, valB, rowptrB, colB);
     if (rc) return rc;
     CU(cudaSetDevice(ctx->device), "cudaSetDevice");
     release_operands(ctx);
-    ctx->As = Csr{rowptrA, colA, valA};
-    ctx->Bs = Csr{rowptrB, colB, valB};
+    const bool values = dtype != BHB200_DTYPE_NONE;   // (structure only: the caller's value pointers are never read)
+    ctx->As = Csr{rowptrA, colA, values ? valA : nullptr};
+    ctx->Bs = Csr{rowptrB, colB, values ? valB : nullptr};
     ctx->dtype = dtype;
     ctx->m = m;
     ctx->k = k;
@@ -1244,6 +1276,7 @@ int bhb200_spgemm_numeric(bhb200_ctx *ctx)
     if (!ctx || !ctx->have_data || !ctx->have_C)
         return fail(ctx, BHB200_ERR_INVALID, "spgemm_numeric needs a completed spgemm on the same operands");
     if (ctx->mask_changed) return fail(ctx, BHB200_ERR_INVALID, "spgemm_numeric: the mask changed since the last spgemm");
+    if (ctx->dtype == BHB200_DTYPE_NONE) return refuse_structure(ctx, "spgemm_numeric");
     int rc = begin_call(ctx);
     if (rc) return rc;
     bhb200_stats &st = ctx->stats;
@@ -1315,6 +1348,7 @@ int bhb200_spgemm_numeric(bhb200_ctx *ctx)
 static int update_values_any(bhb200_ctx *ctx, int dtype, const void *valA, const void *valB)
 {
     if (!ctx || !ctx->have_data) return fail(ctx, BHB200_ERR_INVALID, "update_values before initData");
+    if (ctx->dtype == BHB200_DTYPE_NONE) return refuse_structure(ctx, "update_values");
     if (ctx->borrowed) return fail(ctx, BHB200_ERR_INVALID, "operands are caller-owned device arrays: update them in place");
     if (dtype != ctx->dtype) return fail(ctx, BHB200_ERR_INVALID, "value type differs from initData");
     CU(cudaSetDevice(ctx->device), "cudaSetDevice");
@@ -1453,10 +1487,12 @@ int64_t bhb200_get_nnzC(const bhb200_ctx *ctx)
     return (ctx && ctx->have_C) ? ctx->nnzC : -1;
 }
 
+// dtype BHB200_DTYPE_NONE: the structure of C (any product), valC is null
 static int get_C_any(bhb200_ctx *ctx, int dtype, int32_t *rowptrC, int32_t *colC, void *valC)
 {
     if (!ctx || !ctx->have_C) return fail(ctx, BHB200_ERR_INVALID, "get_C before spgemm");
-    if (dtype != ctx->dtype) return fail(ctx, BHB200_ERR_INVALID, "get_C dtype differs from initData dtype");
+    if (dtype != BHB200_DTYPE_NONE && ctx->dtype == BHB200_DTYPE_NONE) return refuse_structure(ctx, "get_C");
+    if (dtype != BHB200_DTYPE_NONE && dtype != ctx->dtype) return fail(ctx, BHB200_ERR_INVALID, "get_C dtype differs from initData dtype");
     if (ctx->nnzC > 0x7fffffffLL) return fail(ctx, BHB200_ERR_OVERFLOW, "nnz(C) exceeds INT32_MAX; use the int64 row pointers");
     CU(cudaSetDevice(ctx->device), "cudaSetDevice");
     cudaStream_t s = ctx->stream;
@@ -1478,11 +1514,16 @@ int bhb200_get_C_f32(bhb200_ctx *ctx, int32_t *rowptrC, int32_t *colC, float *va
 {
     return get_C_any(ctx, BHB200_DTYPE_F32, rowptrC, colC, valC);
 }
+int bhb200_get_C_structure(bhb200_ctx *ctx, int32_t *rowptrC, int32_t *colC)
+{
+    return get_C_any(ctx, BHB200_DTYPE_NONE, rowptrC, colC, nullptr);
+}
 
 int bhb200_get_C_range(bhb200_ctx *ctx, int64_t first, int64_t count, int32_t *colC, void *valC)
 {
     if (!ctx || !ctx->have_C) return fail(ctx, BHB200_ERR_INVALID, "get_C_range before spgemm");
     if (first < 0 || count < 0 || first + count > ctx->nnzC) return fail(ctx, BHB200_ERR_INVALID, "range outside [0, nnzC]");
+    if (valC && ctx->dtype == BHB200_DTYPE_NONE) return refuse_structure(ctx, "get_C_range with valC");
     CU(cudaSetDevice(ctx->device), "cudaSetDevice");
     cudaStream_t s = ctx->stream;
     const size_t vs = vsize(ctx->dtype);
@@ -1512,13 +1553,14 @@ int bhb200_get_C_device(bhb200_ctx *ctx, const int32_t **rowptr32, const int64_t
     if (rowptr32) *rowptr32 = ctx->nnzC > 0x7fffffffLL ? nullptr : ctx->rowptr32.as<int32_t>();
     if (rowptr64) *rowptr64 = ctx->rowoff64.as<int64_t>();
     if (colC) *colC = ctx->colC.as<int32_t>();
-    if (valC) *valC = ctx->valC.p;
+    if (valC) *valC = ctx->dtype == BHB200_DTYPE_NONE ? nullptr : ctx->valC.p;
     return BHB200_SUCCESS;
 }
 
 int bhb200_copy_C_to_device(bhb200_ctx *ctx, int64_t *rowptrC64, int32_t *colC, void *valC)
 {
     if (!ctx || !ctx->have_C) return fail(ctx, BHB200_ERR_INVALID, "copy_C_to_device before spgemm");
+    if (valC && ctx->dtype == BHB200_DTYPE_NONE) return refuse_structure(ctx, "copy_C_to_device with valC");
     CU(cudaSetDevice(ctx->device), "cudaSetDevice");
     cudaStream_t s = ctx->stream;
     if (rowptrC64)

@@ -187,7 +187,12 @@ bool build_pattern_plan(const int *offsA, int nA, const int *offsB, int nB, int 
             mlog[(size_t)ja * nB + jb] = (unsigned char)o;
             pfull[(size_t)ja * nw + (o >> 5)] |= 1u << (o & 31);
         }
-    choose_layout(nA, nB, nD, mlog, value_size == 8 ? 16 : 32, sums.data(), pos, plan.acc_len);
+    if (value_size > 0) {
+        choose_layout(nA, nB, nD, mlog, value_size == 8 ? 16 : 32, sums.data(), pos, plan.acc_len);
+    } else {   // structure only: k_pat_emit writes the columns from the output masks, there is no accumulator
+        pos.assign(nD, 0);
+        plan.acc_len = 0;
+    }
     for (size_t i = 0; i < mlog.size(); ++i) mphys[i] = pos[mlog[i]];
     // blob: byte tables first, then the 4-byte tables (aligned)
     const size_t nM = (size_t)nA * nB;

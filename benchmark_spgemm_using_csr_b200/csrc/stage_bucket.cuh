@@ -98,7 +98,7 @@ __host__ __device__ constexpr int b3_chunk()
 template <typename VT, int THREADS>
 inline size_t b3_smem_bytes(const int cap, const int nb, const int knots)
 {
-    return (size_t)b3_chunk<THREADS>() * (16 + sizeof(VT)) + (size_t)cap * (sizeof(VT) + 12) + (size_t)(nb + 1) * 4 +
+    return (size_t)b3_chunk<THREADS>() * (16 + value_bytes<VT>) + (size_t)cap * (value_bytes<VT> + 12) + (size_t)(nb + 1) * 4 +
            (size_t)(knots + 1) * 4 + (size_t)(B3_SCRATCH + B3_LONG_CAP) * 4 + (size_t)cap * 2;
 }
 
@@ -219,8 +219,8 @@ k_num_bucket3(const int *__restrict__ queue, const int count, const int *__restr
     extern __shared__ __align__(16) unsigned char smem_raw[];
     int4 *arec = reinterpret_cast<int4 *>(smem_raw);                      // [ACH] {B row start, length, first product index, -}
     VT *aval = reinterpret_cast<VT *>(arec + ACH);                        // [ACH]
-    VT *v = aval + ACH;                                                   // [cap] a*b of product t
-    int *c = reinterpret_cast<int *>(v + cap);                            // [cap] column of product t; later the sorted columns
+    VT *v = aval + ACH * vslots<VT>;                                      // [cap] a*b of product t
+    int *c = reinterpret_cast<int *>(v + cap * vslots<VT>);               // [cap] column of product t; later the sorted columns
     unsigned *meta = reinterpret_cast<unsigned *>(c + cap);               // [cap] bucket << 16 | arrival
     int *key2 = reinterpret_cast<int *>(meta + cap);                      // [cap] columns in bucket order
     int *cnt = key2 + cap;                                                // [nb + 1] counts -> first slot of every bucket
@@ -344,7 +344,7 @@ k_num_bucket3(const int *__restrict__ queue, const int count, const int *__restr
 //   * bucket / arrival / rank / emit as in k_num_bucket3, at warp scope (__syncwarp only), one emit sweep;
 //   * tight direct bins (DirectOut: rows staged `stride` entries apart, stride < product bound): entries beyond the
 //     stride are not written and the row goes to the retry queue, like k_num_direct.
-// Shared memory per warp: CAPW * (sizeof(VT) + 4 + 4 + 2 + 1) + (CAPW/2 + 1) * 4; the 1024-knot CDF once per CTA.
+// Shared memory per warp: CAPW * (value_bytes<VT> + 4 + 4 + 2 + 1) + (CAPW/2 + 1) * 4; the 1024-knot CDF once per CTA.
 // ---------------------------------------------------------------------------------------------------
 constexpr int B3W_KB = 10;
 constexpr int B3W_WARPS = 8;
@@ -352,7 +352,7 @@ constexpr int B3W_WARPS = 8;
 template <typename VT, int CAPW>
 __host__ __device__ constexpr size_t b3w_per_warp()
 {
-    return (((size_t)CAPW * (sizeof(VT) + 4 + 4 + 2 + 1) + (size_t)(CAPW / 2 + 1) * 4) + 15) & ~(size_t)15;
+    return (((size_t)CAPW * (value_bytes<VT> + 4 + 4 + 2 + 1) + (size_t)(CAPW / 2 + 1) * 4) + 15) & ~(size_t)15;
 }
 
 template <typename VT, int CAPW, int SG>
@@ -372,7 +372,7 @@ k_num_bucket3w(const int *__restrict__ queue, const int count, const int *__rest
     const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
     unsigned char *mine = smem_raw + (((size_t)(K + 1) * 4 + 15) & ~(size_t)15) + (size_t)w * b3w_per_warp<VT, CAPW>();
     VT *v = reinterpret_cast<VT *>(mine);                                   // [CAPW]
-    int *c = reinterpret_cast<int *>(v + CAPW);                             // [CAPW] staged columns, later the sorted ones
+    int *c = reinterpret_cast<int *>(v + CAPW * vslots<VT>);               // [CAPW] staged columns, later the sorted ones
     int *key2 = c + CAPW;                                                   // [CAPW]
     int *cnt = key2 + CAPW;                                                 // [NB + 1]
     unsigned short *meta = reinterpret_cast<unsigned short *>(cnt + NB + 1);   // [CAPW] bucket << 8 | arrival
@@ -571,7 +571,7 @@ k_num_bucket_heavy(const int *__restrict__ queue, const int count, const int *__
 {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     VT *vals = reinterpret_cast<VT *>(smem_raw);                              // [cap]
-    int *keys = reinterpret_cast<int *>(smem_raw + (size_t)cap * sizeof(VT));   // [cap]
+    int *keys = reinterpret_cast<int *>(smem_raw + (size_t)cap * value_bytes<VT>);   // [cap]
     int *cnt = keys + cap;                                                    // [nb]
     int *ocnt = cnt + nb;                                                     // [nb + 1]
     int *scratch = ocnt + nb + 1;                                             // [34]
@@ -665,19 +665,21 @@ k_num_bucket_heavy(const int *__restrict__ queue, const int count, const int *__
                         __syncthreads();
                         const int cmin = s_min;
                         if (cmin == 0x7fffffff) break;
-                        double part = 0.0;
-                        for (int j = a0 + (int)(threadIdx.x >> 5); j < a1; j += THREADS / 32) {
-                            const int k = colA[j];
-                            const VT av = valA[j];
-                            for (int e = rowptrB[k] + lane; e < rowptrB[k + 1]; e += 32)
-                                if (colB[e] == cmin) part += (double)(av * valB[e]);
+                        if constexpr (value_bytes<VT> > 0) {
+                            double part = 0.0;
+                            for (int j = a0 + (int)(threadIdx.x >> 5); j < a1; j += THREADS / 32) {
+                                const int k = colA[j];
+                                const VT av = valA[j];
+                                for (int e = rowptrB[k] + lane; e < rowptrB[k + 1]; e += 32)
+                                    if (colB[e] == cmin) part += (double)(av * valB[e]);
+                            }
+                            part = warp_sum(part);
+                            if (lane == 0 && part != 0.0) atomicAdd(&s_sum, part);
+                            __syncthreads();
                         }
-                        part = warp_sum(part);
-                        if (lane == 0 && part != 0.0) atomicAdd(&s_sum, part);
-                        __syncthreads();
                         if (threadIdx.x == 0) {
                             ctcol[o + written] = cmin;
-                            ctval[o + written] = (VT)s_sum;
+                            if constexpr (value_bytes<VT> > 0) ctval[o + written] = (VT)s_sum;
                         }
                         ++written;
                         last = cmin;
@@ -771,7 +773,7 @@ constexpr int H2_MAX_LG = 11;   // at most 2048 slices per row (16.7 M products)
 template <typename VT>
 inline size_t h2_smem_bytes(const int cap, const int nb)
 {
-    return (size_t)cap * (sizeof(VT) + 12) + (size_t)(nb + 1) * 4 + (size_t)(CDF_KNOTS + 1) * 4 + (size_t)B3_SCRATCH * 4 +
+    return (size_t)cap * (value_bytes<VT> + 12) + (size_t)(nb + 1) * 4 + (size_t)(CDF_KNOTS + 1) * 4 + (size_t)B3_SCRATCH * 4 +
            (size_t)((1 << H2_MAX_LG) + 1) * 4 + (size_t)cap * 2;
 }
 
@@ -786,7 +788,7 @@ k_num_bucket_heavy2(const int *__restrict__ queue, const int count, const int *_
 {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     VT *v = reinterpret_cast<VT *>(smem_raw);                                 // [cap]
-    int *c = reinterpret_cast<int *>(v + cap);                                // [cap]
+    int *c = reinterpret_cast<int *>(v + cap * vslots<VT>);                   // [cap]
     unsigned *meta = reinterpret_cast<unsigned *>(c + cap);                   // [cap]
     int *key2 = reinterpret_cast<int *>(meta + cap);                          // [cap]
     int *cnt = key2 + cap;                                                    // [nb + 1]

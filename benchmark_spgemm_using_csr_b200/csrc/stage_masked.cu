@@ -204,7 +204,7 @@ __global__ void __launch_bounds__(256) k_mask_esc(const int *__restrict__ queue,
 template <typename VT, int LOG2T>
 __host__ __device__ constexpr size_t mask_warp_bytes()
 {
-    return (size_t)(1 << LOG2T) / 2 * (sizeof(VT) + 1) + (size_t)(1 << LOG2T) * 8;
+    return (size_t)(1 << LOG2T) / 2 * (value_bytes<VT> + 1) + (size_t)(1 << LOG2T) * 8;
 }
 constexpr int MASK_WARPS = 8;
 
@@ -218,7 +218,7 @@ __global__ void __launch_bounds__(MASK_WARPS * 32) k_mask_warp(const int *__rest
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     unsigned char *mine = smem_raw + (size_t)warp * mask_warp_bytes<VT, LOG2T>();
     VT *vals = reinterpret_cast<VT *>(mine);
-    int *keys = reinterpret_cast<int *>(mine + (size_t)H * sizeof(VT));
+    int *keys = reinterpret_cast<int *>(mine + (size_t)H * value_bytes<VT>);
     int *posv = keys + T;
     unsigned char *flag = reinterpret_cast<unsigned char *>(posv + T);
     const VT *__restrict__ valA = static_cast<const VT *>(A.val);
@@ -337,7 +337,7 @@ __global__ void __launch_bounds__(THREADS) k_mask_cta(const int *__restrict__ qu
     extern __shared__ __align__(16) unsigned char smem_raw[];
     __shared__ MaskCtaShared sh;
     VT *vals = reinterpret_cast<VT *>(smem_raw);
-    int *keys = reinterpret_cast<int *>(smem_raw + (size_t)H * sizeof(VT));
+    int *keys = reinterpret_cast<int *>(smem_raw + (size_t)H * value_bytes<VT>);
     int *posv = keys + T;
     unsigned char *flag = reinterpret_cast<unsigned char *>(posv + T);
     const VT *__restrict__ valA = static_cast<const VT *>(A.val);
@@ -405,7 +405,7 @@ __global__ void __launch_bounds__(MASK_GLOBAL_THREADS) k_mask_global(const int *
     for (int q = blockIdx.x; q < count; q += gridDim.x) {
         const int row = queue[q];
         const int ms = M.rowptr[row], mc = M.rowptr[row + 1] - ms;
-        VT *acc = static_cast<VT *>(o.acc) + ms;
+        VT *acc = static_cast<VT *>(o.acc) + ms * vslots<VT>;
         unsigned char *hit = o.hit + ms;
         const int *mcol = M.col + ms;
         for (int t = threadIdx.x; t < mc; t += blockDim.x) {
@@ -519,6 +519,7 @@ cudaError_t launch_mask_bin(const LaunchCtx &lc, int dtype, int bin, const int *
                             const int4 *brange, MaskCsr M, MaskOut o)
 {
     if (count <= 0) return cudaSuccess;
+    if (dtype == BHB200_DTYPE_NONE) return launch_mask_bin_t<NoVal>(lc, bin, queue, count, A, B, brange, M, o);   // (hit flags only)
     return dtype == BHB200_DTYPE_F64 ? launch_mask_bin_t<double>(lc, bin, queue, count, A, B, brange, M, o)
                                      : launch_mask_bin_t<float>(lc, bin, queue, count, A, B, brange, M, o);
 }

@@ -33,7 +33,7 @@ k_num_group(const int *__restrict__ queue, const int count, const int *__restric
 {
     constexpr int T = 1 << LOG2T;
     constexpr int N = (R > 0) ? G * R : T / 2;   // max nnz(C_i) of the bin (sort capacity); T >= 2N slots
-    constexpr size_t PER_GROUP = (size_t)T * sizeof(VT) + (size_t)T * 4 + (size_t)N * 4;
+    constexpr size_t PER_GROUP = (size_t)T * value_bytes<VT> + (size_t)T * 4 + (size_t)N * 4;
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int lane = threadIdx.x & 31;
     const int gl = threadIdx.x & (G - 1);
@@ -43,7 +43,7 @@ k_num_group(const int *__restrict__ queue, const int count, const int *__restric
     const unsigned gbits = (G == 32) ? FULL : ((1u << (G & 31)) - 1u);
     unsigned char *mine = smem_raw + (size_t)gib * PER_GROUP;
     VT *vals = reinterpret_cast<VT *>(mine);
-    int *keys = reinterpret_cast<int *>(mine + (size_t)T * sizeof(VT));
+    int *keys = reinterpret_cast<int *>(mine + (size_t)T * value_bytes<VT>);
     int *sk = keys + T;
 
     // All loops are WARP-uniform (trip counts are maxima over the 32/G groups of the warp,
@@ -164,7 +164,7 @@ k_num_direct(const int *__restrict__ queue, const int count, const int *__restri
     constexpr int T = 1 << LOG2T;
     constexpr int N = G * R;                 // speculated capacity of a row
     static_assert(T == 2 * N && R > 0, "direct mode uses the register sort and a half-full table");
-    constexpr size_t PER_GROUP = (size_t)T * sizeof(VT) + (size_t)T * 4 + (size_t)N * 4;
+    constexpr size_t PER_GROUP = (size_t)T * value_bytes<VT> + (size_t)T * 4 + (size_t)N * 4;
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int lane = threadIdx.x & 31;
     const int gl = threadIdx.x & (G - 1);
@@ -174,7 +174,7 @@ k_num_direct(const int *__restrict__ queue, const int count, const int *__restri
     const unsigned gbits = (G == 32) ? FULL : ((1u << (G & 31)) - 1u);
     unsigned char *mine = smem_raw + (size_t)gib * PER_GROUP;
     VT *vals = reinterpret_cast<VT *>(mine);
-    int *keys = reinterpret_cast<int *>(mine + (size_t)T * sizeof(VT));
+    int *keys = reinterpret_cast<int *>(mine + (size_t)T * value_bytes<VT>);
     int *sk = keys + T;
 
     for (int q0 = blockIdx.x * groups_per_block + (gib & ~(32 / G - 1)); q0 < count;
@@ -317,11 +317,14 @@ k_copy_ct(const int *__restrict__ queue, const int count, const int64_t *__restr
 }
 
 // CTAs of k_num_block<VT,LOG2T,THREADS> an SM can hold (threads and shared memory); asking the
-// compiler for that many keeps the register count from being the limiter.
+// compiler for that many keeps the register count from being the limiter.  Value-free tables are
+// counted as f32 ones: at T = 16384 their smaller footprint would ask for two 1024-thread CTAs, i.e.
+// 32 registers, and the kernel then spills.
 template <typename VT, int LOG2T, int THREADS>
 constexpr int num_block_min_ctas()
 {
-    constexpr int smem = (1 << LOG2T) * ((int)sizeof(VT) + 4) + (1 << LOG2T) / 2 * 4 + 1024;
+    constexpr int vb = value_bytes<VT> > 4 ? (int)value_bytes<VT> : 4;
+    constexpr int smem = (1 << LOG2T) * (vb + 4) + (1 << LOG2T) / 2 * 4 + 1024;
     constexpr int by_smem = (228 * 1024) / smem;   // 228 KB per SM, 1 KB reserved per CTA
     constexpr int by_threads = 2048 / THREADS;
     return by_smem < by_threads ? (by_smem < 1 ? 1 : by_smem) : by_threads;
@@ -343,7 +346,7 @@ k_num_block(const int *__restrict__ queue, const int count, const int *__restric
     constexpr int CHUNKS = T / (4 * THREADS);   // 16-byte key chunks per thread in the compaction
     extern __shared__ __align__(16) unsigned char smem_raw[];
     VT *vals = reinterpret_cast<VT *>(smem_raw);
-    int *keys = reinterpret_cast<int *>(smem_raw + (size_t)T * sizeof(VT));
+    int *keys = reinterpret_cast<int *>(smem_raw + (size_t)T * value_bytes<VT>);
     int *sk = keys + T;   // no static shared memory: T=4096 must fit four CTAs per SM to the byte
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     constexpr int nwarps = THREADS / 32;
@@ -597,7 +600,7 @@ static cudaError_t launch_num_group_t(const LaunchCtx &lc, const int *queue, int
 {
     constexpr int T = 1 << LOG2T;
     constexpr int N = (R > 0) ? G * R : T / 2;
-    constexpr size_t per_group = (size_t)T * sizeof(VT) + (size_t)T * 4 + (size_t)N * 4;
+    constexpr size_t per_group = (size_t)T * value_bytes<VT> + (size_t)T * 4 + (size_t)N * 4;
     int groups = (int)((56 * 1024) / per_group);
     const int max_groups = 256 / G;
     if (groups > max_groups) groups = max_groups;
@@ -625,7 +628,7 @@ static cudaError_t launch_num_block_t(const LaunchCtx &lc, const int *queue, int
                                       const int64_t *rowoff, int *colC, void *valC)
 {
     constexpr int T = 1 << LOG2T;
-    const size_t smem = (size_t)T * sizeof(VT) + (size_t)T * 4 + (size_t)(T / 2) * 4;
+    const size_t smem = (size_t)T * value_bytes<VT> + (size_t)T * 4 + (size_t)(T / 2) * 4;
     if (smem > 48 * 1024) {
         cudaError_t e = cudaFuncSetAttribute(k_num_block<VT, LOG2T, THREADS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         if (e != cudaSuccess) return e;
@@ -690,7 +693,7 @@ template <typename VT, int LOG2T, int R>
 static cudaError_t launch_num_direct_filtered(const LaunchCtx &lc, const int *queue, int count, Csr A, Csr B, DirectOut d)
 {
     constexpr int T = 1 << LOG2T;
-    constexpr size_t per_group = (size_t)T * sizeof(VT) + (size_t)T * 4 + (size_t)(32 * R) * 4;
+    constexpr size_t per_group = (size_t)T * value_bytes<VT> + (size_t)T * 4 + (size_t)(32 * R) * 4;
     int groups = (int)((56 * 1024) / per_group);
     if (groups > 8) groups = 8;
     if (groups < 1) groups = 1;
@@ -719,7 +722,7 @@ static cudaError_t launch_num_direct_g(const LaunchCtx &lc, const int *queue, in
         if (d.prod) return launch_num_direct_filtered<VT, LOG2T, R>(lc, queue, count, A, B, d);
     }
     constexpr int T = 1 << LOG2T;
-    constexpr size_t per_group = (size_t)T * sizeof(VT) + (size_t)T * 4 + (size_t)(G * R) * 4;
+    constexpr size_t per_group = (size_t)T * value_bytes<VT> + (size_t)T * 4 + (size_t)(G * R) * 4;
     int groups = (int)((56 * 1024) / per_group);
     const int max_groups = 256 / G;
     if (groups > max_groups) groups = max_groups;
@@ -746,7 +749,7 @@ template <typename VT, int LOG2T, int THREADS>
 static cudaError_t launch_num_block_direct_t(const LaunchCtx &lc, const int *queue, int count, Csr A, Csr B, DirectOut d)
 {
     constexpr int T = 1 << LOG2T;
-    const size_t smem = (size_t)T * sizeof(VT) + (size_t)T * 4 + (size_t)(T / 2) * 4;
+    const size_t smem = (size_t)T * value_bytes<VT> + (size_t)T * 4 + (size_t)(T / 2) * 4;
     if (smem > 48 * 1024) {
         cudaError_t e = cudaFuncSetAttribute(k_num_block<VT, LOG2T, THREADS, true>,
                                              cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
@@ -870,10 +873,10 @@ static cudaError_t launch_num_bucket_heavy_t(const LaunchCtx &lc, const int *que
 {
     if (count <= 0) return cudaSuccess;
     constexpr int THREADS = 1024;
-    constexpr int cap = sizeof(VT) == 8 ? 12288 : 16384;   // entries of a slice held on chip
+    constexpr int cap = value_bytes<VT> == 8 ? 12288 : 16384;   // entries of a slice held on chip
     // buckets per slice: half the capacity (measured best on R-MAT 24 rank 0: /2 70.3, /4 72.5, /8 72.8 ms)
     constexpr int nb = cap / 2;
-    const size_t smem = (size_t)cap * (sizeof(VT) + 4) + (size_t)(2 * nb + 1 + 34) * 4 + (size_t)(CDF_KNOTS + 1) * 4;
+    const size_t smem = (size_t)cap * (value_bytes<VT> + 4) + (size_t)(2 * nb + 1 + 34) * 4 + (size_t)(CDF_KNOTS + 1) * 4;
     auto kern = k_num_bucket_heavy<VT, THREADS>;
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;

@@ -736,11 +736,44 @@ static cudaError_t launch_pat_numeric_t(const LaunchCtx &lc, int m, Csr A, Csr B
     return launch_pat_numeric_tbl<VT, G, false>(lc, m, A, B, ta, tb, t, outmask, rowoff, colC, valC);
 }
 
+// Structure-only products: row i of C is i + dcol[o] for the set bits o of its output mask, in ascending o (dcol is
+// sorted, so the columns come out ascending) -- no operand is read and nothing is accumulated.  A warp per row: lane
+// l of step w writes bit l of mask word w at the row's offset plus the popcount of the bits below it (coalesced).
+__global__ void __launch_bounds__(256) k_pat_emit(const int m, const int nD, const int nw, const int *__restrict__ dcol,
+                                                  const unsigned *__restrict__ outmask, const int64_t *__restrict__ rowoff,
+                                                  int *__restrict__ colC)
+{
+    __shared__ int s_dcol[PAT_MAX_OUT];
+    for (int i = threadIdx.x; i < nD; i += blockDim.x) s_dcol[i] = dcol[i];
+    __syncthreads();
+    const int lane = threadIdx.x & 31;
+    const unsigned below = (1u << lane) - 1u;
+    const int warps = (int)((gridDim.x * blockDim.x) >> 5);
+    for (int row = (int)((blockIdx.x * blockDim.x + threadIdx.x) >> 5); row < m; row += warps) {
+        const unsigned mine = lane < nw ? __ldg(outmask + (size_t)row * nw + lane) : 0u;
+        int64_t o = rowoff[row];
+        for (int w = 0; w < nw; ++w) {
+            const unsigned bits = __shfl_sync(FULL, mine, w);
+            if ((bits >> lane) & 1u) colC[o + __popc(bits & below)] = row + s_dcol[(w << 5) + lane];
+            o += __popc(bits);
+        }
+    }
+}
+
 cudaError_t launch_pat_numeric(const LaunchCtx &lc, int dtype, int m, Csr A, Csr B, const unsigned char *ta,
                                const unsigned char *tb, PatTables t, const unsigned *outmask, const int64_t *rowoff,
                                int *colC, void *valC)
 {
     if (m <= 0) return cudaSuccess;
+    if (dtype == BHB200_DTYPE_NONE) {
+        const int threads = 256;
+        long long blocks = ((long long)m * 32 + threads - 1) / threads;
+        const long long cap = (long long)lc.sm_count * resident_blocks(k_pat_emit, threads, 0);
+        if (blocks > cap) blocks = cap;
+        ++*lc.launches;
+        k_pat_emit<<<(int)blocks, threads, 0, lc.stream>>>(m, t.nD, t.nw, t.dcol, outmask, rowoff, colC);
+        return cudaGetLastError();
+    }
     const int G = t.nDB <= 8 ? 8 : t.nDB <= 16 ? 16 : 32;
     if (dtype == BHB200_DTYPE_F64) {
         double *v = (double *)valC;

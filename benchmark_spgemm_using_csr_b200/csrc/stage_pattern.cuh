@@ -63,6 +63,7 @@ cudaError_t launch_pat_codes(const LaunchCtx &lc, int rows, int ncols, const int
 cudaError_t launch_pat_symbolic(const LaunchCtx &lc, int m, Csr A, const unsigned char *ta, const unsigned long long *maskB,
                                 PatTables t, unsigned *outmask, int *rc, int *prod, Counters *ctr, int k, double avg_row,
                                 const unsigned *fullbits);
+// dtype BHB200_DTYPE_NONE: the columns of C from the output masks alone (k_pat_emit); A, B, ta, tb are not read
 cudaError_t launch_pat_numeric(const LaunchCtx &lc, int dtype, int m, Csr A, Csr B, const unsigned char *ta,
                                const unsigned char *tb, PatTables t, const unsigned *outmask, const int64_t *rowoff,
                                int *colC, void *valC);

@@ -191,11 +191,11 @@ k_num_range(const int *__restrict__ queue, const int count, const int *__restric
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nwarps = blockDim.x >> 5;
     const int nwords = nsum * 32;
-    unsigned char *mine = smem_raw + (size_t)warp * num_range_warp_bytes(nsum, nacc, sizeof(VT));
+    unsigned char *mine = smem_raw + (size_t)warp * num_range_warp_bytes(nsum, nacc, value_bytes<VT>);
     unsigned long long *bm64 = reinterpret_cast<unsigned long long *>(mine);   // [nwords] + zero sink + garbage sink
     unsigned *bm32 = reinterpret_cast<unsigned *>(mine);
     VT *acc = reinterpret_cast<VT *>(bm64 + nwords + 2);                        // [nacc] + sink slot
-    int *ocol = reinterpret_cast<int *>(acc + nacc + 4);                        // [nacc]
+    int *ocol = reinterpret_cast<int *>(acc + (nacc + 4) * vslots<VT>);         // [nacc]
     unsigned short *prefix16 = reinterpret_cast<unsigned short *>(ocol + nacc + 4);   // [nwords] + sink
     const int *colB_lane = colB + lane;
     const VT *valB_lane = valB + lane;
@@ -293,7 +293,7 @@ static cudaError_t launch_num_range_t(const LaunchCtx &lc, int nsum, int nacc, c
                                       Csr B, const int *rlo, const int64_t *rowoff, int *colC, void *valC, WordLists wl)
 {
     if (count <= 0) return cudaSuccess;
-    const size_t wb = num_range_warp_bytes(nsum, nacc, sizeof(VT));
+    const size_t wb = num_range_warp_bytes(nsum, nacc, value_bytes<VT>);
     int wpb, bps;
     range_launch_shape(wb, wpb, bps);
     const size_t smem = wb * wpb;

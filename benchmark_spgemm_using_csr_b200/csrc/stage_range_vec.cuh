@@ -184,7 +184,7 @@ k_num_range_vec(const int *__restrict__ queue, const int count, const int *__res
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nwarps = blockDim.x >> 5;
     const int nwords = nsum * 32;
     const int astride = nacc + 4;
-    unsigned char *mine = smem_raw + (size_t)warp * num_range_vec_warp_bytes(nsum, nacc, sizeof(VT));
+    unsigned char *mine = smem_raw + (size_t)warp * num_range_vec_warp_bytes(nsum, nacc, value_bytes<VT>);
     unsigned long long *bm64 = reinterpret_cast<unsigned long long *>(mine);   // [nwords] + zero sink + garbage sink
     unsigned *bm32 = reinterpret_cast<unsigned *>(mine);
     VT *acc = reinterpret_cast<VT *>(bm64 + nwords + 2);                        // RANGE_NG x ([nacc] + sink slot)
@@ -266,7 +266,7 @@ static cudaError_t launch_num_range_vec_t(const LaunchCtx &lc, int nsum, int nac
                                           WordLists wl)
 {
     if (count <= 0) return cudaSuccess;
-    const size_t wb = num_range_vec_warp_bytes(nsum, nacc, sizeof(VT));
+    const size_t wb = num_range_vec_warp_bytes(nsum, nacc, value_bytes<VT>);
     int wpb, bps;
     range_launch_shape(wb, wpb, bps);
     const size_t smem = wb * wpb;
@@ -288,14 +288,17 @@ inline bool range_vec_aligned(const Csr &B)
     return (((uintptr_t)B.col | (uintptr_t)B.val) & 15u) == 0;
 }
 
-// numeric range bins: the vectorised kernel for rows of at most 128 outputs when B is 16-byte aligned
+// numeric range bins: the vectorised kernel for rows of at most 128 outputs when B is 16-byte aligned (its 128-bit loads
+// carry values: structure-only products take the scalar kernel)
 template <typename VT>
 static cudaError_t launch_num_range_pick_t(const LaunchCtx &lc, int nsum, int nacc, const int *queue, int count, Csr A,
                                            Csr B, const int *rlo, const int64_t *rowoff, int *colC, void *valC,
                                            WordLists wl)
 {
-    if (nacc <= 128 && range_vec_aligned(B))
-        return launch_num_range_vec_t<VT>(lc, nsum, nacc, queue, count, A, B, rlo, rowoff, colC, valC, wl);
+    if constexpr (value_bytes<VT> > 0) {
+        if (nacc <= 128 && range_vec_aligned(B))
+            return launch_num_range_vec_t<VT>(lc, nsum, nacc, queue, count, A, B, rlo, rowoff, colC, valC, wl);
+    }
     return launch_num_range_t<VT>(lc, nsum, nacc, queue, count, A, B, rlo, rowoff, colC, valC, wl);
 }
 

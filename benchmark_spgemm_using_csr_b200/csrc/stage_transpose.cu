@@ -370,6 +370,7 @@ int transpose_passes(int cols)
 cudaError_t launch_transpose(const LaunchCtx &lc, int dtype, int rows, int cols, int nnz, Csr X, TransposeOut out,
                              void *scratch, int *bad, int bad_bit)
 {
+    if (dtype == BHB200_DTYPE_NONE) return transpose_typed<NoVal>(lc, rows, cols, nnz, X, out, scratch, bad, bad_bit);
     return dtype == BHB200_DTYPE_F64 ? transpose_typed<double>(lc, rows, cols, nnz, X, out, scratch, bad, bad_bit)
                       : transpose_typed<float>(lc, rows, cols, nnz, X, out, scratch, bad, bad_bit);
 }

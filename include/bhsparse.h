@@ -81,6 +81,18 @@ public:
 #endif
     }
 
+    /* Addition: structure-only products (bhb200_init_data_structure): the pattern of op(A)*op(B) from operands
+     * without values; spgemm() fills csrRowPtrC and get_C(colC, nullptr) the columns. */
+    int initDataStructure(int m, int k, int n, int nnzA, index_type *csrRowPtrA, index_type *csrColIndA, int nnzB,
+                          index_type *csrRowPtrB, index_type *csrColIndB, index_type *csrRowPtrC, bool transA = false,
+                          bool transB = false)
+    {
+        if (!_ctx) return BHB200_ERR_INVALID;
+        _rowptrC = csrRowPtrC;
+        return bhb200_init_data_structure(_ctx, transA ? BHB200_OP_T : BHB200_OP_N, transB ? BHB200_OP_T : BHB200_OP_N, m, k,
+                                          n, nnzA, csrRowPtrA, csrColIndA, nnzB, csrRowPtrB, csrColIndB);
+    }
+
     /* Addition: masked products C = M .* (op(A)*op(B)) on the structure of M (host arrays, copied;
      * bhb200_set_mask), until clearMask() or the next initData. */
     int setMask(int nnzM, index_type *csrRowPtrM, index_type *csrColIndM)
@@ -104,11 +116,7 @@ public:
          * (bhsparse_cuda.h:2787-2808); get_C writes them again (:3016).  Results beyond
          * INT32_MAX entries have no int32 row pointers (get_nnzC() == -1). */
         if (_rowptrC && bhb200_get_nnzC(_ctx) <= 0x7fffffffLL) {
-#ifdef BHSPARSE_VALUE_FLOAT
-            err = bhb200_get_C_f32(_ctx, _rowptrC, nullptr, nullptr);
-#else
-            err = bhb200_get_C_f64(_ctx, _rowptrC, nullptr, nullptr);
-#endif
+            err = bhb200_get_C_structure(_ctx, _rowptrC, nullptr);   /* (valued and structure-only products) */
             if (err != BHSPARSE_SUCCESS) return err;
         }
         if (_verbose) {
@@ -143,6 +151,7 @@ public:
     int get_C(index_type *csrColIndC, value_type *csrValC)   /* bhsparse_cuda.h:3011-3020 */
     {
         if (!_ctx) return BHB200_ERR_INVALID;
+        if (!csrValC) return bhb200_get_C_structure(_ctx, _rowptrC, csrColIndC);   /* (structure-only products too) */
 #ifdef BHSPARSE_VALUE_FLOAT
         return bhb200_get_C_f32(_ctx, _rowptrC, csrColIndC, csrValC);
 #else

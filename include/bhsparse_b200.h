@@ -44,6 +44,9 @@ extern "C" {
 
 #define BHB200_DTYPE_F32 0
 #define BHB200_DTYPE_F64 1
+/* structure only: operands and C have row pointers and columns, no values (see "structure-only
+ * products" below) */
+#define BHB200_DTYPE_NONE 2
 
 /* op(X) of bhb200_init_data_op_* / bhb200_init_data_device_op: X as stored, or its transpose */
 #define BHB200_OP_N 0
@@ -179,6 +182,30 @@ BHB200_API int bhb200_init_data_device_op(bhb200_ctx *ctx, int dtype, int opA, i
                                           int nnzA, const void *valA, const int32_t *rowptrA, const int32_t *colA,
                                           int nnzB, const void *valB, const int32_t *rowptrB, const int32_t *colB);
 
+/* -- structure-only products: the sparsity pattern of op(A)*op(B) (GraphBLAS's boolean product, the
+ * symbolic stage of MKL sp2m / cuSPARSE SpGEMMreuse) -----------------------------------------------------
+ * Operands of type BHB200_DTYPE_NONE have row pointers and columns only, and so has C: C_ij is present iff
+ * some product A_ik*B_kj exists, so rowptrC / colC are bit for bit those of the valued product of the same
+ * operands.  No value is read, multiplied, staged or stored.
+ *   bhb200_init_data_structure  HOST arrays, copied before the call returns; the rules of
+ *                               bhb200_init_data_op_* (transpose flags, stored row counts, the same host
+ *                               arrays for A and B uploaded once).
+ *   bhb200_init_data_device / _device_op with dtype BHB200_DTYPE_NONE: valA / valB are never read and may
+ *                               be NULL; with the arrays of valued device operands this gives their pattern
+ *                               without a copy.
+ *   bhb200_get_C_structure      rowptrC (m+1) and colC (nnzC) into HOST arrays, for any product (valued
+ *                               too); the NULL, BHB200_ERR_INVALID and BHB200_ERR_OVERFLOW rules of
+ *                               bhb200_get_C_f64.
+ * After a structure-only product, bhb200_get_C_f64 / _f32, bhb200_update_values_*, bhb200_spgemm_numeric,
+ * and bhb200_get_C_range / bhb200_copy_C_to_device with a non-NULL valC return BHB200_ERR_INVALID;
+ * bhb200_get_C_device sets *valC = NULL.  Masks and the row pointer, range and device getters work as for
+ * valued products; bhb200_stats.dtype is BHB200_DTYPE_NONE and its byte counts take 0 bytes per value.
+ * Multi-GPU products (bhb200_dist_setup_square) are valued only. */
+BHB200_API int bhb200_init_data_structure(bhb200_ctx *ctx, int opA, int opB, int m, int k, int n,
+                                          int nnzA, const int32_t *rowptrA, const int32_t *colA,
+                                          int nnzB, const int32_t *rowptrB, const int32_t *colB);
+BHB200_API int bhb200_get_C_structure(bhb200_ctx *ctx, int32_t *rowptrC, int32_t *colC);
+
 /* -- masked products: C = M .* (op(A)*op(B)) (GraphBLAS C<M> = A*B) ----------------------------------
  * M is m x n and structural: row pointers (m+1) and column indices, no values; its rows must be sorted
  * and duplicate-free with columns in [0, n), as the rows of B.  C_ij is present iff M_ij is present and
@@ -288,6 +315,7 @@ BHB200_API int bhb200_set_profiling(bhb200_ctx *ctx, int enabled);
 #define BHB200_DIST_ID_BYTES 128
 BHB200_API int bhb200_dist_unique_id(void *id);
 BHB200_API int bhb200_dist_init(bhb200_ctx *ctx, int rank, int nranks, const void *id);
+/* dist_setup_square takes BHB200_DTYPE_F32 or BHB200_DTYPE_F64 only (structure-only products are single-GPU) */
 BHB200_API int bhb200_dist_setup_square(bhb200_ctx *ctx, int root, int dtype, int n, int64_t nnz, const int32_t *rowptr,
                                         const int32_t *col, const void *val);
 BHB200_API int bhb200_dist_spgemm(bhb200_ctx *ctx);
