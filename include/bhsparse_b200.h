@@ -15,6 +15,21 @@
  * bhsparse_cuda.h:1730,1762).  Argument order is val, rowptr, colidx, as in the
  * reference.
  *
+ * Values (DESIGN.md §2, "The value contract").  For an entry C_ij with p products a_ik*b_kj, let
+ * s = sum |a_ik*b_kj| (exact), u the unit roundoff (2^-53 for f64, 2^-24 for f32), lam the smallest normal
+ * number (2^-1022 / 2^-126) and gamma(p) = p*u / (1 - p*u).
+ *  - Finite inputs whose exact partial sums cannot overflow: |c_hat - c| <= gamma(p)*s + 2*p*lam, in every
+ *    kernel and summation order.  The 2*p*lam term covers gradual underflow and the two f32 kernels that flush
+ *    subnormal products and partial sums to zero: k_num_large<float> and k_mask_global<float> add into global
+ *    memory with atomics that flush subnormals (RED/ATOMG.E.ADD.F32.FTZ on sm_100a).
+ *  - Integers with |a|, |b| <= 2^q and p * 2^(2q) <= 2^(t-1) (t = 53 for f64, 24 for f32) are summed exactly
+ *    in any order: the values are equal to the exact ones.
+ *  - Non-finite: any NaN product, or both a +inf and a -inf product, gives NaN; otherwise a +inf or -inf
+ *    product gives that infinity (products in the value type; inf * stored 0 is NaN).  An entry whose
+ *    products are all finite is finite.  Overflow of finite partial sums is unspecified.
+ *  - Not promised: the sign of a zero result, and bitwise identical results from two identical calls (some
+ *    kernels sum in the order atomics decide).
+ *
  * Every function returns BHB200_SUCCESS (0 == BHSPARSE_SUCCESS, common.h:26) or
  * a negative error code; nothing calls exit().  Not thread-safe per context
  * (the reference is not either, bhsparse_cuda.h:100-101); distinct contexts may
