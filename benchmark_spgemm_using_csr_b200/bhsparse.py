@@ -11,8 +11,9 @@ tests read like the reference driver (main.cu:104-135).
     bh.free_mem(); bh.freePlatform()
 
 Host arrays are numpy (or anything exposing a writable buffer of the right
-dtype); the value dtype (float32/float64) is taken from valA -- the reference
-needs a recompile for that (common.h:31, README.md:84-86).  With valA and valB both
+dtype); the value dtype (float32/float64/complex64) is taken from valA -- the reference
+needs a recompile for that (common.h:31, README.md:84-86).  complex128 is refused
+(ERR_INVALID), never converted.  With valA and valB both
 None the product is structure-only (BHB200_DTYPE_NONE): C has row pointers and
 columns, and get_C takes None for the values.
 """
@@ -31,6 +32,17 @@ BHSPARSE_CUDA = 1       # common.h:36
 
 def _ptr(a):
     return ctypes.c_void_p(a.ctypes.data)
+
+
+# value dtype -> (init_data_op, update_values, get_C) entry-point suffix
+_SUFFIX = {np.dtype(np.float64): "f64", np.dtype(np.float32): "f32", np.dtype(np.complex64): "c64"}
+
+
+def _op(trans) -> int:
+    """transA / transB: False / "N", True / "T", or "C" (conjugate transpose, complex64 only)"""
+    if trans == "C":
+        return capi.OP_C
+    return capi.OP_T if trans in (True, "T") else capi.OP_N
 
 
 class bhsparse:
@@ -70,6 +82,7 @@ class bhsparse:
                  nnzB, csrValB, csrRowPtrB, csrColIndB, csrRowPtrC, transA=False, transB=False) -> int:
         """C = op(A)*op(B): m, k, n are the dimensions of op(A) (m x k) and op(B) (k x n); with
         transA / transB the arrays hold A / B as stored, i.e. k x m / n x k (bhb200_init_data_op_*).
+        transA / transB = "C": conjugate transpose (complex64 values).
         csrValA and csrValB both None: structure-only product (bhb200_init_data_structure)."""
         if not self._ctx:
             return capi.ERR_INVALID
@@ -80,12 +93,12 @@ class bhsparse:
             return capi.ERR_INVALID
         else:
             valA = np.ascontiguousarray(csrValA)
-            if valA.dtype == np.float64:
-                fn, dt = self._lib.bhb200_init_data_op_f64, np.float64
-            elif valA.dtype == np.float32:
-                fn, dt = self._lib.bhb200_init_data_op_f32, np.float32
-            else:
+            dt = valA.dtype
+            if dt not in _SUFFIX:   # (complex128 too: never downcast)
                 return capi.ERR_INVALID
+            if dt == np.complex64 and np.asarray(csrValB).dtype != dt:   # (no mixed real x complex operands)
+                return capi.ERR_INVALID
+            fn = getattr(self._lib, "bhb200_init_data_op_" + _SUFFIX[dt])
             valB = np.ascontiguousarray(csrValB, dtype=dt)
         rpA = np.ascontiguousarray(csrRowPtrA, dtype=np.int32)
         cA = np.ascontiguousarray(csrColIndA, dtype=np.int32)
@@ -102,8 +115,7 @@ class bhsparse:
         self._structure = structure
         self._m = m
         # (the same host arrays for A and B stay the same objects here, so the library can upload them once)
-        opA = capi.OP_T if transA else capi.OP_N
-        opB = capi.OP_T if transB else capi.OP_N
+        opA, opB = _op(transA), _op(transB)
         if structure:
             return self._lib.bhb200_init_data_structure(self._ctx, opA, opB, m, k, n, nnzA, _ptr(rpA), _ptr(cA), nnzB,
                                                         _ptr(rpB), _ptr(cB))
@@ -148,7 +160,7 @@ class bhsparse:
         cp = ctypes.c_void_p(csrColIndC.ctypes.data) if csrColIndC is not None else None
         if csrValC is None:
             return self._lib.bhb200_get_C_structure(self._ctx, rp, cp)
-        fn = self._lib.bhb200_get_C_f64 if self._dtype == np.float64 else self._lib.bhb200_get_C_f32
+        fn = getattr(self._lib, "bhb200_get_C_" + _SUFFIX[self._dtype])
         return fn(self._ctx, rp, cp, ctypes.c_void_p(csrValC.ctypes.data))
 
     def free_mem(self) -> int:
@@ -162,7 +174,7 @@ class bhsparse:
         for v in (csrValA, csrValB):
             if v is not None and (v.dtype != self._dtype or not v.flags.c_contiguous):
                 return capi.ERR_INVALID
-        fn = self._lib.bhb200_update_values_f64 if self._dtype == np.float64 else self._lib.bhb200_update_values_f32
+        fn = getattr(self._lib, "bhb200_update_values_" + _SUFFIX[self._dtype])
         ap = ctypes.c_void_p(csrValA.ctypes.data) if csrValA is not None else None
         bp = ctypes.c_void_p(csrValB.ctypes.data) if csrValB is not None else None
         return fn(self._ctx, ap, bp)
@@ -225,12 +237,15 @@ def spgemm(A, B, device: int = 0, return_stats: bool = False, return_row_product
            transA: bool = False, transB: bool = False, mask=None, structure_only: bool = False):
     """Convenience driver following main.cu:104-135: C = op(A)*op(B) for two
     generators.CSR operands (op = transpose with transA / transB); returns
-    (rowptrC int32, colC int32, valC).  mask: a generators.CSR or (rowptr, col)
+    (rowptrC int32, colC int32, valC).  Values float32, float64 or complex64
+    (transA / transB may then be "C", the conjugate transpose).  mask: a generators.CSR or (rowptr, col)
     whose pattern restricts C (masked product, bhb200_set_mask).  structure_only:
     the pattern of C alone, from the operands' patterns (valC is None)."""
     platforms = [False] * NUM_PLATFORMS
     platforms[BHSPARSE_CUDA] = True
     bh = bhsparse(device)
+    if not structure_only and np.asarray(A.val).dtype == np.complex128:
+        raise capi.BhsparseError(capi.ERR_INVALID, "complex128 values are not supported: use complex64")
     m, k = (A.cols, A.rows) if transA else (A.rows, A.cols)
     n = B.rows if transB else B.cols
     rowptrC = np.zeros(m + 1, dtype=np.int32)

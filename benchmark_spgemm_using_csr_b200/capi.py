@@ -22,8 +22,10 @@ ERR_NO_DEVICE = -5
 DTYPE_F32 = 0
 DTYPE_F64 = 1
 DTYPE_NONE = 2   # structure only: row pointers and columns, no values
+DTYPE_C64 = 4    # complex64: two float32 (re, im) per value (3 is not a type)
 OP_N = 0
 OP_T = 1
+OP_C = 2         # conjugate transpose (complex64 operands only)
 NUM_BINS = 24
 NUM_MASK_BINS = 9
 MASK_BIN_NAMES = ["none", "esc<=32", "w64", "w256", "w1024", "c1024", "c4096", "c16384", "global"]
@@ -47,6 +49,7 @@ EXPORTED = [
     "bhb200_init_data_op_f64", "bhb200_init_data_op_f32", "bhb200_init_data_device_op",
     "bhb200_set_mask", "bhb200_set_mask_device", "bhb200_clear_mask",
     "bhb200_init_data_structure", "bhb200_get_C_structure",
+    "bhb200_init_data_op_c64", "bhb200_update_values_c64", "bhb200_get_C_c64",
 ]
 DIST_ID_BYTES = 128
 
@@ -120,6 +123,7 @@ def load(build_if_missing: bool = False):
                                           c_int, c_void_p, c_void_p, c_void_p]
     L.bhb200_init_data_op_f64.argtypes = [ctxp, c_int, c_int] + L.bhb200_init_data_f64.argtypes[1:]
     L.bhb200_init_data_op_f32.argtypes = L.bhb200_init_data_op_f64.argtypes
+    L.bhb200_init_data_op_c64.argtypes = L.bhb200_init_data_op_f64.argtypes
     L.bhb200_init_data_device_op.argtypes = [ctxp, c_int, c_int, c_int] + L.bhb200_init_data_device.argtypes[2:]
     L.bhb200_init_data_structure.argtypes = [ctxp, c_int, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_int,
                                              c_void_p, c_void_p]
@@ -134,11 +138,13 @@ def load(build_if_missing: bool = False):
     L.bhb200_synchronize.argtypes = [ctxp]
     L.bhb200_update_values_f64.argtypes = [ctxp, c_void_p, c_void_p]
     L.bhb200_update_values_f32.argtypes = [ctxp, c_void_p, c_void_p]
+    L.bhb200_update_values_c64.argtypes = [ctxp, c_void_p, c_void_p]
     L.bhb200_spgemm_numeric.argtypes = [ctxp]
     L.bhb200_get_nnzC.argtypes = [ctxp]
     L.bhb200_get_nnzC.restype = c_int64
     L.bhb200_get_C_f64.argtypes = [ctxp, c_void_p, c_void_p, c_void_p]
     L.bhb200_get_C_f32.argtypes = [ctxp, c_void_p, c_void_p, c_void_p]
+    L.bhb200_get_C_c64.argtypes = [ctxp, c_void_p, c_void_p, c_void_p]
     L.bhb200_get_rowptrC_i64.argtypes = [ctxp, c_void_p]
     L.bhb200_get_C_range.argtypes = [ctxp, c_int64, c_int64, c_void_p, c_void_p]
     L.bhb200_get_C_device.argtypes = [ctxp, POINTER(c_void_p), POINTER(c_void_p), POINTER(c_void_p), POINTER(c_void_p)]

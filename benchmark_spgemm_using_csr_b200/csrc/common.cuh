@@ -14,6 +14,7 @@
 #include <cuda_runtime.h>
 #include <stddef.h>
 #include <stdint.h>
+#include <type_traits>
 
 namespace bhb {
 
@@ -22,7 +23,7 @@ constexpr int SORT_PAD = 0x7fffffff;
 constexpr unsigned FULL = 0xffffffffu;
 
 // ---- value types -------------------------------------------------------------
-// The numeric kernels are templates on the value type VT (float, double).  Structure-only
+// The numeric kernels are templates on the value type VT (float, double, c64 below).  Structure-only
 // products (BHB200_DTYPE_NONE) instantiate them with NoVal: an empty type whose arithmetic,
 // shuffles, loads and atomics do nothing, so every value load, store and shared-memory access
 // compiles away and only the column work is left.  Shared-memory layouts are sized with
@@ -42,6 +43,90 @@ __device__ __forceinline__ NoVal __ldg(const NoVal *) { return NoVal(); }
 __device__ __forceinline__ NoVal atomicAdd(NoVal *, NoVal) { return NoVal(); }
 }  // namespace novalue
 using novalue::NoVal;
+
+// Complex products (BHB200_DTYPE_C64) instantiate them with c64: two floats (re, im), 8 bytes and 8-byte
+// aligned like float _Complex / std::complex<float> / torch.complex64, so every table, bin and plan sized for
+// double holds it unchanged.  The product is the naive formula (re = ar*br - ai*bi, im = ar*bi + ai*br; the
+// compiler may contract it into FMAs): each component is a real sum of the 2p real products, which is what the
+// value contract bounds.  Gauss's three-multiplication form would not keep that per-component bound.
+namespace cplx {   // (its own namespace, as novalue: the overloads below are found by argument-dependent lookup)
+struct __align__(8) c64 {
+    float re, im;
+    c64() = default;   // (trivial: c64 lives in extern shared memory and in __shared__ variables)
+    __host__ __device__ constexpr explicit c64(int v) : re((float)v), im(0.f) {}
+    __host__ __device__ constexpr c64(float r, float i) : re(r), im(i) {}
+    __host__ __device__ c64 operator*(const c64 b) const { return c64(re * b.re - im * b.im, re * b.im + im * b.re); }
+    __host__ __device__ c64 operator+(const c64 b) const { return c64(re + b.re, im + b.im); }
+    __host__ __device__ c64 &operator+=(const c64 b)
+    {
+        re += b.re;
+        im += b.im;
+        return *this;
+    }
+};
+// a*b + c, as fma does for the real types (the pattern kernel's long-row path)
+__device__ __forceinline__ c64 fma(const c64 a, const c64 b, const c64 c)
+{
+    return c64(fmaf(a.re, b.re, fmaf(-a.im, b.im, c.re)), fmaf(a.re, b.im, fmaf(a.im, b.re, c.im)));
+}
+__device__ __forceinline__ c64 __shfl_sync(unsigned mask, const c64 v, int src, int width = 32)
+{
+    return c64(::__shfl_sync(mask, v.re, src, width), ::__shfl_sync(mask, v.im, src, width));
+}
+__device__ __forceinline__ c64 __shfl_down_sync(unsigned mask, const c64 v, unsigned d, int width = 32)
+{
+    return c64(::__shfl_down_sync(mask, v.re, d, width), ::__shfl_down_sync(mask, v.im, d, width));
+}
+__device__ __forceinline__ c64 __ldg(const c64 *p)   // one 64-bit read-only load
+{
+    const float2 t = ::__ldg(reinterpret_cast<const float2 *>(p));
+    return c64(t.x, t.y);
+}
+// per component: two float atomics (shared or global memory); returns the old value
+__device__ __forceinline__ c64 atomicAdd(c64 *p, const c64 v)
+{
+    const float r = ::atomicAdd(&p->re, v.re);
+    return c64(r, ::atomicAdd(&p->im, v.im));
+}
+// complex double: the column-by-column reduction of k_num_bucket_heavy sums in double, as it does for the real types
+struct cdbl {
+    double re, im;
+    cdbl() = default;
+    __host__ __device__ constexpr cdbl(double r) : re(r), im(0.0) {}
+    __host__ __device__ constexpr cdbl(double r, double i) : re(r), im(i) {}
+    __host__ __device__ explicit cdbl(const c64 v) : re(v.re), im(v.im) {}
+    __host__ __device__ explicit operator c64() const { return c64((float)re, (float)im); }
+    __host__ __device__ cdbl &operator+=(const cdbl b)
+    {
+        re += b.re;
+        im += b.im;
+        return *this;
+    }
+    __host__ __device__ bool operator!=(const double b) const { return re != b || im != 0.0; }
+};
+__device__ __forceinline__ cdbl __shfl_xor_sync(unsigned mask, const cdbl v, int d, int width = 32)
+{
+    return cdbl(::__shfl_xor_sync(mask, v.re, d, width), ::__shfl_xor_sync(mask, v.im, d, width));
+}
+__device__ __forceinline__ cdbl atomicAdd(cdbl *p, const cdbl v)
+{
+    const double r = ::atomicAdd(&p->re, v.re);
+    return cdbl(r, ::atomicAdd(&p->im, v.im));
+}
+}  // namespace cplx
+using cplx::c64;
+static_assert(sizeof(c64) == 8 && alignof(c64) == 8, "complex64 is two floats, 8-byte aligned");
+
+// the type k_num_bucket_heavy sums one column's products in: double for the real types, cdbl for c64
+template <typename VT>
+struct WideSum {
+    using type = double;
+};
+template <>
+struct WideSum<c64> {
+    using type = cplx::cdbl;
+};
+
 template <typename VT>
 constexpr size_t value_bytes = sizeof(VT);
 template <>
@@ -633,10 +718,11 @@ struct TransposeOut {
 };
 size_t transpose_scratch_bytes(int nnz, int cols);
 int transpose_passes(int cols);
-cudaError_t launch_transpose(const LaunchCtx &lc, int dtype, int rows, int cols, int nnz, Csr X, TransposeOut out,
+// conj: complex64 values are conjugated as they move (BHB200_OP_C)
+cudaError_t launch_transpose(const LaunchCtx &lc, int dtype, bool conj, int rows, int cols, int nnz, Csr X, TransposeOut out,
                              void *scratch, int *bad, int bad_bit);
-// values again through the permutation of the last transposition: valT[p] = val[perm[p]]
-cudaError_t launch_regather(const LaunchCtx &lc, int dtype, int nnz, const void *val, const int *perm, void *valT);
+// values again through the permutation of the last transposition: valT[p] = val[perm[p]] (conjugated with conj)
+cudaError_t launch_regather(const LaunchCtx &lc, int dtype, bool conj, int nnz, const void *val, const int *perm, void *valT);
 // stage_masked.cu: the mask M (m x n, structural) and where the masked kernels put their rows
 struct MaskCsr {
     const int *rowptr;
@@ -680,9 +766,9 @@ int large_scratch_blocks(int sm_count, int n);
 cudaError_t launch_sym_range(const LaunchCtx &lc, int nsum, const int *queue, int count, Csr A, Csr B, const int *rlo,
                              int *rc, Counters *ctr, WordLists wl);
 
-// The numeric kernels of one value type (stage_numeric_f32.cu / _f64.cu / _none.cu); values are float or double
-// as the operands are, or none (NoVal: columns only, value pointers never read).  The three types compile in three
-// translation units, in parallel.
+// The numeric kernels of one value type (stage_numeric_f32.cu / _f64.cu / _none.cu / _c64.cu); values are float,
+// double or complex64 as the operands are, or none (NoVal: columns only, value pointers never read).  The four types
+// compile in four translation units, in parallel.
 struct ColumnCdf {
     const unsigned *cdf;   // [CDF_KNOTS + 1], non-decreasing, cdf[0] = 0
     int shift;             // column >> shift < CDF_KNOTS
@@ -715,10 +801,30 @@ struct NumericKernels {
     cudaError_t (*copy_ct)(const LaunchCtx &lc, const int *queue, int count, const int64_t *rowoff, const long long *ct_off,
                            const int *ctcol, const void *ctval, int *colC, void *valC, double avg_row);
 };
-extern const NumericKernels NUMERIC_F32, NUMERIC_F64, NUMERIC_NONE;
+extern const NumericKernels NUMERIC_F32, NUMERIC_F64, NUMERIC_NONE, NUMERIC_C64;
+
+// The one place a BHB200_DTYPE_* becomes a value type: f(VT()) with VT = float, double, NoVal or c64 (host code;
+// the launchers call it with a generic lambda and take the type as decltype of its argument).
+template <typename F>
+inline decltype(auto) dispatch_value_type(int dtype, F &&f)
+{
+    switch (dtype) {
+    case BHB200_DTYPE_F64: return f(double());
+    case BHB200_DTYPE_NONE: return f(NoVal());
+    case BHB200_DTYPE_C64: return f(c64());
+    default: return f(float());
+    }
+}
+
 inline const NumericKernels &numeric_kernels(int dtype)
 {
-    return dtype == BHB200_DTYPE_F64 ? NUMERIC_F64 : dtype == BHB200_DTYPE_NONE ? NUMERIC_NONE : NUMERIC_F32;
+    return dispatch_value_type(dtype, [](auto v) -> const NumericKernels & {
+        using VT = decltype(v);
+        if constexpr (std::is_same_v<VT, double>) return NUMERIC_F64;
+        else if constexpr (std::is_same_v<VT, NoVal>) return NUMERIC_NONE;
+        else if constexpr (std::is_same_v<VT, c64>) return NUMERIC_C64;
+        else return NUMERIC_F32;
+    });
 }
 
 }  // namespace bhb

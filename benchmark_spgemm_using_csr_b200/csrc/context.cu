@@ -44,7 +44,12 @@ int fail(bhb200_ctx *c, int code, const char *what, cudaError_t e = cudaSuccess)
 
 size_t vsize(int dtype)
 {
-    return dtype == BHB200_DTYPE_F64 ? 8 : dtype == BHB200_DTYPE_NONE ? 0 : 4;
+    return dispatch_value_type(dtype, [](auto v) { return value_bytes<decltype(v)>; });
+}
+
+const char *dtype_name(int dtype)
+{
+    return dtype == BHB200_DTYPE_F64 ? "f64" : dtype == BHB200_DTYPE_C64 ? "c64" : "f32";
 }
 
 int refuse_structure(bhb200_ctx *ctx, const char *what)
@@ -102,10 +107,13 @@ int check_dims(bhb200_ctx *ctx, int dtype, int m, int k, int n, int nnzA, int nn
     return BHB200_SUCCESS;
 }
 
-int check_ops(bhb200_ctx *ctx, int opA, int opB)
+int check_ops(bhb200_ctx *ctx, int dtype, int opA, int opB)
 {
-    if ((opA != BHB200_OP_N && opA != BHB200_OP_T) || (opB != BHB200_OP_N && opB != BHB200_OP_T))
-        return fail(ctx, BHB200_ERR_INVALID, "op must be BHB200_OP_N or BHB200_OP_T");
+    const int last = dtype == BHB200_DTYPE_C64 ? BHB200_OP_C : BHB200_OP_T;
+    if (opA < BHB200_OP_N || opA > last || opB < BHB200_OP_N || opB > last)
+        return fail(ctx, BHB200_ERR_INVALID,
+                    dtype == BHB200_DTYPE_C64 ? "op must be BHB200_OP_N, BHB200_OP_T or BHB200_OP_C"
+                                              : "op must be BHB200_OP_N or BHB200_OP_T (BHB200_OP_C needs complex64 operands)");
     return BHB200_SUCCESS;
 }
 
@@ -157,13 +165,13 @@ int run_transposes(bhb200_ctx *ctx, const LaunchCtx &lc)
     Counters *d_ctr = ctx->counters.as<Counters>();
     CU(cudaMemsetAsync(&d_ctr->bad_T, 0, sizeof(int), lc.stream), "zero transpose flag");
     if (ctx->opA)
-        CU(launch_transpose(lc, ctx->dtype, ctx->k, ctx->m, ctx->nnzA, ctx->As,
+        CU(launch_transpose(lc, ctx->dtype, ctx->opA == BHB200_OP_C, ctx->k, ctx->m, ctx->nnzA, ctx->As,
                             TransposeOut{ctx->at_rowptr.as<int>(), ctx->at_col.as<int>(), keep_perm ? ctx->at_val.p : nullptr,
                                          keep_perm ? ctx->at_perm.as<int>() : scratch_perm},
                             ctx->t_scratch.p, &d_ctr->bad_T, 1),
            "transpose A");
     if (tb)
-        CU(launch_transpose(lc, ctx->dtype, ctx->n, ctx->k, ctx->nnzB, ctx->Bs,
+        CU(launch_transpose(lc, ctx->dtype, ctx->opB == BHB200_OP_C, ctx->n, ctx->k, ctx->nnzB, ctx->Bs,
                             TransposeOut{ctx->bt_rowptr.as<int>(), ctx->bt_col.as<int>(), keep_perm ? ctx->bt_val.p : nullptr,
                                          keep_perm ? ctx->bt_perm.as<int>() : scratch_perm},
                             ctx->t_scratch.p, &d_ctr->bad_T, 2),
@@ -176,9 +184,9 @@ int run_transposes(bhb200_ctx *ctx, const LaunchCtx &lc)
 int run_regathers(bhb200_ctx *ctx, const LaunchCtx &lc)
 {
     if (ctx->opA)
-        CU(launch_regather(lc, ctx->dtype, ctx->nnzA, ctx->As.val, ctx->at_perm.as<int>(), ctx->at_val.p), "re-gather values of A^T");
+        CU(launch_regather(lc, ctx->dtype, ctx->opA == BHB200_OP_C, ctx->nnzA, ctx->As.val, ctx->at_perm.as<int>(), ctx->at_val.p), "re-gather values of A^T");
     if (ctx->opB && !ctx->t_shared)
-        CU(launch_regather(lc, ctx->dtype, ctx->nnzB, ctx->Bs.val, ctx->bt_perm.as<int>(), ctx->bt_val.p), "re-gather values of B^T");
+        CU(launch_regather(lc, ctx->dtype, ctx->opB == BHB200_OP_C, ctx->nnzB, ctx->Bs.val, ctx->bt_perm.as<int>(), ctx->bt_val.p), "re-gather values of B^T");
     return BHB200_SUCCESS;
 }
 
@@ -195,7 +203,7 @@ int init_host(bhb200_ctx *ctx, int dtype, int opA, int opB, int m, int k, int n,
               const int32_t *colB)
 {
     if (!ctx) return BHB200_ERR_INVALID;
-    int rc = check_ops(ctx, opA, opB);
+    int rc = check_ops(ctx, dtype, opA, opB);
     if (rc) return rc;
     rc = check_dims(ctx, dtype, m, k, n, nnzA, nnzB, valA, rowptrA, colA, valB, rowptrB, colB);
     if (rc) return rc;
@@ -241,7 +249,7 @@ int init_host(bhb200_ctx *ctx, int dtype, int opA, int opB, int m, int k, int n,
     ctx->nnzB = nnzB;
     ctx->opA = opA;
     ctx->opB = opB;
-    ctx->t_shared = alias && opA && opB;
+    ctx->t_shared = alias && opA && opA == opB;   // one transposed copy serves (T, T) and (C, C)
     ctx->have_data = false;
     rc = set_effective(ctx);
     if (rc) return rc;
@@ -343,7 +351,6 @@ int run_numeric_bins(bhb200_ctx *ctx, const LaunchCtx &lc, const int *num_bin, c
 {
     int rc = 0;
     const NumericKernels &nk = numeric_kernels(ctx->dtype);
-    const bool f64 = ctx->dtype == BHB200_DTYPE_F64;   // (for the error messages)
     int *queue = ctx->queue.as<int>();
     int64_t *rowoff = ctx->rowoff64.as<int64_t>();
     int *rlo = ctx->rlo.as<int>();
@@ -358,7 +365,7 @@ int run_numeric_bins(bhb200_ctx *ctx, const LaunchCtx &lc, const int *num_bin, c
     for (int b = NB_G64; b <= NB_B16384; ++b) {
         if (num_bin[b] > 0) CU(stamp(ctx, 1, b), "event");
         CU(nk.hash(lc, b, G, queue + no.off[b], num_bin[b], ctx->A, ctx->B, rowoff, colC, valC),
-           f64 ? "numeric hash f64" : "numeric hash f32");
+           (std::string("numeric hash ") + dtype_name(ctx->dtype)).c_str());
     }
     if (num_bin[NB_LARGE] > 0) {
         rc = reserve_large_scratch(ctx, true);
@@ -367,7 +374,7 @@ int run_numeric_bins(bhb200_ctx *ctx, const LaunchCtx &lc, const int *num_bin, c
         CU(stamp(ctx, 1, NB_LARGE), "event");
         CU(nk.large(lc, queue + no.off[NB_LARGE], num_bin[NB_LARGE], ctx->n, ctx->A, ctx->B, rowoff, colC, valC,
                     ctx->bitmap.as<unsigned>(), ctx->prefix.as<int>(), sb),
-           f64 ? "numeric large f64" : "numeric large f32");
+           (std::string("numeric large ") + dtype_name(ctx->dtype)).c_str());
     }
     {
         const int rb[4] = {NB_RANGE_S128, NB_RANGE_S512, NB_RANGE_L128, NB_RANGE_L512};
@@ -378,7 +385,7 @@ int run_numeric_bins(bhb200_ctx *ctx, const LaunchCtx &lc, const int *num_bin, c
             if (num_bin[b] <= 0) continue;
             CU(stamp(ctx, 1, b), "event");
             CU(nk.range(lc, rnsum[i], rnacc[i], queue + no.off[b], num_bin[b], ctx->A, ctx->B, rlo, rowoff, colC, valC, wl),
-               f64 ? "numeric range f64" : "numeric range f32");
+               (std::string("numeric range ") + dtype_name(ctx->dtype)).c_str());
         }
     }
     return BHB200_SUCCESS;
@@ -1110,6 +1117,13 @@ int bhb200_init_data_op_f32(bhb200_ctx *ctx, int opA, int opB, int m, int k, int
     return init_host(ctx, BHB200_DTYPE_F32, opA, opB, m, k, n, nnzA, valA, rowptrA, colA, nnzB, valB, rowptrB, colB);
 }
 
+int bhb200_init_data_op_c64(bhb200_ctx *ctx, int opA, int opB, int m, int k, int n, int nnzA, const float *valA,
+                            const int32_t *rowptrA, const int32_t *colA, int nnzB, const float *valB, const int32_t *rowptrB,
+                            const int32_t *colB)
+{
+    return init_host(ctx, BHB200_DTYPE_C64, opA, opB, m, k, n, nnzA, valA, rowptrA, colA, nnzB, valB, rowptrB, colB);
+}
+
 int bhb200_init_data_structure(bhb200_ctx *ctx, int opA, int opB, int m, int k, int n, int nnzA, const int32_t *rowptrA,
                                const int32_t *colA, int nnzB, const int32_t *rowptrB, const int32_t *colB)
 {
@@ -1129,12 +1143,15 @@ int bhb200_init_data_device_op(bhb200_ctx *ctx, int dtype, int opA, int opB, int
                                const int32_t *rowptrB, const int32_t *colB)
 {
     if (!ctx) return BHB200_ERR_INVALID;
-    if (dtype != BHB200_DTYPE_F32 && dtype != BHB200_DTYPE_F64 && dtype != BHB200_DTYPE_NONE)
+    if (dtype != BHB200_DTYPE_F32 && dtype != BHB200_DTYPE_F64 && dtype != BHB200_DTYPE_NONE && dtype != BHB200_DTYPE_C64)
         return fail(ctx, BHB200_ERR_INVALID, "bad dtype");
-    int rc = check_ops(ctx, opA, opB);
+    int rc = check_ops(ctx, dtype, opA, opB);
     if (rc) return rc;
     rc = check_dims(ctx, dtype, m, k, n, nnzA, nnzB, valA, rowptrA, colA, valB, rowptrB, colB);
     if (rc) return rc;
+    // (checked here, before any kernel reads them: the kernels load complex64 values as 8-byte words)
+    if (dtype == BHB200_DTYPE_C64 && (((uintptr_t)valA | (uintptr_t)valB) & 7u))
+        return fail(ctx, BHB200_ERR_INVALID, "complex64 value arrays must be 8-byte aligned");
     CU(cudaSetDevice(ctx->device), "cudaSetDevice");
     release_operands(ctx);
     const bool values = dtype != BHB200_DTYPE_NONE;   // (structure only: the caller's value pointers are never read)
@@ -1410,6 +1427,11 @@ int bhb200_update_values_f32(bhb200_ctx *ctx, const float *valA, const float *va
     return update_values_any(ctx, BHB200_DTYPE_F32, valA, valB);
 }
 
+int bhb200_update_values_c64(bhb200_ctx *ctx, const float *valA, const float *valB)
+{
+    return update_values_any(ctx, BHB200_DTYPE_C64, valA, valB);
+}
+
 int bhb200_set_profiling(bhb200_ctx *ctx, int enabled)
 {
     if (!ctx) return BHB200_ERR_INVALID;
@@ -1514,6 +1536,11 @@ int bhb200_get_C_f32(bhb200_ctx *ctx, int32_t *rowptrC, int32_t *colC, float *va
 {
     return get_C_any(ctx, BHB200_DTYPE_F32, rowptrC, colC, valC);
 }
+int bhb200_get_C_c64(bhb200_ctx *ctx, int32_t *rowptrC, int32_t *colC, float *valC)
+{
+    return get_C_any(ctx, BHB200_DTYPE_C64, rowptrC, colC, valC);
+}
+
 int bhb200_get_C_structure(bhb200_ctx *ctx, int32_t *rowptrC, int32_t *colC)
 {
     return get_C_any(ctx, BHB200_DTYPE_NONE, rowptrC, colC, nullptr);

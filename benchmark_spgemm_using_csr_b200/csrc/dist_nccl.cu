@@ -284,12 +284,14 @@ int bhb200_dist_setup_square(bhb200_ctx *ctx, int root, int dtype, int n, int64_
     if (!ctx || !ctx->dist) return dfail(ctx, BHB200_ERR_INVALID, "bhb200_dist_init first");
     DistState *d = ctx->dist;
     if (root < 0 || root >= d->nranks || n < 0 || nnz < 0 || nnz > 0x7fffffffLL) return dfail(ctx, BHB200_ERR_INVALID, "bad argument");
-    if (dtype != BHB200_DTYPE_F32 && dtype != BHB200_DTYPE_F64) return dfail(ctx, BHB200_ERR_INVALID, "bad dtype");
+    if (dtype != BHB200_DTYPE_F32 && dtype != BHB200_DTYPE_F64 && dtype != BHB200_DTYPE_C64)
+        return dfail(ctx, BHB200_ERR_INVALID, "bad dtype");
     const bool is_root = d->rank == root;
     if (is_root && (!rowptr || (nnz > 0 && (!col || !val)))) return dfail(ctx, BHB200_ERR_INVALID, "null B on the root");
     DCU(cudaSetDevice(ctx->device), "cudaSetDevice");
     cudaStream_t s = ctx->stream;
-    const size_t vs = dtype == BHB200_DTYPE_F64 ? 8 : 4;
+    const size_t vs = dtype == BHB200_DTYPE_F32 ? 4 : 8;
+    if (is_root && vs == 8 && ((uintptr_t)val & 7u)) return dfail(ctx, BHB200_ERR_INVALID, "valB is not 8-byte aligned");
     // forget the previous operands (library-owned buffers are reused by reserve())
     ctx->have_data = false;
     ctx->have_C = false;
@@ -368,7 +370,8 @@ int bhb200_dist_setup_square(bhb200_ctx *ctx, int root, int dtype, int n, int64_
     DCU(cudaEventRecord(d->ev_ready, s), "event");
     DCU(cudaStreamWaitEvent(d->val_stream, d->ev_ready, 0), "wait");
     if (nnz > 0)
-        DNC(nccl().Broadcast(b_val, b_val, (size_t)nnz, dtype == BHB200_DTYPE_F64 ? ncclFloat64 : ncclFloat32, root, d->comm,
+        // (values only move: complex64 as 8-byte words)
+        DNC(nccl().Broadcast(b_val, b_val, (size_t)nnz, vs == 8 ? ncclFloat64 : ncclFloat32, root, d->comm,
                              d->val_stream),
             "ncclBroadcast(valB)");
     DCU(cudaEventRecord(d->ev_val, d->val_stream), "event");

@@ -587,7 +587,8 @@ k_num_bucket_heavy(const int *__restrict__ queue, const int count, const int *__
     __shared__ int s_stack_lg[40];
     __shared__ long long s_row_base;
     __shared__ int s_min;
-    __shared__ double s_sum;
+    using Wide = typename WideSum<VT>::type;   // (double; two doubles for c64)
+    __shared__ Wide s_sum;
     const int lane = threadIdx.x & 31;
     const int nrows = count_dev ? min(*count_dev, count) : count;   // (retry kernel: the queue was filled on the device)
 
@@ -666,12 +667,12 @@ k_num_bucket_heavy(const int *__restrict__ queue, const int count, const int *__
                         const int cmin = s_min;
                         if (cmin == 0x7fffffff) break;
                         if constexpr (value_bytes<VT> > 0) {
-                            double part = 0.0;
+                            Wide part = 0.0;
                             for (int j = a0 + (int)(threadIdx.x >> 5); j < a1; j += THREADS / 32) {
                                 const int k = colA[j];
                                 const VT av = valA[j];
                                 for (int e = rowptrB[k] + lane; e < rowptrB[k + 1]; e += 32)
-                                    if (colB[e] == cmin) part += (double)(av * valB[e]);
+                                    if (colB[e] == cmin) part += Wide(av * valB[e]);
                             }
                             part = warp_sum(part);
                             if (lane == 0 && part != 0.0) atomicAdd(&s_sum, part);

@@ -519,9 +519,8 @@ cudaError_t launch_mask_bin(const LaunchCtx &lc, int dtype, int bin, const int *
                             const int4 *brange, MaskCsr M, MaskOut o)
 {
     if (count <= 0) return cudaSuccess;
-    if (dtype == BHB200_DTYPE_NONE) return launch_mask_bin_t<NoVal>(lc, bin, queue, count, A, B, brange, M, o);   // (hit flags only)
-    return dtype == BHB200_DTYPE_F64 ? launch_mask_bin_t<double>(lc, bin, queue, count, A, B, brange, M, o)
-                                     : launch_mask_bin_t<float>(lc, bin, queue, count, A, B, brange, M, o);
+    // (NoVal: hit flags only)
+    return dispatch_value_type(dtype, [&](auto v) { return launch_mask_bin_t<decltype(v)>(lc, bin, queue, count, A, B, brange, M, o); });
 }
 
 }  // namespace bhb

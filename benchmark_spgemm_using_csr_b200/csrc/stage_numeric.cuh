@@ -1,5 +1,6 @@
 // stage_numeric.cuh -- numeric kernels (hash accumulate, sort, write C in place),
-// instantiated for float in stage_numeric_f32.cu and double in stage_numeric_f64.cu.
+// instantiated for float in stage_numeric_f32.cu, double in stage_numeric_f64.cu, complex64 in stage_numeric_c64.cu
+// and NoVal in stage_numeric_none.cu.
 //
 // k_num_group<VT,G,LOG2T,R> : a group of G lanes owns a row: T-slot (column,value) table in
 //      shared memory, B rows streamed one per step (columns of one B row are distinct, so the

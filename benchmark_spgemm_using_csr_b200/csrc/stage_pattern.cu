@@ -498,6 +498,16 @@ __device__ __forceinline__ float lds_val(unsigned a, float)
 }
 __device__ __forceinline__ void sts_val(unsigned a, double v) { asm volatile("st.shared.f64 [%0], %1;" ::"r"(a), "d"(v) : "memory"); }
 __device__ __forceinline__ void sts_val(unsigned a, float v) { asm volatile("st.shared.f32 [%0], %1;" ::"r"(a), "f"(v) : "memory"); }
+__device__ __forceinline__ c64 lds_val(unsigned a, c64)
+{
+    c64 v;
+    asm volatile("ld.shared.v2.f32 {%0, %1}, [%2];" : "=f"(v.re), "=f"(v.im) : "r"(a) : "memory");
+    return v;
+}
+__device__ __forceinline__ void sts_val(unsigned a, c64 v)
+{
+    asm volatile("st.shared.v2.f32 [%0], {%1, %2};" ::"r"(a), "f"(v.re), "f"(v.im) : "memory");
+}
 
 // Predicated (not branched) element load and accumulate of the hot loop: inactive lanes issue no memory
 // access at all, and the warp stays converged.
@@ -562,6 +572,27 @@ __device__ __forceinline__ void pat_accum_if(const bool on, const unsigned mp, c
         "r"(mp), "r"(acc_s), "f"(av), "f"(bv)
         : "memory");
 }
+// complex64: the 8-byte accumulator slot of a double, four FMAs (re += ar*br + (-ai)*bi, im += ar*bi + ai*br)
+__device__ __forceinline__ void pat_accum_if(const bool on, const unsigned mp, const unsigned acc_s, const c64 av, const c64 bv)
+{
+    asm volatile(
+        "{\n"
+        ".reg .pred p;\n"
+        ".reg .u32 q, a;\n"
+        ".reg .f32 vr, vi;\n"
+        "setp.ne.s32 p, %0, 0;\n"
+        "@p ld.shared.u8 q, [%1];\n"
+        "@p mad.lo.u32 a, q, 8, %2;\n"
+        "@p ld.shared.v2.f32 {vr, vi}, [a];\n"
+        "@p fma.rn.f32 vr, %3, %5, vr;\n"
+        "@p fma.rn.f32 vr, %7, %6, vr;\n"
+        "@p fma.rn.f32 vi, %3, %6, vi;\n"
+        "@p fma.rn.f32 vi, %4, %5, vi;\n"
+        "@p st.shared.v2.f32 [a], {vr, vi};\n"
+        "}\n" ::"r"((int)on),
+        "r"(mp), "r"(acc_s), "f"(av.re), "f"(av.im), "f"(bv.re), "f"(bv.im), "f"(-av.im)
+        : "memory");
+}
 
 template <typename VT>
 struct PatRec;
@@ -577,6 +608,14 @@ template <>
 struct PatRec<float> {
     static __device__ __forceinline__ int4 pack(int bs, int lj, float v) { return make_int4(bs, lj, __float_as_int(v), 0); }
     static __device__ __forceinline__ float val(const int4 &r) { return __int_as_float(r.z); }
+};
+template <>
+struct PatRec<c64> {   // {bs, lj, re, im}
+    static __device__ __forceinline__ int4 pack(int bs, int lj, c64 v)
+    {
+        return make_int4(bs, lj, __float_as_int(v.re), __float_as_int(v.im));
+    }
+    static __device__ __forceinline__ c64 val(const int4 &r) { return c64(__int_as_float(r.z), __int_as_float(r.w)); }
 };
 
 // LONGB: rows of B may hold more than G entries (only possible for G = 32 with more than 32 diagonals in B)
@@ -775,16 +814,17 @@ cudaError_t launch_pat_numeric(const LaunchCtx &lc, int dtype, int m, Csr A, Csr
         return cudaGetLastError();
     }
     const int G = t.nDB <= 8 ? 8 : t.nDB <= 16 ? 16 : 32;
-    if (dtype == BHB200_DTYPE_F64) {
-        double *v = (double *)valC;
-        if (G == 8) return launch_pat_numeric_t<double, 8>(lc, m, A, B, ta, tb, t, outmask, rowoff, colC, v);
-        if (G == 16) return launch_pat_numeric_t<double, 16>(lc, m, A, B, ta, tb, t, outmask, rowoff, colC, v);
-        return launch_pat_numeric_t<double, 32>(lc, m, A, B, ta, tb, t, outmask, rowoff, colC, v);
-    }
-    float *v = (float *)valC;
-    if (G == 8) return launch_pat_numeric_t<float, 8>(lc, m, A, B, ta, tb, t, outmask, rowoff, colC, v);
-    if (G == 16) return launch_pat_numeric_t<float, 16>(lc, m, A, B, ta, tb, t, outmask, rowoff, colC, v);
-    return launch_pat_numeric_t<float, 32>(lc, m, A, B, ta, tb, t, outmask, rowoff, colC, v);
+    return dispatch_value_type(dtype, [&](auto val) {
+        using VT = decltype(val);
+        if constexpr (value_bytes<VT> == 0) {
+            return cudaErrorInvalidValue;   // (handled above)
+        } else {
+            VT *v = (VT *)valC;
+            if (G == 8) return launch_pat_numeric_t<VT, 8>(lc, m, A, B, ta, tb, t, outmask, rowoff, colC, v);
+            if (G == 16) return launch_pat_numeric_t<VT, 16>(lc, m, A, B, ta, tb, t, outmask, rowoff, colC, v);
+            return launch_pat_numeric_t<VT, 32>(lc, m, A, B, ta, tb, t, outmask, rowoff, colC, v);
+        }
+    });
 }
 
 }  // namespace bhb

@@ -55,6 +55,18 @@ __device__ __forceinline__ void load_vals4(const double *__restrict__ valB, cons
         v[3] = b.y;
     }
 }
+// complex64: 16 bytes hold two values, as for double
+__device__ __forceinline__ void load_vals4(const c64 *__restrict__ valB, const unsigned e0, const unsigned hi, c64 (&v)[4])
+{
+    const float4 a = __ldg(reinterpret_cast<const float4 *>(valB + e0));
+    v[0] = c64(a.x, a.y);
+    v[1] = c64(a.z, a.w);
+    if (e0 + 2u < hi) {
+        const float4 b = __ldg(reinterpret_cast<const float4 *>(valB + e0) + 1);
+        v[2] = c64(b.x, b.y);
+        v[3] = c64(b.z, b.w);
+    }
+}
 __device__ __forceinline__ void load_vals4(const float *__restrict__ valB, const unsigned e0, const unsigned,
                                            float (&v)[4])
 {

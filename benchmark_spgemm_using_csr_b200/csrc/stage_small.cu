@@ -183,9 +183,10 @@ cudaError_t launch_num_esc(const LaunchCtx &lc, int dtype, const int *queue, int
                            const int64_t *rowoff, int *colC, void *valC)
 {
     if (count <= 0) return cudaSuccess;
-    if (dtype == BHB200_DTYPE_NONE) return launch_num_esc_t<NoVal>(lc, queue, count, n, A, B, rowoff, colC, (NoVal *)valC);
-    return dtype == BHB200_DTYPE_F64 ? launch_num_esc_t<double>(lc, queue, count, n, A, B, rowoff, colC, (double *)valC)
-                                     : launch_num_esc_t<float>(lc, queue, count, n, A, B, rowoff, colC, (float *)valC);
+    return dispatch_value_type(dtype, [&](auto v) {
+        using VT = decltype(v);
+        return launch_num_esc_t<VT>(lc, queue, count, n, A, B, rowoff, colC, (VT *)valC);
+    });
 }
 
 template <typename VT>
@@ -204,9 +205,10 @@ cudaError_t launch_num_single(const LaunchCtx &lc, int dtype, const int *queue, 
                               const int64_t *rowoff, int *colC, void *valC)
 {
     if (count <= 0) return cudaSuccess;
-    if (dtype == BHB200_DTYPE_NONE) return launch_num_single_t<NoVal>(lc, queue, count, A, B, rowoff, colC, (NoVal *)valC);
-    return dtype == BHB200_DTYPE_F64 ? launch_num_single_t<double>(lc, queue, count, A, B, rowoff, colC, (double *)valC)
-                                     : launch_num_single_t<float>(lc, queue, count, A, B, rowoff, colC, (float *)valC);
+    return dispatch_value_type(dtype, [&](auto v) {
+        using VT = decltype(v);
+        return launch_num_single_t<VT>(lc, queue, count, A, B, rowoff, colC, (VT *)valC);
+    });
 }
 
 }  // namespace bhb

@@ -36,6 +36,18 @@ __device__ __forceinline__ unsigned lanemask_lt()
     return m;
 }
 
+// Values only move here.  The conjugate transpose of complex64 operands (BHB200_OP_C) moves them as Conj8: 8-byte words
+// with the sign bit of the imaginary part (bit 63) flipped, which conjugates NaN, inf and zero exactly.
+struct Conj8 {
+    unsigned long long bits;
+};
+template <typename V>
+__device__ __forceinline__ V moved(const V v)
+{
+    return v;
+}
+__device__ __forceinline__ Conj8 moved(const Conj8 v) { return Conj8{v.bits ^ 0x8000000000000000ull}; }
+
 __device__ __forceinline__ int masked_key(int key, int cols)
 {
     return (unsigned)key < (unsigned)cols ? key : 0;
@@ -220,7 +232,7 @@ __global__ void __launch_bounds__(TR_THREADS) k_tr_scatter(const int nnz, const 
             idx_out[pos] = src;
             if (LAST) {
                 colT[pos] = rowidx[src];
-                valT[pos] = val[src];
+                valT[pos] = moved(val[src]);
             }
         }
     }
@@ -237,7 +249,7 @@ __global__ void __launch_bounds__(256) k_tr_identity(const int nnz, const int co
     for (long long e = (long long)blockIdx.x * blockDim.x + threadIdx.x; e < nnz; e += (long long)gridDim.x * blockDim.x) {
         badl |= (unsigned)col[e] >= (unsigned)cols;
         perm[e] = (int)e;
-        valT[e] = val[e];
+        valT[e] = moved(val[e]);
     }
     if (badl && bad) atomicOr(bad, bad_bit);
     if (blockIdx.x == 0 && threadIdx.x == 0) {
@@ -266,7 +278,7 @@ __global__ void __launch_bounds__(256) k_tr_gather(const int nnz, const V *__res
                                                    V *__restrict__ valT)
 {
     for (long long p = (long long)blockIdx.x * blockDim.x + threadIdx.x; p < nnz; p += (long long)gridDim.x * blockDim.x)
-        valT[p] = val[perm[p]];
+        valT[p] = moved(val[perm[p]]);
 }
 
 int pass_count(int cols, int *bits_out)
@@ -367,24 +379,38 @@ int transpose_passes(int cols)
     return pass_count(cols, nullptr);
 }
 
-cudaError_t launch_transpose(const LaunchCtx &lc, int dtype, int rows, int cols, int nnz, Csr X, TransposeOut out,
-                             void *scratch, int *bad, int bad_bit)
+// the type the values move as: complex64 as double (8-byte words), Conj8 for conjugation
+template <typename F>
+cudaError_t with_mover(int dtype, bool conj, F &&f)
 {
-    if (dtype == BHB200_DTYPE_NONE) return transpose_typed<NoVal>(lc, rows, cols, nnz, X, out, scratch, bad, bad_bit);
-    return dtype == BHB200_DTYPE_F64 ? transpose_typed<double>(lc, rows, cols, nnz, X, out, scratch, bad, bad_bit)
-                      : transpose_typed<float>(lc, rows, cols, nnz, X, out, scratch, bad, bad_bit);
+    if (conj) return f(Conj8());
+    return dispatch_value_type(dtype, [&](auto v) {
+        using V = decltype(v);
+        return f(std::conditional_t<std::is_same_v<V, c64>, double, V>());
+    });
 }
 
-cudaError_t launch_regather(const LaunchCtx &lc, int dtype, int nnz, const void *val, const int *perm, void *valT)
+cudaError_t launch_transpose(const LaunchCtx &lc, int dtype, bool conj, int rows, int cols, int nnz, Csr X, TransposeOut out,
+                             void *scratch, int *bad, int bad_bit)
+{
+    return with_mover(dtype, conj, [&](auto v) {
+        return transpose_typed<decltype(v)>(lc, rows, cols, nnz, X, out, scratch, bad, bad_bit);
+    });
+}
+
+cudaError_t launch_regather(const LaunchCtx &lc, int dtype, bool conj, int nnz, const void *val, const int *perm, void *valT)
 {
     if (nnz <= 0) return cudaSuccess;
-    ++*lc.launches;
-    const int grid = grid_for(nnz, 256, lc.sm_count);
-    if (dtype == BHB200_DTYPE_F64)
-        k_tr_gather<double><<<grid, 256, 0, lc.stream>>>(nnz, static_cast<const double *>(val), perm, static_cast<double *>(valT));
-    else
-        k_tr_gather<float><<<grid, 256, 0, lc.stream>>>(nnz, static_cast<const float *>(val), perm, static_cast<float *>(valT));
-    return cudaGetLastError();
+    return with_mover(dtype, conj, [&](auto v) {
+        using V = decltype(v);
+        if constexpr (value_bytes<V> > 0) {
+            ++*lc.launches;
+            k_tr_gather<V><<<grid_for(nnz, 256, lc.sm_count), 256, 0, lc.stream>>>(nnz, static_cast<const V *>(val), perm,
+                                                                                 static_cast<V *>(valT));
+            return cudaGetLastError();
+        }
+        return cudaSuccess;   // (structure-only operands have no values to gather)
+    });
 }
 
 }  // namespace bhb

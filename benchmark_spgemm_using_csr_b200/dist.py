@@ -29,7 +29,20 @@ import torch.distributed as dist
 from . import capi
 from .generators import CSR
 
-_NP2T = {np.dtype(np.float32): torch.float32, np.dtype(np.float64): torch.float64}
+_NP2T = {np.dtype(np.float32): torch.float32, np.dtype(np.float64): torch.float64, np.dtype(np.complex64): torch.complex64}
+# value type names (torch dtype without "torch.") -> BHB200_DTYPE_*, torch dtype, array-interface typestr
+_VTYPES = {"float32": (capi.DTYPE_F32, torch.float32, "<f4"), "float64": (capi.DTYPE_F64, torch.float64, "<f8"),
+           "complex64": (capi.DTYPE_C64, torch.complex64, "<c8")}
+
+
+def _vtype(name: str):
+    if name == "complex128":
+        raise capi.BhsparseError(capi.ERR_INVALID, "complex128 values are not supported: use complex64")
+    return _VTYPES.get(name, _VTYPES["float32"])
+
+
+def _vtype_of_dtype(dtype: int):
+    return next(v for v in _VTYPES.values() if v[0] == dtype)
 
 
 def row_products_host(A: CSR, B_rowptr: np.ndarray) -> np.ndarray:
@@ -111,10 +124,10 @@ class CudaEngine:
             self._own.wait_stream(torch.cuda.current_stream(self.device))
 
     def set_operands(self, m, k, n, A, B):
-        """A, B = (rowptr, col, val) torch CUDA tensors (int32, int32, f32/f64)."""
+        """A, B = (rowptr, col, val) torch CUDA tensors (int32, int32, f32/f64/complex64)."""
         self._keep = (A, B)
         self._order_after_producers()
-        dtype = capi.DTYPE_F64 if A[2].dtype == torch.float64 else capi.DTYPE_F32
+        dtype = _vtype(str(A[2].dtype).replace("torch.", ""))[0]
         p = lambda t: ctypes.c_void_p(t.data_ptr())
         capi.check(self.lib, self.ctx, self.lib.bhb200_init_data_device(
             self.ctx, dtype, m, k, n, int(A[1].numel()), p(A[2]), p(A[0]), p(A[1]),
@@ -147,7 +160,7 @@ class CudaEngine:
     def get_C_range(self, first: int, count: int):
         """Entries [first, first+count) of the local C block as host arrays (col int32, val)."""
         col = np.empty(max(count, 0), dtype=np.int32)
-        val = np.empty(max(count, 0), dtype=np.float64 if self.vdtype == torch.float64 else np.float32)
+        val = np.empty(max(count, 0), dtype=str(self.vdtype).replace("torch.", ""))
         capi.check(self.lib, self.ctx, self.lib.bhb200_get_C_range(
             self.ctx, int(first), int(count), ctypes.c_void_p(col.ctypes.data), ctypes.c_void_p(val.ctypes.data)))
         return col, val
@@ -269,7 +282,7 @@ class RowBlockSpGEMM:
             meta = box[0]
         self.meta = meta
         self.bounds = np.asarray(meta["bounds"], dtype=np.int64)
-        vt = torch.float64 if meta["dtype"] == "float64" else torch.float32
+        vt = _vtype(meta["dtype"])[1]
 
         def bcast(t, numel, tdtype):
             if self.rank != root:
@@ -406,7 +419,7 @@ class NcclRowBlockSpGEMM:
         if self.world > 1:
             dist.broadcast_object_list(info, src=root, group=self.group)
         nnz, dname, n = info[0]              # (n is taken from the root's arrays)
-        dtype = capi.DTYPE_F64 if dname == "float64" else capi.DTYPE_F32
+        dtype = _vtype(dname)[0]
         p = (lambda t: ctypes.c_void_p(t.data_ptr())) if self.rank == root else (lambda t: None)
         capi.check(lib, ctx, lib.bhb200_dist_setup_square(
             ctx, root, dtype, n, nnz, p(B_dev[0] if B_dev else None), p(B_dev[1] if B_dev else None),
@@ -420,7 +433,7 @@ class NcclRowBlockSpGEMM:
         capi.check(lib, ctx, lib.bhb200_dist_get_block_products(ctx, bp))
         self.rows = (int(r0.value), int(r1.value))
         self.engine.m = self.rows[1] - self.rows[0]
-        self.engine.vdtype = torch.float64 if dtype == capi.DTYPE_F64 else torch.float32
+        self.engine.vdtype = _vtype(dname)[1]
         self.meta = dict(m=n, k=n, n=n, nnzA=nnz, nnzB=nnz, dtype=dname, products=int(ptot.value),
                          block_products=[int(x) for x in bp])
         return self
@@ -438,12 +451,13 @@ class NcclRowBlockSpGEMM:
         ptr = [ctypes.c_void_p() for _ in range(6)]
         capi.check(lib, ctx, lib.bhb200_get_operands_device(ctx, dims, *(ctypes.byref(x) for x in ptr)))
         m, k, n, nnzA, nnzB, dtype = (int(x) for x in dims)
-        vt = "<f8" if dtype == capi.DTYPE_F64 else "<f4"
+        vt = _vtype_of_dtype(dtype)[2]
         capi.check(lib, ctx, lib.bhb200_synchronize(ctx))
 
         def view(p, numel, ts):
             if numel == 0:
-                return torch.empty(0, dtype={"<i4": torch.int32, "<f8": torch.float64, "<f4": torch.float32}[ts], device=self.device)
+                return torch.empty(0, dtype={"<i4": torch.int32, "<f8": torch.float64, "<f4": torch.float32,
+                                             "<c8": torch.complex64}[ts], device=self.device)
             return torch.as_tensor(_DevicePtr(p.value, numel, ts), device=self.device)
         A = (view(ptr[0], m + 1, "<i4"), view(ptr[1], nnzA, "<i4"), view(ptr[2], nnzA, vt))
         B = (view(ptr[3], k + 1, "<i4"), view(ptr[4], nnzB, "<i4"), view(ptr[5], nnzB, vt))

@@ -3,8 +3,9 @@ driver uses for `-spgemm A.mtx [B.mtx]` (SpGEMM_cuda/main.cu:56-64 via
 cusp::io::read_matrix_market_file, then ref_spgemm::csr_sort_indices,
 ref_spgemm.h:37-62).  Handles real/integer/pattern fields and
 general/symmetric/skew-symmetric symmetry like the hand-rolled reader of the
-OpenCL driver (SpGEMM_opencl/main.cpp:55-208).  Duplicate entries are summed,
-columns come out sorted ascending.
+OpenCL driver (SpGEMM_opencl/main.cpp:55-208), and complex fields (hermitian files
+mirror the conjugate).  Duplicate entries are summed, columns come out sorted ascending.
+A complex file needs a complex dtype: its imaginary parts are never dropped.
 """
 from __future__ import annotations
 
@@ -21,23 +22,29 @@ def read_mtx(path: str, dtype=np.float64) -> CSR:
         fmt, field, symm = header[2].lower(), header[3].lower(), header[4].lower()
         if fmt != "coordinate":
             raise ValueError("only coordinate format is supported")
-        if field not in ("real", "integer", "pattern", "double"):
+        if field not in ("real", "integer", "pattern", "double", "complex"):
             raise ValueError(f"unsupported field {field}")
+        if field == "complex" and not np.issubdtype(np.dtype(dtype), np.complexfloating):
+            raise ValueError(f"complex matrix read into the real dtype {np.dtype(dtype)}: pass dtype=np.complex64")
         line = f.readline()
         while line.startswith("%") or not line.strip():
             line = f.readline()
         rows, cols, nnz = (int(x) for x in line.split()[:3])
-        data = np.loadtxt(f, ndmin=2) if nnz else np.zeros((0, 3))
+        data = np.loadtxt(f, ndmin=2) if nnz else np.zeros((0, 4))
     if data.shape[0] != nnz:
         raise ValueError("entry count does not match the size line")
     r = data[:, 0].astype(np.int64) - 1
     c = data[:, 1].astype(np.int64) - 1
-    v = np.ones(nnz) if field == "pattern" else data[:, 2].astype(np.float64)
+    if field == "pattern":
+        v = np.ones(nnz)
+    elif field == "complex":
+        v = data[:, 2] + 1j * data[:, 3]
+    else:
+        v = data[:, 2].astype(np.float64)
     if symm in ("symmetric", "skew-symmetric", "hermitian"):
         off = r != c
-        sign = -1.0 if symm == "skew-symmetric" else 1.0
-        r, c, v = (np.concatenate([r, c[off]]), np.concatenate([c, r[off]]),
-                   np.concatenate([v, sign * v[off]]))
+        mirror = -v[off] if symm == "skew-symmetric" else np.conj(v[off]) if symm == "hermitian" else v[off]
+        r, c, v = (np.concatenate([r, c[off]]), np.concatenate([c, r[off]]), np.concatenate([v, mirror]))
     elif symm != "general":
         raise ValueError(f"unsupported symmetry {symm}")
     if r.size and (r.min() < 0 or r.max() >= rows or c.min() < 0 or c.max() >= cols):

@@ -29,6 +29,13 @@
  *    products are all finite is finite.  Overflow of finite partial sums is unspecified.
  *  - Not promised: the sign of a zero result, and bitwise identical results from two identical calls (some
  *    kernels sum in the order atomics decide).
+ *  - complex64 (BHB200_DTYPE_C64): each component of C_ij is a real sum of 2p real products of f32 values,
+ *    Re: ar*br and (-ai)*bi, Im: ar*bi and ai*br.  The f32 rules above hold per component with p replaced by
+ *    2p and s by the sum of the magnitudes of those 2p products: |c_hat - c| <= gamma(2p)*s + 4*p*lam.
+ *    Gaussian integers within the f32 budget for 2p products come back equal.  The class of a non-finite
+ *    component follows the real rule applied to its 2p products, provided no finite real product overflows
+ *    (otherwise it is unspecified): this is the naive formula's behaviour, not C99 Annex G's recovery of
+ *    infinities (inf * (0 + 1i) gives NaN components here).
  *
  * Every function returns BHB200_SUCCESS (0 == BHSPARSE_SUCCESS, common.h:26) or
  * a negative error code; nothing calls exit().  Not thread-safe per context
@@ -62,10 +69,17 @@ extern "C" {
 /* structure only: operands and C have row pointers and columns, no values (see "structure-only
  * products" below) */
 #define BHB200_DTYPE_NONE 2
+/* value 3 is not a type (and stays invalid) */
+/* single-precision complex: two floats (re, im) per value, 8 bytes, 8-byte aligned -- the layout of C99
+ * float _Complex, std::complex<float>, cuFloatComplex, numpy / torch complex64.  Value arrays are passed
+ * as float * holding 2*nnz interleaved floats (or void * to the same bytes); see "complex64 products" below. */
+#define BHB200_DTYPE_C64 4
 
-/* op(X) of bhb200_init_data_op_* / bhb200_init_data_device_op: X as stored, or its transpose */
+/* op(X) of bhb200_init_data_op_* / bhb200_init_data_device_op: X as stored, its transpose, or its conjugate
+ * transpose X^H (complex64 operands only: with f32, f64 or structure-only operands OP_C is BHB200_ERR_INVALID) */
 #define BHB200_OP_N 0
 #define BHB200_OP_T 1
+#define BHB200_OP_C 2
 
 #define BHB200_NUM_SYM_BINS 24
 #define BHB200_NUM_NUM_BINS 24
@@ -221,6 +235,33 @@ BHB200_API int bhb200_init_data_structure(bhb200_ctx *ctx, int opA, int opB, int
                                           int nnzB, const int32_t *rowptrB, const int32_t *colB);
 BHB200_API int bhb200_get_C_structure(bhb200_ctx *ctx, int32_t *rowptrC, int32_t *colC);
 
+/* -- complex64 products: C = op(A)*op(B) over single-precision complex values ------------------------------
+ * Values are BHB200_DTYPE_C64 (two floats per value, see the define).  Every path of the real types runs:
+ * the same bins, direct-mode plans, diagonal-pattern mode and masked kernels as f64 (a complex64 value has the
+ * size of a double), with the product of the value contract above.
+ *   bhb200_init_data_op_c64    HOST arrays, the rules of bhb200_init_data_op_f64; valA / valB hold 2*nnz
+ *                              floats.  opA / opB may also be BHB200_OP_C: op(X) = X^H, the transpose with
+ *                              every value conjugated (the imaginary part's sign flipped, which keeps NaN, inf
+ *                              and zero).  With the same host arrays for A and B they are uploaded once; one
+ *                              transposed copy serves both operands when both ops are equal (T, T or C, C), so
+ *                              A*A^H takes one upload and one transposition.
+ *   bhb200_update_values_c64   new values of the host operands (conjugated again into X^H copies).
+ *   bhb200_get_C_c64           rowptrC, colC and valC (2*nnzC floats) into HOST arrays.
+ *   bhb200_init_data_device / _device_op with BHB200_DTYPE_C64: borrowed device operands; value pointers that
+ *                              are not 8-byte aligned return BHB200_ERR_INVALID from the init call.
+ *                              bhb200_spgemm_numeric re-gathers (and re-conjugates) the values of op = T / C
+ *                              operands from the caller's arrays.
+ * bhb200_get_C_range, bhb200_get_C_device, bhb200_copy_C_to_device, masks and the structure getters work with
+ * 8-byte values; bhb200_stats.dtype is BHB200_DTYPE_C64 and its byte counts take 8 bytes per value.
+ * bhb200_dist_setup_square takes BHB200_DTYPE_C64 (values broadcast as 8-byte words).  The real getters and
+ * update_values_f64 / _f32 on a complex64 context, and the _c64 ones on a real context, return
+ * BHB200_ERR_INVALID.  complex128 is not supported. */
+BHB200_API int bhb200_init_data_op_c64(bhb200_ctx *ctx, int opA, int opB, int m, int k, int n,
+                                       int nnzA, const float *valA, const int32_t *rowptrA, const int32_t *colA,
+                                       int nnzB, const float *valB, const int32_t *rowptrB, const int32_t *colB);
+BHB200_API int bhb200_update_values_c64(bhb200_ctx *ctx, const float *valA, const float *valB);
+BHB200_API int bhb200_get_C_c64(bhb200_ctx *ctx, int32_t *rowptrC, int32_t *colC, float *valC);
+
 /* -- masked products: C = M .* (op(A)*op(B)) (GraphBLAS C<M> = A*B) ----------------------------------
  * M is m x n and structural: row pointers (m+1) and column indices, no values; its rows must be sorted
  * and duplicate-free with columns in [0, n), as the rows of B.  C_ij is present iff M_ij is present and
@@ -330,7 +371,8 @@ BHB200_API int bhb200_set_profiling(bhb200_ctx *ctx, int enabled);
 #define BHB200_DIST_ID_BYTES 128
 BHB200_API int bhb200_dist_unique_id(void *id);
 BHB200_API int bhb200_dist_init(bhb200_ctx *ctx, int rank, int nranks, const void *id);
-/* dist_setup_square takes BHB200_DTYPE_F32 or BHB200_DTYPE_F64 only (structure-only products are single-GPU) */
+/* dist_setup_square takes BHB200_DTYPE_F32, BHB200_DTYPE_F64 or BHB200_DTYPE_C64 (structure-only products are
+ * single-GPU) */
 BHB200_API int bhb200_dist_setup_square(bhb200_ctx *ctx, int root, int dtype, int n, int64_t nnz, const int32_t *rowptr,
                                         const int32_t *col, const void *val);
 BHB200_API int bhb200_dist_spgemm(bhb200_ctx *ctx);
