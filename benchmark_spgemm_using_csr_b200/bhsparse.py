@@ -34,8 +34,12 @@ def _ptr(a):
     return ctypes.c_void_p(a.ctypes.data)
 
 
-# value dtype -> (init_data_op, update_values, get_C) entry-point suffix
-_SUFFIX = {np.dtype(np.float64): "f64", np.dtype(np.float32): "f32", np.dtype(np.complex64): "c64"}
+def _suffix(dt) -> str | None:
+    """init_data_op / update_values / get_C entry-point suffix of a value dtype, None if unsupported"""
+    try:
+        return capi.VALUE_TYPES[capi.dtype_of(dt)][0]
+    except capi.BhsparseError:
+        return None
 
 
 def _op(trans) -> int:
@@ -94,18 +98,19 @@ class bhsparse:
         else:
             valA = np.ascontiguousarray(csrValA)
             dt = valA.dtype
-            if dt not in _SUFFIX:   # (complex128 too: never downcast)
+            if _suffix(dt) is None:   # (complex128 too: never downcast)
                 return capi.ERR_INVALID
             if dt == np.complex64 and np.asarray(csrValB).dtype != dt:   # (no mixed real x complex operands)
                 return capi.ERR_INVALID
-            fn = getattr(self._lib, "bhb200_init_data_op_" + _SUFFIX[dt])
+            fn = getattr(self._lib, "bhb200_init_data_op_" + _suffix(dt))
             valB = np.ascontiguousarray(csrValB, dtype=dt)
         rpA = np.ascontiguousarray(csrRowPtrA, dtype=np.int32)
         cA = np.ascontiguousarray(csrColIndA, dtype=np.int32)
         rpB = np.ascontiguousarray(csrRowPtrB, dtype=np.int32)
         cB = np.ascontiguousarray(csrColIndB, dtype=np.int32)
-        rows_a = k if transA else m            # rows of A / B as stored
-        rows_b = n if transB else k
+        opA, opB = _op(transA), _op(transB)
+        rows_a = capi.op_shape(m, k, opA)[0]   # rows of A / B as stored
+        rows_b = capi.op_shape(k, n, opB)[0]
         if rpA.size != rows_a + 1 or rpB.size != rows_b + 1 or cA.size < nnzA or cB.size < nnzB:
             return capi.ERR_INVALID
         if csrRowPtrC is not None and (csrRowPtrC.dtype != np.int32 or csrRowPtrC.size < m + 1):
@@ -115,7 +120,6 @@ class bhsparse:
         self._structure = structure
         self._m = m
         # (the same host arrays for A and B stay the same objects here, so the library can upload them once)
-        opA, opB = _op(transA), _op(transB)
         if structure:
             return self._lib.bhb200_init_data_structure(self._ctx, opA, opB, m, k, n, nnzA, _ptr(rpA), _ptr(cA), nnzB,
                                                         _ptr(rpB), _ptr(cB))
@@ -160,7 +164,7 @@ class bhsparse:
         cp = ctypes.c_void_p(csrColIndC.ctypes.data) if csrColIndC is not None else None
         if csrValC is None:
             return self._lib.bhb200_get_C_structure(self._ctx, rp, cp)
-        fn = getattr(self._lib, "bhb200_get_C_" + _SUFFIX[self._dtype])
+        fn = getattr(self._lib, "bhb200_get_C_" + _suffix(self._dtype))
         return fn(self._ctx, rp, cp, ctypes.c_void_p(csrValC.ctypes.data))
 
     def free_mem(self) -> int:
@@ -174,7 +178,7 @@ class bhsparse:
         for v in (csrValA, csrValB):
             if v is not None and (v.dtype != self._dtype or not v.flags.c_contiguous):
                 return capi.ERR_INVALID
-        fn = getattr(self._lib, "bhb200_update_values_" + _SUFFIX[self._dtype])
+        fn = getattr(self._lib, "bhb200_update_values_" + _suffix(self._dtype))
         ap = ctypes.c_void_p(csrValA.ctypes.data) if csrValA is not None else None
         bp = ctypes.c_void_p(csrValB.ctypes.data) if csrValB is not None else None
         return fn(self._ctx, ap, bp)
@@ -246,8 +250,7 @@ def spgemm(A, B, device: int = 0, return_stats: bool = False, return_row_product
     bh = bhsparse(device)
     if not structure_only and np.asarray(A.val).dtype == np.complex128:
         raise capi.BhsparseError(capi.ERR_INVALID, "complex128 values are not supported: use complex64")
-    m, k = (A.cols, A.rows) if transA else (A.rows, A.cols)
-    n = B.rows if transB else B.cols
+    m, k, n = capi.op_dims(A, B, _op(transA), _op(transB))
     rowptrC = np.zeros(m + 1, dtype=np.int32)
 
     def ok(err, what):

@@ -1,14 +1,16 @@
-"""ctypes binding of the C-ABI in include/bhsparse_b200.h.
+"""ctypes binding of the C-ABI in include/bhsparse_b200.h, and `Context`, the Python owner of one bhb200_ctx.
 
 Loads benchmark_spgemm_using_csr_b200/lib/libbhsparse_b200.so.  There is NO CPU
 fallback: if the library is missing or no sm_100 GPU is visible every compute
-entry point raises.
+entry point raises.  torch is imported only by the methods that take or return device tensors.
 """
 from __future__ import annotations
 
 import ctypes
 import os
 from ctypes import POINTER, c_char_p, c_double, c_float, c_int, c_int32, c_int64, c_void_p
+
+import numpy as np
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(HERE, "lib", "libbhsparse_b200.so")
@@ -175,3 +177,214 @@ def check(lib, ctx, code: int):
     if code != SUCCESS:
         msg = lib.bhb200_last_error(ctx)
         raise BhsparseError(code, msg.decode() if msg else "")
+
+
+# BHB200_DTYPE_* of a valued product -> (suffix of bhb200_init_data_op_*, bhb200_update_values_* and
+# bhb200_get_C_*; numpy and torch dtype name)
+VALUE_TYPES = {DTYPE_F32: ("f32", "float32"), DTYPE_F64: ("f64", "float64"), DTYPE_C64: ("c64", "complex64")}
+_DTYPE_OF_NAME = {name: dt for dt, (_, name) in VALUE_TYPES.items()}
+
+
+def dtype_of(x) -> int:
+    """BHB200_DTYPE_* of a numpy or torch value array, dtype or dtype name.  Other value types raise: complex128 is
+    refused, never converted."""
+    name = str(getattr(x, "dtype", x)).removeprefix("torch.")
+    if name not in _DTYPE_OF_NAME:
+        hint = ": use complex64" if name == "complex128" else ""
+        raise BhsparseError(ERR_INVALID, f"{name} values are not supported{hint}")
+    return _DTYPE_OF_NAME[name]
+
+
+def op_shape(rows: int, cols: int, op: int):
+    """Shape of op(X) for X of shape (rows, cols), and of X for op(X) of that shape."""
+    return (cols, rows) if op != OP_N else (rows, cols)
+
+
+def op_dims(A, B, opA: int = OP_N, opB: int = OP_N):
+    """(m, k, n) of C = op(A)*op(B) for A and B as stored (anything with .rows and .cols)."""
+    m, k = op_shape(A.rows, A.cols, opA)
+    return m, k, op_shape(B.rows, B.cols, opB)[1]
+
+
+class DevicePtr:
+    """A borrowed device pointer as a __cuda_array_interface__ object (typestr e.g. "<i4"), for torch.as_tensor."""
+
+    def __init__(self, ptr: int, numel: int, typestr: str):
+        self.__cuda_array_interface__ = {"shape": (numel,), "typestr": typestr, "data": (ptr, False), "version": 2}
+
+
+def device_view(ptr: int, numel: int, dtype: str, device):
+    """A torch tensor over `numel` elements of device memory at `ptr` that the library owns: no copy, valid until
+    the owning context changes or frees it."""
+    import torch
+    if numel == 0:
+        return torch.empty(0, dtype=getattr(torch, dtype), device=device)
+    return torch.as_tensor(DevicePtr(ptr, numel, np.dtype(dtype).str), device=device)
+
+
+def _ptr(a):
+    """Address of a numpy array, or NULL for None."""
+    return None if a is None else c_void_p(a.ctypes.data)
+
+
+def _dptr(t):
+    """Address of a torch tensor, or NULL for None."""
+    return None if t is None else c_void_p(t.data_ptr())
+
+
+class Context:
+    """One bhb200_ctx.  Every call raises BhsparseError on a nonzero return.  Operands, values and device masks
+    handed to it stay referenced until the next init or close, so borrowed device arrays outlive their use.
+
+    m, n: the shape of C; dtype: the BHB200_DTYPE_* of the operands."""
+
+    def __init__(self, device: int = 0):
+        self.lib = load()
+        self.ctx = c_void_p()
+        self.device = device
+        self.m = self.n = 0
+        self.dtype = DTYPE_F64
+        self._keep = []
+        self._check(self.lib.bhb200_create(ctypes.byref(self.ctx), device))
+
+    def close(self):
+        if self.ctx:
+            self.lib.bhb200_destroy(self.ctx)
+            self.ctx = c_void_p()
+        self._keep = []
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        self.close()
+
+    def _check(self, code: int):
+        check(self.lib, self.ctx, code)
+
+    # -- operands ---------------------------------------------------------------------------------------
+    def init(self, A, B, opA: int = OP_N, opB: int = OP_N, dtype: int | None = None, same: bool = False):
+        """Host CSR operands as stored; C = op(A)*op(B).  dtype None takes the value type from A.val, DTYPE_NONE
+        passes no values.  same=True passes A's arrays for B (the library uploads them once); otherwise B's values
+        are a copy of their own."""
+        m, k, n = op_dims(A, B, opA, opB)
+        dt = dtype_of(A.val) if dtype is None else dtype
+        a = [np.ascontiguousarray(A.rowptr, np.int32), np.ascontiguousarray(A.col, np.int32)]
+        b = a if same else [np.ascontiguousarray(B.rowptr, np.int32), np.ascontiguousarray(B.col, np.int32)]
+        if dt == DTYPE_NONE:
+            self._keep = [a, b]
+            self._check(self.lib.bhb200_init_data_structure(self.ctx, opA, opB, m, k, n, A.nnz, *map(_ptr, a), B.nnz,
+                                                            *map(_ptr, b)))
+        else:
+            suffix, name = VALUE_TYPES[dt]
+            va = np.ascontiguousarray(A.val, name)
+            vb = va if same else np.array(B.val, name)
+            self._keep = [a, b, va, vb]
+            fn = getattr(self.lib, "bhb200_init_data_op_" + suffix)
+            self._check(fn(self.ctx, opA, opB, m, k, n, A.nnz, _ptr(va), *map(_ptr, a), B.nnz, _ptr(vb), *map(_ptr, b)))
+        self.m, self.n, self.dtype = m, n, dt
+
+    def init_device(self, A, B, m: int, k: int, n: int, opA: int = OP_N, opB: int = OP_N, dtype: int | None = None):
+        """Borrowed device operands: A, B = (rowptr, col, val) torch tensors as stored; op(A) is m x k, op(B) k x n.
+        dtype None takes the value type from A's values.  A val of None is passed as a NULL value pointer (for
+        DTYPE_NONE)."""
+        dt = dtype_of(A[2]) if dtype is None else dtype
+        self._keep = [A, B]
+        self._check(self.lib.bhb200_init_data_device_op(self.ctx, dt, opA, opB, m, k, n, int(A[1].numel()), _dptr(A[2]),
+                                                        _dptr(A[0]), _dptr(A[1]), int(B[1].numel()), _dptr(B[2]),
+                                                        _dptr(B[0]), _dptr(B[1])))
+        self.m, self.n, self.dtype = m, n, dt
+
+    def set_mask(self, rowptr, col):
+        """C = M .* (op(A)*op(B)) on the pattern of M, host arrays (copied by the library)."""
+        rp, c = np.ascontiguousarray(rowptr, np.int32), np.ascontiguousarray(col, np.int32)
+        self._check(self.lib.bhb200_set_mask(self.ctx, int(c.size), _ptr(rp), _ptr(c) if c.size else None))
+
+    def set_mask_device(self, rowptr, col):
+        """The mask from borrowed int32 device tensors."""
+        self._keep.append((rowptr, col))
+        self._check(self.lib.bhb200_set_mask_device(self.ctx, int(col.numel()), _dptr(rowptr), _dptr(col)))
+
+    def clear_mask(self):
+        self._check(self.lib.bhb200_clear_mask(self.ctx))
+
+    # -- products ---------------------------------------------------------------------------------------
+    def spgemm(self) -> int:
+        """The product; returns nnz(C)."""
+        self._check(self.lib.bhb200_spgemm(self.ctx))
+        return int(self.lib.bhb200_get_nnzC(self.ctx))
+
+    def update_values(self, va, vb):
+        """New host values of A and B as stored (None: unchanged), same patterns."""
+        name = VALUE_TYPES[self.dtype][1]
+        va, vb = (None if v is None else np.ascontiguousarray(v, name) for v in (va, vb))
+        self._keep.append((va, vb))
+        fn = getattr(self.lib, "bhb200_update_values_" + VALUE_TYPES[self.dtype][0])
+        self._check(fn(self.ctx, _ptr(va), _ptr(vb)))
+
+    def spgemm_numeric(self):
+        self._check(self.lib.bhb200_spgemm_numeric(self.ctx))
+
+    # -- results ----------------------------------------------------------------------------------------
+    def rowptr64_host(self) -> np.ndarray:
+        out = np.empty(self.m + 1, dtype=np.int64)
+        self._check(self.lib.bhb200_get_rowptrC_i64(self.ctx, _ptr(out)))
+        return out
+
+    def get_C_range(self, first: int, count: int):
+        """Entries [first, first+count) of C as host arrays (col int32, val); val is None for structure-only."""
+        col = np.empty(max(count, 0), dtype=np.int32)
+        val = None if self.dtype == DTYPE_NONE else np.empty(max(count, 0), dtype=VALUE_TYPES[self.dtype][1])
+        self._check(self.lib.bhb200_get_C_range(self.ctx, int(first), int(count), _ptr(col), _ptr(val)))
+        return col, val
+
+    def C(self):
+        """C on the host: (rowptr int64, col int32, val), val None for structure-only; any nnz(C)."""
+        rp = self.rowptr64_host()
+        return (rp, *self.get_C_range(0, int(rp[-1])))
+
+    def C_device(self):
+        """Copies of C on the device as torch tensors (rowptr int64, col int32, val); val None for structure-only.
+        The copy is complete when this returns, so any stream may use them."""
+        import torch
+        nnz = int(self.lib.bhb200_get_nnzC(self.ctx))
+        dev = torch.device("cuda", self.device)
+        rowptr = torch.empty(self.m + 1, dtype=torch.int64, device=dev)
+        col = torch.empty(max(nnz, 1), dtype=torch.int32, device=dev)
+        val = None if self.dtype == DTYPE_NONE else \
+            torch.empty(max(nnz, 1), dtype=getattr(torch, VALUE_TYPES[self.dtype][1]), device=dev)
+        self._check(self.lib.bhb200_copy_C_to_device(self.ctx, _dptr(rowptr), _dptr(col), _dptr(val)))
+        return rowptr, col[:nnz], None if val is None else val[:nnz]
+
+    def operands(self):
+        """((m, k, n), op(A), op(B)) as the library holds them: (rowptr, col, val) views of its device memory
+        (device_view), val None for structure-only."""
+        dims = (c_int32 * 6)()
+        ptrs = [c_void_p() for _ in range(6)]
+        self._check(self.lib.bhb200_get_operands_device(self.ctx, dims, *(ctypes.byref(p) for p in ptrs)))
+        self._check(self.lib.bhb200_synchronize(self.ctx))
+        m, k, n, nnzA, nnzB, dt = (int(x) for x in dims)
+        dev = f"cuda:{self.device}"
+
+        def csr(rows, nnz, rp, col, val):
+            return (device_view(rp.value, rows + 1, "int32", dev), device_view(col.value, nnz, "int32", dev),
+                    None if dt == DTYPE_NONE else device_view(val.value, nnz, VALUE_TYPES[dt][1], dev))
+        return (m, k, n), csr(m, nnzA, *ptrs[:3]), csr(k, nnzB, *ptrs[3:])
+
+    def stats(self) -> dict:
+        st = Stats()
+        self._check(self.lib.bhb200_get_stats(self.ctx, ctypes.byref(st)))
+        return st.as_dict()
+
+    def error(self) -> str:
+        return self.lib.bhb200_last_error(self.ctx).decode()
+
+    def aliased(self) -> int:
+        """1 if A and B came from the same arrays and were uploaded once."""
+        return int(self.lib.bhb200_operands_aliased(self.ctx))
+
+    def set_stream(self, cuda_stream_ptr: int):
+        self._check(self.lib.bhb200_set_stream(self.ctx, c_void_p(cuda_stream_ptr)))
+
+    def set_profiling(self, on: bool):
+        self._check(self.lib.bhb200_set_profiling(self.ctx, 1 if on else 0))

@@ -29,20 +29,10 @@ import torch.distributed as dist
 from . import capi
 from .generators import CSR
 
-_NP2T = {np.dtype(np.float32): torch.float32, np.dtype(np.float64): torch.float64, np.dtype(np.complex64): torch.complex64}
-# value type names (torch dtype without "torch.") -> BHB200_DTYPE_*, torch dtype, array-interface typestr
-_VTYPES = {"float32": (capi.DTYPE_F32, torch.float32, "<f4"), "float64": (capi.DTYPE_F64, torch.float64, "<f8"),
-           "complex64": (capi.DTYPE_C64, torch.complex64, "<c8")}
 
-
-def _vtype(name: str):
-    if name == "complex128":
-        raise capi.BhsparseError(capi.ERR_INVALID, "complex128 values are not supported: use complex64")
-    return _VTYPES.get(name, _VTYPES["float32"])
-
-
-def _vtype_of_dtype(dtype: int):
-    return next(v for v in _VTYPES.values() if v[0] == dtype)
+def _torch_dtype(name) -> torch.dtype:
+    """torch dtype of a supported value type (capi.dtype_of raises for others)"""
+    return getattr(torch, capi.VALUE_TYPES[capi.dtype_of(name)][1])
 
 
 def row_products_host(A: CSR, B_rowptr: np.ndarray) -> np.ndarray:
@@ -92,15 +82,11 @@ class LocalResult:
     val: object
 
 
-class CudaEngine:
+class CudaEngine(capi.Context):
     """Runs one row block through the C-ABI with device-resident operands."""
 
     def __init__(self, device: int):
-        self.lib = capi.load()
-        self.ctx = ctypes.c_void_p(None)
-        capi.check(self.lib, self.ctx, self.lib.bhb200_create(ctypes.byref(self.ctx), device))
-        self.device = device
-        self._keep = None
+        super().__init__(device)
         # The library must run on a stream that is ordered after the producers of its operands
         # (torch kernels, NCCL receives) -- not on the context's private non-blocking stream.
         # Default: torch's current stream; the legacy default stream has handle 0, which
@@ -115,7 +101,7 @@ class CudaEngine:
             self.use_stream(cur.cuda_stream)
 
     def use_stream(self, cuda_stream_ptr: int):
-        capi.check(self.lib, self.ctx, self.lib.bhb200_set_stream(self.ctx, ctypes.c_void_p(cuda_stream_ptr)))
+        self.set_stream(cuda_stream_ptr)
         if self._own is not None and cuda_stream_ptr != self._own.cuda_stream:
             self._own = None
 
@@ -123,61 +109,24 @@ class CudaEngine:
         if self._own is not None:
             self._own.wait_stream(torch.cuda.current_stream(self.device))
 
+    @property
+    def vdtype(self):
+        """torch dtype of the values of C"""
+        return getattr(torch, capi.VALUE_TYPES[self.dtype][1])
+
     def set_operands(self, m, k, n, A, B):
         """A, B = (rowptr, col, val) torch CUDA tensors (int32, int32, f32/f64/complex64)."""
-        self._keep = (A, B)
         self._order_after_producers()
-        dtype = _vtype(str(A[2].dtype).replace("torch.", ""))[0]
-        p = lambda t: ctypes.c_void_p(t.data_ptr())
-        capi.check(self.lib, self.ctx, self.lib.bhb200_init_data_device(
-            self.ctx, dtype, m, k, n, int(A[1].numel()), p(A[2]), p(A[0]), p(A[1]),
-            int(B[1].numel()), p(B[2]), p(B[0]), p(B[1])))
-        self.m, self.vdtype = m, A[2].dtype
+        self.init_device(A, B, m, k, n)
 
     def spgemm(self) -> int:
         self._order_after_producers()
-        capi.check(self.lib, self.ctx, self.lib.bhb200_spgemm(self.ctx))
-        return int(self.lib.bhb200_get_nnzC(self.ctx))
+        return super().spgemm()
 
     def result(self) -> LocalResult:
-        """Copies of the device-resident result as torch tensors (device to device; the copy is
-        complete on the host when bhb200_copy_C_to_device returns, so any stream may use them)."""
-        nnzC = int(self.lib.bhb200_get_nnzC(self.ctx))
-        dev = torch.device("cuda", self.device)
-        rowptr = torch.empty(self.m + 1, dtype=torch.int64, device=dev)
-        col = torch.empty(max(nnzC, 1), dtype=torch.int32, device=dev)
-        val = torch.empty(max(nnzC, 1), dtype=self.vdtype, device=dev)
-        capi.check(self.lib, self.ctx, self.lib.bhb200_copy_C_to_device(
-            self.ctx, ctypes.c_void_p(rowptr.data_ptr()), ctypes.c_void_p(col.data_ptr()),
-            ctypes.c_void_p(val.data_ptr())))
-        return LocalResult(nnzC, rowptr, col[:nnzC], val[:nnzC])
-
-    def rowptr64_host(self) -> np.ndarray:
-        out = np.empty(self.m + 1, dtype=np.int64)
-        capi.check(self.lib, self.ctx, self.lib.bhb200_get_rowptrC_i64(self.ctx, ctypes.c_void_p(out.ctypes.data)))
-        return out
-
-    def get_C_range(self, first: int, count: int):
-        """Entries [first, first+count) of the local C block as host arrays (col int32, val)."""
-        col = np.empty(max(count, 0), dtype=np.int32)
-        val = np.empty(max(count, 0), dtype=str(self.vdtype).replace("torch.", ""))
-        capi.check(self.lib, self.ctx, self.lib.bhb200_get_C_range(
-            self.ctx, int(first), int(count), ctypes.c_void_p(col.ctypes.data), ctypes.c_void_p(val.ctypes.data)))
-        return col, val
-
-    def stats(self) -> dict:
-        st = capi.Stats()
-        capi.check(self.lib, self.ctx, self.lib.bhb200_get_stats(self.ctx, ctypes.byref(st)))
-        return st.as_dict()
-
-    def set_profiling(self, on: bool):
-        self.lib.bhb200_set_profiling(self.ctx, 1 if on else 0)
-
-    def close(self):
-        if self.ctx:
-            self.lib.bhb200_destroy(self.ctx)
-            self.ctx = ctypes.c_void_p(None)
-        self._keep = None
+        """Copies of the device-resident result as torch tensors (capi.Context.C_device)."""
+        rowptr, col, val = self.C_device()
+        return LocalResult(int(col.numel()), rowptr, col, val)
 
 
 class RowBlockSpGEMM:
@@ -214,7 +163,7 @@ class RowBlockSpGEMM:
             meta = box[0]
         self.meta = meta
         self.bounds = np.asarray(meta["bounds"], dtype=np.int64)
-        vt = _NP2T[np.dtype(meta["dtype"])]
+        vt = _torch_dtype(meta["dtype"])
 
         # B: three broadcasts (rowptr first: it is all k_row_products needs)
         def bcast(host_arr, numel, tdtype):
@@ -282,7 +231,7 @@ class RowBlockSpGEMM:
             meta = box[0]
         self.meta = meta
         self.bounds = np.asarray(meta["bounds"], dtype=np.int64)
-        vt = _vtype(meta["dtype"])[1]
+        vt = _torch_dtype(meta["dtype"])
 
         def bcast(t, numel, tdtype):
             if self.rank != root:
@@ -419,7 +368,7 @@ class NcclRowBlockSpGEMM:
         if self.world > 1:
             dist.broadcast_object_list(info, src=root, group=self.group)
         nnz, dname, n = info[0]              # (n is taken from the root's arrays)
-        dtype = _vtype(dname)[0]
+        dtype = capi.dtype_of(dname)
         p = (lambda t: ctypes.c_void_p(t.data_ptr())) if self.rank == root else (lambda t: None)
         capi.check(lib, ctx, lib.bhb200_dist_setup_square(
             ctx, root, dtype, n, nnz, p(B_dev[0] if B_dev else None), p(B_dev[1] if B_dev else None),
@@ -432,8 +381,7 @@ class NcclRowBlockSpGEMM:
         bp = (ctypes.c_int64 * self.world)()
         capi.check(lib, ctx, lib.bhb200_dist_get_block_products(ctx, bp))
         self.rows = (int(r0.value), int(r1.value))
-        self.engine.m = self.rows[1] - self.rows[0]
-        self.engine.vdtype = _vtype(dname)[1]
+        self.engine.m, self.engine.dtype = self.rows[1] - self.rows[0], dtype
         self.meta = dict(m=n, k=n, n=n, nnzA=nnz, nnzB=nnz, dtype=dname, products=int(ptot.value),
                          block_products=[int(x) for x in bp])
         return self
@@ -445,32 +393,14 @@ class NcclRowBlockSpGEMM:
         capi.check(lib, ctx, lib.bhb200_dist_spgemm(ctx))
         return int(lib.bhb200_get_nnzC(ctx)), None, None
 
-    def _operands(self):
-        lib, ctx = self.engine.lib, self.engine.ctx
-        dims = (ctypes.c_int32 * 6)()
-        ptr = [ctypes.c_void_p() for _ in range(6)]
-        capi.check(lib, ctx, lib.bhb200_get_operands_device(ctx, dims, *(ctypes.byref(x) for x in ptr)))
-        m, k, n, nnzA, nnzB, dtype = (int(x) for x in dims)
-        vt = _vtype_of_dtype(dtype)[2]
-        capi.check(lib, ctx, lib.bhb200_synchronize(ctx))
-
-        def view(p, numel, ts):
-            if numel == 0:
-                return torch.empty(0, dtype={"<i4": torch.int32, "<f8": torch.float64, "<f4": torch.float32,
-                                             "<c8": torch.complex64}[ts], device=self.device)
-            return torch.as_tensor(_DevicePtr(p.value, numel, ts), device=self.device)
-        A = (view(ptr[0], m + 1, "<i4"), view(ptr[1], nnzA, "<i4"), view(ptr[2], nnzA, vt))
-        B = (view(ptr[3], k + 1, "<i4"), view(ptr[4], nnzB, "<i4"), view(ptr[5], nnzB, vt))
-        return A, B
-
     @property
     def A(self):
         """This rank's row block of A as the library holds it (views of device memory)."""
-        return self._operands()[0]
+        return self.engine.operands()[1]
 
     @property
     def B(self):
-        return self._operands()[1]
+        return self.engine.operands()[2]
 
     def layout(self):
         """(row_begin, row_end, nnz_offset, nnz_total) of this rank -- copies nranks int64 from the device."""
@@ -485,12 +415,7 @@ class NcclRowBlockSpGEMM:
         ptr = ctypes.c_void_p()
         capi.check(lib, ctx, lib.bhb200_dist_get_global_rowptr_device(ctx, ctypes.byref(ptr)))
         capi.check(lib, ctx, lib.bhb200_synchronize(ctx))
-        view = _DevicePtr(ptr.value, self.engine.m + 1, "<i8")
-        return torch.as_tensor(view, device=self.device).clone()
+        return capi.device_view(ptr.value, self.engine.m + 1, "int64", self.device).clone()
 
 
-class _DevicePtr:
-    """A borrowed device pointer as a __cuda_array_interface__ object (read-only use, then clone)."""
-
-    def __init__(self, ptr: int, numel: int, typestr: str):
-        self.__cuda_array_interface__ = {"shape": (numel,), "typestr": typestr, "data": (ptr, False), "version": 2}
+_DevicePtr = capi.DevicePtr   # the name code written against earlier versions of this module imports

@@ -18,7 +18,7 @@ import numpy as np
 
 __all__ = [
     "CSR", "poisson5pt", "poisson9pt", "poisson7pt", "poisson27pt", "rmat",
-    "uniform_rect", "random_csr", "banded_random", "diagonals", "rmat_counter", "rmat_counter_torch", "int_values", "real_values", "transpose_pattern",
+    "uniform_rect", "random_csr", "banded_random", "diagonals", "rmat_counter", "rmat_counter_torch", "int_values", "real_values", "transpose_pattern", "transpose",
 ]
 
 
@@ -241,6 +241,15 @@ def transpose_pattern(A: CSR, value_seed=3, values="int") -> CSR:
     """A^T with fresh values (test helper for rectangular chains)."""
     r = np.repeat(np.arange(A.rows, dtype=np.int64), np.diff(A.rowptr))
     return _from_coo_dedup(A.cols, A.rows, A.col.astype(np.int64), r, value_seed, A.val.dtype, values)
+
+
+def transpose(X: CSR) -> CSR:
+    """X^T by a stable argsort of the columns: the entries of a row of X^T in the stored order of X."""
+    rows = np.repeat(np.arange(X.rows, dtype=np.int64), np.diff(X.rowptr.astype(np.int64)))
+    perm = np.argsort(X.col, kind="stable")
+    rowptr = np.zeros(X.cols + 1, dtype=np.int64)
+    np.cumsum(np.bincount(X.col, minlength=X.cols), out=rowptr[1:])
+    return CSR(X.cols, X.rows, rowptr.astype(np.int32), rows[perm].astype(np.int32), X.val[perm])
 
 
 def diagonals(rows, cols, offsets, keep=1.0, seed=1, value_seed=2, dtype=np.float64, values="int") -> CSR:

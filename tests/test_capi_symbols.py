@@ -56,6 +56,27 @@ def test_no_cpu_fallback_without_gpu():
         spgemm(A, A)
 
 
+def test_context_without_gpu_raises():
+    import torch
+    if torch.cuda.is_available():
+        pytest.skip("GPU present")
+    capi.load(build_if_missing=True)
+    with pytest.raises(capi.BhsparseError) as e:
+        capi.Context()
+    assert e.value.code == capi.ERR_NO_DEVICE
+
+
+@pytest.mark.parametrize("op", [capi.OP_N, capi.OP_T, capi.OP_C])
+def test_op_dims(op):
+    """op(X) of a stored rows x cols X is rows x cols for OP_N and cols x rows for OP_T and OP_C."""
+    from benchmark_spgemm_using_csr_b200.generators import CSR
+    A, B = CSR(3, 5, None, None, None), CSR(7, 11, None, None, None)
+    m, k = (3, 5) if op == capi.OP_N else (5, 3)
+    assert capi.op_dims(A, B, op, capi.OP_N) == (m, k, 11)
+    assert capi.op_dims(A, B, capi.OP_N, op) == (3, 5, 11 if op == capi.OP_N else 7)
+    assert capi.op_shape(*capi.op_shape(3, 5, op), op) == (3, 5)
+
+
 def test_header_is_plain_c_and_links(tmp_path):
     """The boundary is a C ABI: the header must compile as C99 and a C caller must link
     against the shared library (no compute call: there is no GPU here)."""

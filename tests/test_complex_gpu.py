@@ -17,8 +17,8 @@ import exact_ref as xr
 from benchmark_spgemm_using_csr_b200 import capi, generators as gen
 from benchmark_spgemm_using_csr_b200.bhsparse import spgemm
 from benchmark_spgemm_using_csr_b200.generators import CSR
-from test_mask_gpu import host_transpose
-from test_values_gpu import CASES, REBINNED, Ctx, check_values, restrict
+from csr_ref import stored
+from test_values_gpu import CASES, REBINNED, check_values, restrict
 
 pytestmark = pytest.mark.gpu
 
@@ -35,36 +35,6 @@ def lib(tmp_path_factory):
 
 def cplx(X: CSR, v) -> CSR:
     return CSR(X.rows, X.cols, X.rowptr, X.col, np.asarray(v, np.complex64))
-
-
-def stored(X: CSR, op) -> CSR:
-    """the operand to hand to the library so that op(stored) = X"""
-    if op == N:
-        return X
-    t = host_transpose(X)
-    return cplx(t, np.conj(t.val)) if op == C else t
-
-
-class CCtx(Ctx):
-    """test_values_gpu's context with complex64 host operands"""
-
-    def init(self, A, B, opA=N, opB=N):
-        m, k = (A.cols, A.rows) if opA != N else (A.rows, A.cols)
-        n = B.rows if opB != N else B.cols
-        self.m, self.dt = m, np.complex64
-        arrs = [np.ascontiguousarray(x) for x in (A.val, A.rowptr, A.col)]
-        arrs += arrs if B is A else [np.ascontiguousarray(x) for x in (B.val, B.rowptr, B.col)]
-        self._keep = arrs
-        p = [ctypes.c_void_p(a.ctypes.data) for a in arrs]
-        self.check(self.lib.bhb200_init_data_op_c64(self.ctx, opA, opB, m, k, n, A.nnz, *p[:3], B.nnz, *p[3:]))
-
-    def update_numeric(self, va, vb):
-        va = np.ascontiguousarray(va)
-        vb = va if vb is None else np.ascontiguousarray(vb)
-        self._vals = (va, vb)
-        self.check(self.lib.bhb200_update_values_c64(self.ctx, ctypes.c_void_p(va.ctypes.data), ctypes.c_void_p(vb.ctypes.data)))
-        self.check(self.lib.bhb200_spgemm_numeric(self.ctx))
-        return self.C()
 
 
 def check_c(got, refs, what, exact=False):
@@ -95,13 +65,10 @@ def test_values_c64(lib, case, monkeypatch):
             monkeypatch.delenv(k)
         for k, v in case.twin_of.items():
             monkeypatch.setenv(k, v)
-        other = CCtx()
-        try:
+        with capi.Context() as other:
             other.init(stored(A2, opA), stored(B2, opB), opA, opB)
             other.spgemm()
             twin_launches = other.stats()["kernel_launches"] - 3
-        finally:
-            other.close()
         for k in case.twin_of:
             monkeypatch.delenv(k)
         for k, v in case.env.items():
@@ -115,13 +82,13 @@ def test_values_c64(lib, case, monkeypatch):
             {k: st[k] for k in ("num_bin_rows", "direct_rows", "direct_retry_rows", "direct_bin_mask", "pattern_mode",
                                 "spill_bytes", "transposed_ops", "mask_bin_rows", "kernel_launches")})
 
-    ctx = CCtx()
-    try:
+    with capi.Context() as ctx:
         def run(A, B, what, exact=False, ref=None):
             ctx.init(stored(A, opA), stored(B, opB), opA, opB)
             if mask is not None:
                 ctx.set_mask(*mask)
-            got = ctx.spgemm()
+            ctx.spgemm()
+            got = ctx.C()
             prove(ctx.stats(), what)
             check_c(got, reference(A, B) if ref is None else ref, f"{case.name} c64 {what}", exact)
 
@@ -130,14 +97,14 @@ def test_values_c64(lib, case, monkeypatch):
         run(cplx(A, cr.tier1(A.nnz, q, 3)), cplx(B, cr.tier1(B.nnz, q, 4)), f"tier 1 (q={q})", exact=True)
         run(A2, B2, "tier 2", ref=ref2)
         A3, B3 = cplx(A, cr.tier2(A.nnz, 5)), cplx(B, cr.tier2(B.nnz, 6))
-        got = ctx.update_numeric(stored(A3, opA).val, stored(B3, opB).val)
+        ctx.update_values(stored(A3, opA).val, stored(B3, opB).val)
+        ctx.spgemm_numeric()
+        got = ctx.C()
         prove(ctx.stats(), "spgemm_numeric", reuse=True)
         check_c(got, reference(A3, B3), f"{case.name} c64 tier 2 after update_values")
         if case.cancel:
             run(*cr.paired(A2, B2, seed=7), "tier 2 cancelling")
         run(cplx(A, cr.tier3(A.nnz, 8)), cplx(B, cr.tier3(B.nnz, 9)), "tier 3")
-    finally:
-        ctx.close()
 
 
 SAME_PATH = ("sym_bin_rows", "num_bin_rows", "direct_bin_mask", "direct_rows", "direct_retry_rows", "pattern_mode",
@@ -156,18 +123,13 @@ def test_same_path_as_f64(case, monkeypatch):
     opA, opB = case.ops
     stats = {}
     real = lambda X, seed: CSR(X.rows, X.cols, X.rowptr, X.col, xr.tier2(X.nnz, seed, np.float64))
-    for name, make, a, b in (("f64", Ctx, real(A, 1), real(B, 2)),
-                             ("c64", CCtx, cplx(A, cr.tier2(A.nnz, 1)), cplx(B, cr.tier2(B.nnz, 2)))):
-        ctx = make()
-        try:
-            st_a, st_b = (host_transpose(a) if opA == T else a), (host_transpose(b) if opB == T else b)
-            ctx.init(st_a, st_b, opA, opB)
+    for name, a, b in (("f64", real(A, 1), real(B, 2)), ("c64", cplx(A, cr.tier2(A.nnz, 1)), cplx(B, cr.tier2(B.nnz, 2)))):
+        with capi.Context() as ctx:
+            ctx.init(stored(a, opA), stored(b, opB), opA, opB)
             if mask is not None:
                 ctx.set_mask(*mask)
             ctx.spgemm()
             stats[name] = ctx.stats()
-        finally:
-            ctx.close()
     diff = {k: (stats["f64"][k], stats["c64"][k]) for k in SAME_PATH if stats["f64"][k] != stats["c64"][k]}
     assert not diff, f"{case.name}: complex64 took another path than f64: {diff}"
 
@@ -183,18 +145,16 @@ def _rect_ops(opA, opB):
 @pytest.mark.parametrize("ops", [(N, C), (C, N), (C, C), (T, C)], ids=["NC", "CN", "CC", "TC"])
 def test_conjugate_transpose(lib, ops):
     A, B = _rect_ops(*ops)
-    ctx = CCtx()
-    try:
+    with capi.Context() as ctx:
         ctx.init(stored(A, ops[0]), stored(B, ops[1]), *ops)
-        got = ctx.spgemm()
+        ctx.spgemm()
         assert ctx.stats()["transposed_ops"] == (ops[0] != N) | 2 * (ops[1] != N)
-        check_c(got, cr.product(lib, A, B), f"ops {ops}")
+        check_c(ctx.C(), cr.product(lib, A, B), f"ops {ops}")
         # new values as stored: conjugated again into the transposed copies
         A3, B3 = cplx(A, cr.tier2(A.nnz, 65)), cplx(B, cr.tier2(B.nnz, 66))
-        got = ctx.update_numeric(stored(A3, ops[0]).val, stored(B3, ops[1]).val)
-        check_c(got, cr.product(lib, A3, B3), f"ops {ops} after update_values")
-    finally:
-        ctx.close()
+        ctx.update_values(stored(A3, ops[0]).val, stored(B3, ops[1]).val)
+        ctx.spgemm_numeric()
+        check_c(ctx.C(), cr.product(lib, A3, B3), f"ops {ops} after update_values")
 
 
 @pytest.mark.parametrize("ops", [(N, C), (C, C)], ids=["A_AH", "AH_AH"])
@@ -202,25 +162,23 @@ def test_aliased_host_arrays(lib, ops):
     """A*A^H and A^H*A^H from the same host arrays: one upload, one transposed copy when both ops are equal"""
     X = gen.random_csr(600, 600 if ops == (C, C) else 450, 3 + np.arange(600) % 11, seed=67, dtype=F32)
     X = cplx(X, cr.tier2(X.nnz, 68))
-    ctx = CCtx()
-    try:
-        ctx.init(X, X, *ops)
+    with capi.Context() as ctx:
+        ctx.init(X, X, *ops, same=True)
         assert ctx.lib.bhb200_operands_aliased(ctx.ctx) == 1
         eff = [X if o == N else cr.conj_transpose(X) for o in ops]
-        check_c(ctx.spgemm(), cr.product(lib, *eff), f"aliased {ops}")
+        ctx.spgemm()
+        check_c(ctx.C(), cr.product(lib, *eff), f"aliased {ops}")
         assert ctx.stats()["transposed_ops"] == (ops[0] != N) | 2
         X2 = cplx(X, cr.tier2(X.nnz, 69))
-        got = ctx.update_numeric(X2.val, None)
+        ctx.update_values(X2.val, X2.val)
+        ctx.spgemm_numeric()
         eff = [X2 if o == N else cr.conj_transpose(X2) for o in ops]
-        check_c(got, cr.product(lib, *eff), f"aliased {ops} after update_values")
-    finally:
-        ctx.close()
+        check_c(ctx.C(), cr.product(lib, *eff), f"aliased {ops} after update_values")
 
 
 def test_real_operands_refuse_op_c():
-    lib = capi.load()
-    ctx = ctypes.c_void_p()
-    assert lib.bhb200_create(ctypes.byref(ctx), 0) == capi.SUCCESS
+    c = capi.Context()
+    lib, ctx = c.lib, c.ctx
     try:
         X = gen.random_csr(50, 50, 4, seed=1)
         p = [ctypes.c_void_p(np.ascontiguousarray(a).ctypes.data) for a in (X.val, X.rowptr, X.col)]
@@ -231,7 +189,7 @@ def test_real_operands_refuse_op_c():
             assert lib.bhb200_init_data_device_op(ctx, capi.DTYPE_F64, *op, 50, 50, 50, 0, None, p[1], None, 0, None, p[1],
                                                   None) == capi.ERR_INVALID
     finally:
-        lib.bhb200_destroy(ctx)
+        c.close()
 
 
 # ---- borrowed torch.complex64 operands and the interfaces -----------------------------------------------------
@@ -246,14 +204,12 @@ def test_borrowed_device_operands(lib):
     A, B = _rect_ops(N, C)
     Bs = stored(B, C)
     tA, tB = _torch_operands(A, dev), _torch_operands(Bs, dev)
-    L = capi.load()
-    ctx = Ctx()
+    ctx = capi.Context()
+    L = ctx.lib
     p = lambda t: ctypes.c_void_p(t.data_ptr())
     try:
-        ctx.check(L.bhb200_init_data_device_op(ctx.ctx, capi.DTYPE_C64, N, C, A.rows, A.cols, B.cols, A.nnz, p(tA[2]),
-                                               p(tA[0]), p(tA[1]), Bs.nnz, p(tB[2]), p(tB[0]), p(tB[1])))
-        ctx.m, ctx.dt = A.rows, np.complex64
-        ctx.check(L.bhb200_spgemm(ctx.ctx))
+        ctx.init_device(tA, tB, A.rows, A.cols, B.cols, N, C)
+        ctx.spgemm()
         got = ctx.C()
         check_c(got, cr.product(lib, A, B), "borrowed N,C")
         st = ctx.stats()
@@ -263,32 +219,31 @@ def test_borrowed_device_operands(lib):
         tA[2].copy_(torch.from_numpy(A3.val).to(dev))
         tB[2].copy_(torch.from_numpy(stored(B3, C).val).to(dev))
         torch.cuda.synchronize(dev)
-        ctx.check(L.bhb200_spgemm_numeric(ctx.ctx))
+        ctx.spgemm_numeric()
         rp, col, val = ctx.C()
         check_c((rp, col, val), cr.product(lib, A3, B3), "borrowed N,C after spgemm_numeric")
         nnz = col.size
         # get_C_c64, get_C_range of a slice, get_C_device, copy_C_to_device
         rp32, col2, val2 = np.empty(A.rows + 1, np.int32), np.empty(nnz, np.int32), np.empty(nnz, np.complex64)
-        ctx.check(L.bhb200_get_C_c64(ctx.ctx, *(ctypes.c_void_p(a.ctypes.data) for a in (rp32, col2, val2))))
+        capi.check(L, ctx.ctx, L.bhb200_get_C_c64(ctx.ctx, *(ctypes.c_void_p(a.ctypes.data) for a in (rp32, col2, val2))))
         assert np.array_equal(rp32, rp) and np.array_equal(col2, col) and np.array_equal(val2.view(np.uint64), val.view(np.uint64))
         c3, v3 = np.empty(100, np.int32), np.empty(100, np.complex64)
-        ctx.check(L.bhb200_get_C_range(ctx.ctx, nnz - 100, 100, ctypes.c_void_p(c3.ctypes.data), ctypes.c_void_p(v3.ctypes.data)))
+        capi.check(L, ctx.ctx, L.bhb200_get_C_range(ctx.ctx, nnz - 100, 100, ctypes.c_void_p(c3.ctypes.data), ctypes.c_void_p(v3.ctypes.data)))
         assert np.array_equal(c3, col[-100:]) and np.array_equal(v3.view(np.uint64), val[-100:].view(np.uint64))
         dvp = ctypes.c_void_p()
-        ctx.check(L.bhb200_get_C_device(ctx.ctx, None, None, None, ctypes.byref(dvp)))
+        capi.check(L, ctx.ctx, L.bhb200_get_C_device(ctx.ctx, None, None, None, ctypes.byref(dvp)))
         assert dvp.value and dvp.value % 8 == 0
         drp = torch.empty(A.rows + 1, dtype=torch.int64, device=dev)
         dcol = torch.empty(nnz, dtype=torch.int32, device=dev)
         dval = torch.empty(nnz, dtype=torch.complex64, device=dev)
-        ctx.check(L.bhb200_copy_C_to_device(ctx.ctx, p(drp), p(dcol), p(dval)))
+        capi.check(L, ctx.ctx, L.bhb200_copy_C_to_device(ctx.ctx, p(drp), p(dcol), p(dval)))
         assert np.array_equal(drp.cpu().numpy(), rp) and np.array_equal(dcol.cpu().numpy(), col)
         assert np.array_equal(dval.cpu().numpy().view(np.uint64), val.view(np.uint64))
         # the structure of the same borrowed arrays, without values
-        ctx.check(L.bhb200_init_data_device_op(ctx.ctx, capi.DTYPE_NONE, N, T, A.rows, A.cols, B.cols, A.nnz, None,
-                                               p(tA[0]), p(tA[1]), Bs.nnz, None, p(tB[0]), p(tB[1])))
-        ctx.check(L.bhb200_spgemm(ctx.ctx))
+        ctx.init_device((*tA[:2], None), (*tB[:2], None), A.rows, A.cols, B.cols, N, T, capi.DTYPE_NONE)
+        ctx.spgemm()
         srp, scol = np.empty(A.rows + 1, np.int32), np.empty(nnz, np.int32)
-        ctx.check(L.bhb200_get_C_structure(ctx.ctx, ctypes.c_void_p(srp.ctypes.data), ctypes.c_void_p(scol.ctypes.data)))
+        capi.check(L, ctx.ctx, L.bhb200_get_C_structure(ctx.ctx, ctypes.c_void_p(srp.ctypes.data), ctypes.c_void_p(scol.ctypes.data)))
         assert np.array_equal(srp, rp) and np.array_equal(scol, col)
     finally:
         ctx.close()
@@ -300,8 +255,8 @@ def test_misaligned_borrowed_values_are_refused():
     X = cplx(gen.random_csr(100, 100, 5, seed=3, dtype=F32), cr.tier2(500, 4))
     rp, col, val = _torch_operands(X, dev)
     buf = torch.zeros(2 * X.nnz + 2, dtype=torch.float32, device=dev)   # values at an offset of 4 bytes
-    L = capi.load()
-    ctx = Ctx()
+    ctx = capi.Context()
+    L = ctx.lib
     p = lambda t: ctypes.c_void_p(t.data_ptr())
     try:
         rc = L.bhb200_init_data_device(ctx.ctx, capi.DTYPE_C64, 100, 100, 100, X.nnz, ctypes.c_void_p(buf.data_ptr() + 4),
@@ -318,17 +273,17 @@ def test_cross_type_refusals():
     Xc = cplx(X, cr.tier2(X.nnz, 6))
     out = [np.empty(81, np.int32), np.empty(10000, np.int32), np.empty(20000, np.float64)]
     po = [ctypes.c_void_p(a.ctypes.data) for a in out]
-    ctx = CCtx()
+    ctx = capi.Context()
     try:
-        ctx.init(Xc, Xc)
+        ctx.init(Xc, Xc, same=True)
         ctx.spgemm()
         for fn in (L.bhb200_get_C_f64, L.bhb200_get_C_f32):
             assert fn(ctx.ctx, *po) == capi.ERR_INVALID
         for fn in (L.bhb200_update_values_f64, L.bhb200_update_values_f32):
             assert fn(ctx.ctx, po[2], po[2]) == capi.ERR_INVALID
-        real = Ctx()
+        real = capi.Context()
         try:
-            real.init(X, X)
+            real.init(X, X, same=True)
             real.spgemm()
             assert L.bhb200_get_C_c64(real.ctx, *po) == capi.ERR_INVALID
             assert L.bhb200_update_values_c64(real.ctx, po[2], po[2]) == capi.ERR_INVALID

@@ -8,9 +8,9 @@ import ctypes
 import numpy as np
 import pytest
 
-import oracle
 from benchmark_spgemm_using_csr_b200 import capi, generators as gen
 from conftest import assert_csr_equal
+from csr_ref import keys, lower_triangle, product, restrict, symmetrize
 from ref_cases import _kat
 
 pytestmark = pytest.mark.gpu
@@ -19,33 +19,9 @@ N, T = capi.OP_N, capi.OP_T
 
 
 # ---- references -------------------------------------------------------------------------------------
-def host_transpose(X: gen.CSR) -> gen.CSR:
-    rows = np.repeat(np.arange(X.rows, dtype=np.int64), np.diff(X.rowptr.astype(np.int64)))
-    perm = np.argsort(X.col, kind="stable")
-    rowptr = np.zeros(X.cols + 1, dtype=np.int64)
-    np.cumsum(np.bincount(X.col, minlength=X.cols), out=rowptr[1:])
-    return gen.CSR(X.cols, X.rows, rowptr.astype(np.int32), rows[perm].astype(np.int32), X.val[perm])
-
-
 def unmasked(A, B, opA=N, opB=N):
-    a = host_transpose(A) if opA == T else A
-    b = host_transpose(B) if opB == T else B
-    return oracle.spgemm(a.rows, a.cols, b.cols, a.rowptr, a.col, a.val, b.rowptr, b.col, b.val), a.rows, b.cols
-
-
-def keys(rowptr, col, n):
-    rows = np.repeat(np.arange(len(rowptr) - 1, dtype=np.int64), np.diff(np.asarray(rowptr, dtype=np.int64)))
-    return rows * n + col.astype(np.int64)
-
-
-def restrict(C, m, n, rpM, colM):
-    """The unmasked C restricted to the pattern of M."""
-    rp, col, val = C
-    keep = np.isin(keys(rp, col, n), keys(rpM, colM, n))
-    rows = np.repeat(np.arange(m, dtype=np.int64), np.diff(np.asarray(rp, dtype=np.int64)))
-    rowptr = np.zeros(m + 1, dtype=np.int64)
-    np.cumsum(np.bincount(rows[keep], minlength=m), out=rowptr[1:])
-    return rowptr, col[keep], val[keep]
+    m, _, n = capi.op_dims(A, B, opA, opB)
+    return product(A, B, opA, opB), m, n
 
 
 def pattern(rows, cols, rowptr, col):
@@ -71,91 +47,10 @@ def union(p, q, n):
     return rowptr.astype(np.int32), (k % n).astype(np.int32)
 
 
-# ---- a context on the C-ABI -------------------------------------------------------------------------
-class Ctx:
-    def __init__(self):
-        self.lib = capi.load()
-        self.ctx = ctypes.c_void_p()
-        assert self.lib.bhb200_create(ctypes.byref(self.ctx), 0) == capi.SUCCESS
-        self._keep = []
-
-    def init(self, A, B, opA=N, opB=N, same=False):
-        m, k = (A.cols, A.rows) if opA == T else (A.rows, A.cols)
-        n = B.rows if opB == T else B.cols
-        self.m, self.n, self.dt = m, n, A.val.dtype
-        arrs = [np.ascontiguousarray(x) for x in (A.val, A.rowptr, A.col)]
-        brrs = arrs if same else [np.ascontiguousarray(x) for x in (B.val.astype(A.val.dtype), B.rowptr, B.col)]
-        self._keep = [arrs, brrs]
-        p = lambda a: ctypes.c_void_p(a.ctypes.data)
-        fn = self.lib.bhb200_init_data_op_f64 if self.dt == np.float64 else self.lib.bhb200_init_data_op_f32
-        return fn(self.ctx, opA, opB, m, k, n, A.nnz, *map(p, arrs), B.nnz, *map(p, brrs))
-
-    def init_device(self, m, k, n, A, B, opA=N, opB=N):
-        """A, B = (rowptr, col, val) torch CUDA tensors as stored (borrowed)."""
-        import torch
-        self.m, self.n, self.dt = m, n, np.float64 if A[2].dtype == torch.float64 else np.float32
-        self._keep = [A, B]
-        dtype = capi.DTYPE_F64 if self.dt == np.float64 else capi.DTYPE_F32
-        p = lambda t: ctypes.c_void_p(t.data_ptr())
-        return self.lib.bhb200_init_data_device_op(self.ctx, dtype, opA, opB, m, k, n, int(A[1].numel()), p(A[2]), p(A[0]),
-                                                   p(A[1]), int(B[1].numel()), p(B[2]), p(B[0]), p(B[1]))
-
-    def set_mask(self, rp, col):
-        rp = np.ascontiguousarray(rp, dtype=np.int32)
-        col = np.ascontiguousarray(col, dtype=np.int32)
-        return self.lib.bhb200_set_mask(self.ctx, int(col.size), ctypes.c_void_p(rp.ctypes.data),
-                                        ctypes.c_void_p(col.ctypes.data) if col.size else None)
-
-    def set_mask_device(self, rp, col):
-        self._keep.append((rp, col))
-        return self.lib.bhb200_set_mask_device(self.ctx, int(col.numel()), ctypes.c_void_p(rp.data_ptr()),
-                                               ctypes.c_void_p(col.data_ptr()))
-
-    def clear_mask(self):
-        return self.lib.bhb200_clear_mask(self.ctx)
-
-    def check(self, rc):
-        capi.check(self.lib, self.ctx, rc)
-
-    def spgemm(self):
-        return self.lib.bhb200_spgemm(self.ctx)
-
-    def numeric(self):
-        return self.lib.bhb200_spgemm_numeric(self.ctx)
-
-    def update(self, va, vb):
-        fn = self.lib.bhb200_update_values_f64 if self.dt == np.float64 else self.lib.bhb200_update_values_f32
-        p = lambda a: ctypes.c_void_p(a.ctypes.data) if a is not None else None
-        self._vals = (va, vb)
-        return fn(self.ctx, p(va), p(vb))
-
-    def C(self):
-        nnz = int(self.lib.bhb200_get_nnzC(self.ctx))
-        rp = np.zeros(self.m + 1, dtype=np.int64)
-        col = np.empty(nnz, dtype=np.int32)
-        val = np.empty(nnz, dtype=self.dt)
-        self.check(self.lib.bhb200_get_rowptrC_i64(self.ctx, ctypes.c_void_p(rp.ctypes.data)))
-        self.check(self.lib.bhb200_get_C_range(self.ctx, 0, nnz, ctypes.c_void_p(col.ctypes.data),
-                                               ctypes.c_void_p(val.ctypes.data)))
-        return rp, col, val
-
-    def stats(self):
-        st = capi.Stats()
-        self.check(self.lib.bhb200_get_stats(self.ctx, ctypes.byref(st)))
-        return st.as_dict()
-
-    def error(self):
-        return self.lib.bhb200_last_error(self.ctx).decode()
-
-    def close(self):
-        self.lib.bhb200_destroy(self.ctx)
-
-
 @pytest.fixture
 def ctx():
-    c = Ctx()
-    yield c
-    c.close()
+    with capi.Context() as c:
+        yield c
 
 
 def rtol_of(dt, values):
@@ -165,8 +60,8 @@ def rtol_of(dt, values):
 
 
 def check_masked(c, A, B, rpM, colM, what, opA=N, opB=N, values="int"):
-    c.check(c.set_mask(rpM, colM))
-    c.check(c.spgemm())
+    c.set_mask(rpM, colM)
+    c.spgemm()
     C, m, n = unmasked(A, B, opA, opB)
     want = restrict(C, m, n, rpM, colM)
     exact, rtol = rtol_of(A.val.dtype, values)
@@ -223,7 +118,7 @@ def test_masked_product(ctx, name, build, dt):
     for values in ("int", "real"):
         A, B = build(dt, values)
         C, m, n = unmasked(A, B)
-        ctx.check(ctx.init(A, B, same=A is B))
+        ctx.init(A, B, same=A is B)
         for kind in MASKS:
             rpM, colM = make_mask(kind, A, C, m, n)
             check_masked(ctx, A, B, rpM, colM, f"{name}/{values}/{kind}", values=values)
@@ -278,7 +173,7 @@ BIN_ROWS = [
 @pytest.mark.parametrize("dt", [np.float64, np.float32], ids=["f64", "f32"])
 def test_every_masked_bin(ctx, dt):
     A, B, rpM, colM = _bin_operands([r for r, _ in BIN_ROWS], dt)
-    ctx.check(ctx.init(A, B))
+    ctx.init(A, B)
     st = check_masked(ctx, A, B, rpM, colM, "bins", values="int" if dt == np.float64 else "real")
     want = np.bincount([b for _, b in BIN_ROWS], minlength=capi.NUM_MASK_BINS)
     assert st["mask_bin_rows"] == list(want), st["mask_bin_rows"]
@@ -291,41 +186,39 @@ def test_cancellation_keeps_explicit_zero(ctx):
                 np.array([(1.0 if i % 2 == 0 else -1.0) for i in range(k) for _ in (0, 1)]))
     A = gen.CSR(2, k, np.array([0, k, k + 2], np.int32), np.concatenate([np.arange(k), [0, 1]]).astype(np.int32),
                 np.ones(k + 2))
-    ctx.check(ctx.init(A, B))
-    ctx.check(ctx.set_mask(np.array([0, 1, 2], np.int32), np.array([0, 0], np.int32)))
-    ctx.check(ctx.spgemm())
+    ctx.init(A, B)
+    ctx.set_mask(np.array([0, 1, 2], np.int32), np.array([0, 0], np.int32))
+    ctx.spgemm()
     rp, col, val = ctx.C()
     assert list(rp) == [0, 1, 2] and list(col) == [0, 0] and list(val) == [0.0, 0.0]
 
 
 # ---- 3. triangle counting ---------------------------------------------------------------------------
 def _lower(scale):
+    """L = strictly lower triangle of the symmetrized R-MAT graph with values 1, and its triangle count by scipy."""
     sp = pytest.importorskip("scipy.sparse")
-    R = gen.rmat(scale, 16, values="ones")
-    S = sp.csr_matrix((R.val, R.col, R.rowptr), shape=(R.rows, R.cols))
-    S = ((S + S.T) > 0).astype(np.float64)
-    L = sp.tril(S, k=-1, format="csr")
-    L.sort_indices()
-    return L, float((L @ L).multiply(L).sum())
+    L = lower_triangle(symmetrize(gen.rmat(scale, 16)))
+    L = gen.CSR(L.rows, L.cols, L.rowptr, L.col, np.ones(L.nnz))
+    S = sp.csr_matrix((L.val, L.col, L.rowptr), shape=(L.rows, L.cols))
+    return L, float((S @ S).multiply(S).sum())
 
 
 @pytest.mark.parametrize("scale", [12, 13, 14])
 def test_triangle_counting(ctx, scale):
     import torch
-    L, triangles = _lower(scale)
-    n = L.shape[0]
-    X = gen.CSR(n, n, L.indptr.astype(np.int32), L.indices.astype(np.int32), L.data.astype(np.float64))
-    ctx.check(ctx.init(X, X, same=True))
-    ctx.check(ctx.set_mask(X.rowptr, X.col))
-    ctx.check(ctx.spgemm())
+    X, triangles = _lower(scale)
+    n = X.rows
+    ctx.init(X, X, same=True)
+    ctx.set_mask(X.rowptr, X.col)
+    ctx.spgemm()
     assert ctx.C()[2].sum() == triangles
     # device-resident L as A, B and M, no copy
     rp, col, val = (torch.from_numpy(X.rowptr).cuda(), torch.from_numpy(X.col).cuda(), torch.from_numpy(X.val).cuda())
-    d = Ctx()
+    d = capi.Context()
     try:
-        d.check(d.init_device(n, n, n, (rp, col, val), (rp, col, val)))
-        d.check(d.set_mask_device(rp, col))
-        d.check(d.spgemm())
+        d.init_device((rp, col, val), (rp, col, val), n, n, n)
+        d.set_mask_device(rp, col)
+        d.spgemm()
         assert d.C()[2].sum() == triangles
         assert d.stats()["masked"] == 1
     finally:
@@ -339,12 +232,12 @@ def test_a_at_masked(ctx, dt):
     A = gen.random_csr(800, 1200, np.arange(800) % 60, seed=21, dtype=dt)
     C, m, n = unmasked(A, A, N, T)
     rpM, colM = union(subset(np.asarray(C[0], np.int32), C[1], 0.3, 22), make_mask("outside", A, C, m, n, 23), n)
-    ctx.check(ctx.init(A, A, N, T, same=True))
+    ctx.init(A, A, N, T, same=True)
     check_masked(ctx, A, A, rpM, colM, "A*A^T host", N, T)
     dev = tuple(torch.from_numpy(x).cuda() for x in (A.rowptr, A.col, A.val))
-    d = Ctx()
+    d = capi.Context()
     try:
-        d.check(d.init_device(800, 1200, 800, dev, dev, N, T))
+        d.init_device(dev, dev, 800, 1200, 800, N, T)
         check_masked(d, A, A, rpM, colM, "A*A^T borrowed", N, T)
     finally:
         d.close()
@@ -354,45 +247,49 @@ def test_a_at_masked(ctx, dt):
 def test_lifecycle(ctx):
     A = gen.rmat(11, 8)
     C, m, n = unmasked(A, A)
-    ctx.check(ctx.init(A, A, same=True))
+    ctx.init(A, A, same=True)
     m1 = subset(np.asarray(C[0], np.int32), C[1], 0.5, 1)
     m2 = make_mask("outside", A, C, m, n, 2)
     check_masked(ctx, A, A, *m1, "mask 1")
     check_masked(ctx, A, A, *m2, "mask 2 replaces mask 1")
     # clear: the unmasked product, with the launches of a fresh context
-    ctx.check(ctx.clear_mask())
+    ctx.clear_mask()
     assert_csr_equal(ctx.C(), restrict(C, m, n, *m2), what="C readable after clear_mask")
-    assert ctx.numeric() == capi.ERR_INVALID and "mask" in ctx.error()
-    ctx.check(ctx.spgemm())
+    with pytest.raises(capi.BhsparseError, match="mask") as e:
+        ctx.spgemm_numeric()
+    assert e.value.code == capi.ERR_INVALID and "mask" in ctx.error()
+    ctx.spgemm()
     assert_csr_equal(ctx.C(), C, what="after clear_mask")
-    fresh = Ctx()
+    fresh = capi.Context()
     try:
-        fresh.check(fresh.init(A, A, same=True))
-        fresh.check(fresh.spgemm())
+        fresh.init(A, A, same=True)
+        fresh.spgemm()
         assert ctx.stats()["kernel_launches"] == fresh.stats()["kernel_launches"]
         assert ctx.stats()["masked"] == 0
     finally:
         fresh.close()
     # init_data clears the mask
     check_masked(ctx, A, A, *m1, "mask again")
-    ctx.check(ctx.init(A, A, same=True))
-    ctx.check(ctx.spgemm())
+    ctx.init(A, A, same=True)
+    ctx.spgemm()
     assert_csr_equal(ctx.C(), C, what="init_data cleared the mask")
     # set_mask without a new spgemm: no numeric-only update
-    ctx.check(ctx.set_mask(*m1))
-    assert ctx.numeric() == capi.ERR_INVALID and "mask" in ctx.error()
+    ctx.set_mask(*m1)
+    with pytest.raises(capi.BhsparseError, match="mask") as e:
+        ctx.spgemm_numeric()
+    assert e.value.code == capi.ERR_INVALID and "mask" in ctx.error()
     assert_csr_equal(ctx.C(), C, what="C readable after set_mask")
 
 
 @pytest.mark.parametrize("dt", [np.float64, np.float32], ids=["f64", "f32"])
 def test_update_values_and_numeric(ctx, dt):
     A, B, rpM, colM = _bin_operands([r for r, _ in BIN_ROWS], dt)
-    ctx.check(ctx.init(A, B))
+    ctx.init(A, B)
     check_masked(ctx, A, B, rpM, colM, "first values", values="real")
     A2 = gen.CSR(A.rows, A.cols, A.rowptr, A.col, gen.int_values(A.nnz, 31, dt))
     B2 = gen.CSR(B.rows, B.cols, B.rowptr, B.col, gen.int_values(B.nnz, 32, dt))
-    ctx.check(ctx.update(A2.val, B2.val))
-    ctx.check(ctx.numeric())
+    ctx.update_values(A2.val, B2.val)
+    ctx.spgemm_numeric()
     C, m, n = unmasked(A2, B2)
     exact, rtol = rtol_of(dt, "int" if dt == np.float64 else "real")
     assert_csr_equal(ctx.C(), restrict(C, m, n, rpM, colM), exact_values=exact, rtol=rtol, what="numeric after update")
@@ -421,11 +318,15 @@ def _bad_masks(m, n):
 
 def test_mask_errors(ctx):
     A = gen.poisson5pt(8, 8)
-    assert ctx.set_mask(A.rowptr, A.col) == capi.ERR_INVALID and "mask" in ctx.error()   # before init_data
-    ctx.check(ctx.init(A, A, same=True))
+    with pytest.raises(capi.BhsparseError, match="mask") as e:   # before init_data
+        ctx.set_mask(A.rowptr, A.col)
+    assert e.value.code == capi.ERR_INVALID and "mask" in ctx.error()
+    ctx.init(A, A, same=True)
     for what, rp, col, word in _bad_masks(A.rows, A.cols):
-        ctx.check(ctx.set_mask(rp, col))
-        assert ctx.spgemm() == capi.ERR_INVALID, what
+        ctx.set_mask(rp, col)
+        with pytest.raises(capi.BhsparseError) as e:
+            ctx.spgemm()
+        assert e.value.code == capi.ERR_INVALID, what
         assert "mask" in ctx.error() and word in ctx.error(), (what, ctx.error())
     check_masked(ctx, A, A, A.rowptr, A.col, "a good mask after bad ones")
 
@@ -436,13 +337,16 @@ def test_mask_on_dist_context(ctx):
     rc = lib.bhb200_dist_unique_id(uid)
     if rc != capi.SUCCESS:
         pytest.skip("NCCL not available")
-    ctx.check(lib.bhb200_dist_init(ctx.ctx, 0, 1, uid))
+    capi.check(lib, ctx.ctx, lib.bhb200_dist_init(ctx.ctx, 0, 1, uid))
     import torch
     A = gen.poisson5pt(8, 8)
     dev = [torch.from_numpy(x).cuda() for x in (A.rowptr, A.col, A.val)]
-    ctx.check(lib.bhb200_dist_setup_square(ctx.ctx, 0, capi.DTYPE_F64, A.rows, A.nnz, *[ctypes.c_void_p(t.data_ptr()) for t in dev]))
-    assert ctx.set_mask(A.rowptr, A.col) == capi.ERR_INVALID and "mask" in ctx.error()
-    ctx.check(lib.bhb200_dist_finalize(ctx.ctx))
+    capi.check(lib, ctx.ctx, lib.bhb200_dist_setup_square(ctx.ctx, 0, capi.DTYPE_F64, A.rows, A.nnz,
+                                                          *[ctypes.c_void_p(t.data_ptr()) for t in dev]))
+    with pytest.raises(capi.BhsparseError, match="mask") as e:
+        ctx.set_mask(A.rowptr, A.col)
+    assert e.value.code == capi.ERR_INVALID and "mask" in ctx.error()
+    capi.check(lib, ctx.ctx, lib.bhb200_dist_finalize(ctx.ctx))
 
 
 # ---- 7. staging and C in host memory; empty shapes --------------------------------------------------
@@ -452,9 +356,9 @@ def test_device_cap_spills(monkeypatch):
     rpM, colM = union(subset(np.asarray(C[0], np.int32), C[1], 0.5, 3), (A.rowptr, A.col), n)
     want = restrict(C, m, n, rpM, colM)
     monkeypatch.setenv("BHB200_DEBUG_DEVICE_CAP", "4096")
-    c = Ctx()
+    c = capi.Context()
     try:
-        c.check(c.init(A, A, same=True))
+        c.init(A, A, same=True)
         st = check_masked(c, A, A, rpM, colM, "spilled")
         assert st["spill_bytes"] > 0
         assert_csr_equal(c.C(), want, what="spilled")
@@ -465,13 +369,13 @@ def test_device_cap_spills(monkeypatch):
 def test_empty_shapes(ctx):
     E = gen.CSR(0, 5, np.zeros(1, np.int32), np.zeros(0, np.int32), np.zeros(0))
     B = gen.poisson5pt(5, 1)
-    ctx.check(ctx.init(E, B))
-    ctx.check(ctx.set_mask(np.zeros(1, np.int32), np.zeros(0, np.int32)))
-    ctx.check(ctx.spgemm())
+    ctx.init(E, B)
+    ctx.set_mask(np.zeros(1, np.int32), np.zeros(0, np.int32))
+    ctx.spgemm()
     assert ctx.lib.bhb200_get_nnzC(ctx.ctx) == 0
     A = gen.poisson5pt(6, 6)
-    ctx.check(ctx.init(A, A, same=True))
-    ctx.check(ctx.set_mask(np.zeros(A.rows + 1, np.int32), np.zeros(0, np.int32)))
-    ctx.check(ctx.spgemm())
+    ctx.init(A, A, same=True)
+    ctx.set_mask(np.zeros(A.rows + 1, np.int32), np.zeros(0, np.int32))
+    ctx.spgemm()
     assert ctx.lib.bhb200_get_nnzC(ctx.ctx) == 0
     assert list(ctx.C()[0]) == [0] * (A.rows + 1)

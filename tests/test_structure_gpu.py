@@ -13,6 +13,7 @@ import pytest
 import oracle
 from benchmark_spgemm_using_csr_b200 import capi, generators as gen
 from benchmark_spgemm_using_csr_b200.bhsparse import bhsparse, spgemm, NUM_PLATFORMS, BHSPARSE_CUDA
+from csr_ref import lower_triangle, product, restrict, symmetrize
 
 pytestmark = pytest.mark.gpu
 
@@ -20,120 +21,33 @@ N, T = capi.OP_N, capi.OP_T
 SAME_PATH = ["products", "nnzC", "sym_bin_rows", "num_bin_rows", "direct_bin_mask", "pattern_mode"]
 
 
-def host_transpose(X: gen.CSR) -> gen.CSR:
-    rows = np.repeat(np.arange(X.rows, dtype=np.int64), np.diff(X.rowptr.astype(np.int64)))
-    perm = np.argsort(X.col, kind="stable")
-    rowptr = np.zeros(X.cols + 1, dtype=np.int64)
-    np.cumsum(np.bincount(X.col, minlength=X.cols), out=rowptr[1:])
-    return gen.CSR(X.cols, X.rows, rowptr.astype(np.int32), rows[perm].astype(np.int32), X.val[perm])
-
-
-def keys(rowptr, col, n):
-    rows = np.repeat(np.arange(len(rowptr) - 1, dtype=np.int64), np.diff(np.asarray(rowptr, dtype=np.int64)))
-    return rows * n + col.astype(np.int64)
-
-
 def oracle_pattern(A, B, opA=N, opB=N, mask=None):
-    a = host_transpose(A) if opA == T else A
-    b = host_transpose(B) if opB == T else B
-    rp, col, _ = oracle.spgemm(a.rows, a.cols, b.cols, a.rowptr, a.col, a.val.astype(np.float64), b.rowptr, b.col,
-                               b.val.astype(np.float64))
-    rp = np.asarray(rp, dtype=np.int64)
-    if mask is not None:
-        keep = np.isin(keys(rp, col, b.cols), keys(mask[0], mask[1], b.cols))
-        rows = np.repeat(np.arange(a.rows, dtype=np.int64), np.diff(rp))
-        rp = np.zeros(a.rows + 1, dtype=np.int64)
-        np.cumsum(np.bincount(rows[keep], minlength=a.rows), out=rp[1:])
-        col = col[keep]
-    return rp, np.asarray(col, dtype=np.int32)
+    m, _, n = capi.op_dims(A, B, opA, opB)
+    C = product(A.astype(np.float64), B.astype(np.float64), opA, opB)
+    rp, col, _ = restrict(C, m, n, *mask) if mask is not None else C
+    return np.asarray(rp, dtype=np.int64), np.asarray(col, dtype=np.int32)
 
 
-class Ctx:
-    def __init__(self):
-        self.lib = capi.load()
-        self.ctx = ctypes.c_void_p()
-        assert self.lib.bhb200_create(ctypes.byref(self.ctx), 0) == capi.SUCCESS
-        self._keep = []
-
-    def init(self, A, B, dt, opA=N, opB=N, same=False):
-        """dt: np.float32 / np.float64, or None for structure-only host operands."""
-        m, k = (A.cols, A.rows) if opA == T else (A.rows, A.cols)
-        n = B.rows if opB == T else B.cols
-        self.m = m
-        p = lambda a: ctypes.c_void_p(a.ctypes.data)
-        ia = [np.ascontiguousarray(A.rowptr), np.ascontiguousarray(A.col)]
-        ib = ia if same else [np.ascontiguousarray(B.rowptr), np.ascontiguousarray(B.col)]
-        if dt is None:
-            self._keep = [ia, ib]
-            return self.lib.bhb200_init_data_structure(self.ctx, opA, opB, m, k, n, A.nnz, *map(p, ia), B.nnz, *map(p, ib))
-        va = np.ascontiguousarray(A.val.astype(dt))
-        vb = va if same else np.ascontiguousarray(B.val.astype(dt))
-        self._keep = [ia, ib, va, vb]
-        fn = self.lib.bhb200_init_data_op_f64 if dt == np.float64 else self.lib.bhb200_init_data_op_f32
-        return fn(self.ctx, opA, opB, m, k, n, A.nnz, p(va), *map(p, ia), B.nnz, p(vb), *map(p, ib))
-
-    def init_device(self, A, B, dtype, opA=N, opB=N, values=False):
-        """Borrowed device operands; structure-only ones get NULL value pointers unless `values`."""
-        import torch
-        m, k = (A.cols, A.rows) if opA == T else (A.rows, A.cols)
-        n = B.rows if opB == T else B.cols
-        self.m = m
-        dev = lambda x: torch.from_numpy(np.ascontiguousarray(x)).cuda()
-        vt = np.float32 if dtype == capi.DTYPE_F32 else np.float64
-        ta = [dev(A.rowptr), dev(A.col), dev(A.val.astype(vt))]
-        tb = ta if B is A else [dev(B.rowptr), dev(B.col), dev(B.val.astype(vt))]
-        self._keep = [ta, tb]
-        p = lambda t: ctypes.c_void_p(t.data_ptr())
-        vA = p(ta[2]) if values or dtype != capi.DTYPE_NONE else None
-        vB = p(tb[2]) if values or dtype != capi.DTYPE_NONE else None
-        return self.lib.bhb200_init_data_device_op(self.ctx, dtype, opA, opB, m, k, n, A.nnz, vA, p(ta[0]), p(ta[1]),
-                                                   B.nnz, vB, p(tb[0]), p(tb[1]))
-
-    def set_mask(self, rp, col):
-        self._mask = (np.ascontiguousarray(rp, dtype=np.int32), np.ascontiguousarray(col, dtype=np.int32))
-        return self.lib.bhb200_set_mask(self.ctx, int(col.size), ctypes.c_void_p(self._mask[0].ctypes.data),
-                                        ctypes.c_void_p(self._mask[1].ctypes.data) if col.size else None)
-
-    def check(self, rc):
-        capi.check(self.lib, self.ctx, rc)
-
-    def spgemm(self):
-        return self.lib.bhb200_spgemm(self.ctx)
-
-    def structure(self):
-        """(rowptr int64, col int32) through bhb200_get_C_structure (any product)."""
-        nnz = int(self.lib.bhb200_get_nnzC(self.ctx))
-        rp = np.zeros(self.m + 1, dtype=np.int32)
-        col = np.empty(nnz, dtype=np.int32)
-        self.check(self.lib.bhb200_get_C_structure(self.ctx, ctypes.c_void_p(rp.ctypes.data), ctypes.c_void_p(col.ctypes.data)))
-        return rp.astype(np.int64), col
-
-    def stats(self):
-        st = capi.Stats()
-        self.check(self.lib.bhb200_get_stats(self.ctx, ctypes.byref(st)))
-        return st.as_dict()
-
-    def error(self):
-        return self.lib.bhb200_last_error(self.ctx).decode()
-
-    def close(self):
-        self.lib.bhb200_destroy(self.ctx)
+def _device(X, dt):
+    """X on the device as borrowed (rowptr, col, val), val None for structure-only"""
+    import torch
+    dev = lambda x: torch.from_numpy(np.ascontiguousarray(x)).cuda()
+    return dev(X.rowptr), dev(X.col), None if dt is None else dev(X.val.astype(dt))
 
 
 def run(A, B, dt, opA=N, opB=N, same=False, mask=None, device=False):
-    c = Ctx()
-    try:
+    """dt: np.float32 / np.float64, or None for structure-only operands; returns ((rowptr, col) of C, stats)."""
+    dtype = capi.DTYPE_NONE if dt is None else capi.dtype_of(np.dtype(dt))
+    with capi.Context() as c:
         if device:
-            dtype = {None: capi.DTYPE_NONE, np.float32: capi.DTYPE_F32, np.float64: capi.DTYPE_F64}[dt]
-            c.check(c.init_device(A, B, dtype, opA, opB))
+            ta = _device(A, dt)
+            c.init_device(ta, ta if B is A else _device(B, dt), *capi.op_dims(A, B, opA, opB), opA, opB, dtype)
         else:
-            c.check(c.init(A, B, dt, opA, opB, same))
+            c.init(A, B, opA, opB, dtype, same)
         if mask is not None:
-            c.check(c.set_mask(*mask))
-        c.check(c.spgemm())
-        return c.structure(), c.stats()
-    finally:
-        c.close()
+            c.set_mask(*mask)
+        c.spgemm()
+        return c.C()[:2], c.stats()
 
 
 def check_structure(A, B, what, opA=N, opB=N, same=False, mask=None, device=False):
@@ -247,32 +161,13 @@ def test_transposed(ops, device, monkeypatch):
 def test_same_arrays_uploaded_once(ops):
     A = gen.rmat(11, 8, seed=5)
     st = check_structure(A, A, f"A op {ops} A", *ops, same=True)
-    c = Ctx()
-    try:
-        c.check(c.init(A, A, None, *ops, same=True))
+    with capi.Context() as c:
+        c.init(A, A, *ops, capi.DTYPE_NONE, same=True)
         assert c.lib.bhb200_operands_aliased(c.ctx) == 1
-    finally:
-        c.close()
     assert st["transposed_ops"] == (1 if ops[0] == T else 0) | (2 if ops[1] == T else 0)
 
 
 # ---- 4. masked products ------------------------------------------------------------------------------------
-def lower_triangle(A):
-    rows = np.repeat(np.arange(A.rows, dtype=np.int64), np.diff(A.rowptr.astype(np.int64)))
-    keep = A.col < rows
-    rowptr = np.zeros(A.rows + 1, dtype=np.int64)
-    np.cumsum(np.bincount(rows[keep], minlength=A.rows), out=rowptr[1:])
-    return gen.CSR(A.rows, A.cols, rowptr.astype(np.int32), A.col[keep].astype(np.int32), A.val[keep])
-
-
-def symmetrize(A):
-    k = np.union1d(keys(A.rowptr, A.col, A.cols), (A.col.astype(np.int64) * A.cols +
-                                                   np.repeat(np.arange(A.rows), np.diff(A.rowptr.astype(np.int64)))))
-    rowptr = np.zeros(A.rows + 1, dtype=np.int64)
-    np.cumsum(np.bincount(k // A.cols, minlength=A.rows), out=rowptr[1:])
-    return gen.CSR(A.rows, A.cols, rowptr.astype(np.int32), (k % A.cols).astype(np.int32), gen.int_values(k.size, 3))
-
-
 @pytest.mark.parametrize("case", ["triangle", "rmat_pattern_A", "random_mask_dense_rows"])
 def test_masked(case):
     if case == "triangle":                       # (L*L) .* L: every masked bin of a skewed graph, hit flags only
@@ -298,15 +193,13 @@ def test_borrowed_null_values(pattern, monkeypatch):
     check_structure(A, A, f"borrowed stencil pattern={pattern}", device=True)
     R = gen.rmat(12, 16, a=0.57, b=0.19, c=0.19, d=0.05, seed=8)
     check_structure(R, R, f"borrowed rmat pattern={pattern}", device=True)
-    c = Ctx()
-    try:   # valued device arrays read as structure: the values are never touched
-        c.check(c.init_device(R, R, capi.DTYPE_NONE, values=True))
-        c.check(c.spgemm())
+    with capi.Context() as c:   # valued device arrays read as structure: the values are never touched
+        tr = _device(R, np.float64)
+        c.init_device(tr, tr, R.rows, R.cols, R.cols, dtype=capi.DTYPE_NONE)
+        c.spgemm()
         want = oracle_pattern(R, R)
-        got = c.structure()
+        got = c.C()
         assert np.array_equal(got[0], want[0]) and np.array_equal(got[1], want[1])
-    finally:
-        c.close()
 
 
 # ---- 6. host spill ---------------------------------------------------------------------------------------
@@ -326,12 +219,11 @@ def test_context_switches_value_type(pattern, monkeypatch):
     monkeypatch.setenv("BHB200_PATTERN", pattern)
     A = gen.poisson27pt(12, 12, 12)
     want = oracle_pattern(A, A)
-    c = Ctx()
-    try:
+    with capi.Context() as c:
         for dt in (np.float64, None, np.float64, None, np.float32):
-            c.check(c.init(A, A, dt, same=True))
-            c.check(c.spgemm())
-            got = c.structure()
+            c.init(A, A, dtype=capi.DTYPE_NONE if dt is None else capi.dtype_of(np.dtype(dt)), same=True)
+            c.spgemm()
+            got = c.C()
             assert np.array_equal(got[0], want[0]) and np.array_equal(got[1], want[1]), f"{dt}"
             st = c.stats()
             assert st["dtype"] == (capi.DTYPE_NONE if dt is None else capi.DTYPE_F32 if dt == np.float32 else capi.DTYPE_F64)
@@ -339,12 +231,10 @@ def test_context_switches_value_type(pattern, monkeypatch):
             if dt is not None:   # the values are right after a structure-only product on the same context
                 nnz = int(c.lib.bhb200_get_nnzC(c.ctx))
                 val = np.empty(nnz, dtype=dt)
-                c.check(c.lib.bhb200_get_C_range(c.ctx, 0, nnz, None, ctypes.c_void_p(val.ctypes.data)))
+                capi.check(c.lib, c.ctx, c.lib.bhb200_get_C_range(c.ctx, 0, nnz, None, ctypes.c_void_p(val.ctypes.data)))
                 _, _, wv = oracle.spgemm(A.rows, A.cols, A.cols, A.rowptr, A.col, A.val.astype(dt), A.rowptr, A.col,
                                          A.val.astype(dt))
                 assert np.array_equal(val, wv)
-    finally:
-        c.close()
 
 
 # ---- 8. empty shapes -----------------------------------------------------------------------------------------
@@ -364,16 +254,14 @@ def test_empty_shapes():
 # ---- 9. errors and the getters -------------------------------------------------------------------------------
 def test_error_returns_and_getters():
     A = gen.rmat(10, 8, seed=2)
-    c = Ctx()
+    c = capi.Context()
     try:
         lib, ctx = c.lib, c.ctx
-        c.m = A.rows
         rp = np.zeros(A.rows + 1, dtype=np.int32)
         assert lib.bhb200_get_C_structure(ctx, ctypes.c_void_p(rp.ctypes.data), None) == capi.ERR_INVALID   # before spgemm
         assert lib.bhb200_get_C_structure(None, None, None) == capi.ERR_INVALID
-        c.check(c.init(A, A, None, same=True))
-        c.check(c.spgemm())
-        nnz = int(lib.bhb200_get_nnzC(ctx))
+        c.init(A, A, dtype=capi.DTYPE_NONE, same=True)
+        nnz = c.spgemm()
         buf = np.empty(max(nnz, 1), dtype=np.float64)
         vp = ctypes.c_void_p(buf.ctypes.data)
         for call, what in ((lambda: lib.bhb200_get_C_f64(ctx, None, None, vp), "get_C"),
@@ -389,25 +277,26 @@ def test_error_returns_and_getters():
         dval = torch.empty(nnz, dtype=torch.float64, device="cuda")
         assert lib.bhb200_copy_C_to_device(ctx, None, ctypes.c_void_p(dcol.data_ptr()),
                                            ctypes.c_void_p(dval.data_ptr())) == capi.ERR_INVALID
-        c.check(lib.bhb200_copy_C_to_device(ctx, None, ctypes.c_void_p(dcol.data_ptr()), None))
+        capi.check(lib, ctx, lib.bhb200_copy_C_to_device(ctx, None, ctypes.c_void_p(dcol.data_ptr()), None))
         want = oracle_pattern(A, A)
         assert np.array_equal(dcol.cpu().numpy(), want[1])
         # the range getter without values, the int64 row pointers, the device view with valC = NULL
         col = np.empty(nnz, dtype=np.int32)
-        c.check(lib.bhb200_get_C_range(ctx, 0, nnz, ctypes.c_void_p(col.ctypes.data), None))
+        capi.check(lib, ctx, lib.bhb200_get_C_range(ctx, 0, nnz, ctypes.c_void_p(col.ctypes.data), None))
         rp64 = np.empty(A.rows + 1, dtype=np.int64)
-        c.check(lib.bhb200_get_rowptrC_i64(ctx, ctypes.c_void_p(rp64.ctypes.data)))
+        capi.check(lib, ctx, lib.bhb200_get_rowptrC_i64(ctx, ctypes.c_void_p(rp64.ctypes.data)))
         assert np.array_equal(col, want[1]) and np.array_equal(rp64, want[0])
         ptrs = [ctypes.c_void_p() for _ in range(4)]
         ptrs[3] = ctypes.c_void_p(1)
-        c.check(lib.bhb200_get_C_device(ctx, *[ctypes.byref(p) for p in ptrs]))
+        capi.check(lib, ctx, lib.bhb200_get_C_device(ctx, *[ctypes.byref(p) for p in ptrs]))
         assert ptrs[2].value and not ptrs[3].value
         # structure of a valued product, and the valued getters again after re-initialising with values
-        c.check(c.init(A, A, np.float64, same=True))
-        c.check(c.spgemm())
-        got = c.structure()
-        assert np.array_equal(got[0], want[0]) and np.array_equal(got[1], want[1])
-        c.check(lib.bhb200_get_C_f64(ctx, None, None, vp))
+        c.init(A, A, same=True)
+        c.spgemm()
+        srp, scol = np.empty(A.rows + 1, np.int32), np.empty(nnz, np.int32)
+        capi.check(lib, ctx, lib.bhb200_get_C_structure(ctx, ctypes.c_void_p(srp.ctypes.data), ctypes.c_void_p(scol.ctypes.data)))
+        assert np.array_equal(srp, want[0]) and np.array_equal(scol, want[1])
+        capi.check(lib, ctx, lib.bhb200_get_C_f64(ctx, None, None, vp))
         # null columns with nonzeros, bad dtype
         z = np.zeros(A.rows + 1, dtype=np.int32)
         assert lib.bhb200_init_data_structure(ctx, N, N, A.rows, A.cols, A.cols, A.nnz, ctypes.c_void_p(A.rowptr.ctypes.data),

@@ -11,6 +11,7 @@ import pytest
 import oracle
 from benchmark_spgemm_using_csr_b200 import capi, generators as gen
 from conftest import assert_csr_equal
+from csr_ref import product
 
 pytestmark = pytest.mark.gpu
 
@@ -25,24 +26,6 @@ def _path(request, monkeypatch):
 
 
 # ---- host references -----------------------------------------------------------------------------
-def host_transpose(X: gen.CSR) -> gen.CSR:
-    """X^T by a stable argsort of the columns: entries of a row of X^T in stored order of X."""
-    rows = np.repeat(np.arange(X.rows, dtype=np.int64), np.diff(X.rowptr.astype(np.int64)))
-    perm = np.argsort(X.col, kind="stable")
-    rowptr = np.zeros(X.cols + 1, dtype=np.int64)
-    np.cumsum(np.bincount(X.col, minlength=X.cols), out=rowptr[1:])
-    return gen.CSR(X.cols, X.rows, rowptr.astype(np.int32), rows[perm].astype(np.int32), X.val[perm])
-
-
-def op(X, t):
-    return host_transpose(X) if t == T else X
-
-
-def want_product(A, B, opA, opB):
-    a, b = op(A, opA), op(B, opB)
-    return oracle.spgemm(a.rows, a.cols, b.cols, a.rowptr, a.col, a.val, b.rowptr, b.col, b.val)
-
-
 def shuffle_rows(X: gen.CSR, seed=7) -> gen.CSR:
     """Same matrix, entries of every stored row in random order."""
     rng = np.random.Generator(np.random.PCG64(seed))
@@ -53,98 +36,6 @@ def shuffle_rows(X: gen.CSR, seed=7) -> gen.CSR:
     return gen.CSR(X.rows, X.cols, X.rowptr, X.col[order].copy(), X.val[order].copy())
 
 
-def _host(ptr, n, typestr, np_dtype):
-    import torch
-    from benchmark_spgemm_using_csr_b200.dist import _DevicePtr
-    if n == 0:
-        return np.zeros(0, dtype=np_dtype)
-    return torch.as_tensor(_DevicePtr(ptr, n, typestr), device="cuda").cpu().numpy()
-
-
-# ---- a context on the C-ABI -------------------------------------------------------------------------
-class Ctx:
-    def __init__(self):
-        self.lib = capi.load()
-        self.ctx = ctypes.c_void_p()
-        assert self.lib.bhb200_create(ctypes.byref(self.ctx), 0) == capi.SUCCESS
-        self._keep = None
-
-    def init(self, opA, opB, A, B, same=False):
-        """Host operands as stored; same=True passes A's arrays for B too (aliasing)."""
-        m, k = (A.cols, A.rows) if opA == T else (A.rows, A.cols)
-        n = B.rows if opB == T else B.cols
-        self.m, self.dt = m, A.val.dtype
-        arrs = [np.ascontiguousarray(x) for x in (A.val, A.rowptr, A.col)]
-        brrs = arrs if same else [np.ascontiguousarray(x) for x in (B.val.astype(A.val.dtype), B.rowptr, B.col)]
-        self._keep = (arrs, brrs)
-        p = lambda a: ctypes.c_void_p(a.ctypes.data)
-        fn = self.lib.bhb200_init_data_op_f64 if self.dt == np.float64 else self.lib.bhb200_init_data_op_f32
-        return fn(self.ctx, opA, opB, m, k, n, A.nnz, *map(p, arrs), B.nnz, *map(p, brrs))
-
-    def init_device(self, opA, opB, m, k, n, A, B):
-        """A, B = (rowptr, col, val) torch CUDA tensors as stored (borrowed)."""
-        import torch
-        self.m, self.dt = m, np.float64 if A[2].dtype == torch.float64 else np.float32
-        self._keep = (A, B)
-        dtype = capi.DTYPE_F64 if self.dt == np.float64 else capi.DTYPE_F32
-        p = lambda t: ctypes.c_void_p(t.data_ptr())
-        return self.lib.bhb200_init_data_device_op(self.ctx, dtype, opA, opB, m, k, n, int(A[1].numel()), p(A[2]), p(A[0]),
-                                                   p(A[1]), int(B[1].numel()), p(B[2]), p(B[0]), p(B[1]))
-
-    def check(self, rc):
-        capi.check(self.lib, self.ctx, rc)
-
-    def spgemm(self):
-        return self.lib.bhb200_spgemm(self.ctx)
-
-    def numeric(self):
-        return self.lib.bhb200_spgemm_numeric(self.ctx)
-
-    def update(self, va, vb):
-        fn = self.lib.bhb200_update_values_f64 if self.dt == np.float64 else self.lib.bhb200_update_values_f32
-        p = lambda a: ctypes.c_void_p(a.ctypes.data) if a is not None else None
-        self._vals = (va, vb)
-        return fn(self.ctx, p(va), p(vb))
-
-    def C(self):
-        nnz = int(self.lib.bhb200_get_nnzC(self.ctx))
-        rp = np.zeros(self.m + 1, dtype=np.int32)
-        col = np.empty(nnz, dtype=np.int32)
-        val = np.empty(nnz, dtype=self.dt)
-        fn = self.lib.bhb200_get_C_f64 if self.dt == np.float64 else self.lib.bhb200_get_C_f32
-        p = lambda a: ctypes.c_void_p(a.ctypes.data)
-        self.check(fn(self.ctx, p(rp), p(col), p(val)))
-        return rp, col, val
-
-    def operands(self):
-        """The effective operands op(A), op(B) as the library holds them."""
-        dims = (ctypes.c_int32 * 6)()
-        ptrs = [ctypes.c_void_p() for _ in range(6)]
-        self.check(self.lib.bhb200_get_operands_device(self.ctx, dims, *[ctypes.byref(q) for q in ptrs]))
-        self.check(self.lib.bhb200_synchronize(self.ctx))
-        m, k, n, nnzA, nnzB, dtype = list(dims)
-        vt, vd = ("<f8", np.float64) if dtype == capi.DTYPE_F64 else ("<f4", np.float32)
-
-        def csr(rows, cols, nnz, rp, c, v):
-            return gen.CSR(rows, cols, _host(rp.value, rows + 1, "<i4", np.int32), _host(c.value, nnz, "<i4", np.int32),
-                           _host(v.value, nnz, vt, vd))
-        return csr(m, k, nnzA, *ptrs[:3]), csr(k, n, nnzB, *ptrs[3:])
-
-    def stats(self):
-        st = capi.Stats()
-        self.check(self.lib.bhb200_get_stats(self.ctx, ctypes.byref(st)))
-        return st.as_dict()
-
-    def aliased(self):
-        return int(self.lib.bhb200_operands_aliased(self.ctx))
-
-    def error(self):
-        return self.lib.bhb200_last_error(self.ctx).decode()
-
-    def close(self):
-        self.lib.bhb200_destroy(self.ctx)
-
-
 def assert_same_csr(got: gen.CSR, want: gen.CSR, what):
     assert (got.rows, got.cols) == (want.rows, want.cols), what
     assert np.array_equal(got.rowptr, want.rowptr), f"{what}: rowptr"
@@ -152,9 +43,9 @@ def assert_same_csr(got: gen.CSR, want: gen.CSR, what):
     assert got.val.dtype == want.val.dtype and np.array_equal(got.val, want.val), f"{what}: val"
 
 
-def check_product(c: Ctx, A, B, opA, opB, what, exact=True):
-    c.check(c.spgemm())
-    want = want_product(A, B, opA, opB)
+def check_product(c: capi.Context, A, B, opA, opB, what, exact=True):
+    c.spgemm()
+    want = product(A, B, opA, opB)
     rtol = 0 if exact else (1e-12 if A.val.dtype == np.float64 else 1e-5)
     assert_csr_equal(c.C(), want, exact_values=exact, rtol=rtol, what=what)
 
@@ -195,15 +86,16 @@ def test_transpose_bit_exact(name, dt):
     """op(A) = X^T read back from the device: rowptr, col and val (hence perm) equal the stable host transpose."""
     X = _with_real(_CASES[name], dt)
     empty_b = gen.CSR(X.rows, 1, np.zeros(X.rows + 1, dtype=np.int32), np.zeros(0, dtype=np.int32), np.zeros(0, dtype=dt))
-    c = Ctx()
+    c = capi.Context()
     try:
-        c.check(c.init(T, N, X, empty_b))
-        c.check(c.spgemm())
-        effA, _ = c.operands()
-        assert_same_csr(effA, host_transpose(X), f"{name} {dt.__name__}")
+        c.init(X, empty_b, T, N)
+        c.spgemm()
+        (m, k, _), effA, _ = c.operands()
+        effA = gen.CSR(m, k, *(t.cpu().numpy() for t in effA))
+        assert_same_csr(effA, gen.transpose(X), f"{name} {dt.__name__}")
         st = c.stats()
         assert st["transposed_ops"] == 1 and st["nnzC"] == 0
-        c.check(c.spgemm())                     # host operands: transposed once, kept
+        c.spgemm()                     # host operands: transposed once, kept
         assert c.stats()["ms_transpose"] == 0.0
     finally:
         c.close()
@@ -222,9 +114,9 @@ def test_products_diagonals(ops):
     """Nonsymmetric diagonal matrix (pattern mode on the effective operands: X^T has the negated offsets)."""
     D = gen.diagonals(3000, 3000, [-7, -1, 0, 2, 5])
     for same in (True, False):
-        c = Ctx()
+        c = capi.Context()
         try:
-            c.check(c.init(*ops, D, D, same=same))
+            c.init(D, D, *ops, same=same)
             assert c.aliased() == int(same)
             check_product(c, D, D, *ops, f"diagonals {ops} same={same}")
         finally:
@@ -236,17 +128,17 @@ def test_products_random_rect(ops):
     for seed, dt in ((1, np.float64), (3, np.float32)):
         A, B = _rect_pair(*ops, seed)
         A, B = A.astype(dt), B.astype(dt)
-        c = Ctx()
+        c = capi.Context()
         try:
-            c.check(c.init(*ops, A, B))
+            c.init(A, B, *ops)
             check_product(c, A, B, *ops, f"rect {ops} {dt.__name__}")
         finally:
             c.close()
     A, B = _rect_pair(*ops, 9)
     A, B = _with_real(A, np.float64), _with_real(B, np.float64, seed=12)
-    c = Ctx()
+    c = capi.Context()
     try:
-        c.check(c.init(*ops, A, B))
+        c.init(A, B, *ops)
         check_product(c, A, B, *ops, f"rect {ops} real", exact=False)
     finally:
         c.close()
@@ -255,9 +147,9 @@ def test_products_random_rect(ops):
 @pytest.mark.parametrize("dt", [np.float64, np.float32])
 def test_rmat_a_at(dt):
     A = gen.rmat(14, 16, a=0.57, b=0.19, c=0.19, d=0.05, seed=3, dtype=dt)
-    c = Ctx()
+    c = capi.Context()
     try:
-        c.check(c.init(N, T, A, A, same=True))
+        c.init(A, A, N, T, same=True)
         assert c.aliased() == 1
         check_product(c, A, A, N, T, f"rmat14 A*A^T {dt.__name__}")
     finally:
@@ -266,9 +158,9 @@ def test_rmat_a_at(dt):
 
 def test_uniform_rect_at_a():
     A = gen.uniform_rect(40000, 10000, 8)
-    c = Ctx()
+    c = capi.Context()
     try:
-        c.check(c.init(T, N, A, A, same=True))
+        c.init(A, A, T, N, same=True)
         assert c.aliased() == 1
         check_product(c, A, A, T, N, "uniform_rect A^T*A")
         assert c.stats()["transposed_ops"] == 1
@@ -282,15 +174,19 @@ def test_out_of_range_column_is_reported():
     bad = gen.CSR(A.rows, A.cols, A.rowptr, A.col.copy(), A.val)
     bad.col[17] = 200                                      # outside [0, 200)
     B = gen.random_csr(300, 50, 3, seed=3)
-    c = Ctx()
+    c = capi.Context()
     try:
-        c.check(c.init(T, N, bad, B))
-        assert c.spgemm() == capi.ERR_INVALID and "stored A" in c.error()
+        c.init(bad, B, T, N)
+        with pytest.raises(capi.BhsparseError) as e:
+            c.spgemm()
+        assert e.value.code == capi.ERR_INVALID and "stored A" in c.error()
         bad.col[17] = -5
         A2 = gen.random_csr(50, 200, 3, seed=4)            # op(B) = bad^T is 200 x 300
-        c.check(c.init(N, T, A2, bad))
-        assert c.spgemm() == capi.ERR_INVALID and "stored B" in c.error()
-        c.check(c.init(T, N, A, B))                        # the same context then runs a valid product
+        c.init(A2, bad, N, T)
+        with pytest.raises(capi.BhsparseError) as e:
+            c.spgemm()
+        assert e.value.code == capi.ERR_INVALID and "stored B" in c.error()
+        c.init(A, B, T, N)                                 # the same context then runs a valid product
         check_product(c, A, B, T, N, "after the error")
     finally:
         c.close()
@@ -301,10 +197,12 @@ def test_duplicate_in_transposed_b_is_rejected():
     B = gen.random_csr(60, 80, 5, seed=3)                  # stored n x k
     dup = gen.CSR(B.rows, B.cols, B.rowptr, B.col.copy(), B.val)
     dup.col[1] = dup.col[0]                                # the same (row, column) twice
-    c = Ctx()
+    c = capi.Context()
     try:
-        c.check(c.init(N, T, A, dup))
-        assert c.spgemm() == capi.ERR_INVALID
+        c.init(A, dup, N, T)
+        with pytest.raises(capi.BhsparseError) as e:
+            c.spgemm()
+        assert e.value.code == capi.ERR_INVALID
     finally:
         c.close()
 
@@ -312,9 +210,9 @@ def test_duplicate_in_transposed_b_is_rejected():
 def test_unsorted_stored_rows_with_transposed_b():
     A = gen.random_csr(400, 500, 6, seed=2)
     B = shuffle_rows(gen.random_csr(300, 500, 9, seed=3))  # stored n x k, rows in random order
-    c = Ctx()
+    c = capi.Context()
     try:
-        c.check(c.init(N, T, A, B))
+        c.init(A, B, N, T)
         check_product(c, A, B, N, T, "unsorted stored rows of B")
     finally:
         c.close()
@@ -328,17 +226,17 @@ def _vals(nnz, seed, dt):
 @pytest.mark.parametrize("ops", [(N, T), (T, N), (T, T)], ids=["NT", "TN", "TT"])
 def test_aliased_update_values(ops):
     A = gen.random_csr(2000, 2000, 10, seed=8) if ops == (T, T) else gen.random_csr(1500, 2500, 10, seed=8)
-    c = Ctx()
+    c = capi.Context()
     try:
-        c.check(c.init(*ops, A, A, same=True))
+        c.init(A, A, *ops, same=True)
         assert c.aliased() == 1
         check_product(c, A, A, *ops, f"aliased {ops}")
         v, w = _vals(A.nnz, 21, np.float64), _vals(A.nnz, 22, np.float64)
         for va, vb in ((v, v), (v, w)):
-            c.check(c.update(va, vb))
-            c.check(c.numeric())
-            want = want_product(gen.CSR(A.rows, A.cols, A.rowptr, A.col, va),
-                                gen.CSR(A.rows, A.cols, A.rowptr, A.col, vb), *ops)
+            c.update_values(va, vb)
+            c.spgemm_numeric()
+            want = product(gen.CSR(A.rows, A.cols, A.rowptr, A.col, va),
+                           gen.CSR(A.rows, A.cols, A.rowptr, A.col, vb), *ops)
             assert_csr_equal(c.C(), want, what=f"aliased {ops} update")
         assert c.aliased() == 0                            # split by the second update
     finally:
@@ -350,16 +248,16 @@ def test_aliased_update_values(ops):
 def test_reuse_transposed_host_operands(ops, dt):
     A, B = _rect_pair(*ops, 4)
     A, B = A.astype(dt), B.astype(dt)
-    c = Ctx()
+    c = capi.Context()
     try:
-        c.check(c.init(*ops, A, B))
-        c.check(c.spgemm())
+        c.init(A, B, *ops)
+        c.spgemm()
         for r in range(2):
             va, vb = _vals(A.nnz, 30 + r, dt), _vals(B.nnz, 40 + r, dt)
-            c.check(c.update(va, vb))
-            c.check(c.numeric())
-            want = want_product(gen.CSR(A.rows, A.cols, A.rowptr, A.col, va),
-                                gen.CSR(B.rows, B.cols, B.rowptr, B.col, vb), *ops)
+            c.update_values(va, vb)
+            c.spgemm_numeric()
+            want = product(gen.CSR(A.rows, A.cols, A.rowptr, A.col, va),
+                           gen.CSR(B.rows, B.cols, B.rowptr, B.col, vb), *ops)
             assert_csr_equal(c.C(), want, what=f"reuse {ops} round {r}")
             st = c.stats()
             assert st["num_bin_rows"][17] == 0 and st["ms_symbolic"] < 0.05     # no copy bin, no symbolic pass
@@ -388,32 +286,31 @@ def test_galerkin_chain_device_resident():
     tP = [torch.from_numpy(x).to(dev) for x in (P.rowptr, P.col, P.val)]
     stream = torch.cuda.Stream()
     torch.cuda.synchronize()
-    c1, c2 = Ctx(), Ctx()
+    c1, c2 = capi.Context(), capi.Context()
     try:
         for c in (c1, c2):
-            c.check(c.lib.bhb200_set_stream(c.ctx, ctypes.c_void_p(stream.cuda_stream)))
-        c1.check(c1.init_device(N, N, nf, nf, nc, tA, tP))
-        c1.check(c1.spgemm())
+            c.set_stream(stream.cuda_stream)
+        c1.init_device(tA, tP, nf, nf, nc)
+        nnzAP = c1.spgemm()
         rp32, rp64, colC, valC = (ctypes.c_void_p() for _ in range(4))
-        c1.check(c1.lib.bhb200_get_C_device(c1.ctx, ctypes.byref(rp32), ctypes.byref(rp64), ctypes.byref(colC), ctypes.byref(valC)))
-        nnzAP = int(c1.lib.bhb200_get_nnzC(c1.ctx))
+        capi.check(c1.lib, c1.ctx, c1.lib.bhb200_get_C_device(c1.ctx, ctypes.byref(rp32), ctypes.byref(rp64), ctypes.byref(colC),
+                                                              ctypes.byref(valC)))
         dp = lambda q: ctypes.c_void_p(q.value)
         rc = c2.lib.bhb200_init_data_device_op(c2.ctx, capi.DTYPE_F64, T, N, nc, nf, nc, P.nnz, ctypes.c_void_p(tP[2].data_ptr()),
                                                ctypes.c_void_p(tP[0].data_ptr()), ctypes.c_void_p(tP[1].data_ptr()),
                                                nnzAP, dp(valC), dp(rp32), dp(colC))
-        c2.check(rc)
-        c2.m, c2.dt = nc, np.float64
-        c2.check(c2.spgemm())
+        capi.check(c2.lib, c2.ctx, rc)
+        c2.m = nc
+        c2.spgemm()
 
         def want(Av, Pv):
             a = gen.CSR(nf, nf, A.rowptr, A.col, Av)
             p = gen.CSR(nf, nc, P.rowptr, P.col, Pv)
             ap = oracle.spgemm(nf, nf, nc, a.rowptr, a.col, a.val, p.rowptr, p.col, p.val)
-            pt = host_transpose(p)
+            pt = gen.transpose(p)
             return ap, oracle.spgemm(nc, nf, nc, pt.rowptr, pt.col, pt.val, *ap)
 
         ap, rap = want(A.val, P.val)
-        c1.m, c1.dt = nf, np.float64
         assert_csr_equal(c1.C(), ap, what="A*P")
         assert_csr_equal(c2.C(), rap, what="P^T*(A*P)")
         # new values of A and P, written in place on the device; numeric-only refresh of both products
@@ -421,8 +318,8 @@ def test_galerkin_chain_device_resident():
         with torch.cuda.stream(stream):
             tA[2].copy_(torch.from_numpy(Av2).to(dev, non_blocking=False))
             tP[2].copy_(torch.from_numpy(Pv2).to(dev, non_blocking=False))
-        c1.check(c1.numeric())
-        c2.check(c2.numeric())
+        c1.spgemm_numeric()
+        c2.spgemm_numeric()
         ap2, rap2 = want(Av2, Pv2)
         assert_csr_equal(c1.C(), ap2, what="A*P refreshed")
         assert_csr_equal(c2.C(), rap2, what="P^T*(A*P) refreshed")
@@ -438,17 +335,16 @@ def test_nn_op_matches_plain_init():
     B = gen.random_csr(A.cols, 3000, 6, seed=3)
     results = []
     for use_op in (False, True):
-        c = Ctx()
+        c = capi.Context()
         try:
             if use_op:
-                c.check(c.init(N, N, A, B))
+                c.init(A, B, N, N)
             else:
                 p = lambda a: ctypes.c_void_p(a.ctypes.data)
-                c.m, c.dt = A.rows, np.float64
-                c._keep = (A, B)
-                c.check(c.lib.bhb200_init_data_f64(c.ctx, A.rows, A.cols, B.cols, A.nnz, p(A.val), p(A.rowptr), p(A.col),
-                                                   B.nnz, p(B.val), p(B.rowptr), p(B.col)))
-            c.check(c.spgemm())
+                capi.check(c.lib, c.ctx, c.lib.bhb200_init_data_f64(c.ctx, A.rows, A.cols, B.cols, A.nnz, p(A.val), p(A.rowptr),
+                                                                    p(A.col), B.nnz, p(B.val), p(B.rowptr), p(B.col)))
+                c.m = A.rows
+            c.spgemm()
             st = c.stats()
             results.append((c.C(), st["kernel_launches"], st["transposed_ops"], st["ms_transpose"]))
         finally:

@@ -19,7 +19,6 @@ proof of those cases checks instead.
 Most cases hold about 2M products or fewer.  The direct-mode cases are larger because the direct mode samples only
 symbolic bins of at least 4096 rows, so each bin they need takes 4096 rows or more: bucket3_wide (six bins, about
 19M products), bucket3_chunks_long_b (about 29M) and bucket3_hub_column (about 11M)."""
-import ctypes
 from dataclasses import dataclass, field
 from typing import Callable
 
@@ -29,7 +28,8 @@ import pytest
 import exact_ref as xr
 from benchmark_spgemm_using_csr_b200 import capi, generators as gen
 from benchmark_spgemm_using_csr_b200.generators import CSR
-from test_mask_gpu import BIN_ROWS, _bin_operands, host_transpose, keys
+from csr_ref import keys, stored
+from test_mask_gpu import BIN_ROWS, _bin_operands
 
 pytestmark = pytest.mark.gpu
 
@@ -41,63 +41,6 @@ def lib(tmp_path_factory):
     lib = xr.compile_lib(tmp_path_factory.mktemp("exact_ref"))
     assert lib is not None, "gcc is needed to build the quad-precision reference"
     return lib
-
-
-# ---- a context on the C-ABI -------------------------------------------------------------------------
-class Ctx:
-    def __init__(self):
-        self.lib = capi.load()
-        self.ctx = ctypes.c_void_p()
-        assert self.lib.bhb200_create(ctypes.byref(self.ctx), 0) == capi.SUCCESS
-        self._keep = []
-
-    def check(self, rc):
-        capi.check(self.lib, self.ctx, rc)
-
-    def init(self, A, B, opA=N, opB=N):
-        """A, B as stored; C = op(A) * op(B)."""
-        m, k = (A.cols, A.rows) if opA == T else (A.rows, A.cols)
-        n = B.rows if opB == T else B.cols
-        self.m, self.dt = m, A.val.dtype
-        arrs = [np.ascontiguousarray(x) for x in (A.val, A.rowptr, A.col, B.val, B.rowptr, B.col)]
-        self._keep = arrs
-        p = [ctypes.c_void_p(a.ctypes.data) for a in arrs]
-        fn = self.lib.bhb200_init_data_op_f64 if self.dt == np.float64 else self.lib.bhb200_init_data_op_f32
-        self.check(fn(self.ctx, opA, opB, m, k, n, A.nnz, *p[:3], B.nnz, *p[3:]))
-
-    def set_mask(self, rp, col):
-        self._mask = (np.ascontiguousarray(rp, dtype=np.int32), np.ascontiguousarray(col, dtype=np.int32))
-        self.check(self.lib.bhb200_set_mask(self.ctx, int(col.size), *(ctypes.c_void_p(a.ctypes.data) for a in self._mask)))
-
-    def spgemm(self):
-        self.check(self.lib.bhb200_spgemm(self.ctx))
-        return self.C()
-
-    def update_numeric(self, va, vb):
-        va, vb = np.ascontiguousarray(va), np.ascontiguousarray(vb)
-        self._vals = (va, vb)
-        fn = self.lib.bhb200_update_values_f64 if self.dt == np.float64 else self.lib.bhb200_update_values_f32
-        self.check(fn(self.ctx, ctypes.c_void_p(va.ctypes.data), ctypes.c_void_p(vb.ctypes.data)))
-        self.check(self.lib.bhb200_spgemm_numeric(self.ctx))
-        return self.C()
-
-    def C(self):
-        nnz = int(self.lib.bhb200_get_nnzC(self.ctx))
-        rp = np.zeros(self.m + 1, dtype=np.int64)
-        col = np.empty(nnz, dtype=np.int32)
-        val = np.empty(nnz, dtype=self.dt)
-        self.check(self.lib.bhb200_get_rowptrC_i64(self.ctx, ctypes.c_void_p(rp.ctypes.data)))
-        self.check(self.lib.bhb200_get_C_range(self.ctx, 0, nnz, ctypes.c_void_p(col.ctypes.data),
-                                               ctypes.c_void_p(val.ctypes.data)))
-        return rp, col, val
-
-    def stats(self):
-        st = capi.Stats()
-        self.check(self.lib.bhb200_get_stats(self.ctx, ctypes.byref(st)))
-        return st.as_dict()
-
-    def close(self):
-        self.lib.bhb200_destroy(self.ctx)
 
 
 # ---- comparison ------------------------------------------------------------------------------------------
@@ -359,9 +302,6 @@ def test_values(lib, case, dt, monkeypatch):
     mask = case.mask(A, B) if case.mask else None
     opA, opB = case.ops
 
-    def stored(X, op):
-        return host_transpose(X) if op == T else X
-
     def reference(A, B):
         ref = xr.product(lib, A, B)
         return restrict(ref, B.cols, *mask) if mask is not None else ref
@@ -374,13 +314,10 @@ def test_values(lib, case, dt, monkeypatch):
             monkeypatch.delenv(k)
         for k, v in case.twin_of.items():
             monkeypatch.setenv(k, v)
-        other = Ctx()
-        try:
+        with capi.Context() as other:
             other.init(stored(A2, opA), stored(B2, opB), opA, opB)
             other.spgemm()
             twin_launches = other.stats()["kernel_launches"] - 3
-        finally:
-            other.close()
         for k in case.twin_of:
             monkeypatch.delenv(k)
         for k, v in case.env.items():
@@ -393,14 +330,14 @@ def test_values(lib, case, dt, monkeypatch):
             {k: st[k] for k in ("num_bin_rows", "direct_rows", "direct_retry_rows", "direct_bin_mask", "pattern_mode",
                                 "spill_bytes", "transposed_ops", "mask_bin_rows", "kernel_launches")})
 
-    ctx = Ctx()
-    try:
+    with capi.Context() as ctx:
         def run(A, B, what, exact=False, ref=None):
             """A, B: the effective operands with values; a fresh init_data and spgemm."""
             ctx.init(stored(A, opA), stored(B, opB), opA, opB)
             if mask is not None:
                 ctx.set_mask(*mask)
-            got = ctx.spgemm()
+            ctx.spgemm()
+            got = ctx.C()
             prove(ctx.stats(), what)
             check_values(got, reference(A, B) if ref is None else ref, f"{case.name} {np.dtype(dt).name} {what}", exact)
 
@@ -412,14 +349,14 @@ def test_values(lib, case, dt, monkeypatch):
         run(A2, B2, "tier 2", ref=ref2)
         # fresh values on the same context: update_values (values as stored) and spgemm_numeric
         A3, B3 = with_values(A, xr.tier2(A.nnz, 5, dt)), with_values(B, xr.tier2(B.nnz, 6, dt))
-        got = ctx.update_numeric(stored(A3, opA).val, stored(B3, opB).val)
+        ctx.update_values(stored(A3, opA).val, stored(B3, opB).val)
+        ctx.spgemm_numeric()
+        got = ctx.C()
         prove(ctx.stats(), "spgemm_numeric", reuse=True)
         check_values(got, reference(A3, B3), f"{case.name} {np.dtype(dt).name} tier 2 after update_values")
         if case.cancel:
             run(*xr.paired(A2, B2, seed=7), "tier 2 cancelling")
         run(with_values(A, xr.tier3(A.nnz, 8, dt)), with_values(B, xr.tier3(B.nnz, 9, dt)), "tier 3")
-    finally:
-        ctx.close()
 
 
 # ---- masks and non-finite values ---------------------------------------------------------------------------
@@ -442,18 +379,16 @@ def test_nonfinite_outside_mask_stays_outside(lib, dt):
     pick = np.random.default_rng(13).permutation(free)[:free.size // 3]
     v[pick[0::3]], v[pick[1::3]], v[pick[2::3]] = np.inf, -np.inf, np.nan
     B = with_values(B, v)
-    ctx = Ctx()
-    try:
+    with capi.Context() as ctx:
         ctx.init(A, B)
         ctx.set_mask(rpM, colM)
-        got = ctx.spgemm()
+        ctx.spgemm()
+        got = ctx.C()
         assert ctx.stats()["mask_bin_rows"] == MASK_BINS
         ref = restrict(xr.product(lib, A, B), B.cols, rpM, colM)
         assert (ref["cls"] == xr.FINITE).all()
         assert np.isfinite(got[2]).all(), "a non-finite product outside the mask reached C"
         check_values(got, ref, f"mask, non-finite outside {np.dtype(dt).name}")
-    finally:
-        ctx.close()
 
 
 @pytest.mark.parametrize("dt", [np.float64, np.float32], ids=["f64", "f32"])
@@ -464,8 +399,7 @@ def test_masked_cancelling_within_bound(lib, dt):
     A, B = xr.paired(with_values(A, xr.tier2(A.nnz, 21, dt)), with_values(B, xr.tier2(B.nnz, 22, dt)), seed=23)
     ref = xr.product(lib, A, B)
     rng = np.random.default_rng(24)
-    ctx = Ctx()
-    try:
+    with capi.Context() as ctx:
         ctx.init(A, B)
         for keep in (0.05, 0.5):
             sel = rng.random(ref["col"].size) < keep
@@ -474,8 +408,6 @@ def test_masked_cancelling_within_bound(lib, dt):
             np.cumsum(np.bincount(rows[sel], minlength=A.rows), out=rpM[1:])
             colM = ref["col"][sel]
             ctx.set_mask(rpM, colM)
-            got = ctx.spgemm()
+            ctx.spgemm()
             assert ctx.stats()["masked"] == 1
-            check_values(got, restrict(ref, B.cols, rpM, colM), f"mask keep {keep} cancelling {np.dtype(dt).name}")
-    finally:
-        ctx.close()
+            check_values(ctx.C(), restrict(ref, B.cols, rpM, colM), f"mask keep {keep} cancelling {np.dtype(dt).name}")

@@ -22,7 +22,6 @@ Workloads:
 from __future__ import annotations
 
 import argparse
-import ctypes
 import json
 import os
 import sys
@@ -31,82 +30,45 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
-sys.path.insert(0, os.path.join(ROOT, "tools"))
 
 from benchmark_spgemm_using_csr_b200 import capi, generators as gen  # noqa: E402
-from structure_probe import lower_triangle, power_limit  # noqa: E402
+from probe_util import COUNTERS, STAGES, lower_triangle, read_power_limit, run, summary  # noqa: E402
 
-DTYPES = {"c64": capi.DTYPE_C64, "f64": capi.DTYPE_F64, "f32": capi.DTYPE_F32}
-STAGES = ("ms_total", "ms_count", "ms_symbolic", "ms_scan", "ms_numeric", "ms_transpose")
-
-
-class Engine:
-    def __init__(self, dtype):
-        self.dtype = dtype
-        self.lib = capi.load()
-        self.ctx = ctypes.c_void_p()
-        assert self.lib.bhb200_create(ctypes.byref(self.ctx), 0) == capi.SUCCESS
-
-    def check(self, rc):
-        capi.check(self.lib, self.ctx, rc)
-
-    def init(self, m, k, n, A, B, M=None):
-        """A, B = (rowptr, col, val) torch tensors; M = (rowptr, col) or None"""
-        self._keep = (A, B, M)
-        p = lambda t: ctypes.c_void_p(t.data_ptr())
-        self.check(self.lib.bhb200_init_data_device(self.ctx, self.dtype, m, k, n, int(A[1].numel()), p(A[2]), p(A[0]),
-                                                    p(A[1]), int(B[1].numel()), p(B[2]), p(B[0]), p(B[1])))
-        if M is not None:
-            self.check(self.lib.bhb200_set_mask_device(self.ctx, int(M[1].numel()), p(M[0]), p(M[1])))
-
-    def run(self):
-        self.check(self.lib.bhb200_spgemm(self.ctx))
-        st = capi.Stats()
-        self.check(self.lib.bhb200_get_stats(self.ctx, ctypes.byref(st)))
-        return st
-
-    def close(self):
-        self.lib.bhb200_destroy(self.ctx)
-
-
-def summary(sts):
-    med = {key: float(np.median([getattr(s, key) for s in sts])) for key in STAGES}
-    s = sts[-1]
-    med.update({"products": int(s.products), "nnzC": int(s.nnzC), "kernel_launches": int(s.kernel_launches),
-                "pattern_mode": int(s.pattern_mode), "direct_bin_mask": int(s.direct_bin_mask),
-                "workspace_bytes": int(s.workspace_bytes)})
-    return med
+TYPES = ("c64", "f64", "f32")
 
 
 def bin_times(sts):
     """median per-bin kernel times (ms), bins that ran only"""
     out = {}
     for key in ("ms_sym_bin", "ms_num_bin"):
-        med = np.median([list(getattr(s, key)) for s in sts], axis=0)
+        med = np.median([s[key] for s in sts], axis=0)
         out[key] = {str(b): round(float(t), 4) for b, t in enumerate(med) if t > 0}
     return out
 
 
 def probe(torch, name, m, k, n, A, B, M, calls):
     """A, B: {type: (rowptr, col, val)} on the device"""
-    eng = {t: Engine(d) for t, d in DTYPES.items()}
+    eng = {t: capi.Context() for t in TYPES}
     for t, e in eng.items():
-        e.init(m, k, n, A[t], B[t], M)
-        e.run()
-        e.run()
+        e.init_device(A[t], B[t], m, k, n)
+        if M is not None:
+            e.set_mask_device(*M)
+        run(e)
+        run(e)
     rec = {t: [] for t in eng}
     for _ in range(calls):
         for t, e in eng.items():
-            rec[t].append(e.run())
+            rec[t].append(run(e))
     prof = {}
     for t in ("c64", "f64"):
-        eng[t].check(eng[t].lib.bhb200_set_profiling(eng[t].ctx, 1))
-        eng[t].run()
-        prof[t] = bin_times([eng[t].run() for _ in range(calls)])
+        eng[t].set_profiling(True)
+        run(eng[t])
+        prof[t] = bin_times([run(eng[t]) for _ in range(calls)])
     for e in eng.values():
         e.close()
     out = {"workload": name, "m": m, "k": k, "n": n, "calls": calls}
-    out.update({t: summary(v) for t, v in rec.items()})
+    counters = COUNTERS + ("direct_bin_mask", "workspace_bytes")
+    out.update({t: summary(v, STAGES + ("ms_transpose",), counters) for t, v in rec.items()})
     out["bins"] = prof
     for t in ("f64", "f32"):
         out[f"c64_over_{t}"] = out["c64"]["ms_total"] / out[t]["ms_total"] if out[t]["ms_total"] > 0 else None
@@ -123,7 +85,7 @@ def main():
     if not torch.cuda.is_available():
         raise SystemExit("complex_probe: no CUDA device (there is no CPU path)")
     device = torch.cuda.get_device_name(0)
-    plim = power_limit()
+    plim = read_power_limit()
     nx, scale, rect_rows, rect_cols, tscale = (16, 12, 1 << 14, 1 << 12, 12) if args.small else (128, 21, 1 << 22, 1 << 20, 20)
     out = open(args.out, "w") if args.out else None
 

@@ -17,10 +17,8 @@ Workloads:
 from __future__ import annotations
 
 import argparse
-import ctypes
 import json
 import os
-import subprocess
 import sys
 
 import numpy as np
@@ -29,59 +27,16 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 
 from benchmark_spgemm_using_csr_b200 import capi, generators as gen  # noqa: E402
-from benchmark_spgemm_using_csr_b200.dist import _DevicePtr  # noqa: E402
+from probe_util import lower_triangle, read_power_limit, run, summary  # noqa: E402
 
 
-def power_limit():
-    try:
-        r = subprocess.run(["nvidia-smi", "--query-gpu=power.limit", "--format=csv,noheader"], capture_output=True, text=True,
-                           timeout=30)
-        return r.stdout.strip().splitlines()[0]
-    except Exception as e:   # noqa: BLE001
-        return f"unavailable ({e})"
-
-
-class Engine:
-    def __init__(self, torch):
-        self.torch = torch
-        self.lib = capi.load()
-        self.ctx = ctypes.c_void_p()
-        assert self.lib.bhb200_create(ctypes.byref(self.ctx), 0) == capi.SUCCESS
-
-    def check(self, rc):
-        capi.check(self.lib, self.ctx, rc)
-
-    def init(self, m, k, n, A, B, M=None):
-        self._keep = (A, B, M)
-        self.m, self.n = m, n
-        dtype = capi.DTYPE_F64 if A[2].dtype == self.torch.float64 else capi.DTYPE_F32
-        p = lambda t: ctypes.c_void_p(t.data_ptr())
-        self.check(self.lib.bhb200_init_data_device(self.ctx, dtype, m, k, n, int(A[1].numel()), p(A[2]), p(A[0]), p(A[1]),
-                                                    int(B[1].numel()), p(B[2]), p(B[0]), p(B[1])))
-        if M is not None:
-            self.check(self.lib.bhb200_set_mask_device(self.ctx, int(M[1].numel()), p(M[0]), p(M[1])))
-
-    def run(self):
-        self.check(self.lib.bhb200_spgemm(self.ctx))
-        st = capi.Stats()
-        self.check(self.lib.bhb200_get_stats(self.ctx, ctypes.byref(st)))
-        return st
-
-    def C(self):
-        """(rowptr int64, col, val) of the result as torch tensors (copies)."""
-        torch = self.torch
-        ptr = [ctypes.c_void_p() for _ in range(4)]
-        self.check(self.lib.bhb200_get_C_device(self.ctx, *[ctypes.byref(q) for q in ptr]))
-        self.check(self.lib.bhb200_synchronize(self.ctx))
-        nnz = int(self.lib.bhb200_get_nnzC(self.ctx))
-        vt = "<f8" if self._keep[0][2].dtype == torch.float64 else "<f4"
-        view = lambda p, n, ts: torch.as_tensor(_DevicePtr(p.value, n, ts), device="cuda").clone() if n else \
-            torch.zeros(0, device="cuda", dtype=torch.int64 if ts == "<i8" else torch.int32 if ts == "<i4" else
-                        torch.float64 if ts == "<f8" else torch.float32)
-        return view(ptr[1], self.m + 1, "<i8"), view(ptr[2], nnz, "<i4"), view(ptr[3], nnz, vt)
-
-    def close(self):
-        self.lib.bhb200_destroy(self.ctx)
+def context(m, k, n, A, B, M=None):
+    """A capi.Context on borrowed device operands, masked by M = (rowptr, col) unless None."""
+    c = capi.Context()
+    c.init_device(A, B, m, k, n)
+    if M is not None:
+        c.set_mask_device(*M)
+    return c
 
 
 def keys(torch, rowptr, col, n):
@@ -103,48 +58,24 @@ def same_as_filtered(torch, unm, msk, M, n):
     return bool(got_k.numel() == want_k.numel() and torch.equal(got_k, want_k) and torch.equal(msk[2], want_v))
 
 
-def stage(st):
-    return {"ms_total": st.ms_total, "ms_count": st.ms_count, "ms_symbolic": st.ms_symbolic, "ms_scan": st.ms_scan,
-            "ms_numeric": st.ms_numeric}
-
-
 def probe(torch, name, m, k, n, A, B, M, calls):
-    masked, plain = Engine(torch), Engine(torch)
-    masked.init(m, k, n, A, B, M)
-    plain.init(m, k, n, A, B)
+    masked, plain = context(m, k, n, A, B, M), context(m, k, n, A, B)
     for e in (masked, plain):   # warm-up
-        e.run()
-        e.run()
+        run(e)
+        run(e)
     rec_m, rec_u = [], []
     for _ in range(calls):
-        rec_m.append(masked.run())
-        rec_u.append(plain.run())
-
-    def summary(sts):
-        med = {key: float(np.median([stage(s)[key] for s in sts])) for key in stage(sts[0])}
-        s = sts[-1]
-        med.update({"products": int(s.products), "nnzC": int(s.nnzC), "kernel_launches": int(s.kernel_launches),
-                    "pattern_mode": int(s.pattern_mode)})
-        if s.masked:
-            med.update({"nnzM": int(s.nnzM), "mask_bin_rows": dict(zip(capi.MASK_BIN_NAMES, list(s.mask_bin_rows)))})
-        return med
-    cm, cu = masked.C(), plain.C()
+        rec_m.append(run(masked))
+        rec_u.append(run(plain))
+    s = rec_m[-1]
+    sm = dict(summary(rec_m), nnzM=int(s["nnzM"]), mask_bin_rows=dict(zip(capi.MASK_BIN_NAMES, s["mask_bin_rows"])))
+    cm, cu = masked.C_device(), plain.C_device()
     rec = {"workload": name, "m": m, "k": k, "n": n, "dtype": str(A[2].dtype).replace("torch.", ""), "calls": calls,
-           "masked": summary(rec_m), "unmasked": summary(rec_u), "same_as_filtered": same_as_filtered(torch, cu, cm, M, n),
+           "masked": sm, "unmasked": summary(rec_u), "same_as_filtered": same_as_filtered(torch, cu, cm, M, n),
            "masked_sum": float(cm[2].double().sum())}
     masked.close()
     plain.close()
     return rec
-
-
-def lower_triangle(scale):
-    import scipy.sparse as sp
-    R = gen.rmat(scale, 16, values="ones")
-    S = sp.csr_matrix((R.val, R.col, R.rowptr), shape=(R.rows, R.cols))
-    S = ((S + S.T) > 0).astype(np.float64)
-    L = sp.tril(S, k=-1, format="csr")
-    L.sort_indices()
-    return L
 
 
 def main():
@@ -157,7 +88,7 @@ def main():
     if not torch.cuda.is_available():
         raise SystemExit("mask_probe: no CUDA device (there is no CPU path)")
     device = torch.cuda.get_device_name(0)
-    plim = power_limit()
+    plim = read_power_limit()
     dev = lambda *a: tuple(torch.from_numpy(np.ascontiguousarray(x)).cuda() for x in a)
     scale, nx, rect_rows, rect_cols = (12, 16, 1 << 14, 1 << 12) if args.small else (20, 128, 1 << 22, 1 << 20)
     out = open(args.out, "w") if args.out else None
@@ -184,10 +115,9 @@ def main():
     A = gen.uniform_rect(rect_rows, rect_cols, per_row=8, seed=1, dtype=np.float32)
     B = gen.uniform_rect(rect_cols, rect_rows, per_row=8, seed=2, value_seed=3, dtype=np.float32)
     Ad, Bd = dev(A.rowptr, A.col, A.val), dev(B.rowptr, B.col, B.val)
-    e = Engine(torch)
-    e.init(A.rows, A.cols, B.cols, Ad, Bd)
-    e.run()
-    rp, col, _ = e.C()
+    e = context(A.rows, A.cols, B.cols, Ad, Bd)
+    e.spgemm()
+    rp, col, _ = e.C_device()
     e.close()
     g = torch.Generator(device="cuda")
     g.manual_seed(5)

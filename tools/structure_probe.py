@@ -20,10 +20,8 @@ Workloads:
 from __future__ import annotations
 
 import argparse
-import ctypes
 import json
 import os
-import subprocess
 import sys
 
 import numpy as np
@@ -32,91 +30,33 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 
 from benchmark_spgemm_using_csr_b200 import capi, generators as gen  # noqa: E402
-from benchmark_spgemm_using_csr_b200.dist import _DevicePtr  # noqa: E402
+from probe_util import COUNTERS, lower_triangle, read_power_limit, run, summary  # noqa: E402
 
 
-def power_limit():
-    try:
-        r = subprocess.run(["nvidia-smi", "--query-gpu=power.limit", "--format=csv,noheader"], capture_output=True, text=True,
-                           timeout=30)
-        return r.stdout.strip().splitlines()[0]
-    except Exception as e:   # noqa: BLE001
-        return f"unavailable ({e})"
-
-
-class Engine:
-    def __init__(self, torch, structure):
-        self.torch = torch
-        self.structure = structure
-        self.lib = capi.load()
-        self.ctx = ctypes.c_void_p()
-        assert self.lib.bhb200_create(ctypes.byref(self.ctx), 0) == capi.SUCCESS
-
-    def check(self, rc):
-        capi.check(self.lib, self.ctx, rc)
-
-    def init(self, m, k, n, A, B, M=None):
-        self._keep = (A, B, M)
-        self.m = m
-        p = lambda t: ctypes.c_void_p(t.data_ptr())
-        if self.structure:
-            dtype, va, vb = capi.DTYPE_NONE, None, None
-        else:
-            dtype = capi.DTYPE_F64 if A[2].dtype == self.torch.float64 else capi.DTYPE_F32
-            va, vb = p(A[2]), p(B[2])
-        self.check(self.lib.bhb200_init_data_device(self.ctx, dtype, m, k, n, int(A[1].numel()), va, p(A[0]), p(A[1]),
-                                                    int(B[1].numel()), vb, p(B[0]), p(B[1])))
-        if M is not None:
-            self.check(self.lib.bhb200_set_mask_device(self.ctx, int(M[1].numel()), p(M[0]), p(M[1])))
-
-    def run(self):
-        self.check(self.lib.bhb200_spgemm(self.ctx))
-        st = capi.Stats()
-        self.check(self.lib.bhb200_get_stats(self.ctx, ctypes.byref(st)))
-        return st
-
-    def structure_of_C(self):
-        """(rowptr int64, col int32) of the result as torch tensors (copies)."""
-        torch = self.torch
-        ptr = [ctypes.c_void_p() for _ in range(4)]
-        self.check(self.lib.bhb200_get_C_device(self.ctx, *[ctypes.byref(q) for q in ptr]))
-        self.check(self.lib.bhb200_synchronize(self.ctx))
-        nnz = int(self.lib.bhb200_get_nnzC(self.ctx))
-        rp = torch.as_tensor(_DevicePtr(ptr[1].value, self.m + 1, "<i8"), device="cuda").clone()
-        col = torch.as_tensor(_DevicePtr(ptr[2].value, nnz, "<i4"), device="cuda").clone() if nnz else \
-            torch.zeros(0, dtype=torch.int32, device="cuda")
-        return rp, col
-
-    def close(self):
-        self.lib.bhb200_destroy(self.ctx)
-
-
-def stage(st):
-    return {"ms_total": st.ms_total, "ms_count": st.ms_count, "ms_symbolic": st.ms_symbolic, "ms_scan": st.ms_scan,
-            "ms_numeric": st.ms_numeric}
+def context(m, k, n, A, B, M, structure):
+    """A capi.Context on borrowed device operands; structure-only ones get NULL value pointers."""
+    c = capi.Context()
+    if structure:
+        c.init_device((*A[:2], None), (*B[:2], None), m, k, n, dtype=capi.DTYPE_NONE)
+    else:
+        c.init_device(A, B, m, k, n)
+    if M is not None:
+        c.set_mask_device(*M)
+    return c
 
 
 def probe(torch, name, m, k, n, A, B, M, calls):
-    valued, structure = Engine(torch, False), Engine(torch, True)
-    valued.init(m, k, n, A, B, M)
-    structure.init(m, k, n, A, B, M)
+    valued, structure = context(m, k, n, A, B, M, False), context(m, k, n, A, B, M, True)
     for e in (valued, structure):   # warm-up
-        e.run()
-        e.run()
+        run(e)
+        run(e)
     rec_v, rec_s = [], []
     for _ in range(calls):
-        rec_v.append(valued.run())
-        rec_s.append(structure.run())
-
-    def summary(sts):
-        med = {key: float(np.median([stage(s)[key] for s in sts])) for key in stage(sts[0])}
-        s = sts[-1]
-        med.update({"products": int(s.products), "nnzC": int(s.nnzC), "kernel_launches": int(s.kernel_launches),
-                    "pattern_mode": int(s.pattern_mode), "direct_bin_mask": int(s.direct_bin_mask),
-                    "workspace_bytes": int(s.workspace_bytes)})
-        return med
-    cv, cs = valued.structure_of_C(), structure.structure_of_C()
-    sv, ss = summary(rec_v), summary(rec_s)
+        rec_v.append(run(valued))
+        rec_s.append(run(structure))
+    cv, cs = valued.C_device(), structure.C_device()
+    counters = COUNTERS + ("direct_bin_mask", "workspace_bytes")
+    sv, ss = summary(rec_v, counters=counters), summary(rec_s, counters=counters)
     rec = {"workload": name, "m": m, "k": k, "n": n, "dtype": str(A[2].dtype).replace("torch.", ""), "calls": calls,
            "valued": sv, "structure": ss,
            "identical": bool(torch.equal(cv[0], cs[0]) and torch.equal(cv[1], cs[1])),
@@ -124,16 +64,6 @@ def probe(torch, name, m, k, n, A, B, M, calls):
     valued.close()
     structure.close()
     return rec
-
-
-def lower_triangle(scale):
-    import scipy.sparse as sp
-    R = gen.rmat(scale, 16, values="ones")
-    S = sp.csr_matrix((R.val, R.col, R.rowptr), shape=(R.rows, R.cols))
-    S = ((S + S.T) > 0).astype(np.float64)
-    L = sp.tril(S, k=-1, format="csr")
-    L.sort_indices()
-    return L
 
 
 def main():
@@ -146,7 +76,7 @@ def main():
     if not torch.cuda.is_available():
         raise SystemExit("structure_probe: no CUDA device (there is no CPU path)")
     device = torch.cuda.get_device_name(0)
-    plim = power_limit()
+    plim = read_power_limit()
     dev = lambda *a: tuple(torch.from_numpy(np.ascontiguousarray(x)).cuda() for x in a)
     nx, scale, rect_rows, rect_cols, tscale = (16, 12, 1 << 14, 1 << 12, 12) if args.small else (128, 21, 1 << 22, 1 << 20, 20)
     out = open(args.out, "w") if args.out else None

@@ -15,10 +15,8 @@ Workloads: 27-pt 128^3 f64 A*A^T (nonsymmetric values), R-MAT scale 20 A*A^T, un
 from __future__ import annotations
 
 import argparse
-import ctypes
 import json
 import os
-import subprocess
 import sys
 
 import numpy as np
@@ -27,60 +25,7 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 
 from benchmark_spgemm_using_csr_b200 import capi, generators as gen  # noqa: E402
-
-
-def host_transpose(X):
-    rows = np.repeat(np.arange(X.rows, dtype=np.int64), np.diff(X.rowptr.astype(np.int64)))
-    perm = np.argsort(X.col, kind="stable")
-    rowptr = np.zeros(X.cols + 1, dtype=np.int64)
-    np.cumsum(np.bincount(X.col, minlength=X.cols), out=rowptr[1:])
-    return gen.CSR(X.cols, X.rows, rowptr.astype(np.int32), rows[perm].astype(np.int32), X.val[perm])
-
-
-def power_limit():
-    try:
-        r = subprocess.run(["nvidia-smi", "--query-gpu=power.limit", "--format=csv,noheader"], capture_output=True, text=True,
-                           timeout=30)
-        return r.stdout.strip().splitlines()[0]
-    except Exception as e:   # noqa: BLE001
-        return f"unavailable ({e})"
-
-
-class Engine:
-    def __init__(self, torch):
-        self.torch = torch
-        self.lib = capi.load()
-        self.ctx = ctypes.c_void_p()
-        assert self.lib.bhb200_create(ctypes.byref(self.ctx), 0) == capi.SUCCESS
-
-    def check(self, rc):
-        capi.check(self.lib, self.ctx, rc)
-
-    def init(self, opA, opB, m, k, n, A, B):
-        self._keep = (A, B)
-        dtype = capi.DTYPE_F64 if A[2].dtype == self.torch.float64 else capi.DTYPE_F32
-        p = lambda t: ctypes.c_void_p(t.data_ptr())
-        self.check(self.lib.bhb200_init_data_device_op(self.ctx, dtype, opA, opB, m, k, n, int(A[1].numel()), p(A[2]), p(A[0]),
-                                                       p(A[1]), int(B[1].numel()), p(B[2]), p(B[0]), p(B[1])))
-        self.m = m
-
-    def run(self):
-        self.check(self.lib.bhb200_spgemm(self.ctx))
-        st = capi.Stats()
-        self.check(self.lib.bhb200_get_stats(self.ctx, ctypes.byref(st)))
-        return st
-
-    def structure(self):
-        nnz = int(self.lib.bhb200_get_nnzC(self.ctx))
-        rp = np.zeros(self.m + 1, dtype=np.int32)
-        col = np.empty(nnz, dtype=np.int32)
-        dt = self._keep[0][2].dtype
-        fn = self.lib.bhb200_get_C_f64 if dt == self.torch.float64 else self.lib.bhb200_get_C_f32
-        self.check(fn(self.ctx, ctypes.c_void_p(rp.ctypes.data), ctypes.c_void_p(col.ctypes.data), None))
-        return rp, col
-
-    def close(self):
-        self.lib.bhb200_destroy(self.ctx)
+from probe_util import read_power_limit, run  # noqa: E402
 
 
 def copy_ms(torch, X, calls):
@@ -103,32 +48,32 @@ def probe(torch, name, X, mode, calls):
     """mode 'NT': X*X^T, 'TN': X^T*X (X stored)."""
     dev = torch.device("cuda")
     t = lambda C: [torch.from_numpy(np.ascontiguousarray(a)).to(dev) for a in (C.rowptr, C.col, C.val)]
-    XT = host_transpose(X)
+    XT = gen.transpose(X)
     tX, tXT = t(X), t(XT)
     N, T = capi.OP_N, capi.OP_T
     if mode == "NT":
         dims = (X.rows, X.cols, X.rows)
-        op_args = (N, T, *dims, tX, tX)
-        pre_args = (N, N, *dims, tX, tXT)
+        op_args = (tX, tX, *dims, N, T)
+        pre_args = (tX, tXT, *dims, N, N)
     else:
         dims = (X.cols, X.rows, X.cols)
-        op_args = (T, N, *dims, tX, tX)
-        pre_args = (N, N, *dims, tXT, tX)
-    e_op, e_pre = Engine(torch), Engine(torch)
-    e_op.init(*op_args)
-    e_pre.init(*pre_args)
+        op_args = (tX, tX, *dims, T, N)
+        pre_args = (tXT, tX, *dims, N, N)
+    e_op, e_pre = capi.Context(), capi.Context()
+    e_op.init_device(*op_args)
+    e_pre.init_device(*pre_args)
     for e in (e_op, e_pre):   # warm-up
-        e.run()
-        e.run()
+        run(e)
+        run(e)
     ms_t, ms_op, ms_pre, launches = [], [], [], 0
     for _ in range(calls):
-        st = e_op.run()
-        ms_t.append(st.ms_transpose)
-        ms_op.append(st.ms_total)
-        launches = st.kernel_launches
-        st = e_pre.run()
-        ms_pre.append(st.ms_total)
-    a, b = e_op.structure(), e_pre.structure()
+        st = run(e_op)
+        ms_t.append(st["ms_transpose"])
+        ms_op.append(st["ms_total"])
+        launches = st["kernel_launches"]
+        st = run(e_pre)
+        ms_pre.append(st["ms_total"])
+    a, b = e_op.C(), e_pre.C()
     same = bool(np.array_equal(a[0], b[0]) and np.array_equal(a[1], b[1]))
     rec = {
         "workload": name, "product": "A*A^T" if mode == "NT" else "A^T*A", "rows": X.rows, "cols": X.cols, "nnz": X.nnz,
@@ -152,7 +97,7 @@ def main():
     if not torch.cuda.is_available():
         raise SystemExit("transpose_probe: no CUDA device (there is no CPU path)")
     device = torch.cuda.get_device_name(0)
-    plim = power_limit()
+    plim = read_power_limit()
     if args.small:
         work = [("27pt_16^3", gen.poisson27pt(16, 16, 16), "NT"), ("rmat_s12", gen.rmat(12, 16), "NT"),
                 ("uniform_rect_4k_1k", gen.uniform_rect(4096, 1024), "TN")]
