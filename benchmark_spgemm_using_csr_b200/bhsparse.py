@@ -11,9 +11,9 @@ tests read like the reference driver (main.cu:104-135).
     bh.free_mem(); bh.freePlatform()
 
 Host arrays are numpy (or anything exposing a writable buffer of the right
-dtype); the value dtype (float32/float64/complex64) is taken from valA -- the reference
-needs a recompile for that (common.h:31, README.md:84-86).  complex128 is refused
-(ERR_INVALID), never converted.  With valA and valB both
+dtype); the value dtype (float32/float64/complex64/complex128) is taken from valA -- the reference
+needs a recompile for that (common.h:31, README.md:84-86).  A complex valB of another dtype than
+valA, or a complex and a real operand, is refused (ERR_INVALID), never converted.  With valA and valB both
 None the product is structure-only (BHB200_DTYPE_NONE): C has row pointers and
 columns, and get_C takes None for the values.
 """
@@ -43,7 +43,7 @@ def _suffix(dt) -> str | None:
 
 
 def _op(trans) -> int:
-    """transA / transB: False / "N", True / "T", or "C" (conjugate transpose, complex64 only)"""
+    """transA / transB: False / "N", True / "T", or "C" (conjugate transpose, complex values only)"""
     if trans == "C":
         return capi.OP_C
     return capi.OP_T if trans in (True, "T") else capi.OP_N
@@ -86,7 +86,7 @@ class bhsparse:
                  nnzB, csrValB, csrRowPtrB, csrColIndB, csrRowPtrC, transA=False, transB=False) -> int:
         """C = op(A)*op(B): m, k, n are the dimensions of op(A) (m x k) and op(B) (k x n); with
         transA / transB the arrays hold A / B as stored, i.e. k x m / n x k (bhb200_init_data_op_*).
-        transA / transB = "C": conjugate transpose (complex64 values).
+        transA / transB = "C": conjugate transpose (complex64 or complex128 values).
         csrValA and csrValB both None: structure-only product (bhb200_init_data_structure)."""
         if not self._ctx:
             return capi.ERR_INVALID
@@ -98,9 +98,10 @@ class bhsparse:
         else:
             valA = np.ascontiguousarray(csrValA)
             dt = valA.dtype
-            if _suffix(dt) is None:   # (complex128 too: never downcast)
+            if _suffix(dt) is None:
                 return capi.ERR_INVALID
-            if dt == np.complex64 and np.asarray(csrValB).dtype != dt:   # (no mixed real x complex operands)
+            dtB = np.asarray(csrValB).dtype
+            if dtB != dt and (dt.kind == "c" or dtB.kind == "c"):   # (no mixed complex operands: never converted)
                 return capi.ERR_INVALID
             fn = getattr(self._lib, "bhb200_init_data_op_" + _suffix(dt))
             valB = np.ascontiguousarray(csrValB, dtype=dt)
@@ -241,15 +242,18 @@ def spgemm(A, B, device: int = 0, return_stats: bool = False, return_row_product
            transA: bool = False, transB: bool = False, mask=None, structure_only: bool = False):
     """Convenience driver following main.cu:104-135: C = op(A)*op(B) for two
     generators.CSR operands (op = transpose with transA / transB); returns
-    (rowptrC int32, colC int32, valC).  Values float32, float64 or complex64
-    (transA / transB may then be "C", the conjugate transpose).  mask: a generators.CSR or (rowptr, col)
+    (rowptrC int32, colC int32, valC).  Values float32, float64, complex64 or complex128
+    (transA / transB may then be "C", the conjugate transpose); complex operands of two types, or a complex and a
+    real one, are refused.  mask: a generators.CSR or (rowptr, col)
     whose pattern restricts C (masked product, bhb200_set_mask).  structure_only:
     the pattern of C alone, from the operands' patterns (valC is None)."""
     platforms = [False] * NUM_PLATFORMS
     platforms[BHSPARSE_CUDA] = True
     bh = bhsparse(device)
-    if not structure_only and np.asarray(A.val).dtype == np.complex128:
-        raise capi.BhsparseError(capi.ERR_INVALID, "complex128 values are not supported: use complex64")
+    if not structure_only:
+        ta, tb = np.asarray(A.val).dtype, np.asarray(B.val).dtype
+        if ta != tb and (ta.kind == "c" or tb.kind == "c"):
+            raise capi.BhsparseError(capi.ERR_INVALID, f"mixed value types are not supported: {ta} A with {tb} B")
     m, k, n = capi.op_dims(A, B, _op(transA), _op(transB))
     rowptrC = np.zeros(m + 1, dtype=np.int32)
 

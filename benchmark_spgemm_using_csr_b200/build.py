@@ -35,6 +35,7 @@ SOURCES = [
     "stage_numeric_f64.cu",
     "stage_numeric_none.cu",
     "stage_numeric_c64.cu",
+    "stage_numeric_c128.cu",
     "stage_transpose.cu",
     "stage_masked.cu",
 ]

@@ -25,9 +25,10 @@ DTYPE_F32 = 0
 DTYPE_F64 = 1
 DTYPE_NONE = 2   # structure only: row pointers and columns, no values
 DTYPE_C64 = 4    # complex64: two float32 (re, im) per value (3 is not a type)
+DTYPE_C128 = 5   # complex128: two float64 (re, im) per value, 16-byte aligned
 OP_N = 0
 OP_T = 1
-OP_C = 2         # conjugate transpose (complex64 operands only)
+OP_C = 2         # conjugate transpose (complex operands only)
 NUM_BINS = 24
 NUM_MASK_BINS = 9
 MASK_BIN_NAMES = ["none", "esc<=32", "w64", "w256", "w1024", "c1024", "c4096", "c16384", "global"]
@@ -52,6 +53,7 @@ EXPORTED = [
     "bhb200_set_mask", "bhb200_set_mask_device", "bhb200_clear_mask",
     "bhb200_init_data_structure", "bhb200_get_C_structure",
     "bhb200_init_data_op_c64", "bhb200_update_values_c64", "bhb200_get_C_c64",
+    "bhb200_init_data_op_c128", "bhb200_update_values_c128", "bhb200_get_C_c128",
 ]
 DIST_ID_BYTES = 128
 
@@ -126,6 +128,7 @@ def load(build_if_missing: bool = False):
     L.bhb200_init_data_op_f64.argtypes = [ctxp, c_int, c_int] + L.bhb200_init_data_f64.argtypes[1:]
     L.bhb200_init_data_op_f32.argtypes = L.bhb200_init_data_op_f64.argtypes
     L.bhb200_init_data_op_c64.argtypes = L.bhb200_init_data_op_f64.argtypes
+    L.bhb200_init_data_op_c128.argtypes = L.bhb200_init_data_op_f64.argtypes
     L.bhb200_init_data_device_op.argtypes = [ctxp, c_int, c_int, c_int] + L.bhb200_init_data_device.argtypes[2:]
     L.bhb200_init_data_structure.argtypes = [ctxp, c_int, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_int,
                                              c_void_p, c_void_p]
@@ -141,12 +144,14 @@ def load(build_if_missing: bool = False):
     L.bhb200_update_values_f64.argtypes = [ctxp, c_void_p, c_void_p]
     L.bhb200_update_values_f32.argtypes = [ctxp, c_void_p, c_void_p]
     L.bhb200_update_values_c64.argtypes = [ctxp, c_void_p, c_void_p]
+    L.bhb200_update_values_c128.argtypes = [ctxp, c_void_p, c_void_p]
     L.bhb200_spgemm_numeric.argtypes = [ctxp]
     L.bhb200_get_nnzC.argtypes = [ctxp]
     L.bhb200_get_nnzC.restype = c_int64
     L.bhb200_get_C_f64.argtypes = [ctxp, c_void_p, c_void_p, c_void_p]
     L.bhb200_get_C_f32.argtypes = [ctxp, c_void_p, c_void_p, c_void_p]
     L.bhb200_get_C_c64.argtypes = [ctxp, c_void_p, c_void_p, c_void_p]
+    L.bhb200_get_C_c128.argtypes = [ctxp, c_void_p, c_void_p, c_void_p]
     L.bhb200_get_rowptrC_i64.argtypes = [ctxp, c_void_p]
     L.bhb200_get_C_range.argtypes = [ctxp, c_int64, c_int64, c_void_p, c_void_p]
     L.bhb200_get_C_device.argtypes = [ctxp, POINTER(c_void_p), POINTER(c_void_p), POINTER(c_void_p), POINTER(c_void_p)]
@@ -181,17 +186,17 @@ def check(lib, ctx, code: int):
 
 # BHB200_DTYPE_* of a valued product -> (suffix of bhb200_init_data_op_*, bhb200_update_values_* and
 # bhb200_get_C_*; numpy and torch dtype name)
-VALUE_TYPES = {DTYPE_F32: ("f32", "float32"), DTYPE_F64: ("f64", "float64"), DTYPE_C64: ("c64", "complex64")}
+VALUE_TYPES = {DTYPE_F32: ("f32", "float32"), DTYPE_F64: ("f64", "float64"), DTYPE_C64: ("c64", "complex64"),
+               DTYPE_C128: ("c128", "complex128")}
 _DTYPE_OF_NAME = {name: dt for dt, (_, name) in VALUE_TYPES.items()}
 
 
 def dtype_of(x) -> int:
-    """BHB200_DTYPE_* of a numpy or torch value array, dtype or dtype name.  Other value types raise: complex128 is
-    refused, never converted."""
+    """BHB200_DTYPE_* of a numpy or torch value array, dtype or dtype name.  Other value types raise, never
+    converted."""
     name = str(getattr(x, "dtype", x)).removeprefix("torch.")
     if name not in _DTYPE_OF_NAME:
-        hint = ": use complex64" if name == "complex128" else ""
-        raise BhsparseError(ERR_INVALID, f"{name} values are not supported{hint}")
+        raise BhsparseError(ERR_INVALID, f"{name} values are not supported")
     return _DTYPE_OF_NAME[name]
 
 

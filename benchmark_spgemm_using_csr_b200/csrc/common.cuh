@@ -23,7 +23,7 @@ constexpr int SORT_PAD = 0x7fffffff;
 constexpr unsigned FULL = 0xffffffffu;
 
 // ---- value types -------------------------------------------------------------
-// The numeric kernels are templates on the value type VT (float, double, c64 below).  Structure-only
+// The numeric kernels are templates on the value type VT (float, double, c64 and c128 below).  Structure-only
 // products (BHB200_DTYPE_NONE) instantiate them with NoVal: an empty type whose arithmetic,
 // shuffles, loads and atomics do nothing, so every value load, store and shared-memory access
 // compiles away and only the column work is left.  Shared-memory layouts are sized with
@@ -113,9 +113,59 @@ __device__ __forceinline__ cdbl atomicAdd(cdbl *p, const cdbl v)
     const double r = ::atomicAdd(&p->re, v.re);
     return cdbl(r, ::atomicAdd(&p->im, v.im));
 }
+
+// Complex products in double (BHB200_DTYPE_C128) instantiate them with c128: two doubles (re, im), 16 bytes and
+// 16-byte aligned like double _Complex / std::complex<double> / cuDoubleComplex / torch.complex128.  The product is
+// the naive formula, as for c64.  Constructible from a double (a real zero or a real sum), so it is also the type
+// k_num_bucket_heavy reduces a column in (WideSum below): its components are double already.  The on-chip layouts
+// sized for 8-byte values do not all hold it: see the routing next to the bin enums.
+struct __align__(16) c128 {
+    double re, im;
+    c128() = default;   // (trivial, as c64)
+    __host__ __device__ constexpr c128(double r) : re(r), im(0.0) {}
+    __host__ __device__ constexpr c128(double r, double i) : re(r), im(i) {}
+    __host__ __device__ c128 operator*(const c128 b) const { return c128(re * b.re - im * b.im, re * b.im + im * b.re); }
+    __host__ __device__ c128 operator+(const c128 b) const { return c128(re + b.re, im + b.im); }
+    __host__ __device__ c128 &operator+=(const c128 b)
+    {
+        re += b.re;
+        im += b.im;
+        return *this;
+    }
+    __host__ __device__ bool operator!=(const double b) const { return re != b || im != 0.0; }
+};
+__device__ __forceinline__ c128 fma(const c128 a, const c128 b, const c128 c)
+{
+    return c128(::fma(a.re, b.re, ::fma(-a.im, b.im, c.re)), ::fma(a.re, b.im, ::fma(a.im, b.re, c.im)));
+}
+__device__ __forceinline__ c128 __shfl_sync(unsigned mask, const c128 v, int src, int width = 32)
+{
+    return c128(::__shfl_sync(mask, v.re, src, width), ::__shfl_sync(mask, v.im, src, width));
+}
+__device__ __forceinline__ c128 __shfl_down_sync(unsigned mask, const c128 v, unsigned d, int width = 32)
+{
+    return c128(::__shfl_down_sync(mask, v.re, d, width), ::__shfl_down_sync(mask, v.im, d, width));
+}
+__device__ __forceinline__ c128 __shfl_xor_sync(unsigned mask, const c128 v, int d, int width = 32)
+{
+    return c128(::__shfl_xor_sync(mask, v.re, d, width), ::__shfl_xor_sync(mask, v.im, d, width));
+}
+__device__ __forceinline__ c128 __ldg(const c128 *p)   // one 128-bit read-only load
+{
+    const double2 t = ::__ldg(reinterpret_cast<const double2 *>(p));
+    return c128(t.x, t.y);
+}
+// per component: two double atomics (shared or global memory); returns the old value
+__device__ __forceinline__ c128 atomicAdd(c128 *p, const c128 v)
+{
+    const double r = ::atomicAdd(&p->re, v.re);
+    return c128(r, ::atomicAdd(&p->im, v.im));
+}
 }  // namespace cplx
 using cplx::c64;
+using cplx::c128;
 static_assert(sizeof(c64) == 8 && alignof(c64) == 8, "complex64 is two floats, 8-byte aligned");
+static_assert(sizeof(c128) == 16 && alignof(c128) == 16, "complex128 is two doubles, 16-byte aligned");
 
 // the type k_num_bucket_heavy sums one column's products in: double for the real types, cdbl for c64
 template <typename VT>
@@ -125,6 +175,10 @@ struct WideSum {
 template <>
 struct WideSum<c64> {
     using type = cplx::cdbl;
+};
+template <>
+struct WideSum<c128> {
+    using type = c128;
 };
 
 template <typename VT>
@@ -194,6 +248,17 @@ enum NumBin {
 };
 constexpr int MAX_BINS = 24;
 
+// Values of more than 8 bytes (complex128).  The bins above are the rows' shape, computed on the device by kernels
+// that do not know the value type; the largest shared-memory tables are sized for 8-byte values and do not hold
+// 16-byte ones (k_num_block with T = 16384: 352 KB).  So the host runs the rows of every numeric bin after
+// num_hash_last() in the global-bitmap kernel of NB_LARGE: the bins NB_B16384 and NB_LARGE are neighbours in the
+// queue, one launch takes both.  bhb200_stats.num_bin_rows counts those rows under NB_LARGE, where they ran.
+constexpr size_t SMEM_BLOCK_MAX = 227 * 1024;   // dynamic shared memory of one CTA on sm_100a
+inline int num_hash_last(size_t value_size)
+{
+    return value_size > 8 ? NB_B8192 : NB_B16384;
+}
+
 // Masked products (stage_masked.cu): the table size follows m = nnz(M_i), the parallelism p = products
 enum MaskBin {
     MB_ZERO = 0,     // p == 0 or m == 0    -> nnz(C_i) = 0, no kernel
@@ -207,6 +272,12 @@ enum MaskBin {
     MB_GLOBAL = 8,   // beyond the shared-memory tables: binary search in M_i, values in global scratch
     MB_COUNT = 9
 };
+// Values of more than 8 bytes: the table of MB_C16384 (264 KB for 16-byte values) does not fit, its rows run in the
+// kernel of MB_GLOBAL (its neighbour in the queue: one launch); bhb200_stats.mask_bin_rows counts them there.
+inline int mask_table_last(size_t value_size)
+{
+    return value_size > 8 ? MB_C4096 : MB_C16384;
+}
 constexpr int MASK_WARP_MAX_P = 2048;
 constexpr int MASK_TABLE_MAX = 8192;
 __host__ __device__ __forceinline__ int mask_bin_of(int p, int m)
@@ -718,7 +789,7 @@ struct TransposeOut {
 };
 size_t transpose_scratch_bytes(int nnz, int cols);
 int transpose_passes(int cols);
-// conj: complex64 values are conjugated as they move (BHB200_OP_C)
+// conj: complex values are conjugated as they move (BHB200_OP_C)
 cudaError_t launch_transpose(const LaunchCtx &lc, int dtype, bool conj, int rows, int cols, int nnz, Csr X, TransposeOut out,
                              void *scratch, int *bad, int bad_bit);
 // values again through the permutation of the last transposition: valT[p] = val[perm[p]] (conjugated with conj)
@@ -766,9 +837,9 @@ int large_scratch_blocks(int sm_count, int n);
 cudaError_t launch_sym_range(const LaunchCtx &lc, int nsum, const int *queue, int count, Csr A, Csr B, const int *rlo,
                              int *rc, Counters *ctr, WordLists wl);
 
-// The numeric kernels of one value type (stage_numeric_f32.cu / _f64.cu / _none.cu / _c64.cu); values are float,
-// double or complex64 as the operands are, or none (NoVal: columns only, value pointers never read).  The four types
-// compile in four translation units, in parallel.
+// The numeric kernels of one value type (stage_numeric_f32.cu / _f64.cu / _none.cu / _c64.cu / _c128.cu); values
+// are float, double, complex64 or complex128 as the operands are, or none (NoVal: columns only, value pointers never
+// read).  The five types compile in five translation units, in parallel.
 struct ColumnCdf {
     const unsigned *cdf;   // [CDF_KNOTS + 1], non-decreasing, cdf[0] = 0
     int shift;             // column >> shift < CDF_KNOTS
@@ -801,9 +872,9 @@ struct NumericKernels {
     cudaError_t (*copy_ct)(const LaunchCtx &lc, const int *queue, int count, const int64_t *rowoff, const long long *ct_off,
                            const int *ctcol, const void *ctval, int *colC, void *valC, double avg_row);
 };
-extern const NumericKernels NUMERIC_F32, NUMERIC_F64, NUMERIC_NONE, NUMERIC_C64;
+extern const NumericKernels NUMERIC_F32, NUMERIC_F64, NUMERIC_NONE, NUMERIC_C64, NUMERIC_C128;
 
-// The one place a BHB200_DTYPE_* becomes a value type: f(VT()) with VT = float, double, NoVal or c64 (host code;
+// The one place a BHB200_DTYPE_* becomes a value type: f(VT()) with VT = float, double, NoVal, c64 or c128 (host code;
 // the launchers call it with a generic lambda and take the type as decltype of its argument).
 template <typename F>
 inline decltype(auto) dispatch_value_type(int dtype, F &&f)
@@ -812,6 +883,7 @@ inline decltype(auto) dispatch_value_type(int dtype, F &&f)
     case BHB200_DTYPE_F64: return f(double());
     case BHB200_DTYPE_NONE: return f(NoVal());
     case BHB200_DTYPE_C64: return f(c64());
+    case BHB200_DTYPE_C128: return f(c128());
     default: return f(float());
     }
 }
@@ -823,6 +895,7 @@ inline const NumericKernels &numeric_kernels(int dtype)
         if constexpr (std::is_same_v<VT, double>) return NUMERIC_F64;
         else if constexpr (std::is_same_v<VT, NoVal>) return NUMERIC_NONE;
         else if constexpr (std::is_same_v<VT, c64>) return NUMERIC_C64;
+        else if constexpr (std::is_same_v<VT, c128>) return NUMERIC_C128;
         else return NUMERIC_F32;
     });
 }

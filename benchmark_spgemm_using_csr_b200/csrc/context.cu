@@ -49,7 +49,7 @@ size_t vsize(int dtype)
 
 const char *dtype_name(int dtype)
 {
-    return dtype == BHB200_DTYPE_F64 ? "f64" : dtype == BHB200_DTYPE_C64 ? "c64" : "f32";
+    return dtype == BHB200_DTYPE_F64 ? "f64" : dtype == BHB200_DTYPE_C64 ? "c64" : dtype == BHB200_DTYPE_C128 ? "c128" : "f32";
 }
 
 int refuse_structure(bhb200_ctx *ctx, const char *what)
@@ -109,11 +109,12 @@ int check_dims(bhb200_ctx *ctx, int dtype, int m, int k, int n, int nnzA, int nn
 
 int check_ops(bhb200_ctx *ctx, int dtype, int opA, int opB)
 {
-    const int last = dtype == BHB200_DTYPE_C64 ? BHB200_OP_C : BHB200_OP_T;
+    const bool complex = dtype == BHB200_DTYPE_C64 || dtype == BHB200_DTYPE_C128;
+    const int last = complex ? BHB200_OP_C : BHB200_OP_T;
     if (opA < BHB200_OP_N || opA > last || opB < BHB200_OP_N || opB > last)
         return fail(ctx, BHB200_ERR_INVALID,
-                    dtype == BHB200_DTYPE_C64 ? "op must be BHB200_OP_N, BHB200_OP_T or BHB200_OP_C"
-                                              : "op must be BHB200_OP_N or BHB200_OP_T (BHB200_OP_C needs complex64 operands)");
+                    complex ? "op must be BHB200_OP_N, BHB200_OP_T or BHB200_OP_C"
+                            : "op must be BHB200_OP_N or BHB200_OP_T (BHB200_OP_C needs complex operands)");
     return BHB200_SUCCESS;
 }
 
@@ -362,17 +363,21 @@ int run_numeric_bins(bhb200_ctx *ctx, const LaunchCtx &lc, const int *num_bin, c
     if (num_bin[NB_ESC] > 0) CU(stamp(ctx, 1, NB_ESC), "event");
     CU(launch_num_esc(lc, ctx->dtype, queue + no.off[NB_ESC], num_bin[NB_ESC], ctx->n, ctx->A, ctx->B, rowoff, colC, valC),
        "numeric ESC");
-    for (int b = NB_G64; b <= NB_B16384; ++b) {
+    const int last_hash = num_hash_last(vsize(ctx->dtype));
+    for (int b = NB_G64; b <= last_hash; ++b) {
         if (num_bin[b] > 0) CU(stamp(ctx, 1, b), "event");
         CU(nk.hash(lc, b, G, queue + no.off[b], num_bin[b], ctx->A, ctx->B, rowoff, colC, valC),
            (std::string("numeric hash ") + dtype_name(ctx->dtype)).c_str());
     }
-    if (num_bin[NB_LARGE] > 0) {
+    // the bins after last_hash and NB_LARGE are consecutive in the queue: one launch of the global-bitmap kernel
+    int large_rows = 0;
+    for (int b = last_hash + 1; b <= NB_LARGE; ++b) large_rows += num_bin[b];
+    if (large_rows > 0) {
         rc = reserve_large_scratch(ctx, true);
         if (rc) return rc;
         const int sb = large_scratch_blocks(ctx->sm_count, ctx->n);
         CU(stamp(ctx, 1, NB_LARGE), "event");
-        CU(nk.large(lc, queue + no.off[NB_LARGE], num_bin[NB_LARGE], ctx->n, ctx->A, ctx->B, rowoff, colC, valC,
+        CU(nk.large(lc, queue + no.off[last_hash + 1], large_rows, ctx->n, ctx->A, ctx->B, rowoff, colC, valC,
                     ctx->bitmap.as<unsigned>(), ctx->prefix.as<int>(), sb),
            (std::string("numeric large ") + dtype_name(ctx->dtype)).c_str());
     }
@@ -391,6 +396,17 @@ int run_numeric_bins(bhb200_ctx *ctx, const LaunchCtx &lc, const int *num_bin, c
     return BHB200_SUCCESS;
 }
 
+// bhb200_stats of the numeric bins as they ran: the rows num_hash_last sends to NB_LARGE are counted there
+void report_routed_num_bins(bhb200_stats &st, size_t value_size)
+{
+    for (int b = num_hash_last(value_size) + 1; b < NB_LARGE; ++b) {
+        st.num_bin_rows[NB_LARGE] += st.num_bin_rows[b];
+        st.num_bin_products[NB_LARGE] += st.num_bin_products[b];
+        st.num_bin_nnzC[NB_LARGE] += st.num_bin_nnzC[b];
+        st.num_bin_nnzA[NB_LARGE] += st.num_bin_nnzA[b];
+        st.num_bin_rows[b] = st.num_bin_products[b] = st.num_bin_nnzC[b] = st.num_bin_nnzA[b] = 0;
+    }
+}
 
 void finish_stats(bhb200_ctx *ctx)
 {
@@ -846,6 +862,7 @@ int scan_and_bin(bhb200_ctx *ctx, Product &p, unsigned spec_mask, const char *wh
         st.num_bin_nnzC[b] = (int64_t)hc.num_bin_nnzc[b];
         st.num_bin_nnzA[b] = (int64_t)hc.num_bin_nnza[b];
     }
+    report_routed_num_bins(st, vsize(ctx->dtype));
     if ((rc = reserve_C(ctx))) return rc;
     offsets_from_counts(hc.num_bin, p.no);
     CU(launch_bin_scatter(p.lc, true, ctx->m, ctx->prod.as<int>(), ctx->rc.as<int>(), ctx->rspan.as<int>(), spec_mask,
@@ -891,16 +908,31 @@ int stage4_numeric(bhb200_ctx *ctx, const Product &p)
 }
 
 // ---- masked product (stage_masked.cu): the masked kernels of every bin, rows staged at their mask offsets ----
+// rows per masked kernel: the bins after mask_table_last run in MB_GLOBAL's kernel and are counted there
+void routed_mask_bins(const int *bins, size_t value_size, int *rows)
+{
+    for (int b = 0; b < MB_COUNT; ++b) rows[b] = bins[b];
+    for (int b = mask_table_last(value_size) + 1; b < MB_GLOBAL; ++b) {
+        rows[MB_GLOBAL] += rows[b];
+        rows[b] = 0;
+    }
+}
+
 int run_mask_bins(bhb200_ctx *ctx, const LaunchCtx &lc)
 {
     const MaskOut o{ctx->rc.as<int>(), ctx->ct_off.as<long long>(), ctx->ct_col.as<int>(), ctx->ct_val.p, ctx->mask_acc.p,
                     ctx->mask_hit.as<unsigned char>()};
     memset(ctx->ev_bin_used, 0, sizeof(ctx->ev_bin_used));
+    int rows[MB_COUNT];
+    routed_mask_bins(ctx->last_mask_bin, vsize(ctx->dtype), rows);
+    const int last_table = mask_table_last(vsize(ctx->dtype));
     for (int b = MB_ZERO + 1; b < MB_COUNT; ++b) {
-        if (ctx->last_mask_bin[b] <= 0) continue;
+        if (rows[b] <= 0) continue;
+        // (MB_GLOBAL starts at the first bin after last_table: the routed bins are its neighbours in the queue)
+        const int first = b == MB_GLOBAL ? last_table + 1 : b;
         CU(stamp(ctx, 0, b), "event");
-        CU(launch_mask_bin(lc, ctx->dtype, b, ctx->mask_q.as<int>() + ctx->last_mask_off.off[b], ctx->last_mask_bin[b], ctx->A,
-                           ctx->B, ctx->brange.as<int4>(), ctx->M, o),
+        CU(launch_mask_bin(lc, ctx->dtype, b, ctx->mask_q.as<int>() + ctx->last_mask_off.off[first], rows[b], ctx->A, ctx->B,
+                           ctx->brange.as<int4>(), ctx->M, o),
            "masked kernel");
     }
     CU(stamp(ctx, 0, MAX_BINS), "event");
@@ -919,14 +951,16 @@ int stage_masked(bhb200_ctx *ctx, Product &p)
     const int *prod = ctx->prod.as<int>();
     st.masked = 1;
     st.nnzM = (int64_t)nM;
-    for (int b = 0; b < BHB200_NUM_MASK_BINS && b < MB_COUNT; ++b) st.mask_bin_rows[b] = p.hc.mask_bin[b];
+    int rows[MB_COUNT];
+    routed_mask_bins(p.hc.mask_bin, vs, rows);
+    for (int b = 0; b < BHB200_NUM_MASK_BINS && b < MB_COUNT; ++b) st.mask_bin_rows[b] = rows[b];
     // staging: exactly nnzM entries, row i at rowptrM[i]; it may spill to host memory like C
     CU(ctx->ct_off.reserve(m1 * 8, &ctx->dev_bytes), "alloc staging offsets");
     CU(ctx->mask_q.reserve(m1 * 4, &ctx->dev_bytes), "alloc masked bin queue");
     CU(ctx->ct_col.reserve_spillable(nM * 4 + 16, &ctx->dev_bytes, ctx->device_cap, nullptr), "alloc staging columns");
     if (vs) CU(ctx->ct_val.reserve_spillable(nM * vs + 16, &ctx->dev_bytes, ctx->device_cap, nullptr), "alloc staging values");
     st.spill_bytes += spilled_bytes(ctx->ct_col) + (vs ? spilled_bytes(ctx->ct_val) : 0);
-    if (p.hc.mask_bin[MB_GLOBAL] > 0) {   // (structure only: hit flags, no accumulator)
+    if (rows[MB_GLOBAL] > 0) {   // (structure only: hit flags, no accumulator)
         if (vs) CU(ctx->mask_acc.reserve(nM * vs + 16, &ctx->dev_bytes), "alloc masked accumulator");
         CU(ctx->mask_hit.reserve(nM + 16, &ctx->dev_bytes), "alloc masked hit flags");
     }
@@ -1124,6 +1158,13 @@ int bhb200_init_data_op_c64(bhb200_ctx *ctx, int opA, int opB, int m, int k, int
     return init_host(ctx, BHB200_DTYPE_C64, opA, opB, m, k, n, nnzA, valA, rowptrA, colA, nnzB, valB, rowptrB, colB);
 }
 
+int bhb200_init_data_op_c128(bhb200_ctx *ctx, int opA, int opB, int m, int k, int n, int nnzA, const double *valA,
+                             const int32_t *rowptrA, const int32_t *colA, int nnzB, const double *valB,
+                             const int32_t *rowptrB, const int32_t *colB)
+{
+    return init_host(ctx, BHB200_DTYPE_C128, opA, opB, m, k, n, nnzA, valA, rowptrA, colA, nnzB, valB, rowptrB, colB);
+}
+
 int bhb200_init_data_structure(bhb200_ctx *ctx, int opA, int opB, int m, int k, int n, int nnzA, const int32_t *rowptrA,
                                const int32_t *colA, int nnzB, const int32_t *rowptrB, const int32_t *colB)
 {
@@ -1143,7 +1184,8 @@ int bhb200_init_data_device_op(bhb200_ctx *ctx, int dtype, int opA, int opB, int
                                const int32_t *rowptrB, const int32_t *colB)
 {
     if (!ctx) return BHB200_ERR_INVALID;
-    if (dtype != BHB200_DTYPE_F32 && dtype != BHB200_DTYPE_F64 && dtype != BHB200_DTYPE_NONE && dtype != BHB200_DTYPE_C64)
+    if (dtype != BHB200_DTYPE_F32 && dtype != BHB200_DTYPE_F64 && dtype != BHB200_DTYPE_NONE && dtype != BHB200_DTYPE_C64 &&
+        dtype != BHB200_DTYPE_C128)
         return fail(ctx, BHB200_ERR_INVALID, "bad dtype");
     int rc = check_ops(ctx, dtype, opA, opB);
     if (rc) return rc;
@@ -1152,6 +1194,9 @@ int bhb200_init_data_device_op(bhb200_ctx *ctx, int dtype, int opA, int opB, int
     // (checked here, before any kernel reads them: the kernels load complex64 values as 8-byte words)
     if (dtype == BHB200_DTYPE_C64 && (((uintptr_t)valA | (uintptr_t)valB) & 7u))
         return fail(ctx, BHB200_ERR_INVALID, "complex64 value arrays must be 8-byte aligned");
+    // (complex128: 128-bit loads)
+    if (dtype == BHB200_DTYPE_C128 && (((uintptr_t)valA | (uintptr_t)valB) & 15u))
+        return fail(ctx, BHB200_ERR_INVALID, "complex128 value arrays must be 16-byte aligned");
     CU(cudaSetDevice(ctx->device), "cudaSetDevice");
     release_operands(ctx);
     const bool values = dtype != BHB200_DTYPE_NONE;   // (structure only: the caller's value pointers are never read)
@@ -1355,6 +1400,7 @@ int bhb200_spgemm_numeric(bhb200_ctx *ctx)
     CU(stamp(ctx, 1, MAX_BINS), "event");
     CU(cudaEventRecord(ctx->ev[4], s), "event");
     for (int b = 0; b < BHB200_NUM_NUM_BINS && b < MAX_BINS; ++b) st.num_bin_rows[b] = ctx->reuse_num_bin[b];
+    report_routed_num_bins(st, vsize(ctx->dtype));
     st.kernel_launches = ctx->launches;
     st.direct_rows = 0;
     st.direct_retry_rows = 0;
@@ -1432,6 +1478,11 @@ int bhb200_update_values_c64(bhb200_ctx *ctx, const float *valA, const float *va
     return update_values_any(ctx, BHB200_DTYPE_C64, valA, valB);
 }
 
+int bhb200_update_values_c128(bhb200_ctx *ctx, const double *valA, const double *valB)
+{
+    return update_values_any(ctx, BHB200_DTYPE_C128, valA, valB);
+}
+
 int bhb200_set_profiling(bhb200_ctx *ctx, int enabled)
 {
     if (!ctx) return BHB200_ERR_INVALID;
@@ -1472,13 +1523,13 @@ int bhb200_pattern_plan_probe(const int32_t *offsA, int nA, const int32_t *offsB
                               uint8_t *position, int32_t *offsC)
 {
     // host-only: the plan the diagonal-pattern mode would build for these offset sets (tests, tools)
-    if (!offsA || !offsB || !info || (value_size != 4 && value_size != 8)) return BHB200_ERR_INVALID;
+    if (!offsA || !offsB || !info || (value_size != 4 && value_size != 8 && value_size != 16)) return BHB200_ERR_INVALID;
     PatternPlan plan;
     if (!build_pattern_plan(offsA, nA, offsB, nB, value_size, plan)) {
         info[0] = 0;
         return BHB200_SUCCESS;
     }
-    const int nb = value_size == 8 ? 16 : 32;
+    const int nb = pattern_lane_group(value_size);
     const unsigned char *mphys = plan.blob.data() + plan.off_mphys;
     int cost = 0, groups = 0;
     for (int ja = 0; ja < nA; ++ja)
@@ -1539,6 +1590,11 @@ int bhb200_get_C_f32(bhb200_ctx *ctx, int32_t *rowptrC, int32_t *colC, float *va
 int bhb200_get_C_c64(bhb200_ctx *ctx, int32_t *rowptrC, int32_t *colC, float *valC)
 {
     return get_C_any(ctx, BHB200_DTYPE_C64, rowptrC, colC, valC);
+}
+
+int bhb200_get_C_c128(bhb200_ctx *ctx, int32_t *rowptrC, int32_t *colC, double *valC)
+{
+    return get_C_any(ctx, BHB200_DTYPE_C128, rowptrC, colC, valC);
 }
 
 int bhb200_get_C_structure(bhb200_ctx *ctx, int32_t *rowptrC, int32_t *colC)

@@ -40,12 +40,17 @@ DirectPlan plan_direct(const Counters &hc, const DirectSwitches &sw, size_t valu
     if (!sw.direct_mode) return p;
     const bool force = sw.force_cap >= 0;
     bool wide_above = false;
+    bool heavy8192 = false;   // SB_B8192 follows a wide neighbour but its capacity does not fit on chip: HEAVY below
     for (int b = SB_G128; b <= SB_B8192; ++b) {
         DirectBin &d = p.bin[b];
         if (d.rows <= 0) continue;   // (an empty bin leaves wide_above as it is)
         if (b == SB_B8192) {
             // not sampled (the group kernels stop at 4096 slots): follows its neighbour
             if (!wide_above) continue;
+            if (8192 > direct_cap_max(value_size)) {
+                heavy8192 = true;
+                continue;
+            }
             d.mode = DirectMode::WIDE;
             d.cap = 8192;
         } else {
@@ -75,7 +80,7 @@ DirectPlan plan_direct(const Counters &hc, const DirectSwitches &sw, size_t valu
     // rows with more products than the on-chip tables hold follow the largest sampled bin: if that one
     // does not compress they run once through the sliced bucket sort, staged at their product count
     // (BHB200_DEBUG_FORCE_HEAVY: tests send them there whatever the sample says)
-    bool top_wide = sw.force_heavy;
+    bool top_wide = sw.force_heavy || heavy8192;
     for (int b = SB_B8192; b >= SB_G128 && !top_wide; --b)
         if (p.bin[b].rows > 0) {
             top_wide = p.bin[b].mode == DirectMode::WIDE;
@@ -85,7 +90,7 @@ DirectPlan plan_direct(const Counters &hc, const DirectSwitches &sw, size_t valu
     // two-pass tables + global column bitmap, whose cost also grows with n -- profiles/r02_notes.md section 5)
     if (top_wide && sw.direct_wide) {
         p.heavy_base = p.ct_entries;
-        for (int b = SB_B16384; b <= SB_LARGE; ++b) {
+        for (int b = heavy8192 ? SB_B8192 : SB_B16384; b <= SB_LARGE; ++b) {
             if (p.bin[b].rows <= 0) continue;
             p.bin[b].mode = DirectMode::HEAVY;
             p.bin[b].base = p.heavy_base;
@@ -143,10 +148,14 @@ DirectLaunches DirectPlan::launches(int b, int G) const
         ls.at[ls.n++] = DirectLaunch{k, cap, sg, p_lo, p_hi, stride};
     };
     if (d.mode == DirectMode::HEAVY) {
-        // rows of at most 8192 products by k_num_bucket3 itself (SB_B16384: 6144 < products <= 12288), the rest by
-        // k_num_bucket_heavy2, partitioned by slice through the row's own staging area
-        if (b == SB_B16384) add(DirectKernel::BUCKET, 8192, 0, 0, 8192, 0);
-        add(DirectKernel::HEAVY, 0, 0, b == SB_B16384 ? 8192 : 0, DIRECT_P_MAX, 0);
+        // rows of at most cap products by k_num_bucket3 itself when the bin has such rows (8-byte values: SB_B16384,
+        // 6144 < products <= 12288, cap 8192; 16-byte values: SB_B8192, 3072 < products <= 6144, cap 4096), the rest
+        // by k_num_bucket_heavy2, partitioned by slice through the row's own staging area
+        const int cap = direct_cap_max(value_size);
+        const int p_floor = 96 << (b - SB_G256);   // the bin's rows have more products than this (sym_bin_of)
+        const int p_bucket = p_floor < cap ? cap : 0;
+        if (p_bucket) add(DirectKernel::BUCKET, cap, 0, 0, cap, 0);
+        add(DirectKernel::HEAVY, 0, 0, p_bucket, DIRECT_P_MAX, 0);
     } else if (d.warp && bucket_ok) {
         add(DirectKernel::BUCKET3W, b == SB_G128 ? 128 : 256, G, 0, DIRECT_P_MAX, d.cap);
     } else if (d.mode == DirectMode::TIGHT) {

@@ -39,6 +39,15 @@ enum class DirectKernel {
 
 constexpr int DIRECT_P_MAX = 0x7fffffff;
 
+// The largest staging capacity of one row on chip (k_num_block, k_num_bucket3).  At 8192 entries their tables hold
+// 8-byte values (224 / 221 KB) but not 16-byte ones (352 / 289 KB of the 227 KB a CTA may have): with complex128
+// values SB_B8192 rows that would be WIDE at 8192 run as HEAVY, and HEAVY bins hand k_num_bucket3 the rows of at
+// most 4096 products instead of 8192.
+inline int direct_cap_max(size_t value_size)
+{
+    return value_size > 8 ? 4096 : 8192;
+}
+
 struct DirectLaunch {
     DirectKernel kernel;
     int cap;          // table capacity (BUCKET3W: capw); 0 for HEAVY

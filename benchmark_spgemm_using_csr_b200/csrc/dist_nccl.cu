@@ -284,14 +284,15 @@ int bhb200_dist_setup_square(bhb200_ctx *ctx, int root, int dtype, int n, int64_
     if (!ctx || !ctx->dist) return dfail(ctx, BHB200_ERR_INVALID, "bhb200_dist_init first");
     DistState *d = ctx->dist;
     if (root < 0 || root >= d->nranks || n < 0 || nnz < 0 || nnz > 0x7fffffffLL) return dfail(ctx, BHB200_ERR_INVALID, "bad argument");
-    if (dtype != BHB200_DTYPE_F32 && dtype != BHB200_DTYPE_F64 && dtype != BHB200_DTYPE_C64)
+    if (dtype != BHB200_DTYPE_F32 && dtype != BHB200_DTYPE_F64 && dtype != BHB200_DTYPE_C64 && dtype != BHB200_DTYPE_C128)
         return dfail(ctx, BHB200_ERR_INVALID, "bad dtype");
     const bool is_root = d->rank == root;
     if (is_root && (!rowptr || (nnz > 0 && (!col || !val)))) return dfail(ctx, BHB200_ERR_INVALID, "null B on the root");
     DCU(cudaSetDevice(ctx->device), "cudaSetDevice");
     cudaStream_t s = ctx->stream;
-    const size_t vs = dtype == BHB200_DTYPE_F32 ? 4 : 8;
+    const size_t vs = dispatch_value_type(dtype, [](auto v) { return value_bytes<decltype(v)>; });
     if (is_root && vs == 8 && ((uintptr_t)val & 7u)) return dfail(ctx, BHB200_ERR_INVALID, "valB is not 8-byte aligned");
+    if (is_root && vs == 16 && ((uintptr_t)val & 15u)) return dfail(ctx, BHB200_ERR_INVALID, "valB is not 16-byte aligned");
     // forget the previous operands (library-owned buffers are reused by reserve())
     ctx->have_data = false;
     ctx->have_C = false;
@@ -370,9 +371,9 @@ int bhb200_dist_setup_square(bhb200_ctx *ctx, int root, int dtype, int n, int64_
     DCU(cudaEventRecord(d->ev_ready, s), "event");
     DCU(cudaStreamWaitEvent(d->val_stream, d->ev_ready, 0), "wait");
     if (nnz > 0)
-        // (values only move: complex64 as 8-byte words)
-        DNC(nccl().Broadcast(b_val, b_val, (size_t)nnz, vs == 8 ? ncclFloat64 : ncclFloat32, root, d->comm,
-                             d->val_stream),
+        // (values only move: complex64 as one 8-byte word, complex128 as two)
+        DNC(nccl().Broadcast(b_val, b_val, (size_t)nnz * (vs == 16 ? 2 : 1), vs == 4 ? ncclFloat32 : ncclFloat64, root,
+                             d->comm, d->val_stream),
             "ncclBroadcast(valB)");
     DCU(cudaEventRecord(d->ev_val, d->val_stream), "event");
     DCU(cudaStreamSynchronize(s), "partition record");

@@ -8,9 +8,9 @@
 namespace bhb {
 
 // Accumulator layout.  The products of one B row (A offset ja fixed, jb = 0, 1, ...) are issued by
-// consecutive lanes; a shared-memory wavefront serves 32 lanes x 4 bytes or 16 lanes x 8 bytes, so
+// consecutive lanes; a shared-memory wavefront serves 32 lanes x 4 bytes, 16 x 8 or 8 x 16, so
 // the outputs M[ja][jb] of each such lane group should sit in distinct banks.  Greedy colouring of
-// the outputs with `nb` residues (nb = 32 for 4-byte, 16 for 8-byte values) against those groups,
+// the outputs with `nb` residues (pattern_lane_group: 32, 16 or 8) against those groups,
 // then position = residue + nb * (index inside the residue class).  Conflicts that remain only
 // cost replays; correctness does not depend on the layout.
 static void choose_layout(int nDA, int nDB, int nD, const std::vector<unsigned char> &mlog, int nb, const long long *offs,
@@ -188,7 +188,7 @@ bool build_pattern_plan(const int *offsA, int nA, const int *offsB, int nB, int 
             pfull[(size_t)ja * nw + (o >> 5)] |= 1u << (o & 31);
         }
     if (value_size > 0) {
-        choose_layout(nA, nB, nD, mlog, value_size == 8 ? 16 : 32, sums.data(), pos, plan.acc_len);
+        choose_layout(nA, nB, nD, mlog, pattern_lane_group(value_size), sums.data(), pos, plan.acc_len);
     } else {   // structure only: k_pat_emit writes the columns from the output masks, there is no accumulator
         pos.assign(nD, 0);
         plan.acc_len = 0;

@@ -587,7 +587,7 @@ k_num_bucket_heavy(const int *__restrict__ queue, const int count, const int *__
     __shared__ int s_stack_lg[40];
     __shared__ long long s_row_base;
     __shared__ int s_min;
-    using Wide = typename WideSum<VT>::type;   // (double; two doubles for c64)
+    using Wide = typename WideSum<VT>::type;   // (double; two doubles for c64 and c128)
     __shared__ Wide s_sum;
     const int lane = threadIdx.x & 31;
     const int nrows = count_dev ? min(*count_dev, count) : count;   // (retry kernel: the queue was filled on the device)
@@ -772,7 +772,7 @@ k_num_bucket_heavy(const int *__restrict__ queue, const int count, const int *__
 constexpr int H2_MAX_LG = 11;   // at most 2048 slices per row (16.7 M products); longer rows -> retry queue
 
 template <typename VT>
-inline size_t h2_smem_bytes(const int cap, const int nb)
+constexpr size_t h2_smem_bytes(const int cap, const int nb)
 {
     return (size_t)cap * (value_bytes<VT> + 12) + (size_t)(nb + 1) * 4 + (size_t)(CDF_KNOTS + 1) * 4 + (size_t)B3_SCRATCH * 4 +
            (size_t)((1 << H2_MAX_LG) + 1) * 4 + (size_t)cap * 2;

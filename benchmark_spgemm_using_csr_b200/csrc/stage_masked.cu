@@ -473,6 +473,7 @@ cudaError_t launch_persistent(const LaunchCtx &lc, KernelT kern, int threads, si
                               const int *queue, int count, const Csr &A, const Csr &B, const int4 *brange, const MaskCsr &M,
                               const MaskOut &o)
 {
+    if (smem > SMEM_BLOCK_MAX) return cudaErrorInvalidValue;
     if (smem > 48 * 1024) {
         const cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         if (e != cudaSuccess) return e;
@@ -505,8 +506,11 @@ cudaError_t launch_mask_bin_t(const LaunchCtx &lc, int bin, const int *queue, in
     case MB_C4096:
         return launch_persistent(lc, k_mask_cta<VT, 12, 512>, 512, mask_cta_bytes<VT, 12>(), 1, queue, count, A, B, brange, M, o);
     case MB_C16384:
-        return launch_persistent(lc, k_mask_cta<VT, 14, 1024>, 1024, mask_cta_bytes<VT, 14>(), 1, queue, count, A, B, brange, M,
-                                 o);
+        // (16-byte values: no such table, the host runs these rows in k_mask_global -- mask_table_last)
+        if constexpr (value_bytes<VT> <= 8)
+            return launch_persistent(lc, k_mask_cta<VT, 14, 1024>, 1024, mask_cta_bytes<VT, 14>(), 1, queue, count, A, B, brange,
+                                     M, o);
+        return cudaErrorInvalidValue;
     case MB_GLOBAL:
         return launch_persistent(lc, k_mask_global<VT>, MASK_GLOBAL_THREADS, 0, 1, queue, count, A, B, brange, M, o);
     default: return cudaErrorInvalidValue;

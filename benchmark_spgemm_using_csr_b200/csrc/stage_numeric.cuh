@@ -630,6 +630,7 @@ static cudaError_t launch_num_block_t(const LaunchCtx &lc, const int *queue, int
 {
     constexpr int T = 1 << LOG2T;
     const size_t smem = (size_t)T * value_bytes<VT> + (size_t)T * 4 + (size_t)(T / 2) * 4;
+    static_assert((size_t)T * value_bytes<VT> + (size_t)T * 4 + (size_t)(T / 2) * 4 <= SMEM_BLOCK_MAX, "k_num_block table");
     if (smem > 48 * 1024) {
         cudaError_t e = cudaFuncSetAttribute(k_num_block<VT, LOG2T, THREADS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         if (e != cudaSuccess) return e;
@@ -670,7 +671,10 @@ static cudaError_t launch_num_hash_t(const LaunchCtx &lc, int bin, int G, const 
     case NB_G2048: return launch_num_block_t<VT, 11, 256>(lc, queue, count, A, B, rowoff, colC, valC);
     case NB_B4096: return launch_num_block_t<VT, 12, 512>(lc, queue, count, A, B, rowoff, colC, valC);
     case NB_B8192: return launch_num_block_t<VT, 13, 1024>(lc, queue, count, A, B, rowoff, colC, valC);
-    case NB_B16384: return launch_num_block_t<VT, 14, 1024>(lc, queue, count, A, B, rowoff, colC, valC);
+    case NB_B16384:
+        // (16-byte values: no such table, the host runs these rows in k_num_large -- num_hash_last)
+        if constexpr (value_bytes<VT> <= 8) return launch_num_block_t<VT, 14, 1024>(lc, queue, count, A, B, rowoff, colC, valC);
+        return cudaErrorInvalidValue;
     default: return cudaErrorInvalidValue;
     }
 }
@@ -751,6 +755,7 @@ static cudaError_t launch_num_block_direct_t(const LaunchCtx &lc, const int *que
 {
     constexpr int T = 1 << LOG2T;
     const size_t smem = (size_t)T * value_bytes<VT> + (size_t)T * 4 + (size_t)(T / 2) * 4;
+    static_assert((size_t)T * value_bytes<VT> + (size_t)T * 4 + (size_t)(T / 2) * 4 <= SMEM_BLOCK_MAX, "k_num_block table");
     if (smem > 48 * 1024) {
         cudaError_t e = cudaFuncSetAttribute(k_num_block<VT, LOG2T, THREADS, true>,
                                              cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
@@ -778,7 +783,10 @@ static cudaError_t launch_num_direct_t(const LaunchCtx &lc, int cap, int G, cons
     case 1024: return launch_num_block_direct_t<VT, 11, 256>(lc, queue, count, A, B, d);
     case 2048: return launch_num_block_direct_t<VT, 12, 512>(lc, queue, count, A, B, d);
     case 4096: return launch_num_block_direct_t<VT, 13, 1024>(lc, queue, count, A, B, d);
-    case 8192: return launch_num_block_direct_t<VT, 14, 1024>(lc, queue, count, A, B, d);
+    case 8192:
+        // (16-byte values: plan_direct plans no capacity above DirectPlan::table_cap_max)
+        if constexpr (value_bytes<VT> <= 8) return launch_num_block_direct_t<VT, 14, 1024>(lc, queue, count, A, B, d);
+        return cudaErrorInvalidValue;
     case 32:
         return G == 8 ? launch_num_direct_g<VT, 8, 6, 4>(lc, queue, count, A, B, d)
                       : launch_num_direct_g<VT, 32, 6, 1>(lc, queue, count, A, B, d);
@@ -801,6 +809,7 @@ static cudaError_t launch_num_bucket_tt(const LaunchCtx &lc, int cap, const int 
     // below 1024 threads every fourth knot of the CDF: enough for <= 1024 buckets, and what lets two 4096-entry CTAs share an SM
     constexpr int KB = THREADS < 1024 ? 10 : CDF_BITS;
     const size_t smem = b3_smem_bytes<VT, THREADS>(cap, nb, 1 << KB);
+    if (smem > SMEM_BLOCK_MAX) return cudaErrorInvalidValue;   // (16-byte values at cap 8192: plan_direct plans none)
     auto kern = k_num_bucket3<VT, THREADS, KB>;
     if (smem > 48 * 1024) {
         cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
@@ -874,10 +883,12 @@ static cudaError_t launch_num_bucket_heavy_t(const LaunchCtx &lc, const int *que
 {
     if (count <= 0) return cudaSuccess;
     constexpr int THREADS = 1024;
-    constexpr int cap = value_bytes<VT> == 8 ? 12288 : 16384;   // entries of a slice held on chip
+    // entries of a slice held on chip (16-byte values: 8192, 212 KB)
+    constexpr int cap = value_bytes<VT> == 16 ? 8192 : value_bytes<VT> == 8 ? 12288 : 16384;
     // buckets per slice: half the capacity (measured best on R-MAT 24 rank 0: /2 70.3, /4 72.5, /8 72.8 ms)
     constexpr int nb = cap / 2;
-    const size_t smem = (size_t)cap * (value_bytes<VT> + 4) + (size_t)(2 * nb + 1 + 34) * 4 + (size_t)(CDF_KNOTS + 1) * 4;
+    constexpr size_t smem = (size_t)cap * (value_bytes<VT> + 4) + (size_t)(2 * nb + 1 + 34) * 4 + (size_t)(CDF_KNOTS + 1) * 4;
+    static_assert(smem <= SMEM_BLOCK_MAX, "k_num_bucket_heavy slice");
     auto kern = k_num_bucket_heavy<VT, THREADS>;
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
@@ -897,8 +908,10 @@ static cudaError_t launch_num_bucket_heavy2_t(const LaunchCtx &lc, const int *qu
 {
     if (count <= 0) return cudaSuccess;
     constexpr int THREADS = 1024;
-    constexpr int cap = 8192, nb = cap / 2;   // entries of a slice on chip (22 / 18 bytes each), buckets per slice
-    const size_t smem = h2_smem_bytes<VT>(cap, nb);
+    // entries of a slice on chip (22 / 18 bytes each; 16-byte values: 4096 of 30 bytes), buckets per slice
+    constexpr int cap = value_bytes<VT> > 8 ? 4096 : 8192, nb = cap / 2;
+    constexpr size_t smem = h2_smem_bytes<VT>(cap, nb);
+    static_assert(smem <= SMEM_BLOCK_MAX, "k_num_bucket_heavy2 slice");
     auto kern = k_num_bucket_heavy2<VT, THREADS>;
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;

@@ -508,6 +508,16 @@ __device__ __forceinline__ void sts_val(unsigned a, c64 v)
 {
     asm volatile("st.shared.v2.f32 [%0], {%1, %2};" ::"r"(a), "f"(v.re), "f"(v.im) : "memory");
 }
+__device__ __forceinline__ c128 lds_val(unsigned a, c128)
+{
+    c128 v;
+    asm volatile("ld.shared.v2.f64 {%0, %1}, [%2];" : "=d"(v.re), "=d"(v.im) : "r"(a) : "memory");
+    return v;
+}
+__device__ __forceinline__ void sts_val(unsigned a, c128 v)
+{
+    asm volatile("st.shared.v2.f64 [%0], {%1, %2};" ::"r"(a), "d"(v.re), "d"(v.im) : "memory");
+}
 
 // Predicated (not branched) element load and accumulate of the hot loop: inactive lanes issue no memory
 // access at all, and the warp stays converged.
@@ -593,11 +603,38 @@ __device__ __forceinline__ void pat_accum_if(const bool on, const unsigned mp, c
         "r"(mp), "r"(acc_s), "f"(av.re), "f"(av.im), "f"(bv.re), "f"(bv.im), "f"(-av.im)
         : "memory");
 }
+// complex128: a 16-byte accumulator slot, the same four FMAs in double
+__device__ __forceinline__ void pat_accum_if(const bool on, const unsigned mp, const unsigned acc_s, const c128 av, const c128 bv)
+{
+    asm volatile(
+        "{\n"
+        ".reg .pred p;\n"
+        ".reg .u32 q, a;\n"
+        ".reg .f64 vr, vi;\n"
+        "setp.ne.s32 p, %0, 0;\n"
+        "@p ld.shared.u8 q, [%1];\n"
+        "@p mad.lo.u32 a, q, 16, %2;\n"
+        "@p ld.shared.v2.f64 {vr, vi}, [a];\n"
+        "@p fma.rn.f64 vr, %3, %5, vr;\n"
+        "@p fma.rn.f64 vr, %7, %6, vr;\n"
+        "@p fma.rn.f64 vi, %3, %6, vi;\n"
+        "@p fma.rn.f64 vi, %4, %5, vi;\n"
+        "@p st.shared.v2.f64 [a], {vr, vi};\n"
+        "}\n" ::"r"((int)on),
+        "r"(mp), "r"(acc_s), "d"(av.re), "d"(av.im), "d"(bv.re), "d"(bv.im), "d"(-av.im)
+        : "memory");
+}
 
+// The per-lane record of one A entry: its B row start bs, lj = length | (ja * nDB) << 16, and the value.  Values of
+// at most 8 bytes share one 16-byte int4 with bs and lj; a complex128 value takes a 32-byte record of its own layout.
+struct PatRec16 {
+    using Rec = int4;
+    static __device__ __forceinline__ Rec load(unsigned a) { return lds_v4(a); }
+};
 template <typename VT>
 struct PatRec;
 template <>
-struct PatRec<double> {
+struct PatRec<double> : PatRec16 {
     static __device__ __forceinline__ int4 pack(int bs, int lj, double v)
     {
         return make_int4(bs, lj, __double2loint(v), __double2hiint(v));
@@ -605,23 +642,41 @@ struct PatRec<double> {
     static __device__ __forceinline__ double val(const int4 &r) { return __hiloint2double(r.w, r.z); }
 };
 template <>
-struct PatRec<float> {
+struct PatRec<float> : PatRec16 {
     static __device__ __forceinline__ int4 pack(int bs, int lj, float v) { return make_int4(bs, lj, __float_as_int(v), 0); }
     static __device__ __forceinline__ float val(const int4 &r) { return __int_as_float(r.z); }
 };
 template <>
-struct PatRec<c64> {   // {bs, lj, re, im}
+struct PatRec<c64> : PatRec16 {   // {bs, lj, re, im}
     static __device__ __forceinline__ int4 pack(int bs, int lj, c64 v)
     {
         return make_int4(bs, lj, __float_as_int(v.re), __float_as_int(v.im));
     }
     static __device__ __forceinline__ c64 val(const int4 &r) { return c64(__int_as_float(r.z), __int_as_float(r.w)); }
 };
+struct __align__(16) PatRec32 {   // {bs, lj, -, -, re, im}
+    int x, y, z, w;
+    double re, im;
+};
+template <>
+struct PatRec<c128> {
+    using Rec = PatRec32;
+    static __device__ __forceinline__ Rec pack(int bs, int lj, c128 v) { return Rec{bs, lj, 0, 0, v.re, v.im}; }
+    static __device__ __forceinline__ c128 val(const Rec &r) { return c128(r.re, r.im); }
+    static __device__ __forceinline__ Rec load(unsigned a)
+    {
+        const int4 h = lds_v4(a);
+        Rec r{h.x, h.y, h.z, h.w, 0.0, 0.0};
+        asm volatile("ld.shared.v2.f64 {%0, %1}, [%2];" : "=d"(r.re), "=d"(r.im) : "r"(a + 16u) : "memory");
+        return r;
+    }
+};
 
 // LONGB: rows of B may hold more than G entries (only possible for G = 32 with more than 32 diagonals in B)
-// 6 CTAs per SM (40 registers): per-warp memory-level parallelism beat 8 CTAs at 32 registers (profiles/r02_notes.md)
+// 6 CTAs per SM (40 registers): per-warp memory-level parallelism beat 8 CTAs at 32 registers (profiles/r02_notes.md).
+// complex128 takes 4 (64 registers): its 32-byte records and 16-byte values spill 72 / 124 bytes at 40.
 template <typename VT, int G, bool LONGB>
-__global__ void __launch_bounds__(256, 6)
+__global__ void __launch_bounds__(256, value_bytes<VT> > 8 ? 4 : 6)
 k_pat_numeric(const int m, const int *__restrict__ rowptrA, const int *__restrict__ colA, const VT *__restrict__ valA,
               const unsigned char *__restrict__ ta, const int *__restrict__ rowptrB, const unsigned char *__restrict__ tb,
               const VT *__restrict__ valB, const PatTables t, const unsigned *__restrict__ outmask,
@@ -648,10 +703,11 @@ k_pat_numeric(const int m, const int *__restrict__ rowptrA, const int *__restric
     const int gshift = lane & ~(G - 1);
     const unsigned gbits = (G == 32) ? FULL : ((1u << (G & 31)) - 1u);
     const int acc_len = t.acc_len;
-    const size_t per_group = (size_t)acc_len * sizeof(VT) + (size_t)G * 16;   // accumulators | records
+    using Rec = typename PatRec<VT>::Rec;
+    const size_t per_group = (size_t)acc_len * sizeof(VT) + (size_t)G * sizeof(Rec);   // accumulators | records
     unsigned char *mine = smem_raw + tab_bytes + (size_t)gib * per_group;
     VT *acc = reinterpret_cast<VT *>(mine);
-    int4 *rec = reinterpret_cast<int4 *>(mine + (size_t)acc_len * sizeof(VT));
+    Rec *rec = reinterpret_cast<Rec *>(mine + (size_t)acc_len * sizeof(VT));
     const int nDB = t.nDB, nD = t.nD, nw = t.nw;
     (void)gshift;
     (void)gbits;
@@ -674,7 +730,7 @@ k_pat_numeric(const int m, const int *__restrict__ rowptrA, const int *__restric
                 const int len = rowptrB[k + 1] - bs;
                 rec[gl] = PatRec<VT>::pack(bs, len | (((int)ta[a0 + j] * nDB) << 16), valA[a0 + j]);   // (ja * nDB <= 63 * 64)
             } else {
-                rec[gl] = make_int4(0, 0, 0, 0);   // length 0: nothing to do for this slot
+                rec[gl] = Rec{};   // length 0: nothing to do for this slot
             }
             __syncwarp();
             const int cnt = min(G, max_na - base);   // warp-uniform
@@ -682,13 +738,13 @@ k_pat_numeric(const int m, const int *__restrict__ rowptrA, const int *__restric
             // value per lane) are issued before B row tt is accumulated.  Branch-free: lanes beyond the end of
             // their B row are predicated off (no memory access), the warp never diverges and every step is
             // straight-line code.
-            int4 rA, rB;
+            Rec rA, rB;
             int jbA = 0, jbB = 0;
             VT bvA = VT(0), bvB = VT(0);
             bool onA = false, onB = false;
 #define PAT_LOAD(R, JB, BV, ON, TT)                                      \
     do {                                                                  \
-        R = lds_v4(rec_s + (unsigned)(TT) * 16u);                        \
+        R = PatRec<VT>::load(rec_s + (unsigned)(TT) * (unsigned)sizeof(Rec)); \
         ON = gl < (R.y & 0x7fff);                                         \
         /* lanes past the end re-read the row's first element (same cache line, no branch); empty row: element 0 */ \
         const int idx__ = ON ? R.x + gl : ((R.y & 0x7fff) ? R.x : 0);    \
@@ -749,7 +805,8 @@ static cudaError_t launch_pat_numeric_tbl(const LaunchCtx &lc, int m, Csr A, Csr
     const int threads = 256;
     const int groups = threads / G;
     const size_t tab_bytes = ((size_t)t.nD * 4 + (size_t)t.nDA * t.nDB + (size_t)t.nD + 15) & ~(size_t)15;
-    const size_t smem = tab_bytes + (size_t)groups * ((size_t)t.acc_len * sizeof(VT) + (size_t)G * 16);
+    const size_t smem = tab_bytes + (size_t)groups * ((size_t)t.acc_len * sizeof(VT) + (size_t)G * sizeof(typename PatRec<VT>::Rec));
+    if (smem > SMEM_BLOCK_MAX) return cudaErrorInvalidValue;
     auto kern = k_pat_numeric<VT, G, LONGB>;
     if (smem > 48 * 1024) {
         cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);

@@ -301,13 +301,14 @@ inline bool range_vec_aligned(const Csr &B)
 }
 
 // numeric range bins: the vectorised kernel for rows of at most 128 outputs when B is 16-byte aligned (its 128-bit loads
-// carry values: structure-only products take the scalar kernel)
+// carry values: structure-only products take the scalar kernel, and so do complex128 ones, whose 128-bit load would
+// carry one value where the kernel's four-column step wants four)
 template <typename VT>
 static cudaError_t launch_num_range_pick_t(const LaunchCtx &lc, int nsum, int nacc, const int *queue, int count, Csr A,
                                            Csr B, const int *rlo, const int64_t *rowoff, int *colC, void *valC,
                                            WordLists wl)
 {
-    if constexpr (value_bytes<VT> > 0) {
+    if constexpr (value_bytes<VT> > 0 && value_bytes<VT> <= 8) {
         if (nacc <= 128 && range_vec_aligned(B))
             return launch_num_range_vec_t<VT>(lc, nsum, nacc, queue, count, A, B, rlo, rowoff, colC, valC, wl);
     }

@@ -47,6 +47,14 @@ __device__ __forceinline__ V moved(const V v)
     return v;
 }
 __device__ __forceinline__ Conj8 moved(const Conj8 v) { return Conj8{v.bits ^ 0x8000000000000000ull}; }
+// complex128 moves as 16-byte words (Move16); its conjugate as Conj16, bit 63 of the imaginary double flipped
+struct __align__(16) Move16 {
+    unsigned long long re, im;
+};
+struct __align__(16) Conj16 {
+    unsigned long long re, im;
+};
+__device__ __forceinline__ Conj16 moved(const Conj16 v) { return Conj16{v.re, v.im ^ 0x8000000000000000ull}; }
 
 __device__ __forceinline__ int masked_key(int key, int cols)
 {
@@ -379,14 +387,16 @@ int transpose_passes(int cols)
     return pass_count(cols, nullptr);
 }
 
-// the type the values move as: complex64 as double (8-byte words), Conj8 for conjugation
+// the type the values move as: complex64 as double (8-byte words), Conj8 for conjugation; complex128 as Move16,
+// Conj16 for conjugation (conj is only ever set for complex operands: check_ops)
 template <typename F>
 cudaError_t with_mover(int dtype, bool conj, F &&f)
 {
-    if (conj) return f(Conj8());
+    if (conj) return dtype == BHB200_DTYPE_C128 ? f(Conj16()) : f(Conj8());
     return dispatch_value_type(dtype, [&](auto v) {
         using V = decltype(v);
-        return f(std::conditional_t<std::is_same_v<V, c64>, double, V>());
+        if constexpr (std::is_same_v<V, c128>) return f(Move16());
+        else return f(std::conditional_t<std::is_same_v<V, c64>, double, V>());
     });
 }
 

@@ -115,7 +115,7 @@ class CudaEngine(capi.Context):
         return getattr(torch, capi.VALUE_TYPES[self.dtype][1])
 
     def set_operands(self, m, k, n, A, B):
-        """A, B = (rowptr, col, val) torch CUDA tensors (int32, int32, f32/f64/complex64)."""
+        """A, B = (rowptr, col, val) torch CUDA tensors (int32, int32, f32/f64/complex64/complex128)."""
         self._order_after_producers()
         self.init_device(A, B, m, k, n)
 

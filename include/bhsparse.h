@@ -15,14 +15,14 @@
  *     bh->free_mem(); bh->freePlatform();
  *
  * value_type follows the reference's typedef (common.h:31): double unless
- * BHSPARSE_VALUE_FLOAT (float) or BHSPARSE_VALUE_COMPLEX_FLOAT (std::complex<float>, the _c64 entry points) is
- * defined before including this header.
+ * BHSPARSE_VALUE_FLOAT (float), BHSPARSE_VALUE_COMPLEX_FLOAT (std::complex<float>, the _c64 entry points) or
+ * BHSPARSE_VALUE_COMPLEX_DOUBLE (std::complex<double>, the _c128 entry points) is defined before including this header.
  */
 #ifndef BHSPARSE_H
 #define BHSPARSE_H
 
 #include <cstdio>
-#ifdef BHSPARSE_VALUE_COMPLEX_FLOAT
+#if defined(BHSPARSE_VALUE_COMPLEX_FLOAT) || defined(BHSPARSE_VALUE_COMPLEX_DOUBLE)
 #include <complex>
 #endif
 
@@ -35,7 +35,9 @@
 #define BHSPARSE_OPENCL 2
 
 typedef int index_type;      /* common.h:30 */
-#if defined(BHSPARSE_VALUE_COMPLEX_FLOAT)
+#if defined(BHSPARSE_VALUE_COMPLEX_DOUBLE)
+typedef std::complex<double> value_type;   /* two doubles (re, im): BHB200_DTYPE_C128 */
+#elif defined(BHSPARSE_VALUE_COMPLEX_FLOAT)
 typedef std::complex<float> value_type;   /* two floats (re, im): BHB200_DTYPE_C64 */
 #elif defined(BHSPARSE_VALUE_FLOAT)
 typedef float value_type;
@@ -78,7 +80,10 @@ public:
         if (!_ctx) return BHB200_ERR_INVALID;
         _rowptrC = csrRowPtrC;
         const int opA = transA ? BHB200_OP_T : BHB200_OP_N, opB = transB ? BHB200_OP_T : BHB200_OP_N;
-#if defined(BHSPARSE_VALUE_COMPLEX_FLOAT)
+#if defined(BHSPARSE_VALUE_COMPLEX_DOUBLE)
+        return bhb200_init_data_op_c128(_ctx, opA, opB, m, k, n, nnzA, reinterpret_cast<const double *>(csrValA), csrRowPtrA,
+                                        csrColIndA, nnzB, reinterpret_cast<const double *>(csrValB), csrRowPtrB, csrColIndB);
+#elif defined(BHSPARSE_VALUE_COMPLEX_FLOAT)
         return bhb200_init_data_op_c64(_ctx, opA, opB, m, k, n, nnzA, reinterpret_cast<const float *>(csrValA), csrRowPtrA,
                                        csrColIndA, nnzB, reinterpret_cast<const float *>(csrValB), csrRowPtrB, csrColIndB);
 #elif defined(BHSPARSE_VALUE_FLOAT)
@@ -149,7 +154,9 @@ public:
     int update_values(const value_type *csrValA, const value_type *csrValB)
     {
         if (!_ctx) return BHB200_ERR_INVALID;
-#if defined(BHSPARSE_VALUE_COMPLEX_FLOAT)
+#if defined(BHSPARSE_VALUE_COMPLEX_DOUBLE)
+        return bhb200_update_values_c128(_ctx, reinterpret_cast<const double *>(csrValA), reinterpret_cast<const double *>(csrValB));
+#elif defined(BHSPARSE_VALUE_COMPLEX_FLOAT)
         return bhb200_update_values_c64(_ctx, reinterpret_cast<const float *>(csrValA), reinterpret_cast<const float *>(csrValB));
 #elif defined(BHSPARSE_VALUE_FLOAT)
         return bhb200_update_values_f32(_ctx, csrValA, csrValB);
@@ -163,7 +170,9 @@ public:
     {
         if (!_ctx) return BHB200_ERR_INVALID;
         if (!csrValC) return bhb200_get_C_structure(_ctx, _rowptrC, csrColIndC);   /* (structure-only products too) */
-#if defined(BHSPARSE_VALUE_COMPLEX_FLOAT)
+#if defined(BHSPARSE_VALUE_COMPLEX_DOUBLE)
+        return bhb200_get_C_c128(_ctx, _rowptrC, csrColIndC, reinterpret_cast<double *>(csrValC));
+#elif defined(BHSPARSE_VALUE_COMPLEX_FLOAT)
         return bhb200_get_C_c64(_ctx, _rowptrC, csrColIndC, reinterpret_cast<float *>(csrValC));
 #elif defined(BHSPARSE_VALUE_FLOAT)
         return bhb200_get_C_f32(_ctx, _rowptrC, csrColIndC, csrValC);

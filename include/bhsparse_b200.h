@@ -36,6 +36,10 @@
  *    component follows the real rule applied to its 2p products, provided no finite real product overflows
  *    (otherwise it is unspecified): this is the naive formula's behaviour, not C99 Annex G's recovery of
  *    infinities (inf * (0 + 1i) gives NaN components here).
+ *  - complex128 (BHB200_DTYPE_C128): the same per-component rule with the f64 values and constants: each
+ *    component is a real sum of 2p f64 products, |c_hat - c| <= gamma(2p)*s + 4*p*lam with u = 2^-53 and
+ *    lam = 2^-1022.  Gaussian integers within the f64 budget for 2p products come back equal; non-finite
+ *    components follow the naive formula, as for complex64.
  *
  * Every function returns BHB200_SUCCESS (0 == BHSPARSE_SUCCESS, common.h:26) or
  * a negative error code; nothing calls exit().  Not thread-safe per context
@@ -74,9 +78,14 @@ extern "C" {
  * float _Complex, std::complex<float>, cuFloatComplex, numpy / torch complex64.  Value arrays are passed
  * as float * holding 2*nnz interleaved floats (or void * to the same bytes); see "complex64 products" below. */
 #define BHB200_DTYPE_C64 4
+/* double-precision complex: two doubles (re, im) per value, 16 bytes, 16-byte aligned -- the layout of C99
+ * double _Complex, std::complex<double>, cuDoubleComplex, numpy / torch complex128.  Value arrays are passed
+ * as double * holding 2*nnz interleaved doubles (or void * to the same bytes); see "complex128 products" below. */
+#define BHB200_DTYPE_C128 5
 
 /* op(X) of bhb200_init_data_op_* / bhb200_init_data_device_op: X as stored, its transpose, or its conjugate
- * transpose X^H (complex64 operands only: with f32, f64 or structure-only operands OP_C is BHB200_ERR_INVALID) */
+ * transpose X^H (complex64 and complex128 operands only: with f32, f64 or structure-only operands OP_C is
+ * BHB200_ERR_INVALID) */
 #define BHB200_OP_N 0
 #define BHB200_OP_T 1
 #define BHB200_OP_C 2
@@ -255,12 +264,32 @@ BHB200_API int bhb200_get_C_structure(bhb200_ctx *ctx, int32_t *rowptrC, int32_t
  * 8-byte values; bhb200_stats.dtype is BHB200_DTYPE_C64 and its byte counts take 8 bytes per value.
  * bhb200_dist_setup_square takes BHB200_DTYPE_C64 (values broadcast as 8-byte words).  The real getters and
  * update_values_f64 / _f32 on a complex64 context, and the _c64 ones on a real context, return
- * BHB200_ERR_INVALID.  complex128 is not supported. */
+ * BHB200_ERR_INVALID; so do they on a complex128 context. */
 BHB200_API int bhb200_init_data_op_c64(bhb200_ctx *ctx, int opA, int opB, int m, int k, int n,
                                        int nnzA, const float *valA, const int32_t *rowptrA, const int32_t *colA,
                                        int nnzB, const float *valB, const int32_t *rowptrB, const int32_t *colB);
 BHB200_API int bhb200_update_values_c64(bhb200_ctx *ctx, const float *valA, const float *valB);
 BHB200_API int bhb200_get_C_c64(bhb200_ctx *ctx, int32_t *rowptrC, int32_t *colC, float *valC);
+
+/* -- complex128 products: C = op(A)*op(B) over double-precision complex values -----------------------------
+ * Values are BHB200_DTYPE_C128 (two doubles per value, see the define).  The entry points follow the _c64 ones:
+ *   bhb200_init_data_op_c128   HOST arrays, the rules of bhb200_init_data_op_c64; valA / valB hold 2*nnz
+ *                              doubles; opA / opB may be BHB200_OP_C.
+ *   bhb200_update_values_c128  new values of the host operands (conjugated again into X^H copies).
+ *   bhb200_get_C_c128          rowptrC, colC and valC (2*nnzC doubles) into HOST arrays.
+ *   bhb200_init_data_device / _device_op with BHB200_DTYPE_C128: borrowed device operands; value pointers that
+ *                              are not 16-byte aligned return BHB200_ERR_INVALID from the init call.
+ * bhb200_get_C_range, bhb200_get_C_device, bhb200_copy_C_to_device, masks and the structure getters work with
+ * 16-byte values; bhb200_stats.dtype is BHB200_DTYPE_C128 and its byte counts take 16 bytes per value.
+ * bhb200_dist_setup_square takes BHB200_DTYPE_C128.  The on-chip tables sized for 8-byte values do not all hold
+ * 16-byte ones, so some rows run in another kernel than they would in f64 (DESIGN.md 4.13); the statistics
+ * (num_bin_rows, mask_bin_rows, direct_bin_mask) report the kernels that ran.  The real and _c64 getters and
+ * updaters return BHB200_ERR_INVALID on a complex128 context, and the _c128 ones on any other context. */
+BHB200_API int bhb200_init_data_op_c128(bhb200_ctx *ctx, int opA, int opB, int m, int k, int n,
+                                        int nnzA, const double *valA, const int32_t *rowptrA, const int32_t *colA,
+                                        int nnzB, const double *valB, const int32_t *rowptrB, const int32_t *colB);
+BHB200_API int bhb200_update_values_c128(bhb200_ctx *ctx, const double *valA, const double *valB);
+BHB200_API int bhb200_get_C_c128(bhb200_ctx *ctx, int32_t *rowptrC, int32_t *colC, double *valC);
 
 /* -- masked products: C = M .* (op(A)*op(B)) (GraphBLAS C<M> = A*B) ----------------------------------
  * M is m x n and structural: row pointers (m+1) and column indices, no values; its rows must be sorted
@@ -371,7 +400,7 @@ BHB200_API int bhb200_set_profiling(bhb200_ctx *ctx, int enabled);
 #define BHB200_DIST_ID_BYTES 128
 BHB200_API int bhb200_dist_unique_id(void *id);
 BHB200_API int bhb200_dist_init(bhb200_ctx *ctx, int rank, int nranks, const void *id);
-/* dist_setup_square takes BHB200_DTYPE_F32, BHB200_DTYPE_F64 or BHB200_DTYPE_C64 (structure-only products are
+/* dist_setup_square takes BHB200_DTYPE_F32, BHB200_DTYPE_F64, BHB200_DTYPE_C64 or BHB200_DTYPE_C128 (structure-only products are
  * single-GPU) */
 BHB200_API int bhb200_dist_setup_square(bhb200_ctx *ctx, int root, int dtype, int n, int64_t nnz, const int32_t *rowptr,
                                         const int32_t *col, const void *val);
@@ -389,7 +418,9 @@ BHB200_API int bhb200_dist_finalize(bhb200_ctx *ctx);
  * in the product), then info[1..5] = diagonals of C, mask words per row, accumulator length,
  * shared-memory wavefronts of one pass over all (A diagonal, lane group) pairs with the chosen
  * accumulator layout, and their conflict-free minimum.  position (nA*nB bytes, optional): accumulator
- * slot of product (ja, jb), diagonals in ascending order; offsC (<= 256 ints, optional): diagonals of C. */
+ * slot of product (ja, jb), diagonals in ascending order; offsC (<= 256 ints, optional): diagonals of C.
+ * value_size is 4, 8 or 16 (f32; f64 and complex64; complex128): a lane group is the 128 bytes of one
+ * shared-memory wavefront, 32, 16 or 8 lanes. */
 BHB200_API int bhb200_pattern_plan_probe(const int32_t *offsA, int nA, const int32_t *offsB, int nB, int value_size,
                                          int32_t *info, uint8_t *position, int32_t *offsC);
 
